@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: batched audio -> blendshape inference (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp32|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp32|bf16] [--dump-outputs DIR]
 
 One step = ``SequentialDualStreamModel.forward`` (the public call) over 512 synthetic 8.5 s clips (16 kHz, 30 fps, one
 output frame per clip) per GPU.  BASELINE.json quotes configs[1] in "fp32 and bf16": the line's value / dtype are the
@@ -12,6 +12,8 @@ to the bare host->device copy rate measured in the same run; ``roofline`` descri
 short leg so that the timed region keeps its programmatic dependent launches); ``configs`` holds the other workloads of
 BASELINE.json (60 fps, 4096 streams, corpus sweep); ``cpu_baseline`` / ``--impl reference`` time the reference's own CPU
 forward (the unmodified modules staged under oracle/_ref) on this box's host cores.
+``--dump-outputs DIR`` writes the blendshapes the last timed step returned to ``DIR/blendshapes.npy`` (float32; the inputs
+are seeded, so two builds can be compared output for output).
 """
 import argparse
 import json
@@ -23,6 +25,8 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark may run from a read-only checkout: it writes nothing into the tree, compiled bytecode included
+sys.dont_write_bytecode = True
 
 CLIPS_PER_GPU = 512
 CLIP_SAMPLES = 136000          # 8.5 s at 16 kHz
@@ -281,6 +285,14 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------- GPU arm
+def dump_outputs(directory, arrays):
+    """Write each tensor of ``arrays`` to ``directory/<name>.npy`` as float32."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), t.float().cpu().numpy())
+
+
 def _make_model(K, O, torch, dev, fps, precision):
     w = O.make_weights(1234, fps, style="init")
     model = K.SequentialDualStreamModel(target_fps=fps, mel_sequence_length=256 if fps == 30 else 512).to(dev).eval()
@@ -377,6 +389,11 @@ def run_gpu(args):
     barrier()
     clocks = sampler.stop()
     launches = _lib.launch_count()
+    # what the timed path handed its caller in the last step (every rank's block, as gathered), set aside before the legs
+    # below write into `kept` again
+    last_step = None
+    if args.dump_outputs:
+        last_step = (gathered.view(world, K_steps, B, 1, 52)[:, -1] if world > 1 else kept[-1]).reshape(-1, 1, 52).clone()
     mine_ms, gather_ms = t0.elapsed_time(t1), g0.elapsed_time(t1)
     per_rank = torch.tensor([mine_ms, gather_ms, host_submit_ms], device=dev)
     all_ranks = per_rank.clone().unsqueeze(0)
@@ -620,6 +637,8 @@ def run_gpu(args):
             line["configs"] = configs
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline()
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, {"blendshapes": last_step})
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -723,7 +742,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the host-buffer leg")
     ap.add_argument("--no-other-precision", action="store_true", help="skip the secondary (bf16 / fp32) leg")
     ap.add_argument("--no-configs", action="store_true", help="skip the 60 fps / streaming / corpus legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the blendshapes of the last timed step to DIR/blendshapes.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "koemorph_b200":
+        ap.error("--dump-outputs applies to the koemorph_b200 path")
     _claim_stdout()
     if args.impl == "reference":
         run_reference(args)

@@ -1,8 +1,8 @@
-"""Run the UNMODIFIED reference modules from /root/reference (build container only).
+"""Run the UNMODIFIED reference modules of the upstream KoeMorph project (a checkout named by KOEMORPH_REFERENCE).
 
 TEST INFRASTRUCTURE ONLY -- used by ``tests/golden/make_golden.py`` to produce the
-committed golden vectors and by ``tests/test_oracle.py`` (skipped when
-/root/reference is absent, as on the GPU box).
+committed golden vectors and by ``bench.py --impl reference``; the test suite
+reads those stored vectors and never imports the reference itself.
 
 The reference cannot be imported as-is in this image: ``librosa`` and
 ``opensmile`` are not installed (SURVEY.md section 8c).  Following SURVEY.md
