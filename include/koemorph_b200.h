@@ -42,7 +42,8 @@ extern "C" {
 const char* koe_last_error(void);
 int koe_version(void);
 /* sizeof of the public argument structs, for bindings that mirror them (ctypes, cgo, JNI): 0 koe_frontend_config,
- * 1 koe_logmel_args, 2 koe_core_weights, 3 koe_stream_args, 4 koe_forward_args; -1 for any other index */
+ * 1 koe_logmel_args, 2 koe_core_weights, 3 koe_stream_args, 4 koe_forward_args, 5 koe_stream_pool_args; -1 for any
+ * other index */
 int koe_sizeof_struct(int which);
 /* number of kernels launched by this library in this process since load / since the last reset */
 int64_t koe_launch_count(void);
@@ -302,6 +303,60 @@ typedef struct {
   int64_t step;
 } koe_stream_args;
 int koe_stream_push(const koe_stream_args* args, int* emitted, void* stream);
+
+/*
+ * Stream pool: up to `capacity` streams that open, close and advance on their own clocks (a real-time service whose users
+ * connect, leave and send late packets).  Every stream of a pool computes exactly -- bit for bit -- what a one-stream
+ * koe_stream_push computes when fed the same hops from the moment the stream was opened, whatever the other streams do
+ * and whatever its slot held before: it emits from its own window_frames-th hop on, its first frame passes the
+ * smoothing unchanged, and a reused slot carries no audio, mel rows or smoothing state over.
+ *
+ * The pool object (host memory) owns the clock policy: which slots are open, how many hops each stream has pushed and
+ * how many frames it has emitted.  Its entry points return KOE_E_INVALID on misuse (slot out of range or not open, a
+ * slot listed twice in one call, more streams than free slots) before anything is queued.  Device buffers are
+ * caller-owned (koe_stream_pool_args, shapes below with C = capacity, V = 1 + 2 * n_edge buffer variants:
+ * plain, window-start 0, window-end 0, window-start 1, window-end 1).  koe_stream_pool_push uploads its per-call tables
+ * (pushing streams: slot, ring row, first hop; emitting streams: slot, ring base, has smoothing state) with one
+ * cudaMemcpyAsync from pinned staging that the library owns per (device, stream); it cannot be captured into a CUDA graph.
+ */
+typedef struct koe_stream_pool koe_stream_pool_t;
+typedef struct {
+  const koe_frontend_t* frontend;
+  const koe_core_weights* weights;
+  const float* hop_audio;        /* [n][hop]: row i is the next hop of stream slots_host[i] (koe_stream_pool_push) */
+  float* tail;                   /* [C][half_fft + n_edge * hop]: each slot's audio tail (any content when opened) */
+  float* tail_compact;           /* [C][half_fft + n_edge * hop]: the pushing streams' tails, in call order */
+  float* stage;                  /* [V][C][80], */
+  float* stage_max;              /* [V][C]: the new mel rows of the pushing streams, in call order */
+  float* ring_f; float* fmax_f;  /* [C][window_frames][80], [C][window_frames] (as koe_stream_args) */
+  float* ring_r; float* fmax_r;
+  float* row_l; float* fmax_l;   /* [C][80], [C] */
+  float* ring_r2; float* fmax_r2; /* hop < n_fft/2 only, else NULL */
+  float* row_l2; float* fmax_l2;
+  float* expr_sigmoid;           /* [C] */
+  float* expr_compact;           /* [C]: scratch of koe_stream_pool_set_egemaps */
+  float* out;                    /* [C][52]: row w is the frame of the w-th emitting stream of the call */
+  float* ema_state;              /* [C][52], or NULL: no temporal smoothing */
+  int32_t* tables;               /* [6][C] int32: the per-call tables */
+  float alpha;                   /* sigmoid(smoothing_alpha) */
+  int32_t precision;
+} koe_stream_pool_args;
+int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_fft, koe_stream_pool_t** out);
+int koe_stream_pool_destroy(koe_stream_pool_t* pool);
+/* takes the n lowest free slots into slots_host[n]; their clocks start at zero (their expression input is unset until
+ * koe_stream_pool_set_egemaps) */
+int koe_stream_pool_open(koe_stream_pool_t* pool, int n, int32_t* slots_host);
+int koe_stream_pool_close(koe_stream_pool_t* pool, int slot);
+/* the emotion stream for n open streams: egemaps [n][weights->emo_in] -> expr_sigmoid[slots_host[i]] */
+int koe_stream_pool_set_egemaps(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const int32_t* slots_host, int n,
+                                const float* egemaps, void* stream);
+/* advances the n open streams slots_host[0..n) by one hop each.  *n_emitted streams emit a frame: their slots go to
+ * emitted_host[0..*n_emitted) (capacity entries), in call order, and their frames to out rows 0..*n_emitted.  Queues the
+ * tail update, the frontend launches of koe_stream_push on the pushing streams (2 at 30 fps, 4 at 60 fps), the scatter
+ * into their rings and, when a stream emits, the core over the emitting streams and the smoothing: 6 kernels (8 at
+ * 60 fps), 4 (6) when no stream emits, none for n = 0. */
+int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const int32_t* slots_host, int n,
+                         int32_t* emitted_host, int* n_emitted, void* stream);
 
 /*
  * The whole forward of SequentialDualStreamModel.forward (src/model/sequential_dual_stream_model.py:63-167) -- or, with

@@ -75,6 +75,17 @@ class ForwardArgs(C.Structure):
                 ("precision", C.c_int32)]
 
 
+class StreamPoolArgs(C.Structure):
+    """koe_stream_pool_args (include/koemorph_b200.h)."""
+    _fields_ = [("frontend", C.c_void_p), ("weights", C.c_void_p), ("hop_audio", C.c_void_p),
+                ("tail", C.c_void_p), ("tail_compact", C.c_void_p), ("stage", C.c_void_p), ("stage_max", C.c_void_p),
+                ("ring_f", C.c_void_p), ("fmax_f", C.c_void_p), ("ring_r", C.c_void_p), ("fmax_r", C.c_void_p),
+                ("row_l", C.c_void_p), ("fmax_l", C.c_void_p),
+                ("ring_r2", C.c_void_p), ("fmax_r2", C.c_void_p), ("row_l2", C.c_void_p), ("fmax_l2", C.c_void_p),
+                ("expr_sigmoid", C.c_void_p), ("expr_compact", C.c_void_p), ("out", C.c_void_p),
+                ("ema_state", C.c_void_p), ("tables", C.c_void_p), ("alpha", C.c_float), ("precision", C.c_int32)]
+
+
 class FrontendConfig(C.Structure):
     """koe_frontend_config (include/koemorph_b200.h)."""
     _fields_ = [("device", C.c_int32), ("sample_rate", C.c_int32), ("n_fft", C.c_int32), ("n_mels", C.c_int32),
@@ -112,6 +123,14 @@ _SIGNATURES = {
     "koe_sizeof_struct": (C.c_int, [C.c_int]),
     "koe_stream_push": (C.c_int, [C.POINTER(StreamArgs), C.POINTER(C.c_int), C.c_void_p]),
     "koe_forward_windows": (C.c_int, [C.POINTER(ForwardArgs), C.c_void_p]),
+    "koe_stream_pool_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "koe_stream_pool_destroy": (C.c_int, [C.c_void_p]),
+    "koe_stream_pool_open": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "koe_stream_pool_close": (C.c_int, [C.c_void_p, C.c_int]),
+    "koe_stream_pool_set_egemaps": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_int, C.c_void_p,
+                                              C.c_void_p]),
+    "koe_stream_pool_push": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_int, C.c_void_p,
+                                       C.POINTER(C.c_int), C.c_void_p]),
     "koe_affine_rows": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "koe_emotion_stream": (C.c_int, [C.POINTER(CoreWeightsStruct), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "koe_dual_stream_windows": (C.c_int, [C.POINTER(CoreWeightsStruct), C.POINTER(C.c_void_p),

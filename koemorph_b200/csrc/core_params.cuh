@@ -26,6 +26,10 @@ struct CoreParams {
   unsigned early_target;
   int early_items;
   long long* dbg;  // optional phase timestamps of CTA 0 (bring-up / profiling only), NULL in production
+  // stream pool (csrc/stream_pool.cu; the kPool instantiations only): window w reads the rings, edge rows and expression
+  // value of stream pool_slot[w] with ring base pool_base[w], and writes output row w
+  const int* pool_slot;
+  const int* pool_base;
 };
 
 // frame k of window wi of clip b: which buffer and which row (see koe_dual_stream_windows in the header)
@@ -41,6 +45,16 @@ __device__ __forceinline__ long long window_row(const CoreParams& p, int variant
   return variant == 0 ? (long long)b * p.n_frames + (long long)wi * p.stride_frames + k
                       : (long long)b * p.n_out + wi;
 }
+// the same in the stream pool: ring mode with the window's own stream slot and ring base
+__device__ __forceinline__ long long pool_window_row(const CoreParams& p, int variant, int slot, int base, int k) {
+  return variant > 0 && (variant & 1) == 0 ? (long long)slot : (long long)slot * p.ring_frames + (base + k) % p.ring_frames;
+}
+// kPool: (b, wi) of the callers below are the window's stream slot and ring base
+template <bool kPool>
+__device__ __forceinline__ long long core_row(const CoreParams& p, int variant, int b, int wi, int k) {
+  if constexpr (kPool) return pool_window_row(p, variant, b, wi, k);
+  else return window_row(p, variant, b, wi, k);
+}
 
 // emotion stream launch shared by the public entry and the fused forward (csrc/session.cu, which has it write the
 // expression entries of `out`); the core launch that leaves those entries alone (expr_sigmoid == NULL); see dual_stream.cu
@@ -51,6 +65,11 @@ int launch_dual_stream_windows(const koe_core_weights* w, const float* const* po
                                const float* expr_sigmoid, float* out, float* sigmoid_out, float* attn_out, int precision,
                                void* stream, bool expr_by_emotion_kernel, unsigned* early_flag = nullptr,
                                unsigned early_target = 0, int early_items = 0, bool* early_applied = nullptr);
+// the core over the emitting windows of a stream-pool push (csrc/stream_pool.cu): window w is stream slot[w] (device
+// table) with ring base base[w]; output row w
+int launch_dual_stream_pool(const koe_core_weights* w, const float* const* power, const float* const* frame_max, int n_edge,
+                            int n_windows, int ring_frames, const int* slot, const int* base, const float* expr_sigmoid,
+                            float* out, int precision, void* stream);
 // how many SMs' worth of CTAs the tensor-core core launches for n_items windows (the early-release split follows it)
 int dual_stream_tc_grid(int n_items);
 

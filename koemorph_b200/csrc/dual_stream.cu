@@ -108,6 +108,9 @@ constexpr size_t kCoreSmemFloats = (size_t)kABlockRows * kTok      // A block
                                    + 64;                           // reductions
 constexpr size_t kCoreSmem = kCoreSmemFloats * sizeof(float);
 
+// kPool: the stream-pool flavour (window item = stream p.pool_slot[item], ring base p.pool_base[item]); a separate
+// instantiation, so that the kernel every other caller runs stays exactly as it was
+template <bool kPool = false>
 __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreParams p) {
   extern __shared__ __align__(16) float smem[];
   float* s_a = smem;                               // [64][80]
@@ -122,7 +125,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
   const int n_items = p.n_clips * p.n_out;
 
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-    const int b = item / p.n_out, wi = item % p.n_out;
+    const int b = kPool ? __ldg(p.pool_slot + item) : item / p.n_out, wi = kPool ? __ldg(p.pool_base + item) : item % p.n_out;
     const bool prenorm = p.mel_long != nullptr;
 
     // ---- P0: dB reference of this window -------------------------------------------------------
@@ -131,7 +134,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
       float mx = -INFINITY;
       for (int k = tid; k < T; k += kCoreThreads) {
         const int v = window_variant(p, k);
-        mx = fmaxf(mx, p.fmax[v][window_row(p, v, b, wi, k)]);
+        mx = fmaxf(mx, p.fmax[v][core_row<kPool>(p, v, b, wi, k)]);
       }
       mx = warp_max(mx);
       if (tx == 0) s_red[ty] = mx;
@@ -173,7 +176,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
         } else if (k >= 0) {
           const int var = window_variant(p, k);
           const float4 pw =
-              __ldg(reinterpret_cast<const float4*>(p.power[var] + window_row(p, var, b, wi, k) * kTok) + q);
+              __ldg(reinterpret_cast<const float4*>(p.power[var] + core_row<kPool>(p, var, b, wi, k) * kTok) + q);
           v.x = normalise_db(pw.x, ref_db, true);
           v.y = normalise_db(pw.y, ref_db, true);
           v.z = normalise_db(pw.z, ref_db, true);
@@ -772,14 +775,19 @@ static int launch_core(const CoreParams& p_in, int precision, cudaStream_t strea
     KOE_CUDA(cudaGetDevice(&dev));
     KOE_REQUIRE(dev >= 0 && dev < 64, "device index too large");
     if (num_sms[dev] == 0) {
-      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)kCoreSmem));
+      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)kCoreSmem));
       int n = 0;
       KOE_CUDA(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
       num_sms[dev] = n;
     }
     const int grid = std::min(p.n_clips * p.n_out, num_sms[dev]);
-    dual_stream_fp32_kernel<<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
+    if (p.pool_slot != nullptr)
+      dual_stream_fp32_kernel<true><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
+    else
+      dual_stream_fp32_kernel<false><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
     count_launch();
     KOE_CUDA(cudaGetLastError());
     return KOE_OK;
@@ -880,6 +888,38 @@ extern "C" int koe_dual_stream_ring_edges(const koe_core_weights* w, const float
   p.attn_out = attn_out;
   p.ring_frames = ring_frames;
   p.ring_base = ring_base % ring_frames;
+  return launch_core(p, precision, (cudaStream_t)stream);
+}
+
+int koe::launch_dual_stream_pool(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                                 int n_edge, int n_windows, int ring_frames, const int* slot, const int* base,
+                                 const float* expr_sigmoid, float* out, int precision, void* stream) {
+  if (int rc = validate_weights(w)) return rc;
+  KOE_REQUIRE(power != nullptr && frame_max != nullptr && slot != nullptr && base != nullptr && expr_sigmoid != nullptr &&
+                  out != nullptr,
+              "stream pool core: NULL argument");
+  KOE_REQUIRE(n_edge >= 1 && n_edge <= KOE_MAX_EDGE && n_windows >= 0 && ring_frames == w->k_mel - 3,
+              "stream pool core: bad sizes");
+  if (n_windows == 0) return KOE_OK;
+  CoreParams p{};
+  p.w = *w;
+  for (int j = 0; j < 1 + 2 * n_edge; ++j) {
+    KOE_REQUIRE(power[j] != nullptr && frame_max[j] != nullptr, "stream pool core: NULL buffer %d", j);
+    KOE_REQUIRE((reinterpret_cast<uintptr_t>(power[j]) & 15) == 0, "stream pool core: mel rows must be 16-byte aligned");
+    p.power[j] = power[j], p.fmax[j] = frame_max[j];
+  }
+  p.n_edge = n_edge;
+  p.n_clips = n_windows;
+  p.n_frames = ring_frames;
+  p.n_out = 1;
+  p.stride_frames = 1;
+  p.frames_per_window = ring_frames + 1;
+  p.mel_seq = w->k_mel - 3;
+  p.expr_sigmoid = expr_sigmoid;
+  p.out = out;
+  p.ring_frames = ring_frames;
+  p.pool_slot = slot;
+  p.pool_base = base;
   return launch_core(p, precision, (cudaStream_t)stream);
 }
 

@@ -218,8 +218,10 @@ __device__ __forceinline__ void simt_barrier() { asm volatile("bar.sync 1, 256;"
 
 // kEarly: the early-release flavour of the fused forward (see the wait below); a separate instantiation, so that the
 // kernel every other caller runs (streaming, sequences, the public entries) stays exactly as it was: the three extra
-// checks cost that one 4 % through register spills when they were run-time branches
-template <int KMEL, bool kEarly = false>
+// checks cost that one 4 % through register spills when they were run-time branches.  kPool: the stream-pool flavour
+// (csrc/stream_pool.cu), ring mode with a stream slot and a ring base per window (p.pool_slot, p.pool_base), kept apart
+// for the same reason.
+template <int KMEL, bool kEarly = false, bool kPool = false>
 __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams p) {
   using G = Geo<KMEL>;
   constexpr int kKMel = G::kKMel, kA1Chunks = G::kA1Chunks, kA1Sbo = G::kA1Sbo, kLongChunks = G::kLongChunks;
@@ -354,19 +356,20 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       const uint64_t pol_keep = l2_policy_keep(), pol_stream = l2_policy_stream();
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         long long* dp = (p.dbg != nullptr && blockIdx.x == 0 && item < 2 * (int)gridDim.x) ? p.dbg + 32 + 16 * (item / gridDim.x) : nullptr;
-        const int b = item / p.n_out, wi = item % p.n_out;
+        const int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
         if (kEarly && (item == (int)blockIdx.x || item == first_late_item)) {
           if (item == first_late_item) pdl_wait();
           asm volatile("fence.proxy.async.global;" ::: "memory");  // generic-proxy acquire / wait above -> TMA reads below
         }
         const float* base = p.ring_frames > 0 ? p.power[0] + (size_t)b * p.ring_frames * kTok
-                                              : p.power[0] + window_row(p, 0, b, wi, 0) * kTok;
+                                              : p.power[0] + core_row<kPool>(p, 0, b, wi, 0) * kTok;
         // Ring mode (the streaming step): with thousands of streams the rings (82 KB each: 335 MB for 4096 streams) do not
         // stay in L2 from one hop to the next, and a window's six stages pass through two ring slots one HBM latency after
         // the other.  The NEXT window's ring and frame maxima are pulled into L2 now, a whole window ahead (4096 streams:
         // p50 0.4285 -> 0.4175 ms per hop; a steady window is 19.4 k cycles here against 17.6 k in the batch forward).
         if (p.ring_frames > 0 && item + (int)gridDim.x < n_items) {
-          const int nb = item + gridDim.x;   // (n_out == 1 in ring mode: item == stream)
+          // (n_out == 1 in ring mode: item == stream; the pool's next window reads stream pool_slot[item + grid])
+          const int nb = kPool ? p.pool_slot[item + gridDim.x] : item + gridDim.x;
           const char* ring = reinterpret_cast<const char*>(p.power[0] + (size_t)nb * p.ring_frames * kTok);
           const uint32_t ring_bytes = (uint32_t)p.ring_frames * kTok * 4;
           for (uint32_t off = 0; off < ring_bytes; off += 16384) bulk_prefetch_l2(ring + off, min(16384u, ring_bytes - off));
@@ -383,7 +386,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           if (s == n_mel_stages - 1) stamp(dp, 9);
           mbar_expect_tx(bar_full + 8 * slot, bytes);
           if (p.ring_frames > 0) {
-            const int r0 = (p.ring_base + kMelRows * s) % p.ring_frames;
+            const int r0 = ((kPool ? wi : p.ring_base) + kMelRows * s) % p.ring_frames;
             const int n1 = min(n, p.ring_frames - r0);
             bulk_g2s_hint(dst, base + (size_t)r0 * kTok, (uint32_t)n1 * kTok * 4, bar_full + 8 * slot, pol_keep);
             if (n1 < n)
@@ -510,7 +513,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
     auto frame_max_partial = [&](const int item) {
       float mx = -INFINITY;
       if (!prenorm) {
-        const int b = item / p.n_out, wi = item % p.n_out;
+        const int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
         for (int k0 = tid; k0 < T; k0 += 3 * kSimt) {
           float f[3];
 #pragma unroll
@@ -519,7 +522,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
             f[u] = -INFINITY;
             if (k < T) {
               const int v = window_variant(p, k);
-              f[u] = p.fmax[v][window_row(p, v, b, wi, k)];
+              f[u] = p.fmax[v][core_row<kPool>(p, v, b, wi, k)];
             }
           }
           mx = fmaxf(fmaxf(mx, f[0]), fmaxf(f[1], f[2]));
@@ -528,7 +531,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       return mx;
     };
     auto stage_window = [&](const int item, float mx, long long* ds) {
-      const int b = item / p.n_out, wi = item % p.n_out;
+      const int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
       // ---- window dB reference
       float ref_db = 0.0f;
       if (!prenorm) {
@@ -550,14 +553,14 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
             const int k = T >= 3 ? T - 3 + e : (e < T ? e : -1);
             if (k >= 0) {
               const int var = window_variant(p, k);
-              extra[e] = p.power[var][window_row(p, var, b, wi, k) * kTok + tid];
+              extra[e] = p.power[var][core_row<kPool>(p, var, b, wi, k) * kTok + tid];
             } else {
               extra[e] = -INFINITY;
             }
           }
           if (p.n_edge > 0) {
-            extra[3] = __ldg(p.power[1] + window_row(p, 1, b, wi, 0) * kTok + tid);
-            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + window_row(p, 2, b, wi, T - 1) * kTok + tid);
+            extra[3] = __ldg(p.power[1] + core_row<kPool>(p, 1, b, wi, 0) * kTok + tid);
+            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + core_row<kPool>(p, 2, b, wi, T - 1) * kTok + tid);
           }
         }
         for (int s = 0; s < n_mel_stages; ++s) {
@@ -617,12 +620,12 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           // edge frames inside the long-term range see zeros beyond the window edge: patch them in place
           // (frame m and frame T-1-m for m < n_edge: one per side at 30 fps, two at 60 fps)
           for (int m = 0; m < p.n_edge; ++m) {
-            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + window_row(p, 1 + 2 * m, b, wi, m) * kTok + j);
+            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + core_row<kPool>(p, 1 + 2 * m, b, wi, m) * kTok + j);
             *reinterpret_cast<__nv_bfloat16*>(arow + (m >> 3) * 128 + (m & 7) * 2) =
                 __float2bfloat16_rn(normalise_bf16(lo, ref_db, true));
             const int k = T - 1 - m;
             if (k < Tl) {
-              const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + window_row(p, 2 + 2 * m, b, wi, k) * kTok + j);
+              const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + core_row<kPool>(p, 2 + 2 * m, b, wi, k) * kTok + j);
               *reinterpret_cast<__nv_bfloat16*>(arow + (k >> 3) * 128 + (k & 7) * 2) =
                   __float2bfloat16_rn(normalise_bf16(x, ref_db, true));
             }
@@ -685,7 +688,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       stamp(dk, 2);
     }
     for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-      const int b = item / p.n_out;
+      const int b = kPool ? p.pool_slot[item] : item / p.n_out;
       const bool has_next = item + (int)gridDim.x < n_items;
       long long* ds = (p.dbg != nullptr && blockIdx.x == 0 && tid == 0 && item < 2 * (int)gridDim.x) ? p.dbg + 16 * (item / gridDim.x) : nullptr;
       stamp(ds, 0);
@@ -960,6 +963,22 @@ int launch_dual_stream_tc(const CoreParams& p, int precision, cudaStream_t strea
     else
       KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, true>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes,
                                            stream, p));
+  } else if (p.pool_slot != nullptr) {
+    KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
+    static bool configured[64] = {false};
+    if (!configured[dev]) {
+      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<259, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    tc::kSmemBytes));
+      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<515, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    tc::kSmemBytes));
+      configured[dev] = true;
+    }
+    if (p.w.k_mel == 259)
+      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259, false, true>, dim3(grid), dim3(tc::kThreads),
+                                           tc::kSmemBytes, stream, p));
+    else
+      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, false, true>, dim3(grid), dim3(tc::kThreads),
+                                           tc::kSmemBytes, stream, p));
   } else if (p.w.k_mel == 259)
     KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes, stream, p));
   else

@@ -1,0 +1,388 @@
+// Stream pool (koe_stream_pool_* in the header): koe_stream_push for streams that open, close and advance on their own
+// clocks.  The kernels never needed lock-step -- every window is computed on its own and every per-stream state (audio
+// tail, mel rings, smoothing state, expression value) is stored per stream -- only the addressing did: koe_stream_push
+// derives one tail buffer, one ring slot and one ring base from one shared step counter.  Here the pool object keeps a
+// clock per slot, and each push hands the kernels small tables built from those clocks:
+//   pushing stream i:  slot, ring row (the slot of its newest complete frame), first hop or not
+//   emitting stream w: slot, ring base, has smoothing state or not
+// A push of n streams queues: the tail update (in place, per slot) with a compact copy of the tails, the frontend
+// launches of koe_stream_push on the compact tails into compact staging rows, the scatter of those rows into each slot's
+// rings, and -- when at least one stream emits -- the core over the emitting streams only and the smoothing.
+//
+// Stream n's frames are numbered from its own first hop: the newest complete frame after hop n is g = n - lag (lag =
+// n_edge - 1) in ring row g mod W, and the window that ends after hop n starts at ring row (n + 1 - W) mod W -- the
+// arithmetic of koe_stream_push, per stream.
+#include <map>
+#include <mutex>
+#include <utility>
+#include <vector>
+
+#include "core_params.cuh"
+
+struct koe_stream_pool {
+  int capacity, hop, window_frames, half_fft, n_edge, tail_len;
+  std::vector<unsigned char> open;
+  std::vector<int64_t> hops;      // hops pushed since the slot was opened
+  std::vector<int64_t> frames;    // frames emitted since the slot was opened
+  std::vector<int32_t> row;       // ring row of the newest complete frame after the next hop, (hops - lag) mod W: kept as
+                                  // a counter, so that a push of thousands of streams does no division on the host
+  std::vector<uint32_t> listed;   // duplicate check: the call that last listed the slot
+  uint32_t call = 0;
+};
+
+namespace koe {
+
+// pushing stream i: new_tail = [old_tail[hop:], hop_audio[i]] in slot push_slot[i]'s own tail (an opened slot's first
+// hop reads the old tail as zeros: this is where a reused slot forgets its previous stream), copied to compact row i for
+// the frontend.  One CTA per stream row: read, barrier, write.
+__global__ void __launch_bounds__(256) pool_tail_kernel(float* __restrict__ tail, const float* __restrict__ hop_audio,
+                                                         const int* __restrict__ push_slot, const int* __restrict__ push_first,
+                                                         int n, int tail_len, int hop, float* __restrict__ compact) {
+  extern __shared__ float s_tail[];
+  const int keep = tail_len - hop;
+  for (int i = blockIdx.x; i < n; i += gridDim.x) {
+    float* t = tail + (long long)__ldg(push_slot + i) * tail_len;
+    const bool first = __ldg(push_first + i) != 0;
+    const float* x = hop_audio + (long long)i * hop;
+    for (int k = threadIdx.x; k < keep; k += blockDim.x) s_tail[k] = first ? 0.0f : t[hop + k];
+    for (int k = threadIdx.x; k < hop; k += blockDim.x) s_tail[keep + k] = __ldcs(x + k);
+    __syncthreads();
+    float* c = compact + (long long)i * tail_len;
+    for (int k = threadIdx.x; k < tail_len; k += blockDim.x) {
+      const float v = s_tail[k];
+      t[k] = v;
+      c[k] = v;
+    }
+    __syncthreads();
+  }
+}
+
+struct PoolRings {
+  float* power[1 + 2 * KOE_MAX_EDGE];  // plain ring, window-start ring 0, window-end row 0, window-start ring 1, window-end row 1
+  float* fmax[1 + 2 * KOE_MAX_EDGE];
+};
+
+// staged row v of pushing stream i ([n][V][80], maxima [n][V]) -> ring row push_row[i] of slot push_slot[i] (plain and
+// window-start variants) or the slot's own row (window-end variants)
+__global__ void __launch_bounds__(256) pool_scatter_kernel(PoolRings r, const float* __restrict__ stage,
+                                                            const float* __restrict__ stage_max,
+                                                            const int* __restrict__ push_slot,
+                                                            const int* __restrict__ push_row, int n, int n_var, int W) {
+  constexpr int kQuads = KOE_N_MELS / 4;
+  const int total = n * n_var * kQuads;
+  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
+    const int q = idx % kQuads, iv = idx / kQuads, v = iv % n_var, i = iv / n_var;
+    const long long s = __ldg(push_slot + i);
+    const long long row = v > 0 && (v & 1) == 0 ? s : s * W + __ldg(push_row + i);
+    reinterpret_cast<float4*>(r.power[v] + row * KOE_N_MELS)[q] = __ldcs(reinterpret_cast<const float4*>(stage) + (long long)iv * kQuads + q);
+    if (q == 0) r.fmax[v][row] = __ldcs(stage_max + iv);
+  }
+}
+
+// smoothing of the emitting streams: the roundings of ema_step_kernel (koe_ema_scan with n_out = 1), with stream
+// emit_slot[w]'s state for output row w
+__global__ void __launch_bounds__(256) pool_ema_kernel(float* __restrict__ frames, int k, float alpha,
+                                                        float* __restrict__ state, const int* __restrict__ emit_slot,
+                                                        const int* __restrict__ emit_has_state) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= k * KOE_N_BLENDSHAPES) return;
+  const int w = i / KOE_N_BLENDSHAPES, j = i % KOE_N_BLENDSHAPES;
+  float* st = state + (long long)__ldg(emit_slot + w) * KOE_N_BLENDSHAPES + j;
+  const float x = frames[i];
+  const float y = __ldg(emit_has_state + w) ? fmaf(1.0f - alpha, *st, alpha * x) : x;
+  frames[i] = y;
+  *st = y;
+}
+
+__global__ void __launch_bounds__(256) pool_expr_scatter_kernel(const float* __restrict__ compact, const int* __restrict__ slot,
+                                                                 int n, float* __restrict__ expr_sigmoid) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i < n) expr_sigmoid[__ldg(slot + i)] = compact[i];
+}
+
+namespace {
+// Pinned staging of the per-call tables, per (device, stream): a ring of kDepth buffers, each guarded by an event
+// recorded after the copy that reads it, so the host may run kDepth calls ahead of the device before it waits.
+struct PoolStaging {
+  static constexpr int kDepth = 4;
+  struct Buf {
+    int32_t* host = nullptr;
+    size_t ints = 0;
+    cudaEvent_t copied = nullptr;
+  };
+  struct Ring {
+    Buf buf[kDepth];
+    int next = 0;
+  };
+  std::mutex mu;
+  std::map<std::pair<int, void*>, Ring> rings;
+
+  // a buffer of >= ints entries that no queued copy reads any more
+  int acquire(void* stream, size_t ints, Buf** out) {
+    int dev = 0;
+    KOE_CUDA(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lock(mu);
+    Ring& r = rings[{dev, stream}];
+    Buf& b = r.buf[r.next];
+    r.next = (r.next + 1) % kDepth;
+    if (b.copied == nullptr) KOE_CUDA(cudaEventCreateWithFlags(&b.copied, cudaEventDisableTiming));
+    else KOE_CUDA(cudaEventSynchronize(b.copied));
+    if (b.ints < ints) {
+      if (b.host != nullptr) KOE_CUDA(cudaFreeHost(b.host));
+      b.host = nullptr, b.ints = 0;
+      const size_t want = std::max<size_t>(ints, 1024);
+      KOE_CUDA(cudaHostAlloc(&b.host, want * sizeof(int32_t), cudaHostAllocDefault));
+      b.ints = want;
+    }
+    *out = &b;
+    return KOE_OK;
+  }
+};
+PoolStaging g_pool_staging;
+
+// one copy of host[0, ints) to the device tables, then the event that frees the staging buffer
+int upload_tables(PoolStaging::Buf* b, int32_t* dev_tables, size_t ints, cudaStream_t stream) {
+  KOE_CUDA(cudaMemcpyAsync(dev_tables, b->host, ints * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+  KOE_CUDA(cudaEventRecord(b->copied, stream));
+  return KOE_OK;
+}
+
+int num_sms() {
+  static int sms[64] = {0};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
+  if (sms[dev] == 0 && cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
+  return sms[dev];
+}
+
+// every slot of slots[0, n) in range, open and listed once
+int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* what) {
+  KOE_REQUIRE(n >= 0 && n <= pool->capacity, "%s: %d streams for a pool of %d", what, n, pool->capacity);
+  KOE_REQUIRE(n == 0 || slots != nullptr, "%s: NULL slots", what);
+  if (++pool->call == 0) {  // (the stamp wrapped: forget every earlier call)
+    std::fill(pool->listed.begin(), pool->listed.end(), 0u);
+    pool->call = 1;
+  }
+  for (int i = 0; i < n; ++i) {
+    const int s = slots[i];
+    KOE_REQUIRE(s >= 0 && s < pool->capacity, "%s: slot %d out of range [0, %d)", what, s, pool->capacity);
+    KOE_REQUIRE(pool->open[s], "%s: slot %d is not open", what, s);
+    KOE_REQUIRE(pool->listed[s] != pool->call, "%s: slot %d listed twice", what, s);
+    pool->listed[s] = pool->call;
+  }
+  return KOE_OK;
+}
+
+int check_capture(void* stream, const char* what) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  KOE_CUDA(cudaStreamIsCapturing((cudaStream_t)stream, &cap));
+  if (cap != cudaStreamCaptureStatusNone)
+    return fail(KOE_E_UNSUPPORTED, "%s cannot be captured into a CUDA graph: its tables change every call", what);
+  return KOE_OK;
+}
+}  // namespace
+
+}  // namespace koe
+
+using namespace koe;
+
+extern "C" int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_fft, koe_stream_pool_t** out) {
+  KOE_REQUIRE(out != nullptr, "koe_stream_pool_create: NULL argument");
+  *out = nullptr;
+  KOE_REQUIRE(capacity >= 1 && capacity <= (1 << 24) && hop > 0 && window_frames > 0 && half_fft > 0,
+              "koe_stream_pool_create: bad geometry");
+  const int n_edge = (half_fft + hop - 1) / hop;
+  KOE_REQUIRE(n_edge >= 1 && n_edge <= KOE_MAX_EDGE && window_frames + 1 > 2 * n_edge,
+              "koe_stream_pool_create: hop %d needs %d edge frames per window side (max %d)", hop, n_edge, KOE_MAX_EDGE);
+  auto* p = new koe_stream_pool();
+  p->capacity = capacity, p->hop = hop, p->window_frames = window_frames, p->half_fft = half_fft, p->n_edge = n_edge;
+  p->tail_len = half_fft + n_edge * hop;
+  p->open.assign(capacity, 0);
+  p->hops.assign(capacity, 0);
+  p->frames.assign(capacity, 0);
+  p->row.assign(capacity, 0);
+  p->listed.assign(capacity, 0);
+  *out = p;
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_destroy(koe_stream_pool_t* pool) {
+  delete pool;
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_open(koe_stream_pool_t* pool, int n, int32_t* slots_host) {
+  KOE_REQUIRE(pool != nullptr && (n == 0 || slots_host != nullptr), "koe_stream_pool_open: NULL argument");
+  KOE_REQUIRE(n >= 0, "koe_stream_pool_open: negative count");
+  int free_slots = 0;
+  for (int s = 0; s < pool->capacity; ++s) free_slots += pool->open[s] ? 0 : 1;
+  KOE_REQUIRE(n <= free_slots, "koe_stream_pool_open: %d streams asked, %d of %d slots free", n, free_slots, pool->capacity);
+  for (int s = 0, i = 0; i < n; ++s) {
+    if (pool->open[s]) continue;
+    pool->open[s] = 1;
+    pool->hops[s] = 0;
+    pool->frames[s] = 0;
+    pool->row[s] = (pool->window_frames - (pool->n_edge - 1)) % pool->window_frames;
+    slots_host[i++] = s;
+  }
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_close(koe_stream_pool_t* pool, int slot) {
+  KOE_REQUIRE(pool != nullptr, "koe_stream_pool_close: NULL pool");
+  KOE_REQUIRE(slot >= 0 && slot < pool->capacity, "koe_stream_pool_close: slot %d out of range [0, %d)", slot, pool->capacity);
+  KOE_REQUIRE(pool->open[slot], "koe_stream_pool_close: slot %d is not open", slot);
+  pool->open[slot] = 0;
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_set_egemaps(koe_stream_pool_t* pool, const koe_stream_pool_args* a, const int32_t* slots_host,
+                                           int n, const float* egemaps, void* stream) {
+  KOE_REQUIRE(pool != nullptr && a != nullptr, "koe_stream_pool_set_egemaps: NULL argument");
+  if (int rc = check_slots(pool, slots_host, n, "koe_stream_pool_set_egemaps")) return rc;
+  if (n == 0) return KOE_OK;
+  KOE_REQUIRE(a->weights != nullptr && egemaps != nullptr && a->expr_sigmoid != nullptr && a->expr_compact != nullptr &&
+                  a->tables != nullptr,
+              "koe_stream_pool_set_egemaps: NULL buffer");
+  if (int rc = check_capture(stream, "koe_stream_pool_set_egemaps")) return rc;
+  PoolStaging::Buf* b = nullptr;
+  if (int rc = g_pool_staging.acquire(stream, (size_t)n, &b)) return rc;
+  std::copy(slots_host, slots_host + n, b->host);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = upload_tables(b, a->tables, (size_t)n, st)) return rc;
+  if (int rc = launch_emotion_stream(a->weights, egemaps, n, a->expr_compact, nullptr, nullptr, 1, stream, false)) return rc;
+  pool_expr_scatter_kernel<<<(n + 255) / 256, 256, 0, st>>>(a->expr_compact, a->tables, n, a->expr_sigmoid);
+  count_launch();
+  KOE_CUDA(cudaGetLastError());
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_pool_args* a, const int32_t* slots_host, int n,
+                                    int32_t* emitted_host, int* n_emitted, void* stream) {
+  KOE_REQUIRE(pool != nullptr && a != nullptr && n_emitted != nullptr && emitted_host != nullptr,
+              "koe_stream_pool_push: NULL argument");
+  *n_emitted = 0;
+  if (int rc = check_slots(pool, slots_host, n, "koe_stream_pool_push")) return rc;
+  if (n == 0) return KOE_OK;
+  const int W = pool->window_frames, n_edge = pool->n_edge, tail_len = pool->tail_len;
+  const int hop = pool->hop, half = pool->half_fft, V = 1 + 2 * n_edge, lag = n_edge - 1;
+  KOE_REQUIRE(a->frontend != nullptr && a->weights != nullptr, "koe_stream_pool_push: NULL frontend / weights");
+  KOE_REQUIRE(a->weights->k_mel == W + 3, "koe_stream_pool_push: weights for k_mel %d, pool of window_frames %d",
+              a->weights->k_mel, W);
+  KOE_REQUIRE(a->hop_audio && a->tail && a->tail_compact && a->stage && a->stage_max && a->ring_f && a->fmax_f && a->ring_r &&
+                  a->fmax_r && a->row_l && a->fmax_l && a->expr_sigmoid && a->out && a->tables,
+              "koe_stream_pool_push: NULL buffer");
+  KOE_REQUIRE(n_edge == 1 || (a->ring_r2 && a->fmax_r2 && a->row_l2 && a->fmax_l2),
+              "koe_stream_pool_push: hop < n_fft/2 needs the second edge buffers (ring_r2, row_l2)");
+  KOE_REQUIRE(a->ema_state == nullptr || (a->alpha >= 0.0f && a->alpha <= 1.0f), "koe_stream_pool_push: alpha must be in [0, 1]");
+  if (int rc = check_capture(stream, "koe_stream_pool_push")) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+
+  // ---- the per-call tables: [push slot | push ring row | push first hop][emit slot | emit ring base | emit has state]
+  PoolStaging::Buf* b = nullptr;
+  if (int rc = g_pool_staging.acquire(stream, 6 * (size_t)n, &b)) return rc;
+  int32_t* h = b->host;
+  int k = 0;
+  for (int i = 0; i < n; ++i) {
+    const int s = slots_host[i];
+    const int64_t age = pool->hops[s];  // hops before this one
+    h[i] = s;
+    h[n + i] = pool->row[s];
+    h[2 * n + i] = age == 0 ? 1 : 0;
+    if (age + 1 >= W) emitted_host[k++] = s;  // this hop completes a window
+  }
+  // the emit columns are k long, laid out after the push columns; ring base (n + 1 - W) mod W = (row + lag + 1) mod W
+  for (int w = 0; w < k; ++w) {
+    const int s = emitted_host[w];
+    const int base = pool->row[s] + lag + 1;
+    h[3 * n + w] = s;
+    h[3 * n + k + w] = base >= W ? base - W : base;
+    h[3 * n + 2 * k + w] = pool->frames[s] > 0 ? 1 : 0;
+  }
+  const size_t ints = 3 * (size_t)n + 3 * (size_t)k;
+  if (int rc = upload_tables(b, a->tables, ints, st)) return rc;
+  const int* push_slot = a->tables;
+  const int* push_row = a->tables + n;
+  const int* push_first = a->tables + 2 * n;
+  const int* emit_slot = a->tables + 3 * n;
+  const int* emit_base = emit_slot + k;
+  const int* emit_has = emit_slot + 2 * k;
+
+  // ---- 1. tail update + compact copy
+  {
+    const int grid = std::min(n, std::max(num_sms(), 1) * 8);
+    pool_tail_kernel<<<grid, 256, tail_len * sizeof(float), st>>>(a->tail, a->hop_audio, push_slot, push_first, n, tail_len,
+                                                                  hop, a->tail_compact);
+    count_launch();
+    KOE_CUDA(cudaGetLastError());
+  }
+  // ---- 2. the frontend launches of koe_stream_push, on the compact tails, into staging rows [n][V][80]
+  float* stage[1 + 2 * KOE_MAX_EDGE];
+  float* stage_max[1 + 2 * KOE_MAX_EDGE];
+  for (int v = 0; v < V; ++v) stage[v] = a->stage + (size_t)v * KOE_N_MELS, stage_max[v] = a->stage_max + v;
+  koe_logmel_args f = {};
+  f.audio = a->tail_compact;
+  f.audio_stride = tail_len;
+  f.n_clips = n;
+  f.n_samples = tail_len;
+  f.hop = hop;
+  f.frame_offset = 0;
+  f.frame_step = 1;
+  f.pad_mode = 0;
+  f.sample_offset = half;
+  f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = KOE_NO_EDGE;
+  f.power_clip_stride = (int64_t)V * KOE_N_MELS, f.frame_max_clip_stride = V;
+  f.power_b_clip_stride = (int64_t)V * KOE_N_MELS, f.frame_max_b_clip_stride = V;
+  // plain frame g and the frame one hop later (30 fps: the window-end row; 60 fps: the last-but-one frame of the window)
+  f.n_frames = 2;
+  f.power = stage[0], f.frame_max = stage_max[0];
+  f.power_b = n_edge == 1 ? stage[2] : stage[4], f.frame_max_b = n_edge == 1 ? stage_max[2] : stage_max[4];
+  if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
+  f.power_b = nullptr, f.frame_max_b = nullptr;
+  f.n_frames = 1;
+  if (n_edge == 2) {  // the frame centred on the tail's end: the window's last frame
+    f.frame_offset = 2;
+    f.power = stage[2], f.frame_max = stage_max[2];
+    if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
+    f.frame_offset = 0;
+  }
+  for (int m = 0; m < n_edge; ++m) {  // window-start variants of frame g
+    f.lo_rel_hops = -m;
+    f.power = stage[1 + 2 * m], f.frame_max = stage_max[1 + 2 * m];
+    if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
+  }
+  // ---- 3. staging rows -> each slot's rings and window-end rows
+  PoolRings r{};
+  float* const power[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, a->row_l, a->ring_r2, a->row_l2};
+  float* const fmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, a->fmax_l, a->fmax_r2, a->fmax_l2};
+  for (int v = 0; v < V; ++v) r.power[v] = power[v], r.fmax[v] = fmax[v];
+  {
+    const int total = n * V * (KOE_N_MELS / 4);
+    pool_scatter_kernel<<<std::min((total + 255) / 256, std::max(num_sms(), 1) * 8), 256, 0, st>>>(
+        r, a->stage, a->stage_max, push_slot, push_row, n, V, W);
+    count_launch();
+    KOE_CUDA(cudaGetLastError());
+  }
+  // ---- 4. the core over the emitting streams, 5. their smoothing
+  if (k > 0) {
+    const float* cpower[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, a->row_l, a->ring_r2, a->row_l2};
+    const float* cfmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, a->fmax_l, a->fmax_r2, a->fmax_l2};
+    if (int rc = launch_dual_stream_pool(a->weights, cpower, cfmax, n_edge, k, W, emit_slot, emit_base, a->expr_sigmoid,
+                                         a->out, a->precision, stream))
+      return rc;
+    if (a->ema_state != nullptr) {
+      pool_ema_kernel<<<(k * KOE_N_BLENDSHAPES + 255) / 256, 256, 0, st>>>(a->out, k, a->alpha, a->ema_state, emit_slot,
+                                                                          emit_has);
+      count_launch();
+      KOE_CUDA(cudaGetLastError());
+    }
+  }
+  // ---- the clocks advance once everything is queued
+  for (int i = 0; i < n; ++i) {
+    const int s = slots_host[i];
+    if (++pool->hops[s] >= W) ++pool->frames[s];
+    if (++pool->row[s] == W) pool->row[s] = 0;
+  }
+  *n_emitted = k;
+  return KOE_OK;
+}

@@ -16,7 +16,8 @@ L0[n+1] -- 5 FFTs per hop against 513.  F and R rows go into per-stream rings of
 (164 KB per stream), the only audio kept is the last ``n_fft/2 + hop`` samples, and the core kernel addresses the
 rings directly (``koe_dual_stream_ring``).  After the 256th hop every step emits the frame that
 ``SequentialDualStreamModel.forward`` would produce for the window ending at the newest sample, EMA included.
-All streams advance in lockstep (one hop per step each).
+All streams of a StreamingEngine advance in lockstep (one hop per step each); in a StreamPool every stream opens,
+closes and advances on its own clock.
 """
 from __future__ import annotations
 
@@ -207,3 +208,208 @@ class StreamingEngine:
                                             1 if self.emitted > 0 else 0, st), "koe_ema_scan")
         self.emitted += 1
         return self.out
+
+
+class StreamPool:
+    """Up to ``capacity`` concurrent streams that open, close and advance on their own clocks (``koe_stream_pool_*`` in
+    include/koemorph_b200.h): a real-time service whose users connect and leave at any time and whose packets arrive
+    late.  Every stream of the pool computes bit for bit what a one-stream :class:`StreamingEngine` computes when fed
+    the same hops from the moment the stream was opened, whatever the other streams do and whatever its slot held
+    before: it emits from its own W-th hop on (256 at 30 fps, 512 at 60 fps), its first frame passes the smoothing
+    unchanged, and a reused slot carries nothing over.  The clocks live in the native pool object; this class owns the
+    device buffers and checks what it hands over."""
+
+    def __init__(self, model, capacity: int):
+        self.model = model
+        self.capacity = int(capacity)
+        if self.capacity < 1:
+            raise ValueError(f"capacity must be >= 1, got {capacity}")
+        self.dev = next(model.parameters()).device
+        if self.dev.type != "cuda":
+            raise RuntimeError("StreamPool needs the model on a CUDA device")
+        self._dev_index = self.dev.index if self.dev.index is not None else torch.cuda.current_device()
+        self.hop = model.hop_length
+        self.W = model.mel_sequence_length
+        self.half = model.n_fft // 2
+        self.n_edge = -(-self.half // self.hop)            # edge frames per window side (StreamingEngine)
+        if self.n_edge > _lib.MAX_EDGE:
+            raise NotImplementedError(f"hop {self.hop} needs {self.n_edge} edge frames per window side (max {_lib.MAX_EDGE})")
+        self.tail_len = self.half + self.n_edge * self.hop
+        cap, V = self.capacity, 1 + 2 * self.n_edge
+        f32 = dict(dtype=torch.float32, device=self.dev)
+        self.tail = torch.zeros(cap, self.tail_len, **f32)
+        self.tail_compact = torch.empty(cap, self.tail_len, **f32)
+        self.stage = torch.empty(cap, V, 80, **f32)
+        self.stage_max = torch.empty(cap, V, **f32)
+        self.ring_f = torch.zeros(cap, self.W, 80, **f32)
+        self.ring_r = torch.zeros(cap, self.W, 80, **f32)
+        self.fmax_f = torch.zeros(cap, self.W, **f32)
+        self.fmax_r = torch.zeros(cap, self.W, **f32)
+        self.row_l = torch.zeros(cap, 80, **f32)
+        self.fmax_l = torch.zeros(cap, **f32)
+        if self.n_edge == 2:
+            self.ring_r2 = torch.zeros(cap, self.W, 80, **f32)
+            self.fmax_r2 = torch.zeros(cap, self.W, **f32)
+            self.row_l2 = torch.zeros(cap, 80, **f32)
+            self.fmax_l2 = torch.zeros(cap, **f32)
+        else:
+            self.ring_r2 = self.fmax_r2 = self.row_l2 = self.fmax_l2 = None
+        self.expr = torch.zeros(cap, **f32)
+        self.expr_compact = torch.empty(cap, **f32)
+        self.state = torch.zeros(cap, 52, **f32)
+        self.out = torch.zeros(cap, 52, **f32)
+        self.tables = torch.empty(6 * cap, dtype=torch.int32, device=self.dev)
+        self._emitted = torch.empty(cap, dtype=torch.int32)  # host: the slots of the last push's frames
+        self._n_emitted = C.c_int(0)
+        self._n_emitted_ref = C.byref(self._n_emitted)
+        self._lib = _lib.load()
+        h = C.c_void_p()
+        self._check(self._lib.koe_stream_pool_create(cap, self.hop, self.W, self.half, C.byref(h)), "koe_stream_pool_create")
+        self._h = h
+        self._fe = model._frontend(self.dev)
+        self._alpha, self._alpha_key = 0.0, None
+        self._args, self._args_key, self._w_tensors = None, None, []
+        self.pushes = 0
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h is not None and h.value:
+            self._lib.koe_stream_pool_destroy(h)
+            self._h = None
+
+    # ---- public API -------------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def open(self, egemaps: torch.Tensor) -> list:
+        """Opens k streams for egemaps (k, 264) (or (k, 3, 88)); returns their slots.  Their clocks start at zero."""
+        eg = self._egemaps(egemaps)
+        k = eg.shape[0]
+        slots = torch.empty(k, dtype=torch.int32)
+        self._check(self._lib.koe_stream_pool_open(self._h, k, slots.data_ptr()), "koe_stream_pool_open")
+        try:
+            self._set_egemaps(slots, eg)
+        except BaseException:
+            for s in slots.tolist():
+                self._lib.koe_stream_pool_close(self._h, s)
+            raise
+        return slots.tolist()
+
+    def close(self, slot: int) -> None:
+        """Frees the slot of an open stream; the next stream opened there starts from silence."""
+        slot = int(slot)
+        if not 0 <= slot < self.capacity:
+            raise ValueError(f"slot {slot} out of range [0, {self.capacity})")
+        self._check(self._lib.koe_stream_pool_close(self._h, slot), "koe_stream_pool_close")
+
+    @torch.no_grad()
+    def set_egemaps(self, slots, egemaps: torch.Tensor) -> None:
+        """Refreshes the expression input of the listed open streams only: egemaps row i belongs to slots[i]."""
+        s = self._slots(slots)
+        eg = self._egemaps(egemaps)
+        if eg.shape[0] != s.numel():
+            raise ValueError(f"egemaps has {eg.shape[0]} rows for {s.numel()} slots")
+        self._set_egemaps(s, eg)
+
+    @torch.no_grad()
+    def push(self, slots, hop_audio: torch.Tensor):
+        """Advances exactly the listed open streams by one hop each: hop_audio (n, hop) float32 on the model's device,
+        row i the next hop of slots[i].  Returns (emitted_slots, frames): a CPU int64 tensor of the streams that emitted
+        a frame in this call, in call order, and their (k, 52) smoothed frames -- a view reused by the next call."""
+        s = self._slots(slots)
+        n = s.numel()
+        if not isinstance(hop_audio, torch.Tensor):
+            raise ValueError(f"hop_audio must be a torch.Tensor, got {type(hop_audio).__name__}")
+        if hop_audio.device != self.dev or hop_audio.dtype != torch.float32:
+            raise ValueError(f"hop_audio must be float32 on {self.dev}, got {hop_audio.dtype} on {hop_audio.device}")
+        if tuple(hop_audio.shape) != (n, self.hop):
+            raise ValueError(f"hop_audio must be ({n}, {self.hop}) for {n} slots, got {tuple(hop_audio.shape)}")
+        x = hop_audio.contiguous()
+        a = self._current_args()
+        a.hop_audio = x.data_ptr()
+        self._call(self._lib.koe_stream_pool_push, self._h, self._args_ref, s.data_ptr(), n, self._emitted.data_ptr(),
+                   self._n_emitted_ref, what="koe_stream_pool_push")
+        self.pushes += 1
+        k = self._n_emitted.value
+        return self._emitted[:k].to(torch.int64), self.out[:k]
+
+    # ---- helpers ----------------------------------------------------------------------------------------------------
+    def _check(self, rc: int, what: str) -> None:
+        if rc == -1:   # KOE_E_INVALID: misuse (slot out of range / not open / listed twice, pool full)
+            msg = self._lib.koe_last_error()
+            raise ValueError(f"{what}: {msg.decode() if msg else 'invalid argument'}")
+        _lib.check(rc, what)
+
+    def _call(self, fn, *args, what: str) -> None:
+        if torch.cuda.current_device() == self._dev_index:
+            rc = fn(*args, torch.cuda.current_stream(self.dev).cuda_stream)
+        else:
+            with torch.cuda.device(self.dev):
+                rc = fn(*args, torch.cuda.current_stream(self.dev).cuda_stream)
+        self._check(rc, what)
+
+    def _slots(self, slots) -> torch.Tensor:
+        s = slots if isinstance(slots, torch.Tensor) else torch.as_tensor(slots, dtype=torch.int64)
+        if s.device.type != "cpu":
+            raise ValueError("slots must be host (CPU) indices")
+        if s.dim() != 1 or s.is_floating_point() or s.is_complex() or s.dtype == torch.bool:
+            raise ValueError(f"slots must be a 1-D sequence of integers, got {s.dtype} of shape {tuple(s.shape)}")
+        if s.dtype == torch.int32:        # (the library checks the range of every slot itself)
+            return s.contiguous()
+        if s.numel() and (int(s.min()) < 0 or int(s.max()) >= self.capacity):
+            raise ValueError(f"slots must lie in [0, {self.capacity})")
+        return s.to(torch.int32)
+
+    def _egemaps(self, egemaps) -> torch.Tensor:
+        if not isinstance(egemaps, torch.Tensor):
+            raise ValueError(f"egemaps must be a torch.Tensor, got {type(egemaps).__name__}")
+        if egemaps.device != self.dev or egemaps.dtype != torch.float32:
+            raise ValueError(f"egemaps must be float32 on {self.dev}, got {egemaps.dtype} on {egemaps.device}")
+        eg = egemaps.reshape(egemaps.shape[0], -1) if egemaps.dim() == 3 else egemaps
+        if eg.dim() != 2 or eg.shape[1] != 264:
+            raise ValueError(f"egemaps must be (k, 264) or (k, 3, 88), got {tuple(egemaps.shape)}")
+        return eg.contiguous()
+
+    def _set_egemaps(self, s: torch.Tensor, eg: torch.Tensor) -> None:
+        self._current_args()
+        self._call(self._lib.koe_stream_pool_set_egemaps, self._h, self._args_ref, s.data_ptr(), s.numel(), eg.data_ptr(),
+                   what="koe_stream_pool_set_egemaps")
+
+    def _current_args(self):
+        # the folded weights are re-validated against the module's parameters by their in-place version counters every
+        # call, and by the full walk over the module (replaced tensors: .to(), new Parameters) every 256th push
+        m = self.model
+        a = self._args
+        key = (m.precision, m.use_temporal_smoothing, tuple(t._version for t in self._w_tensors))
+        if a is None or self._args_key != key or (self.pushes & 255) == 0:
+            a = self._args = self._build_args()
+            self._args_key = (m.precision, m.use_temporal_smoothing, tuple(t._version for t in self._w_tensors))
+        if m.use_temporal_smoothing:
+            # sigmoid(smoothing_alpha) is read back once per parameter version, not once per hop (a device sync)
+            ver = (m.smoothing_alpha.data_ptr(), m.smoothing_alpha._version)
+            if self._alpha_key != ver:
+                self._alpha = float(torch.sigmoid(m.smoothing_alpha.detach().float()))
+                self._alpha_key = ver
+            a.alpha = self._alpha
+        return a
+
+    def _build_args(self):
+        m = self.model
+        self._weights = m.dual_stream_attention.kernel_weights(m._compression)   # (kept alive: the block points into it)
+        att = m.dual_stream_attention
+        self._w_tensors = [t for _, t in att.named_parameters()] + [t for _, t in att.named_buffers()] + \
+            ([] if m._compression is None else [m._compression["weight"], m._compression["bias"]])
+        a = _lib.StreamPoolArgs()
+        a.frontend, a.weights = self._fe._h, C.cast(C.pointer(self._weights.struct), C.c_void_p)
+        a.tail, a.tail_compact = self.tail.data_ptr(), self.tail_compact.data_ptr()
+        a.stage, a.stage_max = self.stage.data_ptr(), self.stage_max.data_ptr()
+        a.ring_f, a.fmax_f = self.ring_f.data_ptr(), self.fmax_f.data_ptr()
+        a.ring_r, a.fmax_r = self.ring_r.data_ptr(), self.fmax_r.data_ptr()
+        a.row_l, a.fmax_l = self.row_l.data_ptr(), self.fmax_l.data_ptr()
+        if self.n_edge == 2:
+            a.ring_r2, a.fmax_r2 = self.ring_r2.data_ptr(), self.fmax_r2.data_ptr()
+            a.row_l2, a.fmax_l2 = self.row_l2.data_ptr(), self.fmax_l2.data_ptr()
+        a.expr_sigmoid, a.expr_compact, a.out = self.expr.data_ptr(), self.expr_compact.data_ptr(), self.out.data_ptr()
+        a.ema_state, a.alpha = (self.state.data_ptr(), self._alpha) if m.use_temporal_smoothing else (None, 1.0)
+        a.tables = self.tables.data_ptr()
+        a.precision = _lib.PRECISIONS[m.precision]
+        self._args_ref = C.byref(a)
+        return a
