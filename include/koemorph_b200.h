@@ -42,8 +42,8 @@ extern "C" {
 const char* koe_last_error(void);
 int koe_version(void);
 /* sizeof of the public argument structs, for bindings that mirror them (ctypes, cgo, JNI): 0 koe_frontend_config,
- * 1 koe_logmel_args, 2 koe_core_weights, 3 koe_stream_args, 4 koe_forward_args, 5 koe_stream_pool_args; -1 for any
- * other index */
+ * 1 koe_logmel_args, 2 koe_core_weights, 3 koe_stream_args, 4 koe_forward_args, 5 koe_stream_pool_args,
+ * 6 koe_forward_varlen_args; -1 for any other index */
 int koe_sizeof_struct(int which);
 /* number of kernels launched by this library in this process since load / since the last reset */
 int64_t koe_launch_count(void);
@@ -396,6 +396,47 @@ typedef struct {
   int32_t precision;
 } koe_forward_args;
 int koe_forward_windows(const koe_forward_args* args, void* stream);
+
+/*
+ * Packed variable-length batch: SequentialDualStreamModel.forward for clips of different lengths as ONE call.  The clips
+ * lie back to back in `audio` (clip c = samples [sum of lengths_host[0..c), + lengths_host[c])); clip c gets
+ *   n_out_c    = max(1, (L_c / hop - window_frames) / stride_frames + 1)   (floor division, as the model's num_output_frames)
+ *   n_frames_c = (n_out_c - 1) * stride_frames + window_frames + 1 global frames,
+ * and uses the window-edge variants (n_edge = ceil(half_fft / hop) per side) unless it is a single window that spans the
+ * whole clip (n_out_c == 1 and L_c <= window_frames * hop): such a clip reads every frame of its window from the plain
+ * rows, as koe_forward_windows does with n_edge = 0.  Output rows: clip c's frames are rows
+ * [sum of n_out over clips < c, + n_out_c) of out / sigmoid_out / attn_out, each bit for bit what koe_forward_windows
+ * computes for that clip alone (frame pairs of the frontend's complex FFT are formed within each clip, the smoothing
+ * restarts at each clip's first frame).  The call derives the per-clip geometry from lengths_host, validates everything
+ * (lengths in [0, 2^30), fewer than 2^31 frame pairs and windows, workspace large enough) and returns KOE_E_INVALID
+ * before anything is queued.  It uploads its per-clip tables (sample offset, length, first frame, first window, first
+ * frame pair, edge rule) with one cudaMemcpyAsync from pinned staging that the library owns per (device, stream), so it
+ * cannot be captured into a CUDA graph.  Queues the kernels of koe_forward_windows, chained the same way (no early
+ * release): frontend, 2 * n_edge edge-variant launches (none when no clip uses them), emotion stream, core and, when
+ * smooth != 0 and some clip has more than one frame, the smoothing.  Only the default filterbank (sr 16000, 80 mels,
+ * 80..8000 Hz) is implemented; other banks return KOE_E_UNSUPPORTED.
+ */
+typedef struct {
+  const koe_frontend_t* frontend;
+  const koe_core_weights* weights;   /* k_mel == window_frames + 3 */
+  const float* audio;                /* [sum of lengths] */
+  const int64_t* lengths_host;       /* [n_clips] samples per clip, HOST memory */
+  int32_t n_clips, hop, window_frames, stride_frames, half_fft; /* window_frames = mel_sequence_length; half_fft = 512 */
+  int32_t smooth;                    /* != 0: EMA over each clip's frames (first frame passes through) */
+  int32_t precision;
+  float alpha;                       /* sigmoid(smoothing_alpha) */
+  const float* egemaps;              /* [n_clips][weights->emo_in] */
+  void* workspace;                   /* caller-owned device memory of koe_forward_varlen_size's workspace_bytes, 16-byte aligned */
+  int64_t workspace_bytes;
+  float* out;                        /* [n_windows][52] */
+  float* sigmoid_out;                /* [n_windows][52], or NULL */
+  float* attn_out;                   /* [n_windows][28][80], or NULL */
+} koe_forward_varlen_args;
+/* host only (no device work): total output rows, total global frames and the workspace koe_forward_varlen needs for
+ * the lengths and geometry in args (the buffer and output fields are not read); KOE_E_INVALID on the same misuse */
+int koe_forward_varlen_size(const koe_forward_varlen_args* args, int64_t* n_windows, int64_t* n_frames,
+                            int64_t* workspace_bytes);
+int koe_forward_varlen(const koe_forward_varlen_args* args, void* stream);
 
 /*
  * Learnable-alpha exponential smoothing along the frame axis, in place

@@ -86,6 +86,15 @@ class StreamPoolArgs(C.Structure):
                 ("ema_state", C.c_void_p), ("tables", C.c_void_p), ("alpha", C.c_float), ("precision", C.c_int32)]
 
 
+class ForwardVarlenArgs(C.Structure):
+    """koe_forward_varlen_args (include/koemorph_b200.h)."""
+    _fields_ = [("frontend", C.c_void_p), ("weights", C.c_void_p), ("audio", C.c_void_p), ("lengths_host", C.c_void_p),
+                ("n_clips", C.c_int32), ("hop", C.c_int32), ("window_frames", C.c_int32), ("stride_frames", C.c_int32),
+                ("half_fft", C.c_int32), ("smooth", C.c_int32), ("precision", C.c_int32), ("alpha", C.c_float),
+                ("egemaps", C.c_void_p), ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64), ("out", C.c_void_p),
+                ("sigmoid_out", C.c_void_p), ("attn_out", C.c_void_p)]
+
+
 class FrontendConfig(C.Structure):
     """koe_frontend_config (include/koemorph_b200.h)."""
     _fields_ = [("device", C.c_int32), ("sample_rate", C.c_int32), ("n_fft", C.c_int32), ("n_mels", C.c_int32),
@@ -123,6 +132,9 @@ _SIGNATURES = {
     "koe_sizeof_struct": (C.c_int, [C.c_int]),
     "koe_stream_push": (C.c_int, [C.POINTER(StreamArgs), C.POINTER(C.c_int), C.c_void_p]),
     "koe_forward_windows": (C.c_int, [C.POINTER(ForwardArgs), C.c_void_p]),
+    "koe_forward_varlen_size": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
+                                          C.POINTER(C.c_int64)]),
+    "koe_forward_varlen": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.c_void_p]),
     "koe_stream_pool_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "koe_stream_pool_destroy": (C.c_int, [C.c_void_p]),
     "koe_stream_pool_open": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),

@@ -14,7 +14,7 @@ import sys
 
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc")
 LIB = os.path.join(CSRC, "libkoemorph_b200.so")
-SOURCES = ["api.cu", "logmel.cu", "dual_stream.cu", "dual_stream_tc.cu", "session.cu", "stream_pool.cu"]
+SOURCES = ["api.cu", "logmel.cu", "dual_stream.cu", "dual_stream_tc.cu", "session.cu", "stream_pool.cu", "staging.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

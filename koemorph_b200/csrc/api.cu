@@ -13,6 +13,7 @@ extern "C" int koe_sizeof_struct(int which) {
     case 3: return (int)sizeof(koe_stream_args);
     case 4: return (int)sizeof(koe_forward_args);
     case 5: return (int)sizeof(koe_stream_pool_args);
+    case 6: return (int)sizeof(koe_forward_varlen_args);
     default: return -1;
   }
 }

@@ -66,6 +66,27 @@ int launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* args, void* s
     if (!(cond)) return koe::fail(KOE_E_INVALID, __VA_ARGS__);   \
   } while (0)
 
+// Pinned host staging of small per-call tables (csrc/staging.cu): acquire a buffer of >= ints entries that no queued copy
+// reads any more, fill host[0, ints), then upload_tables: one cudaMemcpyAsync to the device tables and the event that frees
+// the buffer again.  check_capture refuses a call whose stream is capturing a CUDA graph (its tables change every call).
+struct TableStaging {
+  int32_t* host = nullptr;
+  size_t ints = 0;
+  cudaEvent_t copied = nullptr;
+};
+int acquire_table_staging(void* stream, size_t ints, TableStaging** out);
+int upload_tables(TableStaging* b, int32_t* dev_tables, size_t ints, cudaStream_t stream);
+int check_capture(void* stream, const char* what);
+
+// Ragged frontend launch of the packed variable-length forward (csrc/logmel.cu, default bank only): frame pair k of the
+// launch is pair k - pair_base[c] of clip c (pair_base[c] <= k < pair_base[c + 1]); clip c is `length[c]` samples at
+// audio + sample_off[c] and has row_base[c + 1] - row_base[c] frames in this launch, frame j centred on sample
+// (frame_offset + j * frame_step) * hop of the clip (window edges as lo_rel_hops / hi_rel_hops), stored to row
+// row_base[c] + j of power / frame_max.  From `a`: audio, hop, frame_offset, frame_step, lo/hi_rel_hops, power, frame_max.
+int launch_logmel_varlen(const koe_frontend_t* fe, const koe_logmel_args* a, const long long* sample_off, const int* length,
+                         const int* pair_base, const int* row_base, int n_clips, long long total_pairs, void* stream,
+                         bool follows_frontend_launch);
+
 // ---- device helpers ----------------------------------------------------------------------------
 // Programmatic dependent launch (sm_90+): a kernel launched with launch_after_primary_starts() may begin while the
 // previous kernel of the stream is still running, as soon as every CTA of that kernel has executed

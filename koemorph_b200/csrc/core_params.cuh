@@ -30,6 +30,13 @@ struct CoreParams {
   // value of stream pool_slot[w] with ring base pool_base[w], and writes output row w
   const int* pool_slot;
   const int* pool_base;
+  // packed variable-length batch (csrc/session.cu; the kVarlen instantiations only): n_clips counts windows (n_out = 1),
+  // item is the global window = output row; clip c owns windows [vl_window_base[c], vl_window_base[c + 1]) and its plain
+  // rows start at vl_frame_base[c]; vl_plain_only[c] != 0: the clip's window reads every frame from the plain rows
+  const int* vl_window_base;
+  const int* vl_frame_base;
+  const int* vl_plain_only;
+  int vl_clips;
 };
 
 // frame k of window wi of clip b: which buffer and which row (see koe_dual_stream_windows in the header)
@@ -49,17 +56,54 @@ __device__ __forceinline__ long long window_row(const CoreParams& p, int variant
 __device__ __forceinline__ long long pool_window_row(const CoreParams& p, int variant, int slot, int base, int k) {
   return variant > 0 && (variant & 1) == 0 ? (long long)slot : (long long)slot * p.ring_frames + (base + k) % p.ring_frames;
 }
-// kPool: (b, wi) of the callers below are the window's stream slot and ring base
-template <bool kPool>
+// kPool: (b, wi) of the callers below are the window's stream slot and ring base; kVarlen: the window's first plain row
+// and its global index (the row of every edge variant)
+template <bool kPool, bool kVarlen = false>
 __device__ __forceinline__ long long core_row(const CoreParams& p, int variant, int b, int wi, int k) {
-  if constexpr (kPool) return pool_window_row(p, variant, b, wi, k);
+  if constexpr (kVarlen) return variant == 0 ? (long long)b + k : (long long)wi;
+  else if constexpr (kPool) return pool_window_row(p, variant, b, wi, k);
   else return window_row(p, variant, b, wi, k);
+}
+
+// varlen: the clip of window `item` (window_base[c] <= item < window_base[c + 1]; every clip has a window).  Scalar binary
+// search, or -- every lane of a warp calling with the same item -- a 32-ary search with one table load per lane and round.
+template <bool kWarp>
+__device__ __forceinline__ int varlen_clip(const CoreParams& p, int item) {
+  const int* wb = p.vl_window_base;
+  int lo = 0, n = p.vl_clips;  // the clip is in [lo, lo + n)
+  if constexpr (kWarp) {
+    while (n > 1) {
+      const int step = (n + 31) >> 5;
+      const int i = lo + (int)(threadIdx.x & 31) * step;
+      const unsigned m = __ballot_sync(0xffffffffu, i < lo + n && __ldg(wb + i) <= item);  // lane 0 always
+      const int k = 31 - __clz(m);
+      lo += k * step;
+      n = min(step, n - k * step);
+    }
+  } else {
+    while (n > 1) {
+      const int half = n >> 1;
+      if (__ldg(wb + lo + half) <= item) lo += half, n -= half;
+      else n = half;
+    }
+  }
+  return lo;
+}
+struct VarlenWindow {
+  int row;          // first plain row
+  bool plain_only;  // no edge variants: every frame from the plain rows
+};
+template <bool kWarp>
+__device__ __forceinline__ VarlenWindow varlen_window(const CoreParams& p, int item) {
+  const int c = varlen_clip<kWarp>(p, item);
+  return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, __ldg(p.vl_plain_only + c) != 0};
 }
 
 // emotion stream launch shared by the public entry and the fused forward (csrc/session.cu, which has it write the
 // expression entries of `out`); the core launch that leaves those entries alone (expr_sigmoid == NULL); see dual_stream.cu
+// (row_base != NULL: the packed variable-length forward, clip c's output rows are [row_base[c], row_base[c + 1]))
 int launch_emotion_stream(const koe_core_weights* w, const float* emo_in, int n_clips, float* expr_sigmoid, float* out,
-                          float* sigmoid_out, int n_out, void* stream, bool after_frontend);
+                          float* sigmoid_out, int n_out, void* stream, bool after_frontend, const int* row_base = nullptr);
 int launch_dual_stream_windows(const koe_core_weights* w, const float* const* power, const float* const* frame_max, int n_edge,
                                int n_clips, int n_frames, int n_out, int stride_frames, int frames_per_window,
                                const float* expr_sigmoid, float* out, float* sigmoid_out, float* attn_out, int precision,
@@ -70,6 +114,16 @@ int launch_dual_stream_windows(const koe_core_weights* w, const float* const* po
 int launch_dual_stream_pool(const koe_core_weights* w, const float* const* power, const float* const* frame_max, int n_edge,
                             int n_windows, int ring_frames, const int* slot, const int* base, const float* expr_sigmoid,
                             float* out, int precision, void* stream);
+// the core over the windows of a packed variable-length batch (csrc/session.cu): window `item` of the n_windows belongs to
+// the clip c with window_base[c] <= item < window_base[c + 1] and writes output row `item`; plain rows from
+// frame_base[c] + (item - window_base[c]) * stride_frames, edge rows at `item` unless plain_only[c]; expression entries
+// are written by the emotion kernel
+int launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                              int n_edge, int n_windows, int n_frames, int stride_frames, int frames_per_window, int n_clips,
+                              const int* window_base, const int* frame_base, const int* plain_only, float* out,
+                              float* sigmoid_out, float* attn_out, int precision, void* stream);
+// segmented EMA of a packed variable-length batch: clip c's frames are rows [row_base[c], row_base[c + 1]) of `frames`
+int launch_ema_scan_varlen(float* frames, int n_clips, const int* row_base, float alpha, void* stream);
 // how many SMs' worth of CTAs the tensor-core core launches for n_items windows (the early-release split follows it)
 int dual_stream_tc_grid(int n_items);
 

@@ -108,9 +108,10 @@ constexpr size_t kCoreSmemFloats = (size_t)kABlockRows * kTok      // A block
                                    + 64;                           // reductions
 constexpr size_t kCoreSmem = kCoreSmemFloats * sizeof(float);
 
-// kPool: the stream-pool flavour (window item = stream p.pool_slot[item], ring base p.pool_base[item]); a separate
-// instantiation, so that the kernel every other caller runs stays exactly as it was
-template <bool kPool = false>
+// kPool: the stream-pool flavour (window item = stream p.pool_slot[item], ring base p.pool_base[item]); kVarlen: the packed
+// variable-length batch (window item of the clip found in p.vl_window_base).  Separate instantiations, so that the kernel
+// every other caller runs stays exactly as it was
+template <bool kPool = false, bool kVarlen = false>
 __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreParams p) {
   extern __shared__ __align__(16) float smem[];
   float* s_a = smem;                               // [64][80]
@@ -125,7 +126,10 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
   const int n_items = p.n_clips * p.n_out;
 
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-    const int b = kPool ? __ldg(p.pool_slot + item) : item / p.n_out, wi = kPool ? __ldg(p.pool_base + item) : item % p.n_out;
+    VarlenWindow vw{0, false};
+    if constexpr (kVarlen) vw = varlen_window<true>(p, item);
+    const int b = kVarlen ? vw.row : kPool ? __ldg(p.pool_slot + item) : item / p.n_out;
+    const int wi = kVarlen ? item : kPool ? __ldg(p.pool_base + item) : item % p.n_out;
     const bool prenorm = p.mel_long != nullptr;
 
     // ---- P0: dB reference of this window -------------------------------------------------------
@@ -133,8 +137,8 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
     if (!prenorm) {
       float mx = -INFINITY;
       for (int k = tid; k < T; k += kCoreThreads) {
-        const int v = window_variant(p, k);
-        mx = fmaxf(mx, p.fmax[v][core_row<kPool>(p, v, b, wi, k)]);
+        const int v = vw.plain_only ? 0 : window_variant(p, k);
+        mx = fmaxf(mx, p.fmax[v][core_row<kPool, kVarlen>(p, v, b, wi, k)]);
       }
       mx = warp_max(mx);
       if (tx == 0) s_red[ty] = mx;
@@ -174,9 +178,9 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
           else if (t < p.n_long)
             v = __ldg(reinterpret_cast<const float4*>(p.mel_long + ((size_t)b * p.n_frames + t) * kTok) + q);
         } else if (k >= 0) {
-          const int var = window_variant(p, k);
+          const int var = vw.plain_only ? 0 : window_variant(p, k);
           const float4 pw =
-              __ldg(reinterpret_cast<const float4*>(p.power[var] + core_row<kPool>(p, var, b, wi, k) * kTok) + q);
+              __ldg(reinterpret_cast<const float4*>(p.power[var] + core_row<kPool, kVarlen>(p, var, b, wi, k) * kTok) + q);
           v.x = normalise_db(pw.x, ref_db, true);
           v.y = normalise_db(pw.y, ref_db, true);
           v.z = normalise_db(pw.z, ref_db, true);
@@ -390,10 +394,13 @@ __device__ __forceinline__ long long global_ns() {
   return (long long)g;
 }
 
-template <int NC>
+// kVarlen: clip c's output rows are [row_base[c], row_base[c + 1]) (the packed variable-length forward) instead of n_out
+// rows from c * n_out; a separate instantiation
+template <int NC, bool kVarlen = false>
 __global__ void __launch_bounds__(kEt2Threads, 1)
 emotion_tiled_kernel(koe_core_weights W, const float* __restrict__ emo_in, int n_clips, float* __restrict__ expr_sigmoid,
-                     float* __restrict__ out, float* __restrict__ sigmoid_out, int n_out, long long* dbg) {
+                     float* __restrict__ out, float* __restrict__ sigmoid_out, int n_out, long long* dbg,
+                     const int* __restrict__ row_base) {
   constexpr int kSlots = Et2<NC>::kSlots, NP = NC / 2;
   extern __shared__ __align__(128) unsigned char et2_smem[];
   unsigned char* s_ring = et2_smem;
@@ -577,7 +584,13 @@ emotion_tiled_kernel(koe_core_weights W, const float* __restrict__ emo_in, int n
       if (out != nullptr && lane < KOE_N_EXPR) {
         const float v = fminf(fmaxf(o_coef * y, 0.0f), 1.0f);
         size_t o = (size_t)(c0 + c) * n_out * KOE_N_BLENDSHAPES + o_idx;
-        for (int wi = 0; wi < n_out; ++wi, o += KOE_N_BLENDSHAPES) {
+        int rows = n_out;
+        if constexpr (kVarlen) {
+          const int r0 = __ldg(row_base + c0 + c);
+          o = (size_t)r0 * KOE_N_BLENDSHAPES + o_idx;
+          rows = __ldg(row_base + c0 + c + 1) - r0;
+        }
+        for (int wi = 0; wi < rows; ++wi, o += KOE_N_BLENDSHAPES) {
           out[o] = v;
           if (sigmoid_out != nullptr) sigmoid_out[o] = y;
         }
@@ -607,11 +620,19 @@ __global__ void __launch_bounds__(256) ema_step_kernel(float* __restrict__ frame
   if (state != nullptr) state[i] = y;
 }
 
+// kVarlen: the segmented scan of a packed variable-length batch, clip b's frames are rows [row_base[b], row_base[b + 1])
+// (tiles counted from each clip's first frame, as for a clip alone); a separate instantiation
+template <bool kVarlen = false>
 __global__ void __launch_bounds__(256) ema_scan_kernel(float* __restrict__ frames, int n_out, float alpha,
-                                                       float* __restrict__ state, int has_state) {
+                                                       float* __restrict__ state, int has_state,
+                                                       const int* __restrict__ row_base) {
   __shared__ float s_t[kEmaTile * kEmaStride];
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   float* x = frames + (size_t)b * n_out * KOE_N_BLENDSHAPES;
+  if constexpr (kVarlen) {
+    x = frames + (size_t)__ldg(row_base + b) * KOE_N_BLENDSHAPES;
+    n_out = __ldg(row_base + b + 1) - __ldg(row_base + b);
+  }
   const float a = 1.0f - alpha;
   float apow[5];  // a^1, a^2, a^4, a^8, a^16
   apow[0] = a;
@@ -689,7 +710,7 @@ static long long* g_tc_debug = nullptr;  // (koe_debug_set_tc_timestamps below)
 // this one is the log-mel frontend, which writes nothing this kernel reads -- only then may it start beside that kernel's
 // last CTAs; `out` != NULL: the expression entries of the n_out output rows of every clip are written here).
 int koe::launch_emotion_stream(const koe_core_weights* w, const float* emo_in, int n_clips, float* expr_sigmoid, float* out,
-                               float* sigmoid_out, int n_out, void* stream, bool after_frontend) {
+                               float* sigmoid_out, int n_out, void* stream, bool after_frontend, const int* row_base) {
   if (int rc = validate_weights(w)) return rc;
   KOE_REQUIRE(n_clips >= 0 && n_out >= 1, "koe_emotion_stream: bad size");
   if (n_clips == 0) return KOE_OK;  // nothing to do: empty buffers may be NULL
@@ -704,6 +725,10 @@ int koe::launch_emotion_stream(const koe_core_weights* w, const float* emo_in, i
   if (!configured[dev]) {
     KOE_CUDA(cudaFuncSetAttribute(emotion_tiled_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Et2<8>::kSmem));
     KOE_CUDA(cudaFuncSetAttribute(emotion_tiled_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Et2<16>::kSmem));
+    KOE_CUDA(cudaFuncSetAttribute(emotion_tiled_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)Et2<8>::kSmem));
+    KOE_CUDA(cudaFuncSetAttribute(emotion_tiled_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)Et2<16>::kSmem));
     configured[dev] = true;
   }
   // every CTA streams all the weights (0.4 MB).  Eight clips per CTA: 64 CTAs of ~9 us for 512 clips, which start on the
@@ -713,13 +738,16 @@ int koe::launch_emotion_stream(const koe_core_weights* w, const float* emo_in, i
   const bool wide = n_clips > 2048;
   const dim3 grid(wide ? (n_clips + 15) / 16 : (n_clips + 7) / 8), block(kEt2Threads);
   const size_t smem = wide ? Et2<16>::kSmem : Et2<8>::kSmem;
-  auto kernel = wide ? emotion_tiled_kernel<16> : emotion_tiled_kernel<8>;
+  KOE_REQUIRE(row_base == nullptr || out != nullptr, "koe_emotion_stream: row_base without out");
+  auto kernel = row_base != nullptr ? (wide ? emotion_tiled_kernel<16, true> : emotion_tiled_kernel<8, true>)
+                                    : (wide ? emotion_tiled_kernel<16> : emotion_tiled_kernel<8>);
   long long* dbg = after_frontend && g_tc_debug != nullptr ? g_tc_debug + 128 + 2 * 148 : nullptr;
   if (after_frontend) {
     KOE_CUDA(launch_after_primary_starts(kernel, grid, block, smem, (cudaStream_t)stream, *w, emo_in, n_clips, expr_sigmoid, out,
-                                         sigmoid_out, n_out, dbg));
+                                         sigmoid_out, n_out, dbg, row_base));
   } else {
-    kernel<<<grid, block, smem, (cudaStream_t)stream>>>(*w, emo_in, n_clips, expr_sigmoid, out, sigmoid_out, n_out, dbg);
+    kernel<<<grid, block, smem, (cudaStream_t)stream>>>(*w, emo_in, n_clips, expr_sigmoid, out, sigmoid_out, n_out, dbg,
+                                                        row_base);
     KOE_CUDA(cudaGetLastError());
   }
   count_launch();
@@ -779,6 +807,8 @@ static int launch_core(const CoreParams& p_in, int precision, cudaStream_t strea
                                     (int)kCoreSmem));
       KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)kCoreSmem));
+      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)kCoreSmem));
       int n = 0;
       KOE_CUDA(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
       num_sms[dev] = n;
@@ -786,6 +816,8 @@ static int launch_core(const CoreParams& p_in, int precision, cudaStream_t strea
     const int grid = std::min(p.n_clips * p.n_out, num_sms[dev]);
     if (p.pool_slot != nullptr)
       dual_stream_fp32_kernel<true><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
+    else if (p.vl_window_base != nullptr)
+      dual_stream_fp32_kernel<false, true><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
     else
       dual_stream_fp32_kernel<false><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
     count_launch();
@@ -923,6 +955,52 @@ int koe::launch_dual_stream_pool(const koe_core_weights* w, const float* const* 
   return launch_core(p, precision, (cudaStream_t)stream);
 }
 
+int koe::launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                                   int n_edge, int n_windows, int n_frames, int stride_frames, int frames_per_window,
+                                   int n_clips, const int* window_base, const int* frame_base, const int* plain_only,
+                                   float* out, float* sigmoid_out, float* attn_out, int precision, void* stream) {
+  if (int rc = validate_weights(w)) return rc;
+  KOE_REQUIRE(power != nullptr && frame_max != nullptr && window_base != nullptr && frame_base != nullptr &&
+                  plain_only != nullptr && out != nullptr,
+              "varlen core: NULL argument");
+  KOE_REQUIRE(n_edge >= 0 && n_edge <= KOE_MAX_EDGE && n_windows >= 0 && n_clips >= 0 && stride_frames >= 1 &&
+                  frames_per_window > 2 * n_edge && frames_per_window == w->k_mel - 2,
+              "varlen core: bad sizes");
+  if (n_windows == 0) return KOE_OK;
+  CoreParams p{};
+  p.w = *w;
+  for (int j = 0; j < 1 + 2 * n_edge; ++j) {
+    KOE_REQUIRE(power[j] != nullptr && frame_max[j] != nullptr, "varlen core: NULL buffer %d", j);
+    KOE_REQUIRE((reinterpret_cast<uintptr_t>(power[j]) & 15) == 0, "varlen core: mel rows must be 16-byte aligned");
+    p.power[j] = power[j], p.fmax[j] = frame_max[j];
+  }
+  p.n_edge = n_edge;
+  p.n_clips = n_windows;
+  p.n_frames = n_frames;
+  p.n_out = 1;
+  p.stride_frames = stride_frames;
+  p.frames_per_window = frames_per_window;
+  p.mel_seq = w->k_mel - 3;
+  p.out = out;
+  p.sigmoid_out = sigmoid_out;
+  p.attn_out = attn_out;
+  p.vl_window_base = window_base;
+  p.vl_frame_base = frame_base;
+  p.vl_plain_only = plain_only;
+  p.vl_clips = n_clips;
+  return launch_core(p, precision, (cudaStream_t)stream);
+}
+
+int koe::launch_ema_scan_varlen(float* frames, int n_clips, const int* row_base, float alpha, void* stream) {
+  KOE_REQUIRE(frames != nullptr && row_base != nullptr && n_clips >= 0, "varlen smoothing: bad argument");
+  KOE_REQUIRE(alpha >= 0.0f && alpha <= 1.0f, "koe_ema_scan: alpha must be in [0, 1]");
+  if (n_clips == 0) return KOE_OK;
+  ema_scan_kernel<true><<<n_clips, 256, 0, (cudaStream_t)stream>>>(frames, 0, alpha, nullptr, 0, row_base);
+  count_launch();
+  KOE_CUDA(cudaGetLastError());
+  return KOE_OK;
+}
+
 extern "C" int koe_dual_stream_ring(const koe_core_weights* w, const float* power_ring, const float* fmax_ring,
                                     const float* power_lo_ring, const float* fmax_lo_ring, const float* power_hi,
                                     const float* fmax_hi, int n_streams, int ring_frames, int ring_base,
@@ -974,7 +1052,7 @@ extern "C" int koe_ema_scan(float* frames, int n_clips, int n_out, float alpha, 
     ema_step_kernel<<<(n_clips * KOE_N_BLENDSHAPES + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
         frames, n_clips * KOE_N_BLENDSHAPES, alpha, state, has_state);
   else
-    ema_scan_kernel<<<n_clips, 256, 0, (cudaStream_t)stream>>>(frames, n_out, alpha, state, has_state);
+    ema_scan_kernel<<<n_clips, 256, 0, (cudaStream_t)stream>>>(frames, n_out, alpha, state, has_state, nullptr);
   count_launch();
   KOE_CUDA(cudaGetLastError());
   return KOE_OK;

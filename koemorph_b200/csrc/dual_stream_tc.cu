@@ -219,9 +219,10 @@ __device__ __forceinline__ void simt_barrier() { asm volatile("bar.sync 1, 256;"
 // kEarly: the early-release flavour of the fused forward (see the wait below); a separate instantiation, so that the
 // kernel every other caller runs (streaming, sequences, the public entries) stays exactly as it was: the three extra
 // checks cost that one 4 % through register spills when they were run-time branches.  kPool: the stream-pool flavour
-// (csrc/stream_pool.cu), ring mode with a stream slot and a ring base per window (p.pool_slot, p.pool_base), kept apart
-// for the same reason.
-template <int KMEL, bool kEarly = false, bool kPool = false>
+// (csrc/stream_pool.cu), ring mode with a stream slot and a ring base per window (p.pool_slot, p.pool_base), and kVarlen: the
+// packed variable-length batch (the window's clip from p.vl_window_base; clips without edge variants read every frame from
+// the plain rows), kept apart for the same reason.
+template <int KMEL, bool kEarly = false, bool kPool = false, bool kVarlen = false>
 __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams p) {
   using G = Geo<KMEL>;
   constexpr int kKMel = G::kKMel, kA1Chunks = G::kA1Chunks, kA1Sbo = G::kA1Sbo, kLongChunks = G::kLongChunks;
@@ -356,13 +357,14 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       const uint64_t pol_keep = l2_policy_keep(), pol_stream = l2_policy_stream();
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         long long* dp = (p.dbg != nullptr && blockIdx.x == 0 && item < 2 * (int)gridDim.x) ? p.dbg + 32 + 16 * (item / gridDim.x) : nullptr;
-        const int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
+        int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
+        if constexpr (kVarlen) b = varlen_window<false>(p, item).row, wi = item;
         if (kEarly && (item == (int)blockIdx.x || item == first_late_item)) {
           if (item == first_late_item) pdl_wait();
           asm volatile("fence.proxy.async.global;" ::: "memory");  // generic-proxy acquire / wait above -> TMA reads below
         }
         const float* base = p.ring_frames > 0 ? p.power[0] + (size_t)b * p.ring_frames * kTok
-                                              : p.power[0] + core_row<kPool>(p, 0, b, wi, 0) * kTok;
+                                              : p.power[0] + core_row<kPool, kVarlen>(p, 0, b, wi, 0) * kTok;
         // Ring mode (the streaming step): with thousands of streams the rings (82 KB each: 335 MB for 4096 streams) do not
         // stay in L2 from one hop to the next, and a window's six stages pass through two ring slots one HBM latency after
         // the other.  The NEXT window's ring and frame maxima are pulled into L2 now, a whole window ahead (4096 streams:
@@ -393,7 +395,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
               bulk_g2s_hint(dst + (uint32_t)n1 * kTok * 4, base, (uint32_t)(n - n1) * kTok * 4, bar_full + 8 * slot, pol_keep);
           } else {
             bulk_g2s_hint(dst, base + (size_t)s * kMelRows * kTok, bytes, bar_full + 8 * slot,
-                          p.n_out > 1 ? pol_keep : pol_stream);  // overlapping windows of a sequence re-read their rows
+                          kVarlen || p.n_out > 1 ? pol_keep : pol_stream);  // overlapping windows of a sequence re-read their rows
           }
           if (++slot == kRing) slot = kWRing, phase ^= 1;
         }
@@ -513,7 +515,12 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
     auto frame_max_partial = [&](const int item) {
       float mx = -INFINITY;
       if (!prenorm) {
-        const int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
+        int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
+        bool plain_only = false;
+        if constexpr (kVarlen) {
+          const VarlenWindow vw = varlen_window<true>(p, item);
+          b = vw.row, wi = item, plain_only = vw.plain_only;
+        }
         for (int k0 = tid; k0 < T; k0 += 3 * kSimt) {
           float f[3];
 #pragma unroll
@@ -521,8 +528,8 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
             const int k = k0 + u * kSimt;
             f[u] = -INFINITY;
             if (k < T) {
-              const int v = window_variant(p, k);
-              f[u] = p.fmax[v][core_row<kPool>(p, v, b, wi, k)];
+              const int v = plain_only ? 0 : window_variant(p, k);
+              f[u] = p.fmax[v][core_row<kPool, kVarlen>(p, v, b, wi, k)];
             }
           }
           mx = fmaxf(fmaxf(mx, f[0]), fmaxf(f[1], f[2]));
@@ -531,7 +538,12 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       return mx;
     };
     auto stage_window = [&](const int item, float mx, long long* ds) {
-      const int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
+      int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
+      bool plain_only = false;  // (varlen) no edge variants: every frame of the window from the plain rows
+      if constexpr (kVarlen) {
+        const VarlenWindow vw = varlen_window<true>(p, item);
+        b = vw.row, wi = item, plain_only = vw.plain_only;
+      }
       // ---- window dB reference
       float ref_db = 0.0f;
       if (!prenorm) {
@@ -552,15 +564,15 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           for (int e = 0; e < 3; ++e) {
             const int k = T >= 3 ? T - 3 + e : (e < T ? e : -1);
             if (k >= 0) {
-              const int var = window_variant(p, k);
-              extra[e] = p.power[var][core_row<kPool>(p, var, b, wi, k) * kTok + tid];
+              const int var = plain_only ? 0 : window_variant(p, k);
+              extra[e] = p.power[var][core_row<kPool, kVarlen>(p, var, b, wi, k) * kTok + tid];
             } else {
               extra[e] = -INFINITY;
             }
           }
-          if (p.n_edge > 0) {
-            extra[3] = __ldg(p.power[1] + core_row<kPool>(p, 1, b, wi, 0) * kTok + tid);
-            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + core_row<kPool>(p, 2, b, wi, T - 1) * kTok + tid);
+          if (!plain_only && p.n_edge > 0) {
+            extra[3] = __ldg(p.power[1] + core_row<kPool, kVarlen>(p, 1, b, wi, 0) * kTok + tid);
+            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + core_row<kPool, kVarlen>(p, 2, b, wi, T - 1) * kTok + tid);
           }
         }
         for (int s = 0; s < n_mel_stages; ++s) {
@@ -619,13 +631,13 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           *reinterpret_cast<uint4*>(arow + (kLongChunks + 1) * 128) = make_uint4(0, 0, 0, 0);
           // edge frames inside the long-term range see zeros beyond the window edge: patch them in place
           // (frame m and frame T-1-m for m < n_edge: one per side at 30 fps, two at 60 fps)
-          for (int m = 0; m < p.n_edge; ++m) {
-            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + core_row<kPool>(p, 1 + 2 * m, b, wi, m) * kTok + j);
+          for (int m = 0; !plain_only && m < p.n_edge; ++m) {
+            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + core_row<kPool, kVarlen>(p, 1 + 2 * m, b, wi, m) * kTok + j);
             *reinterpret_cast<__nv_bfloat16*>(arow + (m >> 3) * 128 + (m & 7) * 2) =
                 __float2bfloat16_rn(normalise_bf16(lo, ref_db, true));
             const int k = T - 1 - m;
             if (k < Tl) {
-              const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + core_row<kPool>(p, 2 + 2 * m, b, wi, k) * kTok + j);
+              const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + core_row<kPool, kVarlen>(p, 2 + 2 * m, b, wi, k) * kTok + j);
               *reinterpret_cast<__nv_bfloat16*>(arow + (k >> 3) * 128 + (k & 7) * 2) =
                   __float2bfloat16_rn(normalise_bf16(x, ref_db, true));
             }
@@ -963,6 +975,22 @@ int launch_dual_stream_tc(const CoreParams& p, int precision, cudaStream_t strea
     else
       KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, true>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes,
                                            stream, p));
+  } else if (p.vl_window_base != nullptr) {
+    KOE_REQUIRE(p.n_out == 1 && p.ring_frames == 0 && p.expr_sigmoid == nullptr, "tensor-core path: bad varlen parameters");
+    static bool configured[64] = {false};
+    if (!configured[dev]) {
+      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<259, false, false, true>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBytes));
+      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<515, false, false, true>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBytes));
+      configured[dev] = true;
+    }
+    if (p.w.k_mel == 259)
+      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259, false, false, true>, dim3(grid), dim3(tc::kThreads),
+                                           tc::kSmemBytes, stream, p));
+    else
+      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, false, false, true>, dim3(grid), dim3(tc::kThreads),
+                                           tc::kSmemBytes, stream, p));
   } else if (p.pool_slot != nullptr) {
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
     static bool configured[64] = {false};

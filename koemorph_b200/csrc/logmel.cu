@@ -30,6 +30,7 @@
 #include <algorithm>
 #include <cmath>
 #include <mutex>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -84,6 +85,15 @@ struct LogmelParams {
   // stored the rows of all its iterations below early_iters -- the core's first rounds of windows need no more than that
   unsigned* early_flag;
   unsigned early_iters;
+  // packed variable-length batch (launch_logmel_varlen, the kVarlen instantiation only): pair k of the launch is pair
+  // k - vl_pair_base[c] of clip c, vl_length[c] samples at audio + vl_sample_off[c], rows vl_row_base[c] ..
+  // vl_row_base[c + 1] - 1; n_clips / n_samples / n_frames / the clip strides are not used
+  const long long* vl_sample_off;
+  const int* vl_length;
+  const int* vl_pair_base;
+  const int* vl_row_base;
+  int vl_clips;
+  unsigned vl_pairs;
 };
 
 __host__ __device__ constexpr int bitrev5(int i) {
@@ -527,6 +537,78 @@ struct PairLocator {
     pi.fb_lo = pi.fa_lo + p.frame_step * p.hop;
     return pi;
   }
+  // the located pair's samples -> registers
+  __device__ __forceinline__ void load(const LogmelParams& p, const PairInfo& pi, int lane, float2 (&v)[32]) const {
+    if (pi.interior) load_interior(p, pi, lane, v);
+    else if (pi.frame >= 0) load_edge(p, pi, lane, v);
+  }
+};
+
+// The same for a packed variable-length batch: clips of their own lengths, pairs numbered clip by clip, each clip's pairs
+// (2j, 2j + 1) formed from its own frames exactly as a launch over that clip alone forms them.  The clip of a pair comes
+// from the pair-base table: it only moves forward (by gridDim.x * kWarps pairs per call), so one 32-wide probe of the
+// table past the current clip finds it, with a binary search only when the probe falls short (tiny clips) and for the
+// warp's first pair.  The pair's geometry is the one-clip geometry with the clip's own length and frame count (masked loads
+// where the frames reach past either end of the clip: the neighbours' samples read as zeros); PairInfo.clip is 0 and
+// PairInfo.frame the global output row, so that the store phase needs no change.
+struct VarlenLocator {
+  int clip = -1;
+  const float* src = nullptr;  // the located clip's first sample
+  int len = 0;                 // its length
+  __device__ __forceinline__ PairInfo locate(const LogmelParams& p, unsigned iter, unsigned n_iters, unsigned total_pairs,
+                                             unsigned, int warp) {
+    const unsigned pair = iter < n_iters ? iter * kWarps + warp : total_pairs;
+    PairInfo pi;
+    if (pair >= total_pairs) {
+      pi.clip = 0;
+      pi.frame = -1;
+      pi.interior = false;
+      return pi;
+    }
+    const int* pb = p.vl_pair_base;
+    int c = clip < 0 ? 0 : clip;  // pb[c] <= pair
+    const int i = c + 1 + (int)(threadIdx.x & 31);
+    const unsigned m = __ballot_sync(kFullMask, i >= p.vl_clips || (unsigned)__ldg(pb + i) > pair);  // (pb[n_clips] = total)
+    if (m != 0) {
+      c += __ffs(m) - 1;
+    } else {  // pb[c + 32] <= pair < pb[n_clips]
+      int lo = c + 32, hi = p.vl_clips;
+      while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if ((unsigned)__ldg(pb + mid) <= pair) lo = mid;
+        else hi = mid;
+      }
+      c = lo;
+    }
+    clip = c;
+    LogmelParams q = p;
+    q.n_samples = len = __ldg(p.vl_length + c);
+    const int row0 = __ldg(p.vl_row_base + c);
+    q.n_frames = __ldg(p.vl_row_base + c + 1) - row0;
+    src = p.audio + __ldg(p.vl_sample_off + c);
+    pi = pair_geometry(q, 0, (int)(pair - (unsigned)__ldg(pb + c)));
+    pi.frame += row0;
+    return pi;
+  }
+  __device__ __forceinline__ void load(const LogmelParams& p, const PairInfo& pi, int lane, float2 (&v)[32]) const {
+    LogmelParams q = p;
+    q.audio = src;
+    q.n_samples = len;
+    if (pi.interior) {
+      load_interior(q, pi, lane, v);
+    } else if (pi.frame >= 0) {
+      // a clip shorter than its window leaves whole pairs past its end: they read nothing but the zeros the masked loads
+      // would give
+      const bool a_off = pi.fa_lo >= pi.hi_a || pi.fa_lo + kFrameLen <= pi.lo_a;
+      const bool b_off = pi.hi_b <= pi.lo_b || pi.fb_lo >= pi.hi_b || pi.fb_lo + kFrameLen <= pi.lo_b;
+      if (a_off && b_off) {
+#pragma unroll
+        for (int n1 = 0; n1 < 32; ++n1) v[n1] = make_float2(0.0f, 0.0f);
+      } else {
+        load_edge(q, pi, lane, v);
+      }
+    }
+  }
 };
 
 // the same for a warp that expects to wait long (the consumers of the warp-specialised kernel wait for the producers most
@@ -679,7 +761,9 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
 constexpr int kWsProducers = kWarps;
 constexpr int ws_launch_regs(int consumers) { return (65536 / ((kWsProducers + consumers) * 32)) & ~7; }
 
-template <int kWsConsumers, int kWsProducerRegs, int kWsConsumerRegs>
+// kVarlen: the packed variable-length batch (VarlenLocator); a separate instantiation, so that the batch kernel every other
+// caller runs stays exactly as it was
+template <int kWsConsumers, int kWsProducerRegs, int kWsConsumerRegs, bool kVarlen = false>
 __global__ void __launch_bounds__((kWsProducers + kWsConsumers) * 32, 1)
 logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
   constexpr int kWsThreads = (kWsProducers + kWsConsumers) * 32;
@@ -709,7 +793,7 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
   pdl_prologue_done(p);
 
   const unsigned ppc = (unsigned)(p.n_frames + 1) >> 1;
-  const unsigned total_pairs = (unsigned)p.n_clips * ppc;
+  const unsigned total_pairs = kVarlen ? p.vl_pairs : (unsigned)p.n_clips * ppc;
   const unsigned n_iters = (total_pairs + kWarps - 1) / kWarps;
   const unsigned first = blockIdx.x, stride = gridDim.x;
   const unsigned n_local = first < n_iters ? (n_iters - first + stride - 1) / stride : 0;
@@ -717,11 +801,10 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
   if (warp < kWsProducers) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kWsProducerRegs));
     float* xb = s_scratch + warp * kScratch;
-    PairLocator loc;
+    std::conditional_t<kVarlen, VarlenLocator, PairLocator> loc;
     float2 v[32];
     PairInfo nxt = loc.locate(p, first, n_iters, total_pairs, ppc, warp);
-    if (nxt.interior) load_interior(p, nxt, lane, v);
-    else if (nxt.frame >= 0) load_edge(p, nxt, lane, v);
+    loc.load(p, nxt, lane, v);
     for (unsigned k = 0; k < n_local; ++k) {
       const PairInfo cur = nxt;
       if (cur.frame >= 0) fft_first_half(v, s_hann, s_tw, lane);
@@ -733,8 +816,7 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
       if (lane == 0) bar_arrive(spec_ready);
       // audio of the next iteration (an L2 prefetch of these lines one iteration ahead changed nothing: 146.7 vs 146.3 us)
       nxt = loc.locate(p, k + 1 < n_local ? first + (k + 1) * stride : n_iters, n_iters, total_pairs, ppc, warp);
-      if (nxt.interior) load_interior(p, nxt, lane, v);
-      else if (nxt.frame >= 0) load_edge(p, nxt, lane, v);
+      loc.load(p, nxt, lane, v);
     }
   } else {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kWsConsumerRegs));
@@ -1086,6 +1168,9 @@ extern "C" int koe_frontend_create_ex(const koe_frontend_config* cfg, koe_fronte
     e = cudaFuncSetAttribute(logmel_power_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelSmem);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(logmel_power_ws_kernel<8, 96, 48>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelWsSmem);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(logmel_power_ws_kernel<8, 96, 48, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)kLogmelWsSmem);
   cudaDeviceProp prop;
   if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, device);
   if (e == cudaSuccess) {
@@ -1242,6 +1327,54 @@ int koe::launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* a, void*
     le = launch_after_primary_starts(logmel_power_kernel<true>, dim3(grid), dim3(kThreads), kLogmelSmem, st, tab, p);
   else
     le = launch_after_primary_starts(logmel_power_kernel<false>, dim3(grid), dim3(kThreads), kLogmelSmem, st, tab, p);
+  count_launch();
+  KOE_CUDA(le);
+  return KOE_OK;
+}
+
+int koe::launch_logmel_varlen(const koe_frontend_t* fe, const koe_logmel_args* a, const long long* sample_off,
+                              const int* length, const int* pair_base, const int* row_base, int n_clips, long long total_pairs,
+                              void* stream, bool follows_frontend_launch) {
+  KOE_REQUIRE(fe != nullptr && a != nullptr, "koe_logmel_power (varlen): NULL argument");
+  if (n_clips == 0 || total_pairs == 0) return KOE_OK;
+  if (!fe->default_bank)
+    return fail(KOE_E_UNSUPPORTED, "packed variable-length batches are implemented for the default filterbank only");
+  KOE_REQUIRE(a->audio != nullptr && a->power != nullptr && a->frame_max != nullptr && sample_off && length && pair_base &&
+                  row_base,
+              "koe_logmel_power (varlen): NULL buffer");
+  KOE_REQUIRE(a->hop > 0 && a->frame_offset >= 0 && a->frame_step >= 1, "koe_logmel_power (varlen): bad geometry");
+  KOE_REQUIRE(total_pairs < (1ll << 31) - kWarps, "koe_logmel_power (varlen): more than 2^31 frame pairs in one call");
+  FrontendTables tab;
+  tab.hann = fe->d_hann;
+  tab.tw = fe->d_tw;
+  tab.binw = fe->d_binw;
+  tab.groups = reinterpret_cast<const int4*>(fe->d_tables);
+  tab.runs = fe->d_tables + 4 * kMaxGroups;
+  tab.n_bins = fe->n_bins;
+  tab.n_groups = fe->n_groups;
+  tab.log_mode = fe->log_mode;
+  tab.log_eps = fe->log_eps;
+  LogmelParams p = {};
+  p.audio = a->audio;
+  p.hop = a->hop;
+  p.lo_rel = a->lo_rel_hops;
+  p.hi_rel = a->hi_rel_hops;
+  p.frame_offset = a->frame_offset;
+  p.frame_step = a->frame_step;
+  p.power = a->power;
+  p.frame_max = a->frame_max;
+  p.store_order = g_k1_store_order;
+  p.wait_at_end = follows_frontend_launch ? 1 : 0;
+  p.vl_sample_off = sample_off;
+  p.vl_length = length;
+  p.vl_pair_base = pair_base;
+  p.vl_row_base = row_base;
+  p.vl_clips = n_clips;
+  p.vl_pairs = (unsigned)total_pairs;
+  const long long n_blocks = (total_pairs + kWarps - 1) / kWarps;
+  const int grid = (int)std::min(n_blocks, (long long)fe->num_sms * fe->occupancy);
+  const cudaError_t le = launch_after_primary_starts(logmel_power_ws_kernel<8, 96, 48, true>, dim3(grid),
+                                                     dim3((kWsProducers + 8) * 32), kLogmelWsSmem, (cudaStream_t)stream, tab, p);
   count_launch();
   KOE_CUDA(le);
   return KOE_OK;

@@ -9,6 +9,7 @@
 // mel rows with their per-frame maxima, one "window ends here" row (L), the smoothing state.  SURVEY.md section 8
 // note E: frame n is centred on sample n * hop; R[n] is the same frame with everything before its centre zeroed; L[n + 1]
 // is centred on (n + 1) * hop with everything from there on zeroed.
+#include <algorithm>
 #include <map>
 #include <mutex>
 #include <utility>
@@ -241,5 +242,176 @@ extern "C" int koe_forward_windows(const koe_forward_args* a, void* stream) {
   if (early_flag != nullptr && !early_applied) KOE_CUDA(cudaMemsetAsync(early_flag, 0, 2 * sizeof(unsigned), (cudaStream_t)stream));
   if (a->smooth && a->n_out > 1)
     if (int rc = koe_ema_scan(a->out, a->n_clips, a->n_out, a->alpha, nullptr, 0, stream)) return rc;
+  return KOE_OK;
+}
+
+// ---- packed variable-length batch (see koe_forward_varlen in the header) -------------------------------------------------
+// Per-clip tables, int32 words (the int64 sample offsets first, so that they are 8-byte aligned):
+//   sample_off [B] int64 | length [B] | frame_base [B + 1] | window_base [B + 1] | pair_base [B + 1] | edge_pair_base [B + 1]
+//   | plain_only [B]
+// pair_base counts the frame pairs of the plain launch (ceil(n_frames_c / 2) per clip), edge_pair_base those of each
+// edge-variant launch (ceil(n_out_c / 2), none for a clip that reads its window from the plain rows).
+// Workspace (16-byte aligned regions): power[0] [F][80] | power[1 .. 2 n_edge] [N][80] each | frame_max[0] [F] |
+// frame_max[1 .. 2 n_edge] [N] each | tables.
+namespace {
+constexpr int kVarlenTableWords = 8;  // table words per clip (+ 4)
+
+struct VarlenPlan {
+  int n_edge = 0;            // edge variants per window side (0: no clip uses them)
+  int max_out = 0;           // most frames of one clip
+  long long windows = 0, frames = 0, pairs = 0, edge_pairs = 0;
+  size_t off_power[1 + 2 * KOE_MAX_EDGE] = {}, off_fmax[1 + 2 * KOE_MAX_EDGE] = {}, off_tables = 0, bytes = 0;
+};
+
+size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// Validates the lengths and geometry of `a`, sums up the per-clip geometry (the rules of SequentialDualStreamModel) and lays
+// out the workspace; with tables != NULL also writes the per-clip tables.
+int plan_varlen(const koe_forward_varlen_args* a, VarlenPlan* pl, int32_t* tables) {
+  KOE_REQUIRE(a != nullptr && pl != nullptr, "koe_forward_varlen: NULL argument");
+  KOE_REQUIRE(a->n_clips >= 0 && (a->n_clips == 0 || a->lengths_host != nullptr), "koe_forward_varlen: bad n_clips / lengths");
+  KOE_REQUIRE(a->n_clips < (1 << 26), "koe_forward_varlen: %d clips (at most 2^26)", a->n_clips);
+  KOE_REQUIRE(a->hop > 0 && a->window_frames > 0 && a->stride_frames >= 1 && a->half_fft > 0,
+              "koe_forward_varlen: bad geometry");
+  const int B = a->n_clips, hop = a->hop, W = a->window_frames, stride = a->stride_frames;
+  const int n_edge = (a->half_fft + hop - 1) / hop;
+  KOE_REQUIRE(n_edge <= KOE_MAX_EDGE && W + 1 > 2 * n_edge,
+              "koe_forward_varlen: hop %d needs %d edge frames per window side (max %d)", hop, n_edge, KOE_MAX_EDGE);
+  int64_t* sample_off = nullptr;
+  int32_t *length = nullptr, *frame_base = nullptr, *window_base = nullptr, *pair_base = nullptr, *edge_pair_base = nullptr,
+          *plain_only = nullptr;
+  if (tables != nullptr) {
+    sample_off = reinterpret_cast<int64_t*>(tables);
+    length = tables + 2 * (size_t)B;
+    frame_base = length + B;
+    window_base = frame_base + B + 1;
+    pair_base = window_base + B + 1;
+    edge_pair_base = pair_base + B + 1;
+    plain_only = edge_pair_base + B + 1;
+  }
+  *pl = VarlenPlan();
+  long long samples = 0;
+  bool any_edge = false;
+  for (int c = 0; c <= B; ++c) {
+    if (tables != nullptr) {
+      frame_base[c] = (int32_t)pl->frames;
+      window_base[c] = (int32_t)pl->windows;
+      pair_base[c] = (int32_t)pl->pairs;
+      edge_pair_base[c] = (int32_t)pl->edge_pairs;
+    }
+    if (c == B) break;
+    const int64_t L = a->lengths_host[c];
+    KOE_REQUIRE(L >= 0 && L < (1ll << 30), "koe_forward_varlen: length %lld of clip %d outside [0, 2^30)", (long long)L, c);
+    // num_output_frames: max(1, floor((L // hop - W) / stride) + 1) -- a negative numerator gives 1 either way
+    const long long rel = L / hop - W;
+    const long long n_out = rel < 0 ? 1 : rel / stride + 1;
+    const long long n_frames = (n_out - 1) * stride + W + 1;
+    const bool plain = n_out == 1 && L <= (long long)W * hop;  // one window spanning the whole clip: no interior edges
+    any_edge = any_edge || !plain;
+    if (tables != nullptr) {
+      sample_off[c] = samples;
+      length[c] = (int32_t)L;
+      plain_only[c] = plain ? 1 : 0;
+    }
+    samples += L;
+    pl->windows += n_out;
+    pl->frames += n_frames;
+    pl->pairs += (n_frames + 1) / 2;
+    pl->edge_pairs += plain ? 0 : (n_out + 1) / 2;
+    pl->max_out = (int)std::max<long long>(pl->max_out, n_out);
+    KOE_REQUIRE(pl->frames < (1ll << 31) - 32 && pl->windows < (1ll << 31), "koe_forward_varlen: more than 2^31 frames or windows");
+  }
+  pl->n_edge = any_edge ? n_edge : 0;
+  size_t off = 0;
+  pl->off_power[0] = off, off += align16((size_t)pl->frames * KOE_N_MELS * sizeof(float));
+  for (int j = 1; j <= 2 * pl->n_edge; ++j) pl->off_power[j] = off, off += align16((size_t)pl->windows * KOE_N_MELS * sizeof(float));
+  pl->off_fmax[0] = off, off += align16((size_t)pl->frames * sizeof(float));
+  for (int j = 1; j <= 2 * pl->n_edge; ++j) pl->off_fmax[j] = off, off += align16((size_t)pl->windows * sizeof(float));
+  pl->off_tables = off, off += align16(((size_t)kVarlenTableWords * B + 4) * sizeof(int32_t));
+  pl->bytes = off;
+  return KOE_OK;
+}
+}  // namespace
+
+extern "C" int koe_forward_varlen_size(const koe_forward_varlen_args* a, int64_t* n_windows, int64_t* n_frames,
+                                       int64_t* workspace_bytes) {
+  KOE_REQUIRE(n_windows != nullptr && n_frames != nullptr && workspace_bytes != nullptr, "koe_forward_varlen_size: NULL argument");
+  VarlenPlan pl;
+  if (int rc = plan_varlen(a, &pl, nullptr)) return rc;
+  *n_windows = pl.windows, *n_frames = pl.frames, *workspace_bytes = (int64_t)pl.bytes;
+  return KOE_OK;
+}
+
+extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream) {
+  VarlenPlan pl;
+  if (int rc = plan_varlen(a, &pl, nullptr)) return rc;
+  if (a->n_clips == 0) return KOE_OK;
+  KOE_REQUIRE(a->frontend != nullptr && a->weights != nullptr, "koe_forward_varlen: NULL frontend / weights");
+  KOE_REQUIRE(a->weights->k_mel == a->window_frames + 3, "koe_forward_varlen: weights for k_mel %d, window_frames %d",
+              a->weights->k_mel, a->window_frames);
+  KOE_REQUIRE(a->audio && a->egemaps && a->workspace && a->out, "koe_forward_varlen: NULL buffer");
+  KOE_REQUIRE((reinterpret_cast<uintptr_t>(a->workspace) & 15) == 0, "koe_forward_varlen: workspace must be 16-byte aligned");
+  KOE_REQUIRE(a->workspace_bytes >= (int64_t)pl.bytes, "koe_forward_varlen: workspace of %lld bytes, %lld needed",
+              (long long)a->workspace_bytes, (long long)pl.bytes);
+  KOE_REQUIRE(!a->smooth || (a->alpha >= 0.0f && a->alpha <= 1.0f), "koe_forward_varlen: alpha must be in [0, 1]");
+  KOE_REQUIRE(a->precision == 0 || a->precision == 2, "koe_forward_varlen: precision must be 0 or 2");
+  if (!koe_frontend_uses_unrolled_bank(a->frontend))
+    return fail(KOE_E_UNSUPPORTED, "koe_forward_varlen: implemented for the default filterbank only");
+  if (int rc = check_capture(stream, "koe_forward_varlen")) return rc;
+  const int B = a->n_clips;
+  char* ws = static_cast<char*>(a->workspace);
+  float* power[1 + 2 * KOE_MAX_EDGE] = {};
+  float* fmax[1 + 2 * KOE_MAX_EDGE] = {};
+  for (int j = 0; j <= 2 * pl.n_edge; ++j)
+    power[j] = reinterpret_cast<float*>(ws + pl.off_power[j]), fmax[j] = reinterpret_cast<float*>(ws + pl.off_fmax[j]);
+  int32_t* dev_tables = reinterpret_cast<int32_t*>(ws + pl.off_tables);
+  const size_t words = (size_t)kVarlenTableWords * B + 4;
+  TableStaging* stage = nullptr;
+  if (int rc = acquire_table_staging(stream, words, &stage)) return rc;
+  if (int rc = plan_varlen(a, &pl, stage->host)) return rc;
+  if (int rc = upload_tables(stage, dev_tables, words, (cudaStream_t)stream)) return rc;
+  const long long* sample_off = reinterpret_cast<const long long*>(dev_tables);
+  const int* length = dev_tables + 2 * (size_t)B;
+  const int* frame_base = length + B;
+  const int* window_base = frame_base + B + 1;
+  const int* pair_base = window_base + B + 1;
+  const int* edge_pair_base = pair_base + B + 1;
+  const int* plain_only = edge_pair_base + B + 1;
+  const int T = a->window_frames + 1;
+
+  koe_logmel_args f = {};
+  f.audio = a->audio;
+  f.hop = a->hop;
+  f.frame_offset = 0, f.frame_step = 1;
+  f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = KOE_NO_EDGE;
+  f.power = power[0], f.frame_max = fmax[0];
+  // every clip's global frames, then the frames within n_fft/2 of a window edge once per window of the clips that use them
+  if (int rc = launch_logmel_varlen(a->frontend, &f, sample_off, length, pair_base, frame_base, B, pl.pairs, stream, false))
+    return rc;
+  for (int m = 0; m < pl.n_edge; ++m) {
+    f.frame_step = a->stride_frames;
+    f.frame_offset = m, f.lo_rel_hops = -m, f.hi_rel_hops = KOE_NO_EDGE;
+    f.power = power[1 + 2 * m], f.frame_max = fmax[1 + 2 * m];
+    if (int rc = launch_logmel_varlen(a->frontend, &f, sample_off, length, edge_pair_base, window_base, B, pl.edge_pairs,
+                                      stream, true))
+      return rc;
+    f.frame_offset = T - 1 - m, f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = m;
+    f.power = power[2 + 2 * m], f.frame_max = fmax[2 + 2 * m];
+    if (int rc = launch_logmel_varlen(a->frontend, &f, sample_off, length, edge_pair_base, window_base, B, pl.edge_pairs,
+                                      stream, true))
+      return rc;
+  }
+  // as in koe_forward_windows: the emotion kernel writes the expression entries of each clip's rows, the core the rest
+  if (int rc = launch_emotion_stream(a->weights, a->egemaps, B, nullptr, a->out, a->sigmoid_out, 1, stream,
+                                     /*after_frontend=*/true, window_base))
+    return rc;
+  const float* cpower[1 + 2 * KOE_MAX_EDGE] = {power[0], power[1], power[2], power[3], power[4]};
+  const float* cfmax[1 + 2 * KOE_MAX_EDGE] = {fmax[0], fmax[1], fmax[2], fmax[3], fmax[4]};
+  if (int rc = launch_dual_stream_varlen(a->weights, cpower, cfmax, pl.n_edge, (int)pl.windows, (int)pl.frames,
+                                         a->stride_frames, T, B, window_base, frame_base, plain_only, a->out, a->sigmoid_out,
+                                         a->attn_out, a->precision, stream))
+    return rc;
+  if (a->smooth && pl.max_out > 1)
+    if (int rc = launch_ema_scan_varlen(a->out, B, window_base, a->alpha, stream)) return rc;
   return KOE_OK;
 }

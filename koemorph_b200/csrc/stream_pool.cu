@@ -12,9 +12,7 @@
 // Stream n's frames are numbered from its own first hop: the newest complete frame after hop n is g = n - lag (lag =
 // n_edge - 1) in ring row g mod W, and the window that ends after hop n starts at ring row (n + 1 - W) mod W -- the
 // arithmetic of koe_stream_push, per stream.
-#include <map>
-#include <mutex>
-#include <utility>
+#include <algorithm>
 #include <vector>
 
 #include "core_params.cuh"
@@ -101,52 +99,6 @@ __global__ void __launch_bounds__(256) pool_expr_scatter_kernel(const float* __r
 }
 
 namespace {
-// Pinned staging of the per-call tables, per (device, stream): a ring of kDepth buffers, each guarded by an event
-// recorded after the copy that reads it, so the host may run kDepth calls ahead of the device before it waits.
-struct PoolStaging {
-  static constexpr int kDepth = 4;
-  struct Buf {
-    int32_t* host = nullptr;
-    size_t ints = 0;
-    cudaEvent_t copied = nullptr;
-  };
-  struct Ring {
-    Buf buf[kDepth];
-    int next = 0;
-  };
-  std::mutex mu;
-  std::map<std::pair<int, void*>, Ring> rings;
-
-  // a buffer of >= ints entries that no queued copy reads any more
-  int acquire(void* stream, size_t ints, Buf** out) {
-    int dev = 0;
-    KOE_CUDA(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(mu);
-    Ring& r = rings[{dev, stream}];
-    Buf& b = r.buf[r.next];
-    r.next = (r.next + 1) % kDepth;
-    if (b.copied == nullptr) KOE_CUDA(cudaEventCreateWithFlags(&b.copied, cudaEventDisableTiming));
-    else KOE_CUDA(cudaEventSynchronize(b.copied));
-    if (b.ints < ints) {
-      if (b.host != nullptr) KOE_CUDA(cudaFreeHost(b.host));
-      b.host = nullptr, b.ints = 0;
-      const size_t want = std::max<size_t>(ints, 1024);
-      KOE_CUDA(cudaHostAlloc(&b.host, want * sizeof(int32_t), cudaHostAllocDefault));
-      b.ints = want;
-    }
-    *out = &b;
-    return KOE_OK;
-  }
-};
-PoolStaging g_pool_staging;
-
-// one copy of host[0, ints) to the device tables, then the event that frees the staging buffer
-int upload_tables(PoolStaging::Buf* b, int32_t* dev_tables, size_t ints, cudaStream_t stream) {
-  KOE_CUDA(cudaMemcpyAsync(dev_tables, b->host, ints * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
-  KOE_CUDA(cudaEventRecord(b->copied, stream));
-  return KOE_OK;
-}
-
 int num_sms() {
   static int sms[64] = {0};
   int dev = 0;
@@ -173,13 +125,6 @@ int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* 
   return KOE_OK;
 }
 
-int check_capture(void* stream, const char* what) {
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  KOE_CUDA(cudaStreamIsCapturing((cudaStream_t)stream, &cap));
-  if (cap != cudaStreamCaptureStatusNone)
-    return fail(KOE_E_UNSUPPORTED, "%s cannot be captured into a CUDA graph: its tables change every call", what);
-  return KOE_OK;
-}
 }  // namespace
 
 }  // namespace koe
@@ -245,8 +190,8 @@ extern "C" int koe_stream_pool_set_egemaps(koe_stream_pool_t* pool, const koe_st
                   a->tables != nullptr,
               "koe_stream_pool_set_egemaps: NULL buffer");
   if (int rc = check_capture(stream, "koe_stream_pool_set_egemaps")) return rc;
-  PoolStaging::Buf* b = nullptr;
-  if (int rc = g_pool_staging.acquire(stream, (size_t)n, &b)) return rc;
+  TableStaging* b = nullptr;
+  if (int rc = acquire_table_staging(stream, (size_t)n, &b)) return rc;
   std::copy(slots_host, slots_host + n, b->host);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = upload_tables(b, a->tables, (size_t)n, st)) return rc;
@@ -279,8 +224,8 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
   cudaStream_t st = (cudaStream_t)stream;
 
   // ---- the per-call tables: [push slot | push ring row | push first hop][emit slot | emit ring base | emit has state]
-  PoolStaging::Buf* b = nullptr;
-  if (int rc = g_pool_staging.acquire(stream, 6 * (size_t)n, &b)) return rc;
+  TableStaging* b = nullptr;
+  if (int rc = acquire_table_staging(stream, 6 * (size_t)n, &b)) return rc;
   int32_t* h = b->host;
   int k = 0;
   for (int i = 0; i < n; ++i) {

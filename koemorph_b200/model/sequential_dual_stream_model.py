@@ -9,9 +9,11 @@ the window grid; the dB reference of a window is the max over ITS frames, taken 
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 from typing import Dict, Optional
 
+import numpy as np
 import torch
 
 from .. import _lib
@@ -70,6 +72,92 @@ class SequentialDualStreamModel(SimplifiedDualStreamModel):
         res["emotion_backend"] = "egemaps_input"
         res["emotion_processing_time"] = 0.0
         return res
+
+    @torch.no_grad()
+    def forward_varlen(self, audio: torch.Tensor, lengths, egemaps: Optional[torch.Tensor] = None,
+                       return_attention: bool = False, out: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """A packed batch of clips of different lengths as one native forward (koe_forward_varlen).
+
+        ``audio``: 1-D float32 CUDA tensor with the clips back to back, ``audio.numel() == sum(lengths)``; ``lengths``:
+        host sequence or CPU integer tensor, one entry >= 0 per clip; ``egemaps``: (B, 264) or (B, 3, 88).  Clip c's
+        ``num_output_frames(lengths[c])`` frames are rows ``frame_offsets[c]:frame_offsets[c + 1]`` of ``blendshapes``
+        (N, 52) (and of the attention / sigmoid outputs), each equal to ``forward`` on that clip alone, smoothing
+        included.  ``out``: a preallocated contiguous (N, 52) float32 tensor.  Afterwards ``prev_blendshapes`` holds every
+        clip's last frame, (B, 52)."""
+        if not isinstance(audio, torch.Tensor) or not audio.is_cuda:
+            raise ValueError("audio must be a 1-D float32 CUDA tensor holding the clips back to back")
+        audio = _lib.require_cuda(audio, "audio")
+        if audio.dim() != 1:
+            raise ValueError(f"audio must be 1-D (the clips back to back), got {tuple(audio.shape)}")
+        lens = self._check_lengths(lengths, audio.numel())
+        B = lens.numel()
+        dev = audio.device
+        eg = self._check_egemaps(egemaps, B, dev)
+        hop, W, stride = self.hop_length, self.window_frames, self.stride_frames
+        n_out = torch.clamp((lens // hop - W) // stride + 1, min=1)     # num_output_frames, per clip
+        offsets = torch.zeros(B + 1, dtype=torch.int64)
+        torch.cumsum(n_out, 0, out=offsets[1:])
+        N = int(offsets[-1])
+        if out is None:
+            out = torch.empty(N, 52, dtype=torch.float32, device=dev)
+        elif out.shape != (N, 52) or out.dtype != torch.float32 or not out.is_contiguous() or out.device != dev:
+            raise ValueError(f"out must be a contiguous float32 ({N}, 52) tensor on {dev}")
+        sig = torch.empty(N, 52, dtype=torch.float32, device=dev) if return_attention else None
+        attn = torch.empty(N, 28, 80, dtype=torch.float32, device=dev) if return_attention else None
+        if B > 0:
+            lib = _lib.load()
+            w = self.dual_stream_attention.kernel_weights(self._compression)
+            a = _lib.ForwardVarlenArgs()
+            a.frontend, a.weights = self._frontend(dev)._h, C.addressof(w.struct)
+            # (a batch of empty clips reads no sample, but the ABI wants a pointer)
+            src = audio if audio.numel() > 0 else torch.zeros(1, dtype=torch.float32, device=dev)
+            a.audio, a.lengths_host, a.n_clips = src.data_ptr(), lens.data_ptr(), B
+            a.hop, a.window_frames, a.stride_frames, a.half_fft = hop, W, stride, self.n_fft // 2
+            a.smooth = 1 if self.use_temporal_smoothing else 0
+            a.alpha = self._alpha() if self.use_temporal_smoothing else 0.0
+            a.precision = _lib.PRECISIONS[self.precision]
+            n_win, n_frames, ws_bytes = C.c_int64(), C.c_int64(), C.c_int64()
+            _lib.check(lib.koe_forward_varlen_size(C.byref(a), C.byref(n_win), C.byref(n_frames), C.byref(ws_bytes)),
+                       "koe_forward_varlen_size")
+            if n_win.value != N:
+                raise RuntimeError(f"koe_forward_varlen_size: {n_win.value} windows, the model counts {N}")
+            ws = torch.empty(ws_bytes.value, dtype=torch.uint8, device=dev)
+            a.egemaps, a.workspace, a.workspace_bytes = eg.data_ptr(), ws.data_ptr(), ws_bytes.value
+            a.out = out.data_ptr()
+            a.sigmoid_out = sig.data_ptr() if sig is not None else None
+            a.attn_out = attn.data_ptr() if attn is not None else None
+            with torch.cuda.device(dev):
+                _lib.check(lib.koe_forward_varlen(C.byref(a), _lib.stream_ptr(dev)), "koe_forward_varlen")
+        # as forward: the smoothing state is each clip's last frame
+        self.prev_blendshapes = None
+        if self.use_temporal_smoothing:
+            # (the row indices go up from pinned memory: a pageable copy would hold the host until the forward is done)
+            self.prev_blendshapes = out[(offsets[1:] - 1).pin_memory().to(dev, non_blocking=True)]
+        res = _package(out, sig, attn, return_attention)
+        res["frame_offsets"] = offsets
+        res["num_frames"] = N
+        res["fps"] = self.target_fps
+        res["emotion_backend"] = "egemaps_input"
+        res["emotion_processing_time"] = 0.0
+        return res
+
+    @staticmethod
+    def _check_lengths(lengths, n_samples: int) -> torch.Tensor:
+        """Clip lengths as a contiguous CPU int64 tensor; they must be >= 0 and add up to the packed audio."""
+        if isinstance(lengths, torch.Tensor):
+            if lengths.device.type != "cpu" or lengths.is_floating_point() or lengths.is_complex() or lengths.dtype == torch.bool:
+                raise ValueError("lengths must be a host sequence or a CPU integer tensor")
+            lens = lengths.to(torch.int64).reshape(-1).contiguous()
+        else:
+            arr = np.asarray(lengths)
+            if arr.size > 0 and arr.dtype.kind not in "iu":
+                raise ValueError(f"lengths must be integers, got {arr.dtype}")
+            lens = torch.from_numpy(arr.astype(np.int64).reshape(-1))
+        if lens.numel() > 0 and int(lens.min()) < 0:
+            raise ValueError(f"lengths must be >= 0, got {int(lens.min())}")
+        if int(lens.sum()) != n_samples:
+            raise ValueError(f"lengths add up to {int(lens.sum())} samples, audio holds {n_samples}")
+        return lens
 
     @torch.no_grad()
     def forward_single_frame(self, audio: torch.Tensor, frame_idx: int = None,
