@@ -56,6 +56,19 @@ inline cudaError_t launch_after_primary_starts(void (*kernel)(KArgs...), dim3 gr
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
+// the number of SMs of the current device, queried once per device
+inline cudaError_t sm_count(int* n) {
+  static std::atomic<int> cached[64];
+  *n = 0;
+  int dev = 0;
+  if (cudaError_t e = cudaGetDevice(&dev)) return e;
+  const bool cacheable = dev >= 0 && dev < 64;
+  if (cacheable && (*n = cached[dev].load(std::memory_order_relaxed)) > 0) return cudaSuccess;
+  if (cudaError_t e = cudaDeviceGetAttribute(n, cudaDevAttrMultiProcessorCount, dev)) return e;
+  if (cacheable) cached[dev].store(*n, std::memory_order_relaxed);
+  return cudaSuccess;
+}
+
 // frontend launch with launch-chaining knowledge of the caller (csrc/logmel.cu; used by csrc/session.cu)
 // early_clips / early_flag / early_target: see "early release of the core" in csrc/session.cu (0 / NULL: off)
 int launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* args, void* stream, bool follows_frontend_launch,

@@ -26,11 +26,11 @@ struct CoreParams {
   unsigned early_target;
   int early_items;
   long long* dbg;  // optional phase timestamps of CTA 0 (bring-up / profiling only), NULL in production
-  // stream pool (csrc/stream_pool.cu; the kPool instantiations only): window w reads the rings, edge rows and expression
-  // value of stream pool_slot[w] with ring base pool_base[w], and writes output row w
+  // stream pool (csrc/stream_pool.cu; CoreMode::Pool only): window w reads the rings, edge rows and expression value of
+  // stream pool_slot[w] with ring base pool_base[w], and writes output row w
   const int* pool_slot;
   const int* pool_base;
-  // packed variable-length batch (csrc/session.cu; the kVarlen instantiations only): n_clips counts windows (n_out = 1),
+  // packed variable-length batch (csrc/session.cu; CoreMode::Varlen only): n_clips counts windows (n_out = 1),
   // item is the global window = output row; clip c owns windows [vl_window_base[c], vl_window_base[c + 1]) and its plain
   // rows start at vl_frame_base[c]; vl_plain_only[c] != 0: the clip's window reads every frame from the plain rows
   const int* vl_window_base;
@@ -39,30 +39,20 @@ struct CoreParams {
   int vl_clips;
 };
 
-// frame k of window wi of clip b: which buffer and which row (see koe_dual_stream_windows in the header)
+// Which flavour of the core a launch runs.  Each is a separate instantiation of both kernels (the fp32 kernel has no
+// Early), so that adding one leaves the code of the others as it was.
+//   Windows  windows of clips, n_out per clip, stride_frames apart; also, by run-time fields of the same instantiation,
+//            the streaming step's per-stream rings (ring_frames > 0) and prenormalised features (mel_long != NULL)
+//   Early    Windows with one window per clip, released early by the frontend (the fused forward; early_flag)
+//   Pool     a stream-pool push: window w reads the rings of stream pool_slot[w] from ring base pool_base[w]
+//   Varlen   a packed variable-length batch: window w belongs to the clip c with vl_window_base[c] <= w < vl_window_base[c + 1]
+enum class CoreMode { Windows, Early, Pool, Varlen };
+
+// frame k of a window: which buffer (variant) holds it (see koe_dual_stream_windows in the header)
 __device__ __forceinline__ int window_variant(const CoreParams& p, int k) {
   if (k < p.n_edge) return 1 + 2 * k;
   if (k >= p.frames_per_window - p.n_edge) return 2 + 2 * (p.frames_per_window - 1 - k);
   return 0;
-}
-__device__ __forceinline__ long long window_row(const CoreParams& p, int variant, int b, int wi, int k) {
-  if (p.ring_frames > 0)  // plain and lo-edge rows are ring slots of the global frame; a hi-edge row (variants 2, 4) is per stream
-    return variant > 0 && (variant & 1) == 0 ? (long long)b
-                                             : (long long)b * p.ring_frames + (p.ring_base + k) % p.ring_frames;
-  return variant == 0 ? (long long)b * p.n_frames + (long long)wi * p.stride_frames + k
-                      : (long long)b * p.n_out + wi;
-}
-// the same in the stream pool: ring mode with the window's own stream slot and ring base
-__device__ __forceinline__ long long pool_window_row(const CoreParams& p, int variant, int slot, int base, int k) {
-  return variant > 0 && (variant & 1) == 0 ? (long long)slot : (long long)slot * p.ring_frames + (base + k) % p.ring_frames;
-}
-// kPool: (b, wi) of the callers below are the window's stream slot and ring base; kVarlen: the window's first plain row
-// and its global index (the row of every edge variant)
-template <bool kPool, bool kVarlen = false>
-__device__ __forceinline__ long long core_row(const CoreParams& p, int variant, int b, int wi, int k) {
-  if constexpr (kVarlen) return variant == 0 ? (long long)b + k : (long long)wi;
-  else if constexpr (kPool) return pool_window_row(p, variant, b, wi, k);
-  else return window_row(p, variant, b, wi, k);
 }
 
 // varlen: the clip of window `item` (window_base[c] <= item < window_base[c + 1]; every clip has a window).  Scalar binary
@@ -89,15 +79,65 @@ __device__ __forceinline__ int varlen_clip(const CoreParams& p, int item) {
   }
   return lo;
 }
-struct VarlenWindow {
-  int row;          // first plain row
-  bool plain_only;  // no edge variants: every frame from the plain rows
+
+// A window as the row addressing of mode M sees it; CoreRows<M> below is the only code that reads its fields.
+struct CoreWindow {
+  int owner;        // whose rows: the clip (Windows, Early; ring mode: the stream), the stream slot (Pool), or the
+                    // window's first plain row (Varlen)
+  int pos;          // where in them: the window within its clip (Windows, Early), the ring base (Pool), or the global
+                    // window, which is also the window's row in every edge-variant buffer (Varlen)
+  bool plain_only;  // Varlen: the clip has no edge variants, every frame comes from the plain rows
 };
-template <bool kWarp>
-__device__ __forceinline__ VarlenWindow varlen_window(const CoreParams& p, int item) {
-  const int c = varlen_clip<kWarp>(p, item);
-  return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, __ldg(p.vl_plain_only + c) != 0};
-}
+
+// The window resolver of each mode: work item `item` is output row `item` and reads the window window<kWarp>(p, item);
+// frame k of it, variant v, is row row(p, w, v, k) of p.power[v] / p.fmax[v].
+template <CoreMode M>
+struct CoreRows {
+  // kWarp: every lane of a converged warp calls with the same item (Varlen searches the clip with the whole warp)
+  template <bool kWarp>
+  static __device__ __forceinline__ CoreWindow window(const CoreParams& p, int item) {
+    if constexpr (M == CoreMode::Pool) {
+      return {p.pool_slot[item], p.pool_base[item], false};
+    } else if constexpr (M == CoreMode::Varlen) {
+      const int c = varlen_clip<kWarp>(p, item);
+      return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, item,
+              __ldg(p.vl_plain_only + c) != 0};
+    } else {
+      return {item / p.n_out, item % p.n_out, false};
+    }
+  }
+  static __device__ __forceinline__ long long row(const CoreParams& p, const CoreWindow& w, int variant, int k) {
+    if constexpr (M == CoreMode::Varlen) {
+      return variant == 0 ? (long long)w.owner + k : (long long)w.pos;
+    } else if constexpr (M == CoreMode::Pool) {
+      return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
+                                               : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
+    } else {
+      if (p.ring_frames > 0)  // plain and lo-edge rows are ring slots of the global frame; a hi-edge row (variants 2, 4) is per stream
+        return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
+                                                 : (long long)w.owner * p.ring_frames + (p.ring_base + k) % p.ring_frames;
+      return variant == 0 ? (long long)w.owner * p.n_frames + (long long)w.pos * p.stride_frames + k
+                          : (long long)w.owner * p.n_out + w.pos;
+    }
+  }
+  // ring modes (ring_frames > 0, n_out == 1): the ring slot of the window's frame 0
+  static __device__ __forceinline__ int ring_base(const CoreParams& p, const CoreWindow& w) {
+    return M == CoreMode::Pool ? w.pos : p.ring_base;
+  }
+  // ring modes: the stream whose ring and frame maxima window `item` reads (the L2 prefetch of the next window)
+  static __device__ __forceinline__ int ring_stream(const CoreParams& p, int item) {
+    return M == CoreMode::Pool ? p.pool_slot[item] : item;
+  }
+  // the clip or stream whose expression value (expr_sigmoid) output row `item` takes
+  static __device__ __forceinline__ int expr_row(const CoreParams& p, int item) {
+    return M == CoreMode::Pool ? p.pool_slot[item] : item / p.n_out;
+  }
+  // the L2 policy of a window's plain rows: `reread` where other windows read them again (the overlapping windows of a
+  // sequence or of a varlen clip), else `once`
+  static __device__ __forceinline__ uint64_t plain_rows_policy(const CoreParams& p, uint64_t reread, uint64_t once) {
+    return M == CoreMode::Varlen || p.n_out > 1 ? reread : once;
+  }
+};
 
 // emotion stream launch shared by the public entry and the fused forward (csrc/session.cu, which has it write the
 // expression entries of `out`); the core launch that leaves those entries alone (expr_sigmoid == NULL); see dual_stream.cu

@@ -108,10 +108,8 @@ constexpr size_t kCoreSmemFloats = (size_t)kABlockRows * kTok      // A block
                                    + 64;                           // reductions
 constexpr size_t kCoreSmem = kCoreSmemFloats * sizeof(float);
 
-// kPool: the stream-pool flavour (window item = stream p.pool_slot[item], ring base p.pool_base[item]); kVarlen: the packed
-// variable-length batch (window item of the clip found in p.vl_window_base).  Separate instantiations, so that the kernel
-// every other caller runs stays exactly as it was
-template <bool kPool = false, bool kVarlen = false>
+// one instantiation per CoreMode except Early; the window of a work item and the rows of its frames come from CoreRows<M>
+template <CoreMode M>
 __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreParams p) {
   extern __shared__ __align__(16) float smem[];
   float* s_a = smem;                               // [64][80]
@@ -126,10 +124,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
   const int n_items = p.n_clips * p.n_out;
 
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-    VarlenWindow vw{0, false};
-    if constexpr (kVarlen) vw = varlen_window<true>(p, item);
-    const int b = kVarlen ? vw.row : kPool ? __ldg(p.pool_slot + item) : item / p.n_out;
-    const int wi = kVarlen ? item : kPool ? __ldg(p.pool_base + item) : item % p.n_out;
+    const CoreWindow win = CoreRows<M>::template window<true>(p, item);
     const bool prenorm = p.mel_long != nullptr;
 
     // ---- P0: dB reference of this window -------------------------------------------------------
@@ -137,8 +132,8 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
     if (!prenorm) {
       float mx = -INFINITY;
       for (int k = tid; k < T; k += kCoreThreads) {
-        const int v = vw.plain_only ? 0 : window_variant(p, k);
-        mx = fmaxf(mx, p.fmax[v][core_row<kPool, kVarlen>(p, v, b, wi, k)]);
+        const int v = win.plain_only ? 0 : window_variant(p, k);
+        mx = fmaxf(mx, p.fmax[v][CoreRows<M>::row(p, win, v, k)]);
       }
       mx = warp_max(mx);
       if (tx == 0) s_red[ty] = mx;
@@ -174,13 +169,12 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
         if (prenorm) {
           if (t >= p.mel_seq)
-            v = __ldg(reinterpret_cast<const float4*>(p.mel_short + ((size_t)b * 3 + (t - p.mel_seq)) * kTok) + q);
+            v = __ldg(reinterpret_cast<const float4*>(p.mel_short + ((size_t)win.owner * 3 + (t - p.mel_seq)) * kTok) + q);
           else if (t < p.n_long)
-            v = __ldg(reinterpret_cast<const float4*>(p.mel_long + ((size_t)b * p.n_frames + t) * kTok) + q);
+            v = __ldg(reinterpret_cast<const float4*>(p.mel_long + ((size_t)win.owner * p.n_frames + t) * kTok) + q);
         } else if (k >= 0) {
-          const int var = vw.plain_only ? 0 : window_variant(p, k);
-          const float4 pw =
-              __ldg(reinterpret_cast<const float4*>(p.power[var] + core_row<kPool, kVarlen>(p, var, b, wi, k) * kTok) + q);
+          const int var = win.plain_only ? 0 : window_variant(p, k);
+          const float4 pw = __ldg(reinterpret_cast<const float4*>(p.power[var] + CoreRows<M>::row(p, win, var, k) * kTok) + q);
           v.x = normalise_db(pw.x, ref_db, true);
           v.y = normalise_db(pw.y, ref_db, true);
           v.z = normalise_db(pw.z, ref_db, true);
@@ -333,7 +327,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
       }
     }
     if (tid < KOE_N_EXPR && p.expr_sigmoid != nullptr) {  // (NULL: the fused forward's emotion kernel writes these)
-      const float y = __ldg(p.expr_sigmoid + b);
+      const float y = __ldg(p.expr_sigmoid + win.owner);
       const int idx = __ldg(W.expr_idx + tid);
       const size_t o_off = (size_t)item * KOE_N_BLENDSHAPES + idx;
       p.out[o_off] = fminf(fmaxf(__ldg(W.coef + idx) * y, 0.0f), 1.0f);
@@ -685,7 +679,7 @@ __global__ void __launch_bounds__(256) ema_scan_kernel(float* __restrict__ frame
   }
 }
 
-int launch_dual_stream_tc(const CoreParams& p, int precision, cudaStream_t stream);  // dual_stream_tc.cu
+int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t stream);  // dual_stream_tc.cu
 
 }  // namespace koe
 
@@ -794,38 +788,61 @@ extern "C" int koe_affine_rows(const float* x, int n_rows, int n_in, const float
 // (globaltimer); NULL (the default) turns the stamps off
 extern "C" void koe_debug_set_tc_timestamps(long long* device_buffer) { g_tc_debug = device_buffer; }
 
-static int launch_core(const CoreParams& p_in, int precision, cudaStream_t stream) {
+// sets the shared-memory size of the instantiation once per device, then launches it
+template <CoreMode M>
+static int launch_fp32(const CoreParams& p, cudaStream_t stream) {
+  static bool configured[64] = {false};
+  int dev = 0, sms = 0;
+  KOE_CUDA(cudaGetDevice(&dev));
+  KOE_REQUIRE(dev >= 0 && dev < 64, "device index too large");
+  if (!configured[dev]) {
+    KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoreSmem));
+    configured[dev] = true;
+  }
+  KOE_CUDA(sm_count(&sms));
+  dual_stream_fp32_kernel<M><<<std::min(p.n_clips * p.n_out, sms), kCoreThreads, kCoreSmem, stream>>>(p);
+  count_launch();
+  KOE_CUDA(cudaGetLastError());
+  return KOE_OK;
+}
+
+static int launch_core(const CoreParams& p_in, CoreMode mode, int precision, cudaStream_t stream) {
   CoreParams p = p_in;
   p.dbg = g_tc_debug;
-  if (precision == 0) {
-    static int num_sms[64] = {0};
-    int dev = 0;
-    KOE_CUDA(cudaGetDevice(&dev));
-    KOE_REQUIRE(dev >= 0 && dev < 64, "device index too large");
-    if (num_sms[dev] == 0) {
-      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)kCoreSmem));
-      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)kCoreSmem));
-      KOE_CUDA(cudaFuncSetAttribute(dual_stream_fp32_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)kCoreSmem));
-      int n = 0;
-      KOE_CUDA(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
-      num_sms[dev] = n;
-    }
-    const int grid = std::min(p.n_clips * p.n_out, num_sms[dev]);
-    if (p.pool_slot != nullptr)
-      dual_stream_fp32_kernel<true><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
-    else if (p.vl_window_base != nullptr)
-      dual_stream_fp32_kernel<false, true><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
-    else
-      dual_stream_fp32_kernel<false><<<grid, kCoreThreads, kCoreSmem, stream>>>(p);
-    count_launch();
-    KOE_CUDA(cudaGetLastError());
-    return KOE_OK;
+  if (precision == 2) return launch_dual_stream_tc(p, mode, stream);
+  if (precision != 0)
+    return fail(KOE_E_INVALID, "precision must be 0 (fp32) or 2 (bf16 operands, tcgen05), got %d", precision);
+  switch (mode) {
+    case CoreMode::Windows: return launch_fp32<CoreMode::Windows>(p, stream);
+    case CoreMode::Pool: return launch_fp32<CoreMode::Pool>(p, stream);
+    case CoreMode::Varlen: return launch_fp32<CoreMode::Varlen>(p, stream);
+    case CoreMode::Early: break;
   }
-  if (precision == 2) return launch_dual_stream_tc(p, precision, stream);
-  return fail(KOE_E_INVALID, "precision must be 0 (fp32) or 2 (bf16 operands, tcgen05), got %d", precision);
+  return fail(KOE_E_INVALID, "early release needs the tensor-core core (precision 2)");
+}
+
+// The part every core entry fills alike: the weights (validated by the caller), the 1 + 2 n_edge mel-power / frame-max
+// buffers -- each non-NULL, the power rows 16-byte aligned; power == NULL: none, the prenormalised features -- and the
+// outputs; one window per clip, frames 1 apart, unless the entry says otherwise.  `what` names the entry in error messages.
+static int core_params(const char* what, const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                       int n_edge, const float* expr_sigmoid, float* out, float* sigmoid_out, float* attn_out,
+                       CoreParams* p) {
+  *p = CoreParams{};
+  p->w = *w;
+  for (int j = 0; power != nullptr && j < 1 + 2 * n_edge; ++j) {
+    KOE_REQUIRE(power[j] != nullptr && frame_max[j] != nullptr, "%s: NULL power[%d] / frame_max[%d]", what, j, j);
+    KOE_REQUIRE((reinterpret_cast<uintptr_t>(power[j]) & 15) == 0, "%s: power[%d] must be 16-byte aligned", what, j);
+    p->power[j] = power[j], p->fmax[j] = frame_max[j];
+  }
+  p->n_edge = n_edge;
+  p->n_out = 1;
+  p->stride_frames = 1;
+  p->mel_seq = w->k_mel - 3;
+  p->expr_sigmoid = expr_sigmoid;
+  p->out = out;
+  p->sigmoid_out = sigmoid_out;
+  p->attn_out = attn_out;
+  return KOE_OK;
 }
 
 extern "C" int koe_dual_stream_windows(const koe_core_weights* w, const float* const* power,
@@ -856,36 +873,25 @@ int koe::launch_dual_stream_windows(const koe_core_weights* w, const float* cons
   KOE_REQUIRE(n_out == 0 || (long long)(n_out - 1) * stride_frames + frames_per_window <= n_frames,
               "koe_dual_stream_windows: windows run past n_frames");
   KOE_REQUIRE((long long)n_clips * n_out < (1ll << 31), "koe_dual_stream_windows: too many windows");
-  if (n_clips == 0 || n_out == 0) return KOE_OK;
-  CoreParams p{};
-  p.w = *w;
-  for (int j = 0; j < 1 + 2 * KOE_MAX_EDGE; ++j) {
-    const bool used = j < 1 + 2 * n_edge;
-    p.power[j] = used ? power[j] : nullptr;
-    p.fmax[j] = used ? frame_max[j] : nullptr;
-    KOE_REQUIRE(!used || (p.power[j] != nullptr && p.fmax[j] != nullptr), "koe_dual_stream_windows: NULL power[%d]", j);
-    KOE_REQUIRE(!used || (reinterpret_cast<uintptr_t>(p.power[j]) & 15) == 0,
-                "koe_dual_stream_windows: power[%d] must be 16-byte aligned", j);
-  }
-  p.n_edge = n_edge;
+  CoreParams p;
+  if (int rc = core_params("koe_dual_stream_windows", w, power, frame_max, n_edge, expr_sigmoid, out, sigmoid_out, attn_out,
+                           &p))
+    return rc;
   p.n_clips = n_clips;
   p.n_frames = n_frames;
   p.n_out = n_out;
   p.stride_frames = stride_frames;
   p.frames_per_window = frames_per_window;
-  p.mel_seq = w->k_mel - 3;
-  p.expr_sigmoid = expr_sigmoid;
-  p.out = out;
-  p.sigmoid_out = sigmoid_out;
-  p.attn_out = attn_out;
+  CoreMode mode = CoreMode::Windows;
   if (early_flag != nullptr && early_target > 0 && early_items > 0 && precision == 2 && n_out == 1 && n_edge == 0 &&
       attn_out == nullptr && (w->k_mel == 259 || w->k_mel == 515)) {
+    mode = CoreMode::Early;
     p.early_flag = early_flag;
     p.early_target = early_target;
     p.early_items = early_items;
   }
-  const int rc = launch_core(p, precision, (cudaStream_t)stream);
-  if (rc == KOE_OK && early_applied != nullptr) *early_applied = p.early_flag != nullptr;
+  const int rc = launch_core(p, mode, precision, (cudaStream_t)stream);
+  if (rc == KOE_OK && early_applied != nullptr) *early_applied = mode == CoreMode::Early;
   return rc;
 }
 
@@ -900,27 +906,15 @@ extern "C" int koe_dual_stream_ring_edges(const koe_core_weights* w, const float
   KOE_REQUIRE(n_streams >= 0 && ring_base >= 0 && frames_per_window > 2 * n_edge && ring_frames >= frames_per_window - 1,
               "koe_dual_stream_ring: bad sizes (the ring must hold every plain frame of a window)");
   if (n_streams == 0) return KOE_OK;
-  CoreParams p{};
-  p.w = *w;
-  for (int j = 0; j < 1 + 2 * n_edge; ++j) {
-    KOE_REQUIRE(power[j] != nullptr && frame_max[j] != nullptr, "koe_dual_stream_ring: NULL buffer %d", j);
-    KOE_REQUIRE((reinterpret_cast<uintptr_t>(power[j]) & 15) == 0, "koe_dual_stream_ring: mel rows must be 16-byte aligned");
-    p.power[j] = power[j], p.fmax[j] = frame_max[j];
-  }
-  p.n_edge = n_edge;
+  CoreParams p;
+  if (int rc = core_params("koe_dual_stream_ring", w, power, frame_max, n_edge, expr_sigmoid, out, sigmoid_out, attn_out, &p))
+    return rc;
   p.n_clips = n_streams;
   p.n_frames = ring_frames;
-  p.n_out = 1;
-  p.stride_frames = 1;
   p.frames_per_window = frames_per_window;
-  p.mel_seq = w->k_mel - 3;
-  p.expr_sigmoid = expr_sigmoid;
-  p.out = out;
-  p.sigmoid_out = sigmoid_out;
-  p.attn_out = attn_out;
   p.ring_frames = ring_frames;
   p.ring_base = ring_base % ring_frames;
-  return launch_core(p, precision, (cudaStream_t)stream);
+  return launch_core(p, CoreMode::Windows, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_dual_stream_pool(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
@@ -933,26 +927,15 @@ int koe::launch_dual_stream_pool(const koe_core_weights* w, const float* const* 
   KOE_REQUIRE(n_edge >= 1 && n_edge <= KOE_MAX_EDGE && n_windows >= 0 && ring_frames == w->k_mel - 3,
               "stream pool core: bad sizes");
   if (n_windows == 0) return KOE_OK;
-  CoreParams p{};
-  p.w = *w;
-  for (int j = 0; j < 1 + 2 * n_edge; ++j) {
-    KOE_REQUIRE(power[j] != nullptr && frame_max[j] != nullptr, "stream pool core: NULL buffer %d", j);
-    KOE_REQUIRE((reinterpret_cast<uintptr_t>(power[j]) & 15) == 0, "stream pool core: mel rows must be 16-byte aligned");
-    p.power[j] = power[j], p.fmax[j] = frame_max[j];
-  }
-  p.n_edge = n_edge;
+  CoreParams p;
+  if (int rc = core_params("stream pool core", w, power, frame_max, n_edge, expr_sigmoid, out, nullptr, nullptr, &p)) return rc;
   p.n_clips = n_windows;
   p.n_frames = ring_frames;
-  p.n_out = 1;
-  p.stride_frames = 1;
   p.frames_per_window = ring_frames + 1;
-  p.mel_seq = w->k_mel - 3;
-  p.expr_sigmoid = expr_sigmoid;
-  p.out = out;
   p.ring_frames = ring_frames;
   p.pool_slot = slot;
   p.pool_base = base;
-  return launch_core(p, precision, (cudaStream_t)stream);
+  return launch_core(p, CoreMode::Pool, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
@@ -967,28 +950,17 @@ int koe::launch_dual_stream_varlen(const koe_core_weights* w, const float* const
                   frames_per_window > 2 * n_edge && frames_per_window == w->k_mel - 2,
               "varlen core: bad sizes");
   if (n_windows == 0) return KOE_OK;
-  CoreParams p{};
-  p.w = *w;
-  for (int j = 0; j < 1 + 2 * n_edge; ++j) {
-    KOE_REQUIRE(power[j] != nullptr && frame_max[j] != nullptr, "varlen core: NULL buffer %d", j);
-    KOE_REQUIRE((reinterpret_cast<uintptr_t>(power[j]) & 15) == 0, "varlen core: mel rows must be 16-byte aligned");
-    p.power[j] = power[j], p.fmax[j] = frame_max[j];
-  }
-  p.n_edge = n_edge;
+  CoreParams p;
+  if (int rc = core_params("varlen core", w, power, frame_max, n_edge, nullptr, out, sigmoid_out, attn_out, &p)) return rc;
   p.n_clips = n_windows;
   p.n_frames = n_frames;
-  p.n_out = 1;
   p.stride_frames = stride_frames;
   p.frames_per_window = frames_per_window;
-  p.mel_seq = w->k_mel - 3;
-  p.out = out;
-  p.sigmoid_out = sigmoid_out;
-  p.attn_out = attn_out;
   p.vl_window_base = window_base;
   p.vl_frame_base = frame_base;
   p.vl_plain_only = plain_only;
   p.vl_clips = n_clips;
-  return launch_core(p, precision, (cudaStream_t)stream);
+  return launch_core(p, CoreMode::Varlen, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_ema_scan_varlen(float* frames, int n_clips, const int* row_base, float alpha, void* stream) {
@@ -1022,24 +994,17 @@ extern "C" int koe_dual_stream_features(const koe_core_weights* w, const float* 
               "koe_dual_stream_features: NULL argument");
   KOE_REQUIRE(((reinterpret_cast<uintptr_t>(mel_long) | reinterpret_cast<uintptr_t>(mel_short)) & 15) == 0,
               "koe_dual_stream_features: features must be 16-byte aligned");
-  if (n_clips == 0) return KOE_OK;
-  CoreParams p{};
-  p.w = *w;
+  CoreParams p;
+  if (int rc = core_params("koe_dual_stream_features", w, nullptr, nullptr, 0, expr_sigmoid, out, sigmoid_out, attn_out, &p))
+    return rc;
   p.n_clips = n_clips;
-  p.n_out = 1;
-  p.stride_frames = 1;
   p.frames_per_window = 1;
-  p.mel_seq = w->k_mel - 3;
-  p.expr_sigmoid = expr_sigmoid;
-  p.out = out;
-  p.sigmoid_out = sigmoid_out;
-  p.attn_out = attn_out;
   p.mel_long = mel_long;
   p.mel_short = mel_short;
   p.n_long = n_long < p.mel_seq ? n_long : p.mel_seq;
   // rows of a longer mel_long are still addressed with its true length
   p.n_frames = n_long;
-  return launch_core(p, precision, (cudaStream_t)stream);
+  return launch_core(p, CoreMode::Windows, precision, (cudaStream_t)stream);
 }
 
 extern "C" int koe_ema_scan(float* frames, int n_clips, int n_out, float alpha, float* state, int has_state,

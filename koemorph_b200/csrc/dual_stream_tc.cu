@@ -216,15 +216,13 @@ __device__ __forceinline__ void stamp(long long* dbg, int slot) {
 
 __device__ __forceinline__ void simt_barrier() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 
-// kEarly: the early-release flavour of the fused forward (see the wait below); a separate instantiation, so that the
-// kernel every other caller runs (streaming, sequences, the public entries) stays exactly as it was: the three extra
-// checks cost that one 4 % through register spills when they were run-time branches.  kPool: the stream-pool flavour
-// (csrc/stream_pool.cu), ring mode with a stream slot and a ring base per window (p.pool_slot, p.pool_base), and kVarlen: the
-// packed variable-length batch (the window's clip from p.vl_window_base; clips without edge variants read every frame from
-// the plain rows), kept apart for the same reason.
-template <int KMEL, bool kEarly = false, bool kPool = false, bool kVarlen = false>
+// One instantiation per CoreMode; the window of a work item and the rows of its frames come from CoreRows<M>.  Early is
+// the early-release flavour of the fused forward (see the wait below): as run-time branches its extra checks cost the
+// kernel every other caller runs 4 % through register spills.
+template <int KMEL, CoreMode M>
 __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams p) {
   using G = Geo<KMEL>;
+  using Rows = CoreRows<M>;
   constexpr int kKMel = G::kKMel, kA1Chunks = G::kA1Chunks, kA1Sbo = G::kA1Sbo, kLongChunks = G::kLongChunks;
   constexpr int kStagesG1 = G::kStagesG1, kStagesPerWindow = G::kStagesPerWindow;
   constexpr bool kStageAhead = G::kStageAhead;
@@ -234,7 +232,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
   const koe_core_weights& W = p.w;
   // early release: a first look at the flag now, so that its L2 round trip runs beside the prologue (used below)
   unsigned early_seen = 0;
-  if (kEarly && lane == 0) asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(early_seen) : "l"(p.early_flag) : "memory");
+  if (M == CoreMode::Early && lane == 0) asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(early_seen) : "l"(p.early_flag) : "memory");
   long long* dk = (p.dbg != nullptr && blockIdx.x == 0 && tid == 0) ? p.dbg + 120 : nullptr;
   stamp(dk, 0);
   if (p.dbg != nullptr && tid == 0) {  // per-CTA wall-clock span (ns) for the launch-level picture
@@ -296,7 +294,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
   // CTAs leave them, and with the flag they start their first windows at once instead of idling until the frontend's
   // slowest CTA is done.  Acquire: one lane per warp polls, the warp barrier orders the other lanes behind it; the mel-row
   // producer adds a proxy fence (its reads are TMA copies).  Items from early_items on wait for griddepcontrol.wait.
-  if (kEarly) {
+  if constexpr (M == CoreMode::Early) {
     if (lane == 0) {
       unsigned seen = early_seen;
       for (uint32_t spin = 0; seen < p.early_target; ++spin) {
@@ -312,7 +310,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
     pdl_wait();
   }
   // (early_items is a multiple of the grid: a CTA's first item that the flag does not cover is early_items + blockIdx.x)
-  const int first_late_item = kEarly ? p.early_items + (int)blockIdx.x : 0;
+  const int first_late_item = M == CoreMode::Early ? p.early_items + (int)blockIdx.x : 0;
   // (no griddepcontrol.launch_dependents here: released early, the next forward's frontend CTAs take the SMs that this
   // kernel's last partial round of windows leaves idle and the step gets 11 us SLOWER -- measured, 198.6 vs 209.5 us)
 
@@ -357,21 +355,19 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       const uint64_t pol_keep = l2_policy_keep(), pol_stream = l2_policy_stream();
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         long long* dp = (p.dbg != nullptr && blockIdx.x == 0 && item < 2 * (int)gridDim.x) ? p.dbg + 32 + 16 * (item / gridDim.x) : nullptr;
-        int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
-        if constexpr (kVarlen) b = varlen_window<false>(p, item).row, wi = item;
-        if (kEarly && (item == (int)blockIdx.x || item == first_late_item)) {
+        const CoreWindow win = Rows::template window<false>(p, item);
+        if (M == CoreMode::Early && (item == (int)blockIdx.x || item == first_late_item)) {
           if (item == first_late_item) pdl_wait();
           asm volatile("fence.proxy.async.global;" ::: "memory");  // generic-proxy acquire / wait above -> TMA reads below
         }
-        const float* base = p.ring_frames > 0 ? p.power[0] + (size_t)b * p.ring_frames * kTok
-                                              : p.power[0] + core_row<kPool, kVarlen>(p, 0, b, wi, 0) * kTok;
+        const float* base = p.ring_frames > 0 ? p.power[0] + (size_t)win.owner * p.ring_frames * kTok
+                                              : p.power[0] + Rows::row(p, win, 0, 0) * kTok;
         // Ring mode (the streaming step): with thousands of streams the rings (82 KB each: 335 MB for 4096 streams) do not
         // stay in L2 from one hop to the next, and a window's six stages pass through two ring slots one HBM latency after
         // the other.  The NEXT window's ring and frame maxima are pulled into L2 now, a whole window ahead (4096 streams:
         // p50 0.4285 -> 0.4175 ms per hop; a steady window is 19.4 k cycles here against 17.6 k in the batch forward).
         if (p.ring_frames > 0 && item + (int)gridDim.x < n_items) {
-          // (n_out == 1 in ring mode: item == stream; the pool's next window reads stream pool_slot[item + grid])
-          const int nb = kPool ? p.pool_slot[item + gridDim.x] : item + gridDim.x;
+          const int nb = Rows::ring_stream(p, item + gridDim.x);
           const char* ring = reinterpret_cast<const char*>(p.power[0] + (size_t)nb * p.ring_frames * kTok);
           const uint32_t ring_bytes = (uint32_t)p.ring_frames * kTok * 4;
           for (uint32_t off = 0; off < ring_bytes; off += 16384) bulk_prefetch_l2(ring + off, min(16384u, ring_bytes - off));
@@ -388,14 +384,14 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           if (s == n_mel_stages - 1) stamp(dp, 9);
           mbar_expect_tx(bar_full + 8 * slot, bytes);
           if (p.ring_frames > 0) {
-            const int r0 = ((kPool ? wi : p.ring_base) + kMelRows * s) % p.ring_frames;
+            const int r0 = (Rows::ring_base(p, win) + kMelRows * s) % p.ring_frames;
             const int n1 = min(n, p.ring_frames - r0);
             bulk_g2s_hint(dst, base + (size_t)r0 * kTok, (uint32_t)n1 * kTok * 4, bar_full + 8 * slot, pol_keep);
             if (n1 < n)
               bulk_g2s_hint(dst + (uint32_t)n1 * kTok * 4, base, (uint32_t)(n - n1) * kTok * 4, bar_full + 8 * slot, pol_keep);
           } else {
             bulk_g2s_hint(dst, base + (size_t)s * kMelRows * kTok, bytes, bar_full + 8 * slot,
-                          kVarlen || p.n_out > 1 ? pol_keep : pol_stream);  // overlapping windows of a sequence re-read their rows
+                          Rows::plain_rows_policy(p, pol_keep, pol_stream));
           }
           if (++slot == kRing) slot = kWRing, phase ^= 1;
         }
@@ -515,12 +511,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
     auto frame_max_partial = [&](const int item) {
       float mx = -INFINITY;
       if (!prenorm) {
-        int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
-        bool plain_only = false;
-        if constexpr (kVarlen) {
-          const VarlenWindow vw = varlen_window<true>(p, item);
-          b = vw.row, wi = item, plain_only = vw.plain_only;
-        }
+        const CoreWindow win = Rows::template window<true>(p, item);
         for (int k0 = tid; k0 < T; k0 += 3 * kSimt) {
           float f[3];
 #pragma unroll
@@ -528,8 +519,8 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
             const int k = k0 + u * kSimt;
             f[u] = -INFINITY;
             if (k < T) {
-              const int v = plain_only ? 0 : window_variant(p, k);
-              f[u] = p.fmax[v][core_row<kPool, kVarlen>(p, v, b, wi, k)];
+              const int v = win.plain_only ? 0 : window_variant(p, k);
+              f[u] = p.fmax[v][Rows::row(p, win, v, k)];
             }
           }
           mx = fmaxf(fmaxf(mx, f[0]), fmaxf(f[1], f[2]));
@@ -538,12 +529,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       return mx;
     };
     auto stage_window = [&](const int item, float mx, long long* ds) {
-      int b = kPool ? p.pool_slot[item] : item / p.n_out, wi = kPool ? p.pool_base[item] : item % p.n_out;
-      bool plain_only = false;  // (varlen) no edge variants: every frame of the window from the plain rows
-      if constexpr (kVarlen) {
-        const VarlenWindow vw = varlen_window<true>(p, item);
-        b = vw.row, wi = item, plain_only = vw.plain_only;
-      }
+      const CoreWindow win = Rows::template window<true>(p, item);
       // ---- window dB reference
       float ref_db = 0.0f;
       if (!prenorm) {
@@ -564,15 +550,15 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           for (int e = 0; e < 3; ++e) {
             const int k = T >= 3 ? T - 3 + e : (e < T ? e : -1);
             if (k >= 0) {
-              const int var = plain_only ? 0 : window_variant(p, k);
-              extra[e] = p.power[var][core_row<kPool, kVarlen>(p, var, b, wi, k) * kTok + tid];
+              const int var = win.plain_only ? 0 : window_variant(p, k);
+              extra[e] = p.power[var][Rows::row(p, win, var, k) * kTok + tid];
             } else {
               extra[e] = -INFINITY;
             }
           }
-          if (!plain_only && p.n_edge > 0) {
-            extra[3] = __ldg(p.power[1] + core_row<kPool, kVarlen>(p, 1, b, wi, 0) * kTok + tid);
-            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + core_row<kPool, kVarlen>(p, 2, b, wi, T - 1) * kTok + tid);
+          if (!win.plain_only && p.n_edge > 0) {
+            extra[3] = __ldg(p.power[1] + Rows::row(p, win, 1, 0) * kTok + tid);
+            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + Rows::row(p, win, 2, T - 1) * kTok + tid);
           }
         }
         for (int s = 0; s < n_mel_stages; ++s) {
@@ -631,13 +617,13 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           *reinterpret_cast<uint4*>(arow + (kLongChunks + 1) * 128) = make_uint4(0, 0, 0, 0);
           // edge frames inside the long-term range see zeros beyond the window edge: patch them in place
           // (frame m and frame T-1-m for m < n_edge: one per side at 30 fps, two at 60 fps)
-          for (int m = 0; !plain_only && m < p.n_edge; ++m) {
-            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + core_row<kPool, kVarlen>(p, 1 + 2 * m, b, wi, m) * kTok + j);
+          for (int m = 0; !win.plain_only && m < p.n_edge; ++m) {
+            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + Rows::row(p, win, 1 + 2 * m, m) * kTok + j);
             *reinterpret_cast<__nv_bfloat16*>(arow + (m >> 3) * 128 + (m & 7) * 2) =
                 __float2bfloat16_rn(normalise_bf16(lo, ref_db, true));
             const int k = T - 1 - m;
             if (k < Tl) {
-              const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + core_row<kPool, kVarlen>(p, 2 + 2 * m, b, wi, k) * kTok + j);
+              const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + Rows::row(p, win, 2 + 2 * m, k) * kTok + j);
               *reinterpret_cast<__nv_bfloat16*>(arow + (k >> 3) * 128 + (k & 7) * 2) =
                   __float2bfloat16_rn(normalise_bf16(x, ref_db, true));
             }
@@ -660,9 +646,9 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
               // TMA mel ring above)
               if (t < kKMel) {
                 if (t >= p.mel_seq)
-                  x = __ldg(reinterpret_cast<const float4*>(p.mel_short + ((size_t)b * 3 + (t - p.mel_seq)) * kTok) + q);
+                  x = __ldg(reinterpret_cast<const float4*>(p.mel_short + ((size_t)win.owner * 3 + (t - p.mel_seq)) * kTok) + q);
                 else if (t < p.n_long)
-                  x = __ldg(reinterpret_cast<const float4*>(p.mel_long + ((size_t)b * p.n_frames + t) * kTok) + q);
+                  x = __ldg(reinterpret_cast<const float4*>(p.mel_long + ((size_t)win.owner * p.n_frames + t) * kTok) + q);
               }
               r[e] = x;
             }
@@ -700,19 +686,19 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       stamp(dk, 2);
     }
     for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-      const int b = kPool ? p.pool_slot[item] : item / p.n_out;
+      const int expr_row = Rows::expr_row(p, item);
       const bool has_next = item + (int)gridDim.x < n_items;
       long long* ds = (p.dbg != nullptr && blockIdx.x == 0 && tid == 0 && item < 2 * (int)gridDim.x) ? p.dbg + 16 * (item / gridDim.x) : nullptr;
       stamp(ds, 0);
       if (!kStageAhead) {
-        if (kEarly && item == first_late_item) pdl_wait();  // (early release: this window's clip is not covered by the flag)
+        if (M == CoreMode::Early && item == first_late_item) pdl_wait();  // (early release: this window's clip is not covered by the flag)
         stage_window(item, frame_max_partial(item), ds);
         fence_async_smem();
         mbar_arrive(bar_go);
       }
       stamp(ds, 1);
       // (early release: the next window is this CTA's first whose clip the flag does not cover -- it is read from here on)
-      if (kEarly && has_next && item + (int)gridDim.x == first_late_item) pdl_wait();
+      if (M == CoreMode::Early && has_next && item + (int)gridDim.x == first_late_item) pdl_wait();
       const float mx_next = kStageAhead && has_next ? frame_max_partial(item + gridDim.x) : -INFINITY;
 
       // ---- E1: bias + LayerNorm of token row tid -> enc (bf16, K-major) -------------------------------
@@ -888,7 +874,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           if (p.sigmoid_out != nullptr) p.sigmoid_out[o_off] = y;
         }
       } else if (warp == 1 && lane < KOE_N_EXPR && p.expr_sigmoid != nullptr) {  // (NULL: the emotion kernel writes these)
-        const float y = __ldg(p.expr_sigmoid + b);
+        const float y = __ldg(p.expr_sigmoid + expr_row);
         const int idx = __ldg(W.expr_idx + lane);
         const size_t o_off = (size_t)item * KOE_N_BLENDSHAPES + idx;
         p.out[o_off] = fminf(fmaxf(__ldg(W.coef + idx) * y, 0.0f), 1.0f);
@@ -906,7 +892,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem));
   }
-  if (kEarly) {
+  if constexpr (M == CoreMode::Early) {
     // this kernel must not complete before the kernels ahead of it have (what follows waits on this kernel only); the
     // last CTA out clears the flag and the exit counter for the next forward on this stream
     pdl_wait();
@@ -925,92 +911,60 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
 }  // namespace tc
 
 int dual_stream_tc_grid(int n_items) {
-  static int sms[64] = {0};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
-  if (sms[dev] == 0 && cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  return std::min(n_items, sms[dev]);
+  int sms = 0;
+  if (sm_count(&sms) != cudaSuccess) return 0;
+  return std::min(n_items, sms);
 }
 
-int launch_dual_stream_tc(const CoreParams& p, int precision, cudaStream_t stream) {
-  if (precision != 2)
-    return fail(KOE_E_UNSUPPORTED, "tensor-core path: only precision 2 (bf16 operands) is built; tf32 is not");
+// sets the shared-memory size of the instantiation once per device, then launches it behind the previous kernel
+template <int KMEL, CoreMode M>
+static int launch_tc(const CoreParams& p, int grid, cudaStream_t stream) {
+  static bool configured[64] = {false};
+  int dev = 0;
+  KOE_CUDA(cudaGetDevice(&dev));
+  KOE_REQUIRE(dev >= 0 && dev < 64, "device index too large");
+  if (!configured[dev]) {
+    KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<KMEL, M>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  tc::kSmemBytes));
+    configured[dev] = true;
+  }
+  KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<KMEL, M>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes,
+                                       stream, p));
+  return KOE_OK;
+}
+template <CoreMode M>
+static int launch_tc(const CoreParams& p, int grid, cudaStream_t stream) {
+  return p.w.k_mel == 259 ? launch_tc<259, M>(p, grid, stream) : launch_tc<515, M>(p, grid, stream);
+}
+
+int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t stream) {
   if (p.w.k_mel != 259 && p.w.k_mel != 515)
     return fail(KOE_E_UNSUPPORTED, "tensor-core path is built for k_mel = 259 (30 fps) and 515 (60 fps); got %d", p.w.k_mel);
   const int need_stages = p.w.k_mel == 259 ? tc::Geo<259>::kStagesPerWindow : tc::Geo<515>::kStagesPerWindow;
   if (p.w.tc_bf16 == nullptr || p.w.tc_bv == nullptr || p.w.tc_stages != need_stages)
     return fail(KOE_E_INVALID, "tensor-core path: koe_core_weights.tc_bf16 is missing (%d stages, need %d)",
                 p.w.tc_stages, need_stages);
-  static int num_sms[64] = {0};
-  int dev = 0;
-  KOE_CUDA(cudaGetDevice(&dev));
-  KOE_REQUIRE(dev >= 0 && dev < 64, "device index too large");
-  if (num_sms[dev] == 0) {
-    KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<259>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  tc::kSmemBytes));
-    KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<515>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  tc::kSmemBytes));
-    int n = 0;
-    KOE_CUDA(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
-    num_sms[dev] = n;
-  }
+  int sms = 0;
+  KOE_CUDA(sm_count(&sms));
+  const int grid = std::min(p.n_clips * p.n_out, sms);
+  if (mode == CoreMode::Early)
+    KOE_REQUIRE(p.n_out == 1 && p.early_items > 0 && p.early_items % grid == 0 && p.early_target > 0,
+                "tensor-core path: bad early-release parameters");
+  if (mode == CoreMode::Varlen)
+    KOE_REQUIRE(p.n_out == 1 && p.ring_frames == 0 && p.expr_sigmoid == nullptr, "tensor-core path: bad varlen parameters");
+  if (mode == CoreMode::Pool)
+    KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
   if (p.attn_out != nullptr)  // head-average is accumulated with atomics
     KOE_CUDA(cudaMemsetAsync(p.attn_out, 0, (size_t)p.n_clips * p.n_out * KOE_N_MOUTH * tc::kTok * sizeof(float),
                              stream));
-  const int grid = std::min(p.n_clips * p.n_out, num_sms[dev]);
-  if (p.early_flag != nullptr) {
-    KOE_REQUIRE(p.n_out == 1 && p.early_items > 0 && p.early_items % grid == 0 && p.early_target > 0,
-                "tensor-core path: bad early-release parameters");
-    static bool configured[64] = {false};
-    if (!configured[dev]) {
-      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<259, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    tc::kSmemBytes));
-      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<515, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    tc::kSmemBytes));
-      configured[dev] = true;
-    }
-    if (p.w.k_mel == 259)
-      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259, true>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes,
-                                           stream, p));
-    else
-      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, true>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes,
-                                           stream, p));
-  } else if (p.vl_window_base != nullptr) {
-    KOE_REQUIRE(p.n_out == 1 && p.ring_frames == 0 && p.expr_sigmoid == nullptr, "tensor-core path: bad varlen parameters");
-    static bool configured[64] = {false};
-    if (!configured[dev]) {
-      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<259, false, false, true>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBytes));
-      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<515, false, false, true>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBytes));
-      configured[dev] = true;
-    }
-    if (p.w.k_mel == 259)
-      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259, false, false, true>, dim3(grid), dim3(tc::kThreads),
-                                           tc::kSmemBytes, stream, p));
-    else
-      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, false, false, true>, dim3(grid), dim3(tc::kThreads),
-                                           tc::kSmemBytes, stream, p));
-  } else if (p.pool_slot != nullptr) {
-    KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
-    static bool configured[64] = {false};
-    if (!configured[dev]) {
-      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<259, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    tc::kSmemBytes));
-      KOE_CUDA(cudaFuncSetAttribute(tc::dual_stream_tc_kernel<515, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    tc::kSmemBytes));
-      configured[dev] = true;
-    }
-    if (p.w.k_mel == 259)
-      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259, false, true>, dim3(grid), dim3(tc::kThreads),
-                                           tc::kSmemBytes, stream, p));
-    else
-      KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515, false, true>, dim3(grid), dim3(tc::kThreads),
-                                           tc::kSmemBytes, stream, p));
-  } else if (p.w.k_mel == 259)
-    KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<259>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes, stream, p));
-  else
-    KOE_CUDA(launch_after_primary_starts(tc::dual_stream_tc_kernel<515>, dim3(grid), dim3(tc::kThreads), tc::kSmemBytes, stream, p));
+  int rc = KOE_OK;
+  switch (mode) {
+    case CoreMode::Windows: rc = launch_tc<CoreMode::Windows>(p, grid, stream); break;
+    case CoreMode::Early: rc = launch_tc<CoreMode::Early>(p, grid, stream); break;
+    case CoreMode::Pool: rc = launch_tc<CoreMode::Pool>(p, grid, stream); break;
+    case CoreMode::Varlen: rc = launch_tc<CoreMode::Varlen>(p, grid, stream); break;
+  }
+  if (rc != KOE_OK) return rc;
   count_launch();
   KOE_CUDA(cudaGetLastError());
   return KOE_OK;

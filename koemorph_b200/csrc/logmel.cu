@@ -1449,9 +1449,8 @@ extern "C" int koe_pcm16_to_float(const int16_t* pcm, int64_t n_samples, float* 
   KOE_REQUIRE(pcm != nullptr && audio != nullptr, "koe_pcm16_to_float: NULL argument");
   KOE_REQUIRE(((reinterpret_cast<uintptr_t>(pcm) | reinterpret_cast<uintptr_t>(audio)) & 15) == 0,
               "koe_pcm16_to_float: buffers must be 16-byte aligned");
-  int dev = 0, sms = 0;
-  KOE_CUDA(cudaGetDevice(&dev));
-  KOE_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  int sms = 0;
+  KOE_CUDA(koe::sm_count(&sms));
   const long long want = ((n_samples >> 3) + 255) / 256;
   const int grid = (int)std::max<long long>(1, std::min<long long>(want, (long long)sms * 8));
   koe::pcm16_to_float_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(pcm, (long long)n_samples, audio);

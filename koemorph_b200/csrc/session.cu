@@ -58,9 +58,8 @@ extern "C" int koe_stream_push(const koe_stream_args* a, int* emitted, void* str
   const float* old_tail = a->tail[n & 1];
   float* tail = a->tail[(n + 1) & 1];
   {
-    int dev = 0, sms = 0;
-    KOE_CUDA(cudaGetDevice(&dev));
-    KOE_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    KOE_CUDA(sm_count(&sms));
     const int grid = std::min(S, sms * 8);
     stream_tail_shift_kernel<<<grid, 256, 0, stream>>>(old_tail, a->hop_audio, S, tail_len, hop, tail);
     count_launch();

@@ -99,14 +99,6 @@ __global__ void __launch_bounds__(256) pool_expr_scatter_kernel(const float* __r
 }
 
 namespace {
-int num_sms() {
-  static int sms[64] = {0};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
-  if (sms[dev] == 0 && cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  return sms[dev];
-}
-
 // every slot of slots[0, n) in range, open and listed once
 int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* what) {
   KOE_REQUIRE(n >= 0 && n <= pool->capacity, "%s: %d streams for a pool of %d", what, n, pool->capacity);
@@ -221,6 +213,8 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
               "koe_stream_pool_push: hop < n_fft/2 needs the second edge buffers (ring_r2, row_l2)");
   KOE_REQUIRE(a->ema_state == nullptr || (a->alpha >= 0.0f && a->alpha <= 1.0f), "koe_stream_pool_push: alpha must be in [0, 1]");
   if (int rc = check_capture(stream, "koe_stream_pool_push")) return rc;
+  int sms = 0;
+  KOE_CUDA(sm_count(&sms));
   cudaStream_t st = (cudaStream_t)stream;
 
   // ---- the per-call tables: [push slot | push ring row | push first hop][emit slot | emit ring base | emit has state]
@@ -255,7 +249,7 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
 
   // ---- 1. tail update + compact copy
   {
-    const int grid = std::min(n, std::max(num_sms(), 1) * 8);
+    const int grid = std::min(n, sms * 8);
     pool_tail_kernel<<<grid, 256, tail_len * sizeof(float), st>>>(a->tail, a->hop_audio, push_slot, push_first, n, tail_len,
                                                                   hop, a->tail_compact);
     count_launch();
@@ -303,7 +297,7 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
   for (int v = 0; v < V; ++v) r.power[v] = power[v], r.fmax[v] = fmax[v];
   {
     const int total = n * V * (KOE_N_MELS / 4);
-    pool_scatter_kernel<<<std::min((total + 255) / 256, std::max(num_sms(), 1) * 8), 256, 0, st>>>(
+    pool_scatter_kernel<<<std::min((total + 255) / 256, sms * 8), 256, 0, st>>>(
         r, a->stage, a->stage_max, push_slot, push_row, n, V, W);
     count_launch();
     KOE_CUDA(cudaGetLastError());
