@@ -69,11 +69,6 @@ inline cudaError_t sm_count(int* n) {
   return cudaSuccess;
 }
 
-// frontend launch with launch-chaining knowledge of the caller (csrc/logmel.cu; used by csrc/session.cu)
-// early_clips / early_flag / early_target: see "early release of the core" in csrc/session.cu (0 / NULL: off)
-int launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* args, void* stream, bool follows_frontend_launch,
-                  int early_clips, unsigned* early_flag, unsigned* early_target);
-
 #define KOE_REQUIRE(cond, ...)                                   \
   do {                                                           \
     if (!(cond)) return koe::fail(KOE_E_INVALID, __VA_ARGS__);   \
@@ -91,14 +86,51 @@ int acquire_table_staging(void* stream, size_t ints, TableStaging** out);
 int upload_tables(TableStaging* b, int32_t* dev_tables, size_t ints, cudaStream_t stream);
 int check_capture(void* stream, const char* what);
 
-// Ragged frontend launch of the packed variable-length forward (csrc/logmel.cu, default bank only): frame pair k of the
-// launch is pair k - pair_base[c] of clip c (pair_base[c] <= k < pair_base[c + 1]); clip c is `length[c]` samples at
-// audio + sample_off[c] and has row_base[c + 1] - row_base[c] frames in this launch, frame j centred on sample
-// (frame_offset + j * frame_step) * hop of the clip (window edges as lo_rel_hops / hi_rel_hops), stored to row
-// row_base[c] + j of power / frame_max.  From `a`: audio, hop, frame_offset, frame_step, lo/hi_rel_hops, power, frame_max.
-int launch_logmel_varlen(const koe_frontend_t* fe, const koe_logmel_args* a, const long long* sample_off, const int* length,
-                         const int* pair_base, const int* row_base, int n_clips, long long total_pairs, void* stream,
-                         bool follows_frontend_launch);
+// ---- log-mel frontend launches (csrc/logmel.cu) -------------------------------------------------------------------------
+enum class FrontendMode {
+  Frames,      // frame j of clip c to row j of clip c's block of power / frame_max
+  SplitPairs,  // the same for the even frames; frame 2j + 1 to row j of power_b / frame_max_b (the streaming step)
+  Varlen,      // a packed variable-length batch (VarlenTables; default bank only)
+};
+
+// Packed variable-length batch: frame pair k of the launch is pair k - pair_base[c] of clip c (pair_base[c] <= k <
+// pair_base[c + 1], `pairs` in all); clip c is `length[c]` samples at audio + sample_off[c] and has row_base[c + 1] -
+// row_base[c] frames in this launch, frame j centred on sample (frame_offset + j * frame_step) * hop of the clip (window
+// edges as lo_rel_hops / hi_rel_hops), stored to row row_base[c] + j of power / frame_max.  Of the koe_logmel_args it
+// reads audio, hop, frame_offset, frame_step, lo/hi_rel_hops, power and frame_max.
+struct VarlenTables {
+  const long long* sample_off;
+  const int* length;
+  const int* pair_base;
+  const int* row_base;
+  int n_clips;
+  long long pairs;
+};
+
+// Early release of the core (csrc/session.cu): the frontend counts up *flag once clips [0, clips) are stored.  The
+// launcher sets `target` to the count that means so, or to 0 when this launch does not signal.
+struct EarlyRelease {
+  int clips;
+  unsigned* flag;
+  unsigned target;
+};
+
+// One frontend launch.  `follows_frontend_launch`: the kernel queued just before this one on `stream` is another frontend
+// launch of the same forward, writing other buffers.  `early`: only a Frames launch with the default bank signals.
+int launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* a, FrontendMode mode, bool follows_frontend_launch,
+                  void* stream, EarlyRelease* early = nullptr, const VarlenTables* varlen = nullptr);
+
+// Destination of one mel-row variant: clip c's rows at power + c * power_stride, its maxima at frame_max + c * fmax_stride.
+struct MelRows {
+  float* power;
+  float* frame_max;
+  int64_t power_stride, fmax_stride;
+};
+
+// The frontend launches of one streaming hop (csrc/session.cu) over n_streams tails of tail_len samples, the newest
+// complete frame centred `half` samples in: rows[v] receives mel-row variant v = F, R0, L0, R1, L1 (1 + 2 n_edge of them).
+int launch_hop_frontend(const koe_frontend_t* fe, const float* tail, int n_streams, int tail_len, int half, int hop,
+                        int n_edge, const MelRows* rows, void* stream);
 
 // ---- device helpers ----------------------------------------------------------------------------
 // Programmatic dependent launch (sm_90+): a kernel launched with launch_after_primary_starts() may begin while the

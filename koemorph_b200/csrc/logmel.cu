@@ -79,13 +79,12 @@ struct LogmelParams {
   int edge_lo, edge_hi;          // leading / trailing frame pairs of a clip that need masked loads (launch order only)
   int mid_pairs;                 // interior pairs per clip (0: no edge grouping, every pair is located the slow way)
   int step_clips, step_pairs;    // gridDim.x * kWarps pairs, as whole clips of mid_pairs + a remainder
-  int store_order;               // 2 bits per warp class (warp / 4): where its store phase sits (see the kernel)
   int wait_at_end;               // launch chaining: this launch follows another frontend launch of the same forward (below)
   // early release of the core (csrc/session.cu): every consumer warp adds one to *early_flag (release) when its CTA has
   // stored the rows of all its iterations below early_iters -- the core's first rounds of windows need no more than that
   unsigned* early_flag;
   unsigned early_iters;
-  // packed variable-length batch (launch_logmel_varlen, the kVarlen instantiation only): pair k of the launch is pair
+  // packed variable-length batch (FrontendMode::Varlen, VarlenLocator only): pair k of the launch is pair
   // k - vl_pair_base[c] of clip c, vl_length[c] samples at audio + vl_sample_off[c], rows vl_row_base[c] ..
   // vl_row_base[c + 1] - 1; n_clips / n_samples / n_frames / the clip strides are not used
   const long long* vl_sample_off;
@@ -352,29 +351,6 @@ __device__ __forceinline__ void mel_phase_generic(int g, int gend, const int4* s
   }
 }
 
-// ---- mbarrier (shared-memory barrier object): arrive now, wait later -----------------------------------------------
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void bar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void bar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// bounded spin: a protocol bug traps (error to the host) instead of hanging the GPU
-__device__ __forceinline__ void bar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok = 0;
-  for (uint32_t spin = 0; !ok; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (!ok && spin > (1u << 22)) __trap();
-  }
-}
-
 // Launch chaining of the frontend kernels (programmatic dependent launch, common.cuh).  Both kernels are launched with
 // the programmatic attribute: their CTAs take SMs as the previous kernel of the stream (the core / smoothing kernel of the
 // previous forward, another frontend launch, the streaming step's tail shift) drains, and the prologue above -- tables
@@ -511,6 +487,9 @@ __device__ __forceinline__ void store_pair_rows(const FrontendTables& tab, const
 // (gridDim.x * kWarps), so clip and pair are kept incrementally: no division in the loop.
 struct PairLocator {
   int in_clip = -1, in_j = 0;  // interior position of the pair located last (-1: none yet)
+  __device__ __forceinline__ static unsigned total_pairs(const LogmelParams& p) {
+    return (unsigned)p.n_clips * ((unsigned)(p.n_frames + 1) >> 1);
+  }
   __device__ __forceinline__ PairInfo locate(const LogmelParams& p, unsigned iter, unsigned n_iters, unsigned total_pairs,
                                              unsigned ppc, int warp) {
     const unsigned n_edge_pairs = p.mid_pairs > 0 ? (unsigned)p.n_clips * (unsigned)(p.edge_lo + p.edge_hi) : total_pairs;
@@ -555,6 +534,7 @@ struct VarlenLocator {
   int clip = -1;
   const float* src = nullptr;  // the located clip's first sample
   int len = 0;                 // its length
+  __device__ __forceinline__ static unsigned total_pairs(const LogmelParams& p) { return p.vl_pairs; }
   __device__ __forceinline__ PairInfo locate(const LogmelParams& p, unsigned iter, unsigned n_iters, unsigned total_pairs,
                                              unsigned, int warp) {
     const unsigned pair = iter < n_iters ? iter * kWarps + warp : total_pairs;
@@ -642,10 +622,10 @@ __device__ __forceinline__ void bar_wait_parked(uint32_t bar, uint32_t parity) {
 //   B  __syncthreads: all 32 spectra of the iteration are in the tiles
 //   M  mel phase: lane = frame, warp = run of bins -> mel tiles; arrive on the mbarrier
 //   S  store phase of the PREVIOUS iteration's rows (the tiles hold them until the next B), placed per warp class
-//      (warp / 4, one warp of every class on each scheduler) either before F, between T and L, or after L: the classes
-//      then run the FFT a store phase apart, so that the FMA-bound and the shared-memory-bound stretches of different
-//      warps overlap instead of all 16 warps queueing for the same pipe at the same time.
-template <bool kDefaultBank, bool kSplitB = false>
+//      (warp / 4, one warp of every class on each scheduler): classes 0 and 2 before F, classes 1 and 3 after L.  The
+//      classes then run the FFT a store phase apart, so that the FMA-bound and the shared-memory-bound stretches of
+//      different warps overlap instead of all 16 warps queueing for the same pipe at the same time.
+template <bool kDefaultBank, bool kSplitB>
 __global__ void __launch_bounds__(kThreads, 1)
 logmel_power_kernel(FrontendTables tab, LogmelParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -667,19 +647,19 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
   if (tid <= kWarps) s_runs[tid] = tab.runs[tid];
   // cells that no group writes (filter 0's rising half; filters without a falling / rising group in sparse banks) stay 0
   for (int i = tid; i < 2 * kSlots * kTileStride; i += kThreads) s_tiles[i] = 0.0f;
-  const uint32_t mel_done = smem_addr(s_bar);
+  const uint32_t mel_done = smem_u32addr(s_bar);
   if (tid == 0) {
-    bar_init(mel_done, kWarps);
+    mbarrier_init(mel_done, kWarps);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
   pdl_prologue_done(p);
 
   const unsigned ppc = (unsigned)(p.n_frames + 1) >> 1;  // frame pairs per clip
-  const unsigned total_pairs = (unsigned)p.n_clips * ppc;
+  const unsigned total_pairs = PairLocator::total_pairs(p);
   const unsigned n_iters = (total_pairs + kWarps - 1) / kWarps;
   float* xb = s_scratch + warp * kScratch;
-  const int order = (p.store_order >> (2 * (warp >> 2))) & 3;  // 0: S before F; 1: S after L; 2: S between T and L
+  const bool store_first = ((warp >> 2) & 1) == 0;  // S before F (classes 0, 2) or after L (classes 1, 3)
 
   auto store_rows = [&](int clip, int frame, bool has_b, const float* tiles) {  // warp w owns tile rows 2w, 2w + 1
     store_pair_rows<kSplitB>(tab, p, clip, frame, has_b, tiles, 2 * warp, lane);
@@ -690,8 +670,7 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
   float2 v[32];
   unsigned it = blockIdx.x;
   PairInfo nxt = locate(it);
-  if (nxt.interior) load_interior(p, nxt, lane, v);
-  else if (nxt.frame >= 0) load_edge(p, nxt, lane, v);
+  loc.load(p, nxt, lane, v);
   int pend_clip = 0, pend_frame = -1;  // the pair whose mel rows wait in the tiles for their store phase
   bool pend_has_b = false;
   unsigned k = 0;                      // iterations done by this CTA: parity of the mbarrier phase / tile buffer
@@ -700,8 +679,8 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
     // the mel tiles hold the previous iteration's rows until the next mel phase, i.e. until the __syncthreads below:
     // every store phase, early or late, comes before it
     const float* prev_tiles = s_tiles;
-    if (order == 0 && pend_frame >= 0) {
-      bar_wait(mel_done, (k + 1) & 1);  // the previous mel phase, by every warp
+    if (store_first && pend_frame >= 0) {
+      mbarrier_wait(mel_done, (k + 1) & 1);  // the previous mel phase, by every warp
       store_rows(pend_clip, pend_frame, pend_has_b, prev_tiles);
       pend_frame = -1;
     }
@@ -709,23 +688,14 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
     const PairInfo cur = nxt;
     if (cur.frame >= 0) fft_first_half(v, s_hann, s_tw, lane);
     // the tile still holds this warp's spectra of the previous iteration until every warp has finished that mel phase
-    if (k > 0) bar_wait(mel_done, (k + 1) & 1);
+    if (k > 0) mbarrier_wait(mel_done, (k + 1) & 1);
     if (cur.frame >= 0) fft_second_half(v, xb, lane);
-    if (order == 2 && pend_frame >= 0) {
-      store_rows(pend_clip, pend_frame, pend_has_b, prev_tiles);
-      pend_frame = -1;
-    }
     // audio of the next iteration: in flight during the mel / store phases
     nxt = locate(it + gridDim.x);
-    if (nxt.interior) load_interior(p, nxt, lane, v);
-    else if (nxt.frame >= 0) load_edge(p, nxt, lane, v);
-    if (order == 1 && pend_frame >= 0) {
+    loc.load(p, nxt, lane, v);
+    if (!store_first && pend_frame >= 0) {
       store_rows(pend_clip, pend_frame, pend_has_b, prev_tiles);
       pend_frame = -1;
-    }
-    if (p.store_order & 0x100) {  // timing probe (scripts/k1_variants.py): FFT + loads only, free running, no results
-      if (lane == 0) bar_arrive(mel_done);
-      continue;
     }
     __syncthreads();
 
@@ -740,11 +710,11 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
         mel_phase_generic(s_runs[warp], s_runs[warp + 1], s_groups, s_binw, spec, tlo, thi);
     }
     __syncwarp();
-    if (lane == 0) bar_arrive(mel_done);
+    if (lane == 0) mbarrier_arrive(mel_done);
     pend_clip = cur.clip, pend_frame = cur.frame, pend_has_b = cur.has_b;
   }
   if (pend_frame >= 0) {
-    bar_wait(mel_done, (k + 1) & 1);
+    mbarrier_wait(mel_done, (k + 1) & 1);
     store_rows(pend_clip, pend_frame, pend_has_b, s_tiles);
   }
   pdl_epilogue(p);
@@ -759,18 +729,20 @@ logmel_power_kernel(FrontendTables tab, LogmelParams p) {
 // shared memory), spec_free (8 consumer arrivals: nobody reads the spectra of iteration k any more, the producers may
 // overwrite their tiles with the next transposition); the consumers meet at a named barrier between mel and store phase.
 constexpr int kWsProducers = kWarps;
-constexpr int ws_launch_regs(int consumers) { return (65536 / ((kWsProducers + consumers) * 32)) & ~7; }
+constexpr int kWsConsumers = 8;
+constexpr int kWsThreads = (kWsProducers + kWsConsumers) * 32;
+constexpr int kWsLaunchRegs = (65536 / kWsThreads) & ~7;
+constexpr int kWsProducerRegs = 96;
+constexpr int kWsConsumerRegs = 48;
+static_assert(kWsProducers * kWsProducerRegs + kWsConsumers * kWsConsumerRegs <=
+                  (kWsProducers + kWsConsumers) * kWsLaunchRegs,
+              "setmaxnreg redistributes the launch allocation");
+static_assert(kWarps % kWsConsumers == 0, "whole runs per consumer");
 
-// kVarlen: the packed variable-length batch (VarlenLocator); a separate instantiation, so that the batch kernel every other
-// caller runs stays exactly as it was
-template <int kWsConsumers, int kWsProducerRegs, int kWsConsumerRegs, bool kVarlen = false>
-__global__ void __launch_bounds__((kWsProducers + kWsConsumers) * 32, 1)
+// Locator: PairLocator (clips of one length) or VarlenLocator (the packed variable-length batch)
+template <class Locator>
+__global__ void __launch_bounds__(kWsThreads, 1)
 logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
-  constexpr int kWsThreads = (kWsProducers + kWsConsumers) * 32;
-  static_assert(kWsProducers * kWsProducerRegs + kWsConsumers * kWsConsumerRegs <=
-                    (kWsProducers + kWsConsumers) * ws_launch_regs(kWsConsumers),
-                "setmaxnreg redistributes the launch allocation");
-  static_assert(kWarps % kWsConsumers == 0, "whole runs per consumer");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* s_hann = reinterpret_cast<float*>(smem_raw);              // 1024
   float2* s_tw = reinterpret_cast<float2*>(s_hann + kFrameLen);    // 1024 float2
@@ -783,17 +755,17 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
   for (int i = tid; i < kFrameLen; i += kWsThreads) s_hann[i] = tab.hann[i];
   for (int i = tid; i < 1024; i += kWsThreads) s_tw[i] = tab.tw[i];
   for (int i = tid; i < 4 * kSlots * kTileStride; i += kWsThreads) s_tiles[i] = 0.0f;
-  const uint32_t spec_ready = smem_addr(s_bar), spec_free = smem_addr(s_bar + 1);
+  const uint32_t spec_ready = smem_u32addr(s_bar), spec_free = smem_u32addr(s_bar + 1);
   if (tid == 0) {
-    bar_init(spec_ready, kWsProducers);
-    bar_init(spec_free, kWsConsumers);
+    mbarrier_init(spec_ready, kWsProducers);
+    mbarrier_init(spec_free, kWsConsumers);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
   pdl_prologue_done(p);
 
   const unsigned ppc = (unsigned)(p.n_frames + 1) >> 1;
-  const unsigned total_pairs = kVarlen ? p.vl_pairs : (unsigned)p.n_clips * ppc;
+  const unsigned total_pairs = Locator::total_pairs(p);
   const unsigned n_iters = (total_pairs + kWarps - 1) / kWarps;
   const unsigned first = blockIdx.x, stride = gridDim.x;
   const unsigned n_local = first < n_iters ? (n_iters - first + stride - 1) / stride : 0;
@@ -801,7 +773,7 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
   if (warp < kWsProducers) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kWsProducerRegs));
     float* xb = s_scratch + warp * kScratch;
-    std::conditional_t<kVarlen, VarlenLocator, PairLocator> loc;
+    Locator loc;
     float2 v[32];
     PairInfo nxt = loc.locate(p, first, n_iters, total_pairs, ppc, warp);
     loc.load(p, nxt, lane, v);
@@ -809,11 +781,11 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
       const PairInfo cur = nxt;
       if (cur.frame >= 0) fft_first_half(v, s_hann, s_tw, lane);
       // the tile holds this warp's spectra of iteration k - 1 until every consumer has finished that mel phase
-      if (k > 0 && !(p.store_order & 0x200)) bar_wait(spec_free, (k + 1) & 1);  // (0x200: timing probe, results invalid)
+      if (k > 0) mbarrier_wait(spec_free, (k + 1) & 1);
       if (cur.frame >= 0) fft_second_half(v, xb, lane);
       if (lane == 0) s_pair[(k & 1) * kWarps + warp] = make_int4(cur.clip, cur.frame, cur.has_b ? 1 : 0, 0);
       __syncwarp();
-      if (lane == 0) bar_arrive(spec_ready);
+      if (lane == 0) mbarrier_arrive(spec_ready);
       // audio of the next iteration (an L2 prefetch of these lines one iteration ahead changed nothing: 146.7 vs 146.3 us)
       nxt = loc.locate(p, k + 1 < n_local ? first + (k + 1) * stride : n_iters, n_iters, total_pairs, ppc, warp);
       loc.load(p, nxt, lane, v);
@@ -833,7 +805,7 @@ logmel_power_ws_kernel(FrontendTables tab, LogmelParams p) {
           mel_phase_default(run, spec, tlo, thi);
       }
       __syncwarp();
-      if (lane == 0) bar_arrive(spec_free);
+      if (lane == 0) mbarrier_arrive(spec_free);
       asm volatile("bar.sync 1, %0;" ::"n"(kWsConsumers * 32) : "memory");  // every run of this iteration is in the tiles
 #pragma unroll 1
       for (int w = c * (kWarps / kWsConsumers); w < (c + 1) * (kWarps / kWsConsumers); ++w) {
@@ -863,6 +835,12 @@ constexpr size_t kLogmelWsSmem = sizeof(float) * kFrameLen + sizeof(float2) * 10
 constexpr size_t kLogmelSmem = sizeof(float) * kFrameLen + sizeof(float2) * 1024 + sizeof(float2) * kMaxBins +
                                sizeof(int4) * kMaxGroups + sizeof(int) * 32 +
                                sizeof(float) * (2 * kSlots * kTileStride + kWarps * kScratch) + 16;
+
+// The grid is one CTA per SM (launch_logmel): that is all either kernel's shared memory admits (228 KB per SM on sm_100,
+// 1 KB of it reserved per CTA).
+constexpr size_t kSmemPerSm = 228 * 1024, kSmemReservedPerCta = 1024;
+static_assert(2 * (kLogmelSmem + kSmemReservedPerCta) > kSmemPerSm, "logmel_power_kernel: more than one CTA per SM");
+static_assert(2 * (kLogmelWsSmem + kSmemReservedPerCta) > kSmemPerSm, "logmel_power_ws_kernel: more than one CTA per SM");
 
 // ---- dB normalisation: ref = clip max, clamp, rescale; emits long-term and last-3 short-term features
 __global__ void logmel_normalise_kernel(const float* __restrict__ power, const float* __restrict__ frame_max,
@@ -983,7 +961,6 @@ struct koe_frontend {
   int* d_tables = nullptr;  // groups[kMaxGroups] (int4) | runs[kWarps + 1 -> 32]
   int n_bins = 0, n_groups = 0;
   bool default_bank = false;  // structure == melbank_default.inc: the unrolled filterbank phase applies
-  int num_sms = 0, occupancy = 0;
   std::vector<float> fb_host;
 };
 
@@ -1158,31 +1135,11 @@ extern "C" int koe_frontend_create_ex(const koe_frontend_config* cfg, koe_fronte
   binw.resize(kMaxBins, make_float2(0.f, 0.f));
   up((void**)&fe->d_binw, binw.data(), binw.size() * sizeof(float2));
   up((void**)&fe->d_tables, tables.data(), tables.size() * sizeof(int));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(logmel_power_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelSmem);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(logmel_power_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelSmem);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(logmel_power_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelSmem);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(logmel_power_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelSmem);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(logmel_power_ws_kernel<8, 96, 48>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLogmelWsSmem);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(logmel_power_ws_kernel<8, 96, 48, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)kLogmelWsSmem);
-  cudaDeviceProp prop;
-  if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, device);
-  if (e == cudaSuccess) {
-    fe->num_sms = prop.multiProcessorCount;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fe->occupancy, logmel_power_kernel<true>, kThreads, kLogmelSmem);
-  }
   cudaSetDevice(prev);
   if (e != cudaSuccess) {
     koe_frontend_destroy(fe);
     return fail((int)e, "koe_frontend_create: %s", cudaGetErrorString(e));
   }
-  if (fe->occupancy < 1) fe->occupancy = 1;
   *out = fe;
   return KOE_OK;
 }
@@ -1205,179 +1162,170 @@ extern "C" int koe_frontend_filterbank_host(const koe_frontend_t* fe, float* fb_
   return KOE_OK;
 }
 
-// experiment switch of the log-mel kernel (scripts/k1_variants.py): placement of the store phase per warp class
-static int g_k1_store_order = 0x44;  // classes 0, 2: before the FFT; classes 1, 3: after the next pair's loads
-static int g_k1_warp_specialised = 1;
-extern "C" int koe_debug_k1_variant(int store_order, int warp_specialised) {
-  g_k1_store_order = store_order;
-  g_k1_warp_specialised = warp_specialised;
+extern "C" int koe_logmel_power_ex(const koe_frontend_t* fe, const koe_logmel_args* a, void* stream) {
+  const FrontendMode mode = a != nullptr && a->power_b != nullptr ? FrontendMode::SplitPairs : FrontendMode::Frames;
+  return koe::launch_logmel(fe, a, mode, /*follows_frontend_launch=*/false, stream);
+}
+
+namespace koe {
+namespace {
+// sets the shared-memory size of the instantiation once per device, then launches it behind the previous kernel
+template <void (*Kernel)(FrontendTables, LogmelParams)>
+int launch_instantiation(const FrontendTables& tab, const LogmelParams& p, int grid, int threads, size_t smem,
+                         cudaStream_t stream) {
+  static bool configured[64] = {false};
+  int dev = 0;
+  KOE_CUDA(cudaGetDevice(&dev));
+  KOE_REQUIRE(dev >= 0 && dev < 64, "device index too large");
+  if (!configured[dev]) {
+    KOE_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    configured[dev] = true;
+  }
+  const cudaError_t e = launch_after_primary_starts(Kernel, dim3(grid), dim3(threads), smem, stream, tab, p);
+  count_launch();
+  KOE_CUDA(e);
   return KOE_OK;
 }
 
-extern "C" int koe_logmel_power_ex(const koe_frontend_t* fe, const koe_logmel_args* a, void* stream) {
-  return koe::launch_logmel(fe, a, stream, /*follows_frontend_launch=*/false, 0, nullptr, nullptr);
+// the instantiation of each (mode, bank): the warp-specialised kernel where it exists, the lock-step one elsewhere
+int launch_power(FrontendMode mode, bool default_bank, const FrontendTables& tab, const LogmelParams& p, int grid,
+                 cudaStream_t stream) {
+  switch (mode) {
+    case FrontendMode::Frames:
+      if (default_bank)
+        return launch_instantiation<logmel_power_ws_kernel<PairLocator>>(tab, p, grid, kWsThreads, kLogmelWsSmem, stream);
+      return launch_instantiation<logmel_power_kernel<false, false>>(tab, p, grid, kThreads, kLogmelSmem, stream);
+    case FrontendMode::SplitPairs:
+      if (default_bank)
+        return launch_instantiation<logmel_power_kernel<true, true>>(tab, p, grid, kThreads, kLogmelSmem, stream);
+      return launch_instantiation<logmel_power_kernel<false, true>>(tab, p, grid, kThreads, kLogmelSmem, stream);
+    case FrontendMode::Varlen:
+      if (default_bank)
+        return launch_instantiation<logmel_power_ws_kernel<VarlenLocator>>(tab, p, grid, kWsThreads, kLogmelWsSmem, stream);
+      return fail(KOE_E_UNSUPPORTED, "packed variable-length batches are implemented for the default filterbank only");
+  }
+  return fail(KOE_E_INVALID, "koe_logmel_power: unknown frontend mode %d", (int)mode);
 }
+
+// the frontend's tables, and the launch parameters every mode takes from the arguments
+void launch_setup(const koe_frontend_t* fe, const koe_logmel_args* a, bool follows_frontend_launch, FrontendTables* tab,
+                  LogmelParams* p) {
+  tab->hann = fe->d_hann;
+  tab->tw = fe->d_tw;
+  tab->binw = fe->d_binw;
+  tab->groups = reinterpret_cast<const int4*>(fe->d_tables);
+  tab->runs = fe->d_tables + 4 * kMaxGroups;
+  tab->n_bins = fe->n_bins;
+  tab->n_groups = fe->n_groups;
+  tab->log_mode = fe->log_mode;
+  tab->log_eps = fe->log_eps;
+  *p = LogmelParams{};
+  p->audio = a->audio;
+  p->audio_stride = a->audio_stride;
+  p->n_clips = a->n_clips;
+  p->n_samples = a->n_samples;
+  p->hop = a->hop;
+  p->n_frames = a->n_frames;
+  p->lo_rel = a->lo_rel_hops;
+  p->hi_rel = a->hi_rel_hops;
+  p->frame_offset = a->frame_offset;
+  p->frame_step = a->frame_step;
+  p->sample_offset = a->sample_offset;
+  p->pad_mode = a->pad_mode;
+  p->power = a->power;
+  p->frame_max = a->frame_max;
+  p->power_clip_stride = a->power_clip_stride;
+  p->fmax_clip_stride = a->frame_max_clip_stride;
+  p->power_b = a->power_b;
+  p->power_b_clip_stride = a->power_b_clip_stride;
+  p->frame_max_b = a->frame_max_b;
+  p->fmax_b_clip_stride = a->frame_max_b_clip_stride;
+  p->wait_at_end = follows_frontend_launch ? 1 : 0;
+}
+}  // namespace
+}  // namespace koe
 
 // `follows_frontend_launch`: the kernel queued just before this one on `stream` is another frontend launch of the same
 // forward, writing other buffers (see pdl_prologue_done in the kernels)
-int koe::launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* a, void* stream, bool follows_frontend_launch,
-                       int early_clips, unsigned* early_flag, unsigned* early_target) {
-  KOE_REQUIRE(fe != nullptr && a != nullptr, "koe_logmel_power: NULL argument");
-  KOE_REQUIRE(a->n_clips >= 0 && a->n_samples >= 0 && a->n_frames >= 0, "koe_logmel_power: negative size");
-  if (a->n_clips == 0 || a->n_frames == 0) return KOE_OK;  // nothing to do: empty buffers may be NULL
-  KOE_REQUIRE(a->audio != nullptr && a->power != nullptr, "koe_logmel_power: NULL buffer");
-  KOE_REQUIRE(a->hop > 0 && a->audio_stride >= a->n_samples, "koe_logmel_power: bad hop/stride");
-  KOE_REQUIRE(a->frame_offset >= 0 && a->frame_step >= 1 && a->sample_offset >= 0,
-              "koe_logmel_power: bad frame_offset/frame_step/sample_offset");
-  KOE_REQUIRE((long long)a->sample_offset +
-                      ((long long)a->frame_offset + (long long)(a->n_frames + 1) * a->frame_step + KOE_MAX_EDGE + 1) *
-                          a->hop < (1ll << 31) && a->n_samples < (1 << 30),
-              "koe_logmel_power: clip too long for 32-bit sample indices");
-  KOE_REQUIRE(a->pad_mode == 0 || a->pad_mode == 1, "koe_logmel_power: pad_mode must be 0 (constant) or 1 (reflect)");
-  KOE_REQUIRE(a->pad_mode == 0 || (a->lo_rel_hops == KOE_NO_EDGE && a->hi_rel_hops == KOE_NO_EDGE &&
-                                   a->n_samples > KOE_N_FFT / 2),
-              "koe_logmel_power: reflect padding needs n_samples > n_fft/2 and no window edges");
-  KOE_REQUIRE(a->power_clip_stride >= (int64_t)a->n_frames * KOE_N_MELS && a->power_clip_stride % 4 == 0,
-              "koe_logmel_power: bad power_clip_stride");
-  KOE_REQUIRE(a->frame_max == nullptr || a->frame_max_clip_stride >= a->n_frames,
-              "koe_logmel_power: bad frame_max_clip_stride");
-  if (a->n_clips == 0 || a->n_frames == 0) return KOE_OK;
-  FrontendTables tab;
-  tab.hann = fe->d_hann;
-  tab.tw = fe->d_tw;
-  tab.binw = fe->d_binw;
-  tab.groups = reinterpret_cast<const int4*>(fe->d_tables);
-  tab.runs = fe->d_tables + 4 * kMaxGroups;
-  tab.n_bins = fe->n_bins;
-  tab.n_groups = fe->n_groups;
-  tab.log_mode = fe->log_mode;
-  tab.log_eps = fe->log_eps;
-  LogmelParams p;
-  p.audio = a->audio;
-  p.audio_stride = a->audio_stride;
-  p.n_clips = a->n_clips;
-  p.n_samples = a->n_samples;
-  p.hop = a->hop;
-  p.n_frames = a->n_frames;
-  p.lo_rel = a->lo_rel_hops;
-  p.hi_rel = a->hi_rel_hops;
-  p.frame_offset = a->frame_offset;
-  p.frame_step = a->frame_step;
-  p.sample_offset = a->sample_offset;
-  p.pad_mode = a->pad_mode;
-  p.power = a->power;
-  p.frame_max = a->frame_max;
-  p.power_clip_stride = a->power_clip_stride;
-  p.fmax_clip_stride = a->frame_max_clip_stride;
-  p.power_b = a->power_b;
-  p.power_b_clip_stride = a->power_b_clip_stride;
-  p.frame_max_b = a->frame_max_b;
-  p.fmax_b_clip_stride = a->frame_max_b_clip_stride;
-  KOE_REQUIRE(a->power_b == nullptr || (a->frame_max == nullptr) == (a->frame_max_b == nullptr),
-              "koe_logmel_power_ex: power_b needs frame_max_b whenever frame_max is given");
-  {
-    const int ppc = (p.n_frames + 1) / 2;
-    p.edge_lo = 0;
-    while (p.edge_lo < ppc && !pair_geometry(p, 0, p.edge_lo).interior) ++p.edge_lo;
-    p.edge_hi = 0;
-    while (p.edge_lo + p.edge_hi < ppc && !pair_geometry(p, 0, ppc - 1 - p.edge_hi).interior) ++p.edge_hi;
+int koe::launch_logmel(const koe_frontend_t* fe, const koe_logmel_args* a, FrontendMode mode, bool follows_frontend_launch,
+                       void* stream, EarlyRelease* early, const VarlenTables* vl) {
+  if (early != nullptr) early->target = 0;
+  long long pairs = 0;
+  if (mode == FrontendMode::Varlen) {
+    KOE_REQUIRE(fe != nullptr && a != nullptr && vl != nullptr, "koe_logmel_power (varlen): NULL argument");
+    if (vl->n_clips == 0 || vl->pairs == 0) return KOE_OK;
+    KOE_REQUIRE(a->audio != nullptr && a->power != nullptr && a->frame_max != nullptr && vl->sample_off && vl->length &&
+                    vl->pair_base && vl->row_base,
+                "koe_logmel_power (varlen): NULL buffer");
+    KOE_REQUIRE(a->hop > 0 && a->frame_offset >= 0 && a->frame_step >= 1, "koe_logmel_power (varlen): bad geometry");
+    pairs = vl->pairs;
+  } else {
+    KOE_REQUIRE(fe != nullptr && a != nullptr, "koe_logmel_power: NULL argument");
+    KOE_REQUIRE(a->n_clips >= 0 && a->n_samples >= 0 && a->n_frames >= 0, "koe_logmel_power: negative size");
+    if (a->n_clips == 0 || a->n_frames == 0) return KOE_OK;  // nothing to do: empty buffers may be NULL
+    KOE_REQUIRE(a->audio != nullptr && a->power != nullptr, "koe_logmel_power: NULL buffer");
+    KOE_REQUIRE(a->hop > 0 && a->audio_stride >= a->n_samples, "koe_logmel_power: bad hop/stride");
+    KOE_REQUIRE(a->frame_offset >= 0 && a->frame_step >= 1 && a->sample_offset >= 0,
+                "koe_logmel_power: bad frame_offset/frame_step/sample_offset");
+    KOE_REQUIRE((long long)a->sample_offset +
+                        ((long long)a->frame_offset + (long long)(a->n_frames + 1) * a->frame_step + KOE_MAX_EDGE + 1) *
+                            a->hop < (1ll << 31) && a->n_samples < (1 << 30),
+                "koe_logmel_power: clip too long for 32-bit sample indices");
+    KOE_REQUIRE(a->pad_mode == 0 || a->pad_mode == 1, "koe_logmel_power: pad_mode must be 0 (constant) or 1 (reflect)");
+    KOE_REQUIRE(a->pad_mode == 0 || (a->lo_rel_hops == KOE_NO_EDGE && a->hi_rel_hops == KOE_NO_EDGE &&
+                                     a->n_samples > KOE_N_FFT / 2),
+                "koe_logmel_power: reflect padding needs n_samples > n_fft/2 and no window edges");
+    KOE_REQUIRE(a->power_clip_stride >= (int64_t)a->n_frames * KOE_N_MELS && a->power_clip_stride % 4 == 0,
+                "koe_logmel_power: bad power_clip_stride");
+    KOE_REQUIRE(a->frame_max == nullptr || a->frame_max_clip_stride >= a->n_frames,
+                "koe_logmel_power: bad frame_max_clip_stride");
+    KOE_REQUIRE(a->power_b == nullptr || (a->frame_max == nullptr) == (a->frame_max_b == nullptr),
+                "koe_logmel_power_ex: power_b needs frame_max_b whenever frame_max is given");
+    pairs = (long long)a->n_clips * ((a->n_frames + 1) / 2);
   }
-  const long long ppc = (a->n_frames + 1) / 2;
-  KOE_REQUIRE((long long)a->n_clips * ppc < (1ll << 31) - kWarps, "koe_logmel_power: more than 2^31 frame pairs in one call");
-  const long long n_blocks = ((long long)a->n_clips * ppc + kWarps - 1) / kWarps;
-  const long long max_grid = (long long)fe->num_sms * fe->occupancy;
-  const int grid = (int)std::min(n_blocks, max_grid);
-  p.store_order = g_k1_store_order;
-  p.wait_at_end = follows_frontend_launch ? 1 : 0;
-  p.early_flag = nullptr, p.early_iters = 0;
-  p.mid_pairs = 0, p.step_clips = 0, p.step_pairs = 0;
-  if (p.edge_lo + p.edge_hi > 0 && p.edge_lo + p.edge_hi < (int)ppc) {
-    p.mid_pairs = (int)ppc - p.edge_lo - p.edge_hi;
+  KOE_REQUIRE(pairs < (1ll << 31) - kWarps, "koe_logmel_power: more than 2^31 frame pairs in one call");
+  FrontendTables tab;
+  LogmelParams p;
+  launch_setup(fe, a, follows_frontend_launch, &tab, &p);
+  int sms = 0;
+  KOE_CUDA(sm_count(&sms));
+  const long long n_blocks = (pairs + kWarps - 1) / kWarps;
+  const int grid = (int)std::min<long long>(n_blocks, sms);
+  if (mode == FrontendMode::Varlen) {
+    p.vl_sample_off = vl->sample_off;
+    p.vl_length = vl->length;
+    p.vl_pair_base = vl->pair_base;
+    p.vl_row_base = vl->row_base;
+    p.vl_clips = vl->n_clips;
+    p.vl_pairs = (unsigned)pairs;
+    return launch_power(mode, fe->default_bank, tab, p, grid, (cudaStream_t)stream);
+  }
+  const int ppc = (p.n_frames + 1) / 2;
+  while (p.edge_lo < ppc && !pair_geometry(p, 0, p.edge_lo).interior) ++p.edge_lo;
+  while (p.edge_lo + p.edge_hi < ppc && !pair_geometry(p, 0, ppc - 1 - p.edge_hi).interior) ++p.edge_hi;
+  if (p.edge_lo + p.edge_hi > 0 && p.edge_lo + p.edge_hi < ppc) {
+    p.mid_pairs = ppc - p.edge_lo - p.edge_hi;
     const long long step = (long long)grid * kWarps;
     p.step_clips = (int)(step / p.mid_pairs);
     p.step_pairs = (int)(step % p.mid_pairs);
   }
-  // Early release of the core: the clips [0, early_clips) are complete once every pair ahead of clip `early_clips` in the
-  // launch order is stored -- all edge pairs (they come first) and the interior pairs of those clips -- i.e. once every
-  // CTA has finished its iterations below early_iters.  Only the warp-specialised kernel signals; every CTA must own an
-  // iteration below the threshold and one at or above it.
-  if (early_target != nullptr) *early_target = 0;
-  if (early_flag != nullptr && early_clips > 0 && early_clips < a->n_clips && p.power_b == nullptr && fe->default_bank &&
-      g_k1_warp_specialised == 1) {
-    const long long before = p.mid_pairs > 0 ? (long long)a->n_clips * (p.edge_lo + p.edge_hi) + (long long)early_clips * p.mid_pairs
-                                             : (long long)early_clips * ppc;
+  // Early release of the core: the clips [0, early->clips) are complete once every pair ahead of clip `early->clips` in
+  // the launch order is stored -- all edge pairs (they come first) and the interior pairs of those clips -- i.e. once
+  // every CTA has finished its iterations below early_iters.  Only the warp-specialised kernel signals; every CTA must own
+  // an iteration below the threshold and one at or above it.
+  if (early != nullptr && early->flag != nullptr && early->clips > 0 && early->clips < a->n_clips &&
+      mode == FrontendMode::Frames && fe->default_bank) {
+    const long long before = p.mid_pairs > 0
+                                 ? (long long)a->n_clips * (p.edge_lo + p.edge_hi) + (long long)early->clips * p.mid_pairs
+                                 : (long long)early->clips * ppc;
     const long long iters = (before + kWarps - 1) / kWarps;
     if (iters >= grid && iters + grid <= n_blocks) {
-      p.early_flag = early_flag;
+      p.early_flag = early->flag;
       p.early_iters = (unsigned)iters;
-      *early_target = (unsigned)grid * 8u;  // consumer warps per CTA (logmel_power_ws_kernel<8, ...>)
+      early->target = (unsigned)grid * kWsConsumers;  // one arrival per consumer warp
     }
   }
-  cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t le;
-  if (p.power_b != nullptr) {
-    if (fe->default_bank)
-      le = launch_after_primary_starts(logmel_power_kernel<true, true>, dim3(grid), dim3(kThreads), kLogmelSmem, st, tab, p);
-    else
-      le = launch_after_primary_starts(logmel_power_kernel<false, true>, dim3(grid), dim3(kThreads), kLogmelSmem, st, tab, p);
-  } else if (fe->default_bank && g_k1_warp_specialised == 1)
-    le = launch_after_primary_starts(logmel_power_ws_kernel<8, 96, 48>, dim3(grid), dim3((kWsProducers + 8) * 32), kLogmelWsSmem,
-                                     st, tab, p);
-  else if (fe->default_bank)
-    le = launch_after_primary_starts(logmel_power_kernel<true>, dim3(grid), dim3(kThreads), kLogmelSmem, st, tab, p);
-  else
-    le = launch_after_primary_starts(logmel_power_kernel<false>, dim3(grid), dim3(kThreads), kLogmelSmem, st, tab, p);
-  count_launch();
-  KOE_CUDA(le);
-  return KOE_OK;
-}
-
-int koe::launch_logmel_varlen(const koe_frontend_t* fe, const koe_logmel_args* a, const long long* sample_off,
-                              const int* length, const int* pair_base, const int* row_base, int n_clips, long long total_pairs,
-                              void* stream, bool follows_frontend_launch) {
-  KOE_REQUIRE(fe != nullptr && a != nullptr, "koe_logmel_power (varlen): NULL argument");
-  if (n_clips == 0 || total_pairs == 0) return KOE_OK;
-  if (!fe->default_bank)
-    return fail(KOE_E_UNSUPPORTED, "packed variable-length batches are implemented for the default filterbank only");
-  KOE_REQUIRE(a->audio != nullptr && a->power != nullptr && a->frame_max != nullptr && sample_off && length && pair_base &&
-                  row_base,
-              "koe_logmel_power (varlen): NULL buffer");
-  KOE_REQUIRE(a->hop > 0 && a->frame_offset >= 0 && a->frame_step >= 1, "koe_logmel_power (varlen): bad geometry");
-  KOE_REQUIRE(total_pairs < (1ll << 31) - kWarps, "koe_logmel_power (varlen): more than 2^31 frame pairs in one call");
-  FrontendTables tab;
-  tab.hann = fe->d_hann;
-  tab.tw = fe->d_tw;
-  tab.binw = fe->d_binw;
-  tab.groups = reinterpret_cast<const int4*>(fe->d_tables);
-  tab.runs = fe->d_tables + 4 * kMaxGroups;
-  tab.n_bins = fe->n_bins;
-  tab.n_groups = fe->n_groups;
-  tab.log_mode = fe->log_mode;
-  tab.log_eps = fe->log_eps;
-  LogmelParams p = {};
-  p.audio = a->audio;
-  p.hop = a->hop;
-  p.lo_rel = a->lo_rel_hops;
-  p.hi_rel = a->hi_rel_hops;
-  p.frame_offset = a->frame_offset;
-  p.frame_step = a->frame_step;
-  p.power = a->power;
-  p.frame_max = a->frame_max;
-  p.store_order = g_k1_store_order;
-  p.wait_at_end = follows_frontend_launch ? 1 : 0;
-  p.vl_sample_off = sample_off;
-  p.vl_length = length;
-  p.vl_pair_base = pair_base;
-  p.vl_row_base = row_base;
-  p.vl_clips = n_clips;
-  p.vl_pairs = (unsigned)total_pairs;
-  const long long n_blocks = (total_pairs + kWarps - 1) / kWarps;
-  const int grid = (int)std::min(n_blocks, (long long)fe->num_sms * fe->occupancy);
-  const cudaError_t le = launch_after_primary_starts(logmel_power_ws_kernel<8, 96, 48, true>, dim3(grid),
-                                                     dim3((kWsProducers + 8) * 32), kLogmelWsSmem, (cudaStream_t)stream, tab, p);
-  count_launch();
-  KOE_CUDA(le);
-  return KOE_OK;
+  return launch_power(mode, fe->default_bank, tab, p, grid, (cudaStream_t)stream);
 }
 
 extern "C" int koe_logmel_power(const koe_frontend_t* fe, const float* audio, int64_t audio_stride, int n_clips,

@@ -32,6 +32,52 @@ __global__ void __launch_bounds__(256) stream_tail_shift_kernel(const float* __r
   }
 }
 
+// The tail ends at sample (n + 1) * hop.  The newest frame whose samples are all there is global frame g = n - lag,
+// lag = n_edge - 1, centred `half` samples into the tail; the frames centred one hop further each are the window-end
+// variants of the window that ends now: beyond the end of the tail the clip reads as zeros, which is exactly their mask.
+int launch_hop_frontend(const koe_frontend_t* fe, const float* tail, int n_streams, int tail_len, int half, int hop,
+                        int n_edge, const MelRows* rows, void* stream) {
+  koe_logmel_args f = {};
+  f.audio = tail;
+  f.audio_stride = tail_len;
+  f.n_clips = n_streams;
+  f.n_samples = tail_len;
+  f.hop = hop;
+  f.frame_offset = 0;
+  f.frame_step = 1;
+  f.pad_mode = 0;
+  f.sample_offset = half;
+  f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = KOE_NO_EDGE;
+  auto to = [&f](const MelRows& r) {
+    f.power = r.power, f.power_clip_stride = r.power_stride;
+    f.frame_max = r.frame_max, f.frame_max_clip_stride = r.fmax_stride;
+  };
+  // plain frame g and the frame one hop later as ONE pair of one launch: at 30 fps that second frame is the window-end
+  // variant L0 (centred on the tail's end), at 60 fps the last-but-one frame of the window (L1)
+  const MelRows& second = rows[n_edge == 1 ? 2 : 4];
+  f.n_frames = 2;
+  to(rows[0]);
+  f.power_b = second.power, f.power_b_clip_stride = second.power_stride;
+  f.frame_max_b = second.frame_max, f.frame_max_b_clip_stride = second.fmax_stride;
+  if (int rc = launch_logmel(fe, &f, FrontendMode::SplitPairs, /*follows_frontend_launch=*/false, stream)) return rc;
+  f.power_b = nullptr, f.frame_max_b = nullptr;
+  f.n_frames = 1;
+  if (n_edge == 2) {  // the frame centred on the tail's end: the window's last frame
+    f.frame_offset = 2;
+    to(rows[2]);
+    if (int rc = launch_logmel(fe, &f, FrontendMode::Frames, /*follows_frontend_launch=*/false, stream)) return rc;
+    f.frame_offset = 0;
+  }
+  // window-start variants of frame g: nothing before its centre (first frame of the window that starts at g), and at
+  // 60 fps nothing before the centre of frame g - 1 (second frame of the window that starts at g - 1)
+  for (int m = 0; m < n_edge; ++m) {
+    f.lo_rel_hops = -m;
+    to(rows[1 + 2 * m]);
+    if (int rc = launch_logmel(fe, &f, FrontendMode::Frames, /*follows_frontend_launch=*/false, stream)) return rc;
+  }
+  return KOE_OK;
+}
+
 }  // namespace koe
 
 using namespace koe;
@@ -65,54 +111,22 @@ extern "C" int koe_stream_push(const koe_stream_args* a, int* emitted, void* str
     count_launch();
     KOE_CUDA(cudaGetLastError());
   }
-  // The tail ends at sample (n + 1) * hop.  The newest frame whose samples are all there is global frame g = n - lag,
-  // lag = n_edge - 1, centred `half` samples into the tail; the frames centred one hop further each are the window-end
-  // variants of the window that ends now: beyond the end of the tail the clip reads as zeros, which is exactly their mask.
-  const int lag = n_edge - 1;
-  const int64_t g = n - lag;
-  koe_logmel_args f = {};
-  f.audio = tail;
-  f.audio_stride = tail_len;
-  f.n_clips = S;
-  f.n_samples = tail_len;
-  f.hop = hop;
-  f.frame_offset = 0;
-  f.frame_step = 1;
-  f.pad_mode = 0;
-  f.sample_offset = half;
-  f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = KOE_NO_EDGE;
-  f.power_clip_stride = (int64_t)W * KOE_N_MELS, f.frame_max_clip_stride = W;
-  f.power_b_clip_stride = KOE_N_MELS, f.frame_max_b_clip_stride = 1;
+  // frame g = n - (n_edge - 1) goes to ring slot g mod W (plain and window-start variants), the window-end variants to the
+  // stream's own row
+  const int64_t g = n - (n_edge - 1);
   const int slot = (int)(((g % W) + W) % W);
-  // plain frame g (-> ring slot) and the frame one hop later as ONE pair of one launch: at 30 fps that second frame is the
-  // window-end variant L (centred on the tail's end), at 60 fps the last-but-one frame of the window (row_l2)
-  f.n_frames = 2;
-  f.power = a->ring_f + (size_t)slot * KOE_N_MELS, f.frame_max = a->fmax_f + slot;
-  f.power_b = n_edge == 1 ? a->row_l : a->row_l2, f.frame_max_b = n_edge == 1 ? a->fmax_l : a->fmax_l2;
-  if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
-  f.power_b = nullptr, f.frame_max_b = nullptr;
-  if (n_edge == 2) {  // the frame centred on the tail's end: the window's last frame
-    f.n_frames = 1;
-    f.frame_offset = 2;
-    f.power = a->row_l, f.power_clip_stride = KOE_N_MELS;
-    f.frame_max = a->fmax_l, f.frame_max_clip_stride = 1;
-    if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
-    f.frame_offset = 0;
-    f.power_clip_stride = (int64_t)W * KOE_N_MELS, f.frame_max_clip_stride = W;
+  float* const power[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, a->row_l, a->ring_r2, a->row_l2};
+  float* const fmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, a->fmax_l, a->fmax_r2, a->fmax_l2};
+  MelRows rows[1 + 2 * KOE_MAX_EDGE] = {};
+  for (int v = 0; v < 1 + 2 * n_edge; ++v) {
+    if (v > 0 && v % 2 == 0)
+      rows[v] = {power[v], fmax[v], KOE_N_MELS, 1};
+    else
+      rows[v] = {power[v] + (size_t)slot * KOE_N_MELS, fmax[v] + slot, (int64_t)W * KOE_N_MELS, W};
   }
-  // window-start variants of frame g: nothing before its centre (first frame of the window that starts at g), and at
-  // 60 fps nothing before the centre of frame g - 1 (second frame of the window that starts at g - 1)
-  f.n_frames = 1;
-  for (int m = 0; m < n_edge; ++m) {
-    f.lo_rel_hops = -m;
-    f.power = (m == 0 ? a->ring_r : a->ring_r2) + (size_t)slot * KOE_N_MELS;
-    f.frame_max = (m == 0 ? a->fmax_r : a->fmax_r2) + slot;
-    if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
-  }
+  if (int rc = launch_hop_frontend(a->frontend, tail, S, tail_len, half, hop, n_edge, rows, stream)) return rc;
   if (n + 1 < W) return KOE_OK;  // the context is not full yet
   const int base = (int)((n + 1 - W) % W);  // ring slot of the first frame of the window that ends now
-  const float* power[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, a->row_l, a->ring_r2, a->row_l2};
-  const float* fmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, a->fmax_l, a->fmax_r2, a->fmax_l2};
   if (int rc = koe_dual_stream_ring_edges(a->weights, power, fmax, n_edge, S, W, base, W + 1, a->expr_sigmoid, a->out,
                                           nullptr, nullptr, a->precision, stream))
     return rc;
@@ -191,20 +205,18 @@ extern "C" int koe_forward_windows(const koe_forward_args* a, void* stream) {
   f.frame_max = a->frame_max[0], f.frame_max_clip_stride = a->n_frames;
   // early release of the core (above): one window per clip, tensor-core core, no attention output, more than one round
   static const bool early_off = getenv("KOE_NO_EARLY_CORE") != nullptr;  // experiment switch
-  unsigned* early_flag = nullptr;
-  unsigned early_target = 0;
-  int early_clips = 0;
+  EarlyRelease early = {0, nullptr, 0};
   if (!early_off && a->n_out == 1 && a->n_edge == 0 && a->precision == 2 && a->attn_out == nullptr &&
       (a->weights->k_mel == 259 || a->weights->k_mel == 515)) {
     const int G = dual_stream_tc_grid(a->n_clips);
     if (G > 0 && a->n_clips > G) {
-      early_clips = G * ((a->n_clips - 1) / G);
-      early_flag = g_early.get(stream);
+      early.clips = G * ((a->n_clips - 1) / G);
+      early.flag = g_early.get(stream);
     }
   }
-  if (int rc = launch_logmel(a->frontend, &f, stream, /*follows_frontend_launch=*/false, early_clips, early_flag, &early_target))
+  if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Frames, /*follows_frontend_launch=*/false, stream, &early))
     return rc;
-  if (early_target == 0) early_flag = nullptr;
+  unsigned* const early_flag = early.target != 0 ? early.flag : nullptr;
   bool early_applied = false;
   // the frames within n_fft/2 of a window edge, once per window (SURVEY.md section 8 note E)
   for (int m = 0; m < a->n_edge; ++m) {
@@ -216,10 +228,10 @@ extern "C" int koe_forward_windows(const koe_forward_args* a, void* stream) {
     // (these launches follow a frontend launch of this forward and touch none of its buffers: they do not wait for it)
     f.frame_offset = m, f.lo_rel_hops = -m, f.hi_rel_hops = KOE_NO_EDGE;
     f.power = a->power[1 + 2 * m], f.frame_max = a->frame_max[1 + 2 * m];
-    if (int rc = launch_logmel(a->frontend, &f, stream, /*follows_frontend_launch=*/true, 0, nullptr, nullptr)) return rc;
+    if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Frames, /*follows_frontend_launch=*/true, stream)) return rc;
     f.frame_offset = a->frames_per_window - 1 - m, f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = m;
     f.power = a->power[2 + 2 * m], f.frame_max = a->frame_max[2 + 2 * m];
-    if (int rc = launch_logmel(a->frontend, &f, stream, /*follows_frontend_launch=*/true, 0, nullptr, nullptr)) return rc;
+    if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Frames, /*follows_frontend_launch=*/true, stream)) return rc;
   }
   // The mouth entries of every output row come from the mel stream (the core) and the expression entries from the emotion
   // stream alone, so the two kernels do not depend on each other's results: the emotion kernel writes its entries of `out`
@@ -233,7 +245,7 @@ extern "C" int koe_forward_windows(const koe_forward_args* a, void* stream) {
   if (int rc = launch_dual_stream_windows(a->weights, a->power, a->frame_max, a->n_edge, a->n_clips, a->n_frames, a->n_out,
                                           a->stride_frames, a->frames_per_window, nullptr, a->out, a->sigmoid_out,
                                           a->attn_out, a->precision, stream, /*expr_by_emotion_kernel=*/true, early_flag,
-                                          early_target, early_clips, &early_applied)) {
+                                          early.target, early.clips, &early_applied)) {
     if (early_flag != nullptr) cudaMemsetAsync(early_flag, 0, 2 * sizeof(unsigned), (cudaStream_t)stream);  // frontend counted, nobody clears
     return rc;
   }
@@ -385,19 +397,22 @@ extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream
   f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = KOE_NO_EDGE;
   f.power = power[0], f.frame_max = fmax[0];
   // every clip's global frames, then the frames within n_fft/2 of a window edge once per window of the clips that use them
-  if (int rc = launch_logmel_varlen(a->frontend, &f, sample_off, length, pair_base, frame_base, B, pl.pairs, stream, false))
+  const VarlenTables frames = {sample_off, length, pair_base, frame_base, B, pl.pairs};
+  const VarlenTables edges = {sample_off, length, edge_pair_base, window_base, B, pl.edge_pairs};
+  if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Varlen, /*follows_frontend_launch=*/false, stream, nullptr,
+                             &frames))
     return rc;
   for (int m = 0; m < pl.n_edge; ++m) {
     f.frame_step = a->stride_frames;
     f.frame_offset = m, f.lo_rel_hops = -m, f.hi_rel_hops = KOE_NO_EDGE;
     f.power = power[1 + 2 * m], f.frame_max = fmax[1 + 2 * m];
-    if (int rc = launch_logmel_varlen(a->frontend, &f, sample_off, length, edge_pair_base, window_base, B, pl.edge_pairs,
-                                      stream, true))
+    if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Varlen, /*follows_frontend_launch=*/true, stream, nullptr,
+                               &edges))
       return rc;
     f.frame_offset = T - 1 - m, f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = m;
     f.power = power[2 + 2 * m], f.frame_max = fmax[2 + 2 * m];
-    if (int rc = launch_logmel_varlen(a->frontend, &f, sample_off, length, edge_pair_base, window_base, B, pl.edge_pairs,
-                                      stream, true))
+    if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Varlen, /*follows_frontend_launch=*/true, stream, nullptr,
+                               &edges))
       return rc;
   }
   // as in koe_forward_windows: the emotion kernel writes the expression entries of each clip's rows, the core the rest

@@ -256,40 +256,9 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
     KOE_CUDA(cudaGetLastError());
   }
   // ---- 2. the frontend launches of koe_stream_push, on the compact tails, into staging rows [n][V][80]
-  float* stage[1 + 2 * KOE_MAX_EDGE];
-  float* stage_max[1 + 2 * KOE_MAX_EDGE];
-  for (int v = 0; v < V; ++v) stage[v] = a->stage + (size_t)v * KOE_N_MELS, stage_max[v] = a->stage_max + v;
-  koe_logmel_args f = {};
-  f.audio = a->tail_compact;
-  f.audio_stride = tail_len;
-  f.n_clips = n;
-  f.n_samples = tail_len;
-  f.hop = hop;
-  f.frame_offset = 0;
-  f.frame_step = 1;
-  f.pad_mode = 0;
-  f.sample_offset = half;
-  f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = KOE_NO_EDGE;
-  f.power_clip_stride = (int64_t)V * KOE_N_MELS, f.frame_max_clip_stride = V;
-  f.power_b_clip_stride = (int64_t)V * KOE_N_MELS, f.frame_max_b_clip_stride = V;
-  // plain frame g and the frame one hop later (30 fps: the window-end row; 60 fps: the last-but-one frame of the window)
-  f.n_frames = 2;
-  f.power = stage[0], f.frame_max = stage_max[0];
-  f.power_b = n_edge == 1 ? stage[2] : stage[4], f.frame_max_b = n_edge == 1 ? stage_max[2] : stage_max[4];
-  if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
-  f.power_b = nullptr, f.frame_max_b = nullptr;
-  f.n_frames = 1;
-  if (n_edge == 2) {  // the frame centred on the tail's end: the window's last frame
-    f.frame_offset = 2;
-    f.power = stage[2], f.frame_max = stage_max[2];
-    if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
-    f.frame_offset = 0;
-  }
-  for (int m = 0; m < n_edge; ++m) {  // window-start variants of frame g
-    f.lo_rel_hops = -m;
-    f.power = stage[1 + 2 * m], f.frame_max = stage_max[1 + 2 * m];
-    if (int rc = koe_logmel_power_ex(a->frontend, &f, stream)) return rc;
-  }
+  MelRows stage[1 + 2 * KOE_MAX_EDGE] = {};
+  for (int v = 0; v < V; ++v) stage[v] = {a->stage + (size_t)v * KOE_N_MELS, a->stage_max + v, (int64_t)V * KOE_N_MELS, V};
+  if (int rc = launch_hop_frontend(a->frontend, a->tail_compact, n, tail_len, half, hop, n_edge, stage, stream)) return rc;
   // ---- 3. staging rows -> each slot's rings and window-end rows
   PoolRings r{};
   float* const power[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, a->row_l, a->ring_r2, a->row_l2};

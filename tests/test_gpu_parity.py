@@ -348,7 +348,7 @@ def test_pcm16_conversion_is_exact_and_host_pipeline_accepts_it(K):
         pipe(torch.zeros(2, 136000, dtype=torch.float64), torch.from_numpy(eg[:2]))
 
 
-@pytest.mark.parametrize("L,hop,n_frames,frame_offset,pad_mode", [
+RAGGED_SHAPES = [  # L, hop, n_frames, frame_offset, pad_mode
     (136000, 533, 257, 0, "constant"),   # bench shape: frame 255 and 256 run past the clip (three edge pairs)
     (136000, 533, 256, 0, "constant"),
     (20000, 533, 38, 0, "constant"),     # short clip: 1 + L // hop frames
@@ -358,7 +358,10 @@ def test_pcm16_conversion_is_exact_and_host_pipeline_accepts_it(K):
     (1500, 533, 1, 1, "constant"),       # a single frame = a single half-empty pair
     (20000, 266, 76, 0, "constant"),     # 60 fps hop: two leading / trailing edge frames
     (20000, 533, 38, 0, "reflect"),      # MelSlidingWindowExtractor padding
-])
+]
+
+
+@pytest.mark.parametrize("L,hop,n_frames,frame_offset,pad_mode", RAGGED_SHAPES)
 def test_logmel_launch_order_over_ragged_shapes(K, L, hop, n_frames, frame_offset, pad_mode):
     """The frontend launches a clip's padding-touching frame pairs ahead of its interior ones (they take masked loads);
     whatever the split -- no edge pairs, only edge pairs, odd frame counts, several clips -- every output row must still be
@@ -380,6 +383,29 @@ def test_logmel_launch_order_over_ragged_shapes(K, L, hop, n_frames, frame_offse
         if big.any():
             assert np.abs(db[b, :have] - 10 * np.log10(np.maximum(ref, 1e-10)))[big].max() < 8.7e-4
         np.testing.assert_allclose(fmax[b].cpu().numpy(), db[b].max(axis=1), rtol=1e-6)
+
+
+@pytest.mark.parametrize("bank", ["default", "generic"])
+@pytest.mark.parametrize("L,hop,n_frames,frame_offset",
+                         [s[:4] for s in RAGGED_SHAPES if s[4] == "constant" and s[2] >= 2])
+def test_logmel_split_pairs_equal_plain_frames(K, L, hop, n_frames, frame_offset, bank):
+    """The two organisations of the frontend kernel compute the same rows bit for bit.  A plain launch runs the
+    warp-specialised kernel for the default bank and the lock-step kernel for any other; a launch that sends each pair's
+    second frame to its own buffer (out_b, the streaming step) runs the lock-step kernel for both."""
+    from koemorph_b200.features.mel_frontend import LogMelFrontend
+    B = 5
+    audio, _ = O.make_inputs(1000 + L + n_frames, B, L, "speechlike")
+    audio = torch.from_numpy(audio).cuda()
+    fe = LogMelFrontend.get("cuda") if bank == "default" else LogMelFrontend.get("cuda", f_min=60.0, f_max=7600.0)
+    assert fe.uses_unrolled_bank() == (bank == "default")
+    db, fmax = fe.power(audio, hop, n_frames, frame_offset=frame_offset)
+    db_b = torch.empty((B, n_frames // 2, 80), dtype=torch.float32, device="cuda")
+    fmax_b = torch.empty((B, n_frames // 2), dtype=torch.float32, device="cuda")
+    db_a, fmax_a = fe.power(audio, hop, n_frames, frame_offset=frame_offset, out_b=(db_b, fmax_b))
+    assert torch.equal(db_a[:, 0::2], db[:, 0::2])
+    assert torch.equal(fmax_a[:, 0::2], fmax[:, 0::2])
+    assert torch.equal(db_b, db[:, 1::2])
+    assert torch.equal(fmax_b, fmax[:, 1::2])
 
 
 # ---- round 2: host pipeline state handling, fused native forward, public emotion entry, weight-cache invalidation --------
