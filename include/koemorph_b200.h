@@ -314,34 +314,40 @@ int koe_stream_push(const koe_stream_args* args, int* emitted, void* stream);
  * The pool object (host memory) owns the clock policy: which slots are open, how many hops each stream has pushed and
  * how many frames it has emitted.  Its entry points return KOE_E_INVALID on misuse (slot out of range or not open, a
  * slot listed twice in one call, more streams than free slots) before anything is queued.  Device buffers are
- * caller-owned (koe_stream_pool_args, shapes below with C = capacity, V = 1 + 2 * n_edge buffer variants:
- * plain, window-start 0, window-end 0, window-start 1, window-end 1).  koe_stream_pool_push uploads its per-call tables
- * (pushing streams: slot, ring row, first hop; emitting streams: slot, ring base, has smoothing state) with one
- * cudaMemcpyAsync from pinned staging that the library owns per (device, stream); it cannot be captured into a CUDA graph.
+ * caller-owned (koe_stream_pool_args, shapes below with C = capacity, H = max_hops (1 for koe_stream_pool_create),
+ * R = window_frames + H - 1 ring rows, V = 1 + 2 * n_edge buffer variants: plain, window-start 0, window-end 0,
+ * window-start 1, window-end 1).  The pushes upload their per-call tables (which stream, ring row and smoothing state
+ * each pushed hop and each emitted frame belongs to) with one cudaMemcpyAsync from pinned staging that the library owns
+ * per (device, stream); they cannot be captured into a CUDA graph.
  */
 typedef struct koe_stream_pool koe_stream_pool_t;
 typedef struct {
   const koe_frontend_t* frontend;
   const koe_core_weights* weights;
-  const float* hop_audio;        /* [n][hop]: row i is the next hop of stream slots_host[i] (koe_stream_pool_push) */
+  const float* hop_audio;        /* [sum of counts][hop]: the pushed hops, stream by stream in call order */
   float* tail;                   /* [C][half_fft + n_edge * hop]: each slot's audio tail (any content when opened) */
-  float* tail_compact;           /* [C][half_fft + n_edge * hop]: the pushing streams' tails, in call order */
-  float* stage;                  /* [V][C][80], */
-  float* stage_max;              /* [V][C]: the new mel rows of the pushing streams, in call order */
-  float* ring_f; float* fmax_f;  /* [C][window_frames][80], [C][window_frames] (as koe_stream_args) */
+  float* tail_compact;           /* [C * H][half_fft + n_edge * hop]: the tail after each pushed hop, in call order */
+  float* stage;                  /* [C * H][V][80], */
+  float* stage_max;              /* [C * H][V]: the new mel rows of each pushed hop, in call order */
+  float* ring_f; float* fmax_f;  /* [C][R][80], [C][R] */
   float* ring_r; float* fmax_r;
-  float* row_l; float* fmax_l;   /* [C][80], [C] */
+  float* row_l; float* fmax_l;   /* [C][80], [C]: koe_stream_pool_push with H = 1 only, else not read */
   float* ring_r2; float* fmax_r2; /* hop < n_fft/2 only, else NULL */
-  float* row_l2; float* fmax_l2;
+  float* row_l2; float* fmax_l2;  /* hop < n_fft/2 and H = 1 only, else NULL */
   float* expr_sigmoid;           /* [C] */
   float* expr_compact;           /* [C]: scratch of koe_stream_pool_set_egemaps */
-  float* out;                    /* [C][52]: row w is the frame of the w-th emitting stream of the call */
+  float* out;                    /* [C * H][52]: row r is the r-th frame emitted by the call */
   float* ema_state;              /* [C][52], or NULL: no temporal smoothing */
-  int32_t* tables;               /* [6][C] int32: the per-call tables */
+  int32_t* tables;               /* [6][C * H] int32: the per-call tables */
   float alpha;                   /* sigmoid(smoothing_alpha) */
   int32_t precision;
 } koe_stream_pool_args;
+/* a pool whose streams advance by one hop per push: koe_stream_pool_create_ex with max_hops = 1 */
 int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_fft, koe_stream_pool_t** out);
+/* a pool whose streams may advance by up to max_hops hops in one koe_stream_pool_push_hops (1 <= max_hops,
+ * capacity * max_hops <= 2^24): its rings hold R = window_frames + max_hops - 1 rows, because every row of a burst is
+ * written before the core reads the burst's first window */
+int koe_stream_pool_create_ex(int capacity, int hop, int window_frames, int half_fft, int max_hops, koe_stream_pool_t** out);
 int koe_stream_pool_destroy(koe_stream_pool_t* pool);
 /* takes the n lowest free slots into slots_host[n]; their clocks start at zero (their expression input is unset until
  * koe_stream_pool_set_egemaps) */
@@ -354,9 +360,24 @@ int koe_stream_pool_set_egemaps(koe_stream_pool_t* pool, const koe_stream_pool_a
  * emitted_host[0..*n_emitted) (capacity entries), in call order, and their frames to out rows 0..*n_emitted.  Queues the
  * tail update, the frontend launches of koe_stream_push on the pushing streams (2 at 30 fps, 4 at 60 fps), the scatter
  * into their rings and, when a stream emits, the core over the emitting streams and the smoothing: 6 kernels (8 at
- * 60 fps), 4 (6) when no stream emits, none for n = 0. */
+ * 60 fps), 4 (6) when no stream emits, none for n = 0.  On a pool with max_hops > 1 this is koe_stream_pool_push_hops
+ * with every count 1 (the same frames, the same number of kernels). */
 int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const int32_t* slots_host, int n,
                          int32_t* emitted_host, int* n_emitted, void* stream);
+/* advances the n open streams slots_host[0..n) by counts_host[i] hops each, 1 <= counts_host[i] <= max_hops (host
+ * memory): hop_audio holds sum(counts) hops, stream 0's in order, then stream 1's, ...  Every frame is bit for bit the
+ * frame that one koe_stream_pool_push per hop would give.  *n_emitted frames come out: row r of out is a frame of stream
+ * emitted_slot_host[r], the one that completes at its hop emitted_hop_host[r] (counted from 0 since the stream was opened:
+ * the first frame comes at hop window_frames - 1); rows are grouped by stream in call order, hops ascending within a
+ * stream (both host arrays take C * H entries).  All windows of a burst use the stream's expression value at the time of
+ * the call: a koe_stream_pool_set_egemaps meant to take effect between two hops of a stream needs two calls.  Queues
+ * the same kernels as koe_stream_pool_push, whatever the counts: a tail kernel that writes the tail after every pushed
+ * hop, the frontend launches over all pushed hops, the scatter into the rings and, when a frame completes, the core over
+ * all completing windows and the smoothing, which runs each stream's frames in order.  Misuse (a count outside
+ * [1, max_hops], a slot out of range, not open or listed twice) returns KOE_E_INVALID before anything is queued. */
+int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const int32_t* slots_host,
+                              const int32_t* counts_host, int n, int32_t* emitted_slot_host, int64_t* emitted_hop_host,
+                              int* n_emitted, void* stream);
 
 /*
  * The whole forward of SequentialDualStreamModel.forward (src/model/sequential_dual_stream_model.py:63-167) -- or, with

@@ -136,6 +136,7 @@ _SIGNATURES = {
                                           C.POINTER(C.c_int64)]),
     "koe_forward_varlen": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.c_void_p]),
     "koe_stream_pool_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "koe_stream_pool_create_ex": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "koe_stream_pool_destroy": (C.c_int, [C.c_void_p]),
     "koe_stream_pool_open": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "koe_stream_pool_close": (C.c_int, [C.c_void_p, C.c_int]),
@@ -143,6 +144,8 @@ _SIGNATURES = {
                                               C.c_void_p]),
     "koe_stream_pool_push": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_int, C.c_void_p,
                                        C.POINTER(C.c_int), C.c_void_p]),
+    "koe_stream_pool_push_hops": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_void_p, C.c_int,
+                                            C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "koe_affine_rows": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "koe_emotion_stream": (C.c_int, [C.POINTER(CoreWeightsStruct), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "koe_dual_stream_windows": (C.c_int, [C.POINTER(CoreWeightsStruct), C.POINTER(C.c_void_p),

@@ -37,6 +37,14 @@ struct CoreParams {
   const int* vl_frame_base;
   const int* vl_plain_only;
   int vl_clips;
+  // stream-pool bursts (csrc/stream_pool.cu; CoreMode::PoolHops only): the hops of a koe_stream_pool_push_hops call are
+  // staged in call order.  Window w completes at staged hop e = hop_end[w], a hop of stream slot hop_slot[e] whose newest
+  // plain row went to ring row hop_row[e]; the window starts hop_base_shift rows after that (mod ring_frames), and its
+  // window-end rows (variants 2, 4) are hop e's staged rows: row e * (1 + 2 n_edge) of power[2] / power[4]
+  const int* hop_end;
+  const int* hop_slot;
+  const int* hop_row;
+  int hop_base_shift;
 };
 
 // Which flavour of the core a launch runs.  Each is a separate instantiation of both kernels (the fp32 kernel has no
@@ -46,7 +54,9 @@ struct CoreParams {
 //   Early    Windows with one window per clip, released early by the frontend (the fused forward; early_flag)
 //   Pool     a stream-pool push: window w reads the rings of stream pool_slot[w] from ring base pool_base[w]
 //   Varlen   a packed variable-length batch: window w belongs to the clip c with vl_window_base[c] <= w < vl_window_base[c + 1]
-enum class CoreMode { Windows, Early, Pool, Varlen };
+//   PoolHops a stream-pool burst: window w reads the rings of stream hop_slot[hop_end[w]] (ring_frames rows each) and
+//            the window-end rows that hop hop_end[w] staged
+enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops };
 
 // frame k of a window: which buffer (variant) holds it (see koe_dual_stream_windows in the header)
 __device__ __forceinline__ int window_variant(const CoreParams& p, int k) {
@@ -82,11 +92,12 @@ __device__ __forceinline__ int varlen_clip(const CoreParams& p, int item) {
 
 // A window as the row addressing of mode M sees it; CoreRows<M> below is the only code that reads its fields.
 struct CoreWindow {
-  int owner;        // whose rows: the clip (Windows, Early; ring mode: the stream), the stream slot (Pool), or the
-                    // window's first plain row (Varlen)
-  int pos;          // where in them: the window within its clip (Windows, Early), the ring base (Pool), or the global
-                    // window, which is also the window's row in every edge-variant buffer (Varlen)
+  int owner;        // whose rows: the clip (Windows, Early; ring mode: the stream), the stream slot (Pool, PoolHops), or
+                    // the window's first plain row (Varlen)
+  int pos;          // where in them: the window within its clip (Windows, Early), the ring base (Pool, PoolHops), or the
+                    // global window, which is also the window's row in every edge-variant buffer (Varlen)
   bool plain_only;  // Varlen: the clip has no edge variants, every frame comes from the plain rows
+  int hop;          // PoolHops: the staged hop at which the window completes (its window-end rows)
 };
 
 // The window resolver of each mode: work item `item` is output row `item` and reads the window window<kWarp>(p, item);
@@ -98,6 +109,10 @@ struct CoreRows {
   static __device__ __forceinline__ CoreWindow window(const CoreParams& p, int item) {
     if constexpr (M == CoreMode::Pool) {
       return {p.pool_slot[item], p.pool_base[item], false};
+    } else if constexpr (M == CoreMode::PoolHops) {
+      const int e = p.hop_end[item];
+      const int base = p.hop_row[e] + p.hop_base_shift;  // both < ring_frames
+      return {p.hop_slot[e], base >= p.ring_frames ? base - p.ring_frames : base, false, e};
     } else if constexpr (M == CoreMode::Varlen) {
       const int c = varlen_clip<kWarp>(p, item);
       return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, item,
@@ -112,6 +127,9 @@ struct CoreRows {
     } else if constexpr (M == CoreMode::Pool) {
       return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
                                                : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
+    } else if constexpr (M == CoreMode::PoolHops) {
+      return variant > 0 && (variant & 1) == 0 ? (long long)w.hop * (1 + 2 * p.n_edge)
+                                               : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
     } else {
       if (p.ring_frames > 0)  // plain and lo-edge rows are ring slots of the global frame; a hi-edge row (variants 2, 4) is per stream
         return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
@@ -122,14 +140,16 @@ struct CoreRows {
   }
   // ring modes (ring_frames > 0, n_out == 1): the ring slot of the window's frame 0
   static __device__ __forceinline__ int ring_base(const CoreParams& p, const CoreWindow& w) {
-    return M == CoreMode::Pool ? w.pos : p.ring_base;
+    return M == CoreMode::Pool || M == CoreMode::PoolHops ? w.pos : p.ring_base;
   }
   // ring modes: the stream whose ring and frame maxima window `item` reads (the L2 prefetch of the next window)
   static __device__ __forceinline__ int ring_stream(const CoreParams& p, int item) {
+    if constexpr (M == CoreMode::PoolHops) return p.hop_slot[p.hop_end[item]];
     return M == CoreMode::Pool ? p.pool_slot[item] : item;
   }
   // the clip or stream whose expression value (expr_sigmoid) output row `item` takes
   static __device__ __forceinline__ int expr_row(const CoreParams& p, int item) {
+    if constexpr (M == CoreMode::PoolHops) return p.hop_slot[p.hop_end[item]];
     return M == CoreMode::Pool ? p.pool_slot[item] : item / p.n_out;
   }
   // the L2 policy of a window's plain rows: `reread` where other windows read them again (the overlapping windows of a
@@ -154,6 +174,13 @@ int launch_dual_stream_windows(const koe_core_weights* w, const float* const* po
 int launch_dual_stream_pool(const koe_core_weights* w, const float* const* power, const float* const* frame_max, int n_edge,
                             int n_windows, int ring_frames, const int* slot, const int* base, const float* expr_sigmoid,
                             float* out, int precision, void* stream);
+// the core over the windows of a stream-pool burst (csrc/stream_pool.cu): window w completes at staged hop hop_end[w] (device
+// tables as CoreParams::hop_*), rings of ring_frames rows, window-end rows power[2], power[4] at row hop * (1 + 2 n_edge);
+// output row w
+int launch_dual_stream_pool_hops(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                                 int n_edge, int n_windows, int ring_frames, const int* hop_end, const int* hop_slot,
+                                 const int* hop_row, int hop_base_shift, const float* expr_sigmoid, float* out, int precision,
+                                 void* stream);
 // the core over the windows of a packed variable-length batch (csrc/session.cu): window `item` of the n_windows belongs to
 // the clip c with window_base[c] <= item < window_base[c + 1] and writes output row `item`; plain rows from
 // frame_base[c] + (item - window_base[c]) * stride_frames, edge rows at `item` unless plain_only[c]; expression entries

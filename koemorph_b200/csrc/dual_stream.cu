@@ -816,6 +816,7 @@ static int launch_core(const CoreParams& p_in, CoreMode mode, int precision, cud
     case CoreMode::Windows: return launch_fp32<CoreMode::Windows>(p, stream);
     case CoreMode::Pool: return launch_fp32<CoreMode::Pool>(p, stream);
     case CoreMode::Varlen: return launch_fp32<CoreMode::Varlen>(p, stream);
+    case CoreMode::PoolHops: return launch_fp32<CoreMode::PoolHops>(p, stream);
     case CoreMode::Early: break;
   }
   return fail(KOE_E_INVALID, "early release needs the tensor-core core (precision 2)");
@@ -936,6 +937,32 @@ int koe::launch_dual_stream_pool(const koe_core_weights* w, const float* const* 
   p.pool_slot = slot;
   p.pool_base = base;
   return launch_core(p, CoreMode::Pool, precision, (cudaStream_t)stream);
+}
+
+int koe::launch_dual_stream_pool_hops(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                                      int n_edge, int n_windows, int ring_frames, const int* hop_end, const int* hop_slot,
+                                      const int* hop_row, int hop_base_shift, const float* expr_sigmoid, float* out,
+                                      int precision, void* stream) {
+  if (int rc = validate_weights(w)) return rc;
+  KOE_REQUIRE(power != nullptr && frame_max != nullptr && hop_end != nullptr && hop_slot != nullptr && hop_row != nullptr &&
+                  expr_sigmoid != nullptr && out != nullptr,
+              "stream pool burst core: NULL argument");
+  KOE_REQUIRE(n_edge >= 1 && n_edge <= KOE_MAX_EDGE && n_windows >= 0 && ring_frames >= w->k_mel - 3 &&
+                  hop_base_shift >= 0 && hop_base_shift < ring_frames,
+              "stream pool burst core: bad sizes");
+  if (n_windows == 0) return KOE_OK;
+  CoreParams p;
+  if (int rc = core_params("stream pool burst core", w, power, frame_max, n_edge, expr_sigmoid, out, nullptr, nullptr, &p))
+    return rc;
+  p.n_clips = n_windows;
+  p.n_frames = ring_frames;
+  p.frames_per_window = w->k_mel - 2;
+  p.ring_frames = ring_frames;
+  p.hop_end = hop_end;
+  p.hop_slot = hop_slot;
+  p.hop_row = hop_row;
+  p.hop_base_shift = hop_base_shift;
+  return launch_core(p, CoreMode::PoolHops, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,

@@ -10,8 +10,16 @@
 // rings, and -- when at least one stream emits -- the core over the emitting streams only and the smoothing.
 //
 // Stream n's frames are numbered from its own first hop: the newest complete frame after hop n is g = n - lag (lag =
-// n_edge - 1) in ring row g mod W, and the window that ends after hop n starts at ring row (n + 1 - W) mod W -- the
-// arithmetic of koe_stream_push, per stream.
+// n_edge - 1) in ring row g mod R, and the window that ends after hop n starts at ring row (n + 1 - W) mod R -- the
+// arithmetic of koe_stream_push, per stream.  R = ring_frames = W + max_hops - 1: W for a pool of koe_stream_pool_create.
+//
+// A burst (koe_stream_pool_push_hops) advances stream i by counts[i] hops in the same number of launches.  Its hops are
+// staged in call order (stream by stream, hops in order); staged hop e gets its own compact tail -- the tail as it is right
+// after that hop -- so the frontend runs on exactly the tails, and forms exactly the frame pairs, of one push per hop.  All
+// rows of a burst are in the rings before the core reads the burst's first window; that window reaches back W + k - 1 - lag
+// rows from the newest one, which is why the rings hold W + max_hops - 1.  Window-end rows are read by the one window that
+// completes at their hop only, so the core reads them in the staging rows.  The smoothing runs each stream's frames of the
+// call one after the other with the roundings of one push per hop (a scan would round differently).
 #include <algorithm>
 #include <vector>
 
@@ -19,13 +27,16 @@
 
 struct koe_stream_pool {
   int capacity, hop, window_frames, half_fft, n_edge, tail_len;
+  int max_hops, ring_frames;      // hops one stream may advance per call; rows per ring, window_frames + max_hops - 1
   std::vector<unsigned char> open;
   std::vector<int64_t> hops;      // hops pushed since the slot was opened
   std::vector<int64_t> frames;    // frames emitted since the slot was opened
-  std::vector<int32_t> row;       // ring row of the newest complete frame after the next hop, (hops - lag) mod W: kept as
+  std::vector<int32_t> row;       // ring row of the newest complete frame after the next hop, (hops - lag) mod R: kept as
                                   // a counter, so that a push of thousands of streams does no division on the host
   std::vector<uint32_t> listed;   // duplicate check: the call that last listed the slot
   uint32_t call = 0;
+  std::vector<int32_t> ones;      // koe_stream_pool_push on a pool with max_hops > 1: counts of 1 ...
+  std::vector<int64_t> emit_hop;  // ... and the emitting hops it does not return
 };
 
 namespace koe {
@@ -98,6 +109,81 @@ __global__ void __launch_bounds__(256) pool_expr_scatter_kernel(const float* __r
   if (i < n) expr_sigmoid[__ldg(slot + i)] = compact[i];
 }
 
+// ---- bursts (koe_stream_pool_push_hops).  Staged hop e is hop j = e - first[i] of pushing stream i, first[i] <= e <
+// first[i + 1] (first[n] = n_hops): hop_audio row e, compact tail e, staging rows e.
+
+// pushing stream i: X = [its old tail (zeros on its first hop) | its hops]; compact tail e = the tail right after hop j,
+// X[(j + 1) hop, (j + 1) hop + tail_len); the slot's own tail becomes the one after the stream's last hop.  One CTA per
+// stream: the old tail's last tail_len - hop samples to shared memory, barrier, write.
+__global__ void __launch_bounds__(256) pool_hops_tail_kernel(float* __restrict__ tail, const float* __restrict__ hop_audio,
+                                                              const int* __restrict__ hop_slot, const int* __restrict__ first,
+                                                              const int* __restrict__ fresh, int n, int n_hops, int tail_len,
+                                                              int hop, float* __restrict__ compact) {
+  extern __shared__ float s_old[];  // X[hop, tail_len)
+  const int keep = tail_len - hop;
+  for (int i = blockIdx.x; i < n; i += gridDim.x) {
+    const int e0 = __ldg(first + i), e1 = i + 1 < n ? __ldg(first + i + 1) : n_hops;
+    float* t = tail + (long long)__ldg(hop_slot + e0) * tail_len;
+    const bool zero = __ldg(fresh + i) != 0;
+    for (int k = threadIdx.x; k < keep; k += blockDim.x) s_old[k] = zero ? 0.0f : t[hop + k];
+    __syncthreads();
+    const float* x = hop_audio + (long long)e0 * hop;  // the stream's hops, back to back
+    for (int e = e0; e < e1; ++e) {
+      float* c = compact + (long long)e * tail_len;
+      for (int k = threadIdx.x; k < tail_len; k += blockDim.x) {
+        const int q = (e - e0) * hop + k;  // sample X[hop + q]
+        const float v = q < keep ? s_old[q] : __ldg(x + (q - keep));
+        c[k] = v;
+        if (e == e1 - 1) t[k] = v;
+      }
+    }
+    __syncthreads();
+  }
+}
+
+// staged rows of hop e ([n_hops][V][80], maxima [n_hops][V]): the plain and window-start variants (0, 1, 3) -> ring row
+// hop_row[e] of slot hop_slot[e]; the window-end variants stay in staging, where the core reads them
+__global__ void __launch_bounds__(256) pool_hops_scatter_kernel(PoolRings r, const float* __restrict__ stage,
+                                                                 const float* __restrict__ stage_max,
+                                                                 const int* __restrict__ hop_slot,
+                                                                 const int* __restrict__ hop_row, int n_hops, int n_edge,
+                                                                 int ring_frames) {
+  constexpr int kQuads = KOE_N_MELS / 4;
+  const int n_ring = 1 + n_edge, V = 1 + 2 * n_edge;
+  const int total = n_hops * n_ring * kQuads;
+  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
+    const int q = idx % kQuads, im = idx / kQuads, m = im % n_ring, e = im / n_ring;
+    const int v = m == 0 ? 0 : 2 * m - 1;
+    const long long row = (long long)__ldg(hop_slot + e) * ring_frames + __ldg(hop_row + e);
+    const long long src = (long long)e * V + v;
+    reinterpret_cast<float4*>(r.power[v] + row * KOE_N_MELS)[q] = __ldcs(reinterpret_cast<const float4*>(stage) + src * kQuads + q);
+    if (q == 0) r.fmax[v][row] = __ldcs(stage_max + src);
+  }
+}
+
+// smoothing of a burst's frames: a stream's frames of the call are consecutive output rows; thread (w, j), w the first of
+// them, runs them in order with the roundings of pool_ema_kernel -- exactly one push per hop.  has_state[w] == 0 only for
+// a stream's first frame since it was opened.
+__global__ void __launch_bounds__(256) pool_hops_ema_kernel(float* __restrict__ frames, int k, float alpha,
+                                                             float* __restrict__ state, const int* __restrict__ hop_end,
+                                                             const int* __restrict__ hop_slot,
+                                                             const int* __restrict__ has_state) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= k * KOE_N_BLENDSHAPES) return;
+  const int w = i / KOE_N_BLENDSHAPES, j = i % KOE_N_BLENDSHAPES;
+  const int s = __ldg(hop_slot + __ldg(hop_end + w));
+  if (w > 0 && __ldg(hop_slot + __ldg(hop_end + w - 1)) == s) return;  // not the stream's first frame of the call
+  float* st = state + (long long)s * KOE_N_BLENDSHAPES + j;
+  float y = *st;
+  for (int r = w; r < k && (r == w || __ldg(hop_slot + __ldg(hop_end + r)) == s); ++r) {
+    float* f = frames + (long long)r * KOE_N_BLENDSHAPES + j;
+    const float x = *f;
+    y = __ldg(has_state + r) ? fmaf(1.0f - alpha, y, alpha * x) : x;
+    *f = y;
+  }
+  *st = y;
+}
+
 namespace {
 // every slot of slots[0, n) in range, open and listed once
 int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* what) {
@@ -123,24 +209,38 @@ int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* 
 
 using namespace koe;
 
-extern "C" int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_fft, koe_stream_pool_t** out) {
+extern "C" int koe_stream_pool_create_ex(int capacity, int hop, int window_frames, int half_fft, int max_hops,
+                                         koe_stream_pool_t** out) {
   KOE_REQUIRE(out != nullptr, "koe_stream_pool_create: NULL argument");
   *out = nullptr;
   KOE_REQUIRE(capacity >= 1 && capacity <= (1 << 24) && hop > 0 && window_frames > 0 && half_fft > 0,
               "koe_stream_pool_create: bad geometry");
+  KOE_REQUIRE(max_hops >= 1 && (int64_t)capacity * max_hops <= (1 << 24) && (int64_t)window_frames + max_hops - 1 <= INT32_MAX,
+              "koe_stream_pool_create: max_hops %d for %d streams (need 1 <= max_hops, capacity * max_hops <= 2^24)",
+              max_hops, capacity);
   const int n_edge = (half_fft + hop - 1) / hop;
   KOE_REQUIRE(n_edge >= 1 && n_edge <= KOE_MAX_EDGE && window_frames + 1 > 2 * n_edge,
               "koe_stream_pool_create: hop %d needs %d edge frames per window side (max %d)", hop, n_edge, KOE_MAX_EDGE);
   auto* p = new koe_stream_pool();
   p->capacity = capacity, p->hop = hop, p->window_frames = window_frames, p->half_fft = half_fft, p->n_edge = n_edge;
   p->tail_len = half_fft + n_edge * hop;
+  p->max_hops = max_hops;
+  p->ring_frames = window_frames + max_hops - 1;
   p->open.assign(capacity, 0);
   p->hops.assign(capacity, 0);
   p->frames.assign(capacity, 0);
   p->row.assign(capacity, 0);
   p->listed.assign(capacity, 0);
+  if (max_hops > 1) {
+    p->ones.assign(capacity, 1);
+    p->emit_hop.assign(capacity, 0);
+  }
   *out = p;
   return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_fft, koe_stream_pool_t** out) {
+  return koe_stream_pool_create_ex(capacity, hop, window_frames, half_fft, 1, out);
 }
 
 extern "C" int koe_stream_pool_destroy(koe_stream_pool_t* pool) {
@@ -159,7 +259,7 @@ extern "C" int koe_stream_pool_open(koe_stream_pool_t* pool, int n, int32_t* slo
     pool->open[s] = 1;
     pool->hops[s] = 0;
     pool->frames[s] = 0;
-    pool->row[s] = (pool->window_frames - (pool->n_edge - 1)) % pool->window_frames;
+    pool->row[s] = (pool->ring_frames - (pool->n_edge - 1)) % pool->ring_frames;
     slots_host[i++] = s;
   }
   return KOE_OK;
@@ -199,6 +299,9 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
   KOE_REQUIRE(pool != nullptr && a != nullptr && n_emitted != nullptr && emitted_host != nullptr,
               "koe_stream_pool_push: NULL argument");
   *n_emitted = 0;
+  if (pool->max_hops > 1)  // rings of W + max_hops - 1 rows: a burst of one hop per stream
+    return koe_stream_pool_push_hops(pool, a, slots_host, pool->ones.data(), n, emitted_host, pool->emit_hop.data(),
+                                     n_emitted, stream);
   if (int rc = check_slots(pool, slots_host, n, "koe_stream_pool_push")) return rc;
   if (n == 0) return KOE_OK;
   const int W = pool->window_frames, n_edge = pool->n_edge, tail_len = pool->tail_len;
@@ -290,6 +393,132 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
     const int s = slots_host[i];
     if (++pool->hops[s] >= W) ++pool->frames[s];
     if (++pool->row[s] == W) pool->row[s] = 0;
+  }
+  *n_emitted = k;
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stream_pool_args* a, const int32_t* slots_host,
+                                         const int32_t* counts_host, int n, int32_t* emitted_slot_host,
+                                         int64_t* emitted_hop_host, int* n_emitted, void* stream) {
+  KOE_REQUIRE(pool != nullptr && a != nullptr && n_emitted != nullptr && emitted_slot_host != nullptr &&
+                  emitted_hop_host != nullptr,
+              "koe_stream_pool_push_hops: NULL argument");
+  *n_emitted = 0;
+  if (int rc = check_slots(pool, slots_host, n, "koe_stream_pool_push_hops")) return rc;
+  if (n == 0) return KOE_OK;
+  KOE_REQUIRE(counts_host != nullptr, "koe_stream_pool_push_hops: NULL counts");
+  const int W = pool->window_frames, R = pool->ring_frames, H = pool->max_hops, n_edge = pool->n_edge;
+  const int tail_len = pool->tail_len, hop = pool->hop, half = pool->half_fft, V = 1 + 2 * n_edge, lag = n_edge - 1;
+  int n_hops = 0, k = 0;  // staged hops, windows that complete (<= capacity * max_hops <= 2^24)
+  for (int i = 0; i < n; ++i) {
+    const int c = counts_host[i];
+    KOE_REQUIRE(c >= 1 && c <= H, "koe_stream_pool_push_hops: count %d for slot %d outside [1, %d]", c, slots_host[i], H);
+    const int64_t after = pool->hops[slots_host[i]] + c;  // hops after this call; windows complete at hops W - 1, W, ...
+    n_hops += c;
+    k += (int)std::min<int64_t>(c, std::max<int64_t>(0, after - (W - 1)));
+  }
+  KOE_REQUIRE(a->frontend != nullptr && a->weights != nullptr, "koe_stream_pool_push_hops: NULL frontend / weights");
+  KOE_REQUIRE(a->weights->k_mel == W + 3, "koe_stream_pool_push_hops: weights for k_mel %d, pool of window_frames %d",
+              a->weights->k_mel, W);
+  KOE_REQUIRE(a->hop_audio && a->tail && a->tail_compact && a->stage && a->stage_max && a->ring_f && a->fmax_f && a->ring_r &&
+                  a->fmax_r && a->expr_sigmoid && a->out && a->tables,
+              "koe_stream_pool_push_hops: NULL buffer");
+  KOE_REQUIRE(n_edge == 1 || (a->ring_r2 && a->fmax_r2), "koe_stream_pool_push_hops: hop < n_fft/2 needs ring_r2");
+  KOE_REQUIRE(a->ema_state == nullptr || (a->alpha >= 0.0f && a->alpha <= 1.0f),
+              "koe_stream_pool_push_hops: alpha must be in [0, 1]");
+  if (int rc = check_capture(stream, "koe_stream_pool_push_hops")) return rc;
+  int sms = 0;
+  KOE_CUDA(sm_count(&sms));
+  cudaStream_t st = (cudaStream_t)stream;
+
+  // ---- the per-call tables: [hop slot | hop ring row] per staged hop, [first staged hop | first hop since open] per
+  // pushing stream, [staged hop | has smoothing state] per window; 2 n_hops + 2 n + 2 k <= 6 capacity * max_hops
+  TableStaging* b = nullptr;
+  const size_t ints = 2 * (size_t)n_hops + 2 * (size_t)n + 2 * (size_t)k;
+  if (int rc = acquire_table_staging(stream, ints, &b)) return rc;
+  int32_t* const h_slot = b->host;
+  int32_t* const h_row = h_slot + n_hops;
+  int32_t* const h_first = h_row + n_hops;
+  int32_t* const h_fresh = h_first + n;
+  int32_t* const h_end = h_fresh + n;
+  int32_t* const h_has = h_end + k;
+  for (int i = 0, e = 0, w = 0; i < n; ++i) {
+    const int s = slots_host[i], c = counts_host[i];
+    const int64_t age = pool->hops[s];  // hops before this call
+    int64_t frames = pool->frames[s];
+    int r = pool->row[s];
+    h_first[i] = e;
+    h_fresh[i] = age == 0 ? 1 : 0;
+    for (int j = 0; j < c; ++j, ++e) {
+      h_slot[e] = s;
+      h_row[e] = r;
+      if (++r == R) r = 0;
+      if (age + j + 1 >= W) {  // hop age + j completes a window
+        h_end[w] = e;
+        h_has[w] = frames++ > 0 ? 1 : 0;
+        emitted_slot_host[w] = s;
+        emitted_hop_host[w++] = age + j;
+      }
+    }
+  }
+  if (int rc = upload_tables(b, a->tables, ints, st)) return rc;
+  const int* hop_slot = a->tables;
+  const int* hop_row = hop_slot + n_hops;
+  const int* first = hop_row + n_hops;
+  const int* fresh = first + n;
+  const int* hop_end = fresh + n;
+  const int* has_state = hop_end + k;
+
+  // ---- 1. one compact tail per staged hop, each slot's tail after its last hop
+  {
+    const int grid = std::min(n, sms * 8);
+    pool_hops_tail_kernel<<<grid, 256, (tail_len - hop) * sizeof(float), st>>>(a->tail, a->hop_audio, hop_slot, first, fresh,
+                                                                               n, n_hops, tail_len, hop, a->tail_compact);
+    count_launch();
+    KOE_CUDA(cudaGetLastError());
+  }
+  // ---- 2. the frontend launches of koe_stream_push on the compact tails, into staging rows [n_hops][V][80]
+  MelRows stage[1 + 2 * KOE_MAX_EDGE] = {};
+  for (int v = 0; v < V; ++v) stage[v] = {a->stage + (size_t)v * KOE_N_MELS, a->stage_max + v, (int64_t)V * KOE_N_MELS, V};
+  if (int rc = launch_hop_frontend(a->frontend, a->tail_compact, n_hops, tail_len, half, hop, n_edge, stage, stream)) return rc;
+  // ---- 3. plain and window-start rows -> each slot's rings
+  {
+    PoolRings r{};
+    float* const power[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, nullptr, a->ring_r2, nullptr};
+    float* const fmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, nullptr, a->fmax_r2, nullptr};
+    for (int v = 0; v < V; ++v) r.power[v] = power[v], r.fmax[v] = fmax[v];
+    const int total = n_hops * (1 + n_edge) * (KOE_N_MELS / 4);
+    pool_hops_scatter_kernel<<<std::min((total + 255) / 256, sms * 8), 256, 0, st>>>(r, a->stage, a->stage_max, hop_slot,
+                                                                                    hop_row, n_hops, n_edge, R);
+    count_launch();
+    KOE_CUDA(cudaGetLastError());
+  }
+  // ---- 4. the core over the windows that complete, window-end rows from staging; 5. the smoothing
+  if (k > 0) {
+    const float* cpower[1 + 2 * KOE_MAX_EDGE] = {a->ring_f, a->ring_r, a->stage + 2 * KOE_N_MELS, a->ring_r2,
+                                                 n_edge == 2 ? a->stage + 4 * KOE_N_MELS : nullptr};
+    const float* cfmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, a->stage_max + 2, a->fmax_r2,
+                                                n_edge == 2 ? a->stage_max + 4 : nullptr};
+    // the window that completes at hop n starts at frame n + 1 - W = g + lag + 1 - W: ring row (row + lag + H) mod R
+    if (int rc = launch_dual_stream_pool_hops(a->weights, cpower, cfmax, n_edge, k, R, hop_end, hop_slot, hop_row, lag + H,
+                                              a->expr_sigmoid, a->out, a->precision, stream))
+      return rc;
+    if (a->ema_state != nullptr) {
+      pool_hops_ema_kernel<<<(k * KOE_N_BLENDSHAPES + 255) / 256, 256, 0, st>>>(a->out, k, a->alpha, a->ema_state, hop_end,
+                                                                               hop_slot, has_state);
+      count_launch();
+      KOE_CUDA(cudaGetLastError());
+    }
+  }
+  // ---- the clocks advance once everything is queued
+  for (int i = 0; i < n; ++i) {
+    const int s = slots_host[i], c = counts_host[i];
+    const int64_t after = pool->hops[s] + c;
+    pool->frames[s] += std::min<int64_t>(c, std::max<int64_t>(0, after - (W - 1)));
+    pool->hops[s] = after;
+    pool->row[s] += c;
+    if (pool->row[s] >= R) pool->row[s] -= R;
   }
   *n_emitted = k;
   return KOE_OK;

@@ -17,11 +17,12 @@ L0[n+1] -- 5 FFTs per hop against 513.  F and R rows go into per-stream rings of
 rings directly (``koe_dual_stream_ring``).  After the 256th hop every step emits the frame that
 ``SequentialDualStreamModel.forward`` would produce for the window ending at the newest sample, EMA included.
 All streams of a StreamingEngine advance in lockstep (one hop per step each); in a StreamPool every stream opens,
-closes and advances on its own clock.
+closes and advances on its own clock, by one hop per push or by several in one push_hops.
 """
 from __future__ import annotations
 
 import ctypes as C
+import operator
 from typing import Optional
 
 import torch
@@ -217,13 +218,23 @@ class StreamPool:
     the same hops from the moment the stream was opened, whatever the other streams do and whatever its slot held
     before: it emits from its own W-th hop on (256 at 30 fps, 512 at 60 fps), its first frame passes the smoothing
     unchanged, and a reused slot carries nothing over.  The clocks live in the native pool object; this class owns the
-    device buffers and checks what it hands over."""
+    device buffers and checks what it hands over.
 
-    def __init__(self, model, capacity: int):
+    ``max_hops`` > 1 lets :meth:`push_hops` advance a stream by up to that many hops in one call (late packets after a
+    jitter buffer drains, chunked audio, a backlog): the rings then hold ``W + max_hops - 1`` rows, and the per-call
+    buffers are sized for ``capacity * max_hops`` hops."""
+
+    def __init__(self, model, capacity: int, max_hops: int = 1):
         self.model = model
         self.capacity = int(capacity)
         if self.capacity < 1:
             raise ValueError(f"capacity must be >= 1, got {capacity}")
+        try:
+            self.max_hops = operator.index(max_hops)
+        except TypeError:
+            raise ValueError(f"max_hops must be an integer, got {type(max_hops).__name__}") from None
+        if isinstance(max_hops, bool) or self.max_hops < 1:
+            raise ValueError(f"max_hops must be an integer >= 1, got {max_hops!r}")
         self.dev = next(model.parameters()).device
         if self.dev.type != "cuda":
             raise RuntimeError("StreamPool needs the model on a CUDA device")
@@ -236,20 +247,22 @@ class StreamPool:
             raise NotImplementedError(f"hop {self.hop} needs {self.n_edge} edge frames per window side (max {_lib.MAX_EDGE})")
         self.tail_len = self.half + self.n_edge * self.hop
         cap, V = self.capacity, 1 + 2 * self.n_edge
+        hops = cap * self.max_hops                          # hops one call may push
+        self.ring_frames = R = self.W + self.max_hops - 1
         f32 = dict(dtype=torch.float32, device=self.dev)
         self.tail = torch.zeros(cap, self.tail_len, **f32)
-        self.tail_compact = torch.empty(cap, self.tail_len, **f32)
-        self.stage = torch.empty(cap, V, 80, **f32)
-        self.stage_max = torch.empty(cap, V, **f32)
-        self.ring_f = torch.zeros(cap, self.W, 80, **f32)
-        self.ring_r = torch.zeros(cap, self.W, 80, **f32)
-        self.fmax_f = torch.zeros(cap, self.W, **f32)
-        self.fmax_r = torch.zeros(cap, self.W, **f32)
+        self.tail_compact = torch.empty(hops, self.tail_len, **f32)
+        self.stage = torch.empty(hops, V, 80, **f32)
+        self.stage_max = torch.empty(hops, V, **f32)
+        self.ring_f = torch.zeros(cap, R, 80, **f32)
+        self.ring_r = torch.zeros(cap, R, 80, **f32)
+        self.fmax_f = torch.zeros(cap, R, **f32)
+        self.fmax_r = torch.zeros(cap, R, **f32)
         self.row_l = torch.zeros(cap, 80, **f32)
         self.fmax_l = torch.zeros(cap, **f32)
         if self.n_edge == 2:
-            self.ring_r2 = torch.zeros(cap, self.W, 80, **f32)
-            self.fmax_r2 = torch.zeros(cap, self.W, **f32)
+            self.ring_r2 = torch.zeros(cap, R, 80, **f32)
+            self.fmax_r2 = torch.zeros(cap, R, **f32)
             self.row_l2 = torch.zeros(cap, 80, **f32)
             self.fmax_l2 = torch.zeros(cap, **f32)
         else:
@@ -257,14 +270,16 @@ class StreamPool:
         self.expr = torch.zeros(cap, **f32)
         self.expr_compact = torch.empty(cap, **f32)
         self.state = torch.zeros(cap, 52, **f32)
-        self.out = torch.zeros(cap, 52, **f32)
-        self.tables = torch.empty(6 * cap, dtype=torch.int32, device=self.dev)
-        self._emitted = torch.empty(cap, dtype=torch.int32)  # host: the slots of the last push's frames
+        self.out = torch.zeros(hops, 52, **f32)
+        self.tables = torch.empty(6 * hops, dtype=torch.int32, device=self.dev)
+        self._emitted = torch.empty(hops, dtype=torch.int32)     # host: the slots of the last push's frames
+        self._emitted_hop = torch.empty(hops, dtype=torch.int64)  # host: the hop of each (push_hops)
         self._n_emitted = C.c_int(0)
         self._n_emitted_ref = C.byref(self._n_emitted)
         self._lib = _lib.load()
         h = C.c_void_p()
-        self._check(self._lib.koe_stream_pool_create(cap, self.hop, self.W, self.half, C.byref(h)), "koe_stream_pool_create")
+        self._check(self._lib.koe_stream_pool_create_ex(cap, self.hop, self.W, self.half, self.max_hops, C.byref(h)),
+                    "koe_stream_pool_create_ex")
         self._h = h
         self._fe = model._frontend(self.dev)
         self._alpha, self._alpha_key = 0.0, None
@@ -330,6 +345,45 @@ class StreamPool:
         self.pushes += 1
         k = self._n_emitted.value
         return self._emitted[:k].to(torch.int64), self.out[:k]
+
+    @torch.no_grad()
+    def push_hops(self, slots, audio: torch.Tensor, counts):
+        """Advances each listed open stream by several hops in one call: slots[i] by counts[i] hops, 1 <= counts[i] <=
+        max_hops (host integers).  audio: float32 on the model's device, the sum(counts) hops back to back, stream by
+        stream in call order -- a 1-D tensor of sum(counts) * hop samples or an (sum(counts), hop) tensor.  Every frame
+        is bit for bit what one :meth:`push` per hop gives.  Returns (slots, hops, frames): two CPU int64 tensors and a
+        (k, 52) view reused by the next call; row r is the frame of stream slots[r] that completes at its hop hops[r]
+        (counted from 0 since the stream was opened; its first frame comes at hop W - 1).  Rows are grouped by stream in
+        call order, hops ascending.  All frames of the call use each stream's expression input as it is now."""
+        s = self._slots(slots)
+        n = s.numel()
+        c = counts if isinstance(counts, torch.Tensor) else torch.as_tensor(counts, dtype=torch.int64)
+        if c.device.type != "cpu":
+            raise ValueError("counts must be host (CPU) integers")
+        if c.dim() != 1 or c.is_floating_point() or c.is_complex() or c.dtype == torch.bool:
+            raise ValueError(f"counts must be a 1-D sequence of integers, got {c.dtype} of shape {tuple(c.shape)}")
+        if c.numel() != n:
+            raise ValueError(f"{c.numel()} counts for {n} slots")
+        if n and (int(c.min()) < 1 or int(c.max()) > self.max_hops):
+            raise ValueError(f"counts must lie in [1, {self.max_hops}] (max_hops)")
+        c = c.to(torch.int32).contiguous()
+        total = int(c.sum()) if n else 0
+        if not isinstance(audio, torch.Tensor):
+            raise ValueError(f"audio must be a torch.Tensor, got {type(audio).__name__}")
+        if audio.device != self.dev or audio.dtype != torch.float32:
+            raise ValueError(f"audio must be float32 on {self.dev}, got {audio.dtype} on {audio.device}")
+        if tuple(audio.shape) not in ((total * self.hop,), (total, self.hop)):
+            raise ValueError(f"audio must hold sum(counts) = {total} hops of {self.hop} samples: ({total * self.hop},) or "
+                             f"({total}, {self.hop}), got {tuple(audio.shape)}")
+        x = audio.contiguous()
+        a = self._current_args()
+        a.hop_audio = x.data_ptr()
+        self._call(self._lib.koe_stream_pool_push_hops, self._h, self._args_ref, s.data_ptr(), c.data_ptr(), n,
+                   self._emitted.data_ptr(), self._emitted_hop.data_ptr(), self._n_emitted_ref,
+                   what="koe_stream_pool_push_hops")
+        self.pushes += 1
+        k = self._n_emitted.value
+        return self._emitted[:k].to(torch.int64), self._emitted_hop[:k].clone(), self.out[:k]
 
     # ---- helpers ----------------------------------------------------------------------------------------------------
     def _check(self, rc: int, what: str) -> None:
