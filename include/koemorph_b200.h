@@ -331,14 +331,15 @@ typedef struct {
   float* stage_max;              /* [C * H][V]: the new mel rows of each pushed hop, in call order */
   float* ring_f; float* fmax_f;  /* [C][R][80], [C][R] */
   float* ring_r; float* fmax_r;
-  float* row_l; float* fmax_l;   /* [C][80], [C]: koe_stream_pool_push with H = 1 only, else not read */
+  float* row_l; float* fmax_l;   /* [C][80], [C]: koe_stream_pool_push with H = 1 and no KOE_POOL_WARMUP only, else not
+                                    read */
   float* ring_r2; float* fmax_r2; /* hop < n_fft/2 only, else NULL */
-  float* row_l2; float* fmax_l2;  /* hop < n_fft/2 and H = 1 only, else NULL */
+  float* row_l2; float* fmax_l2;  /* hop < n_fft/2, H = 1 and no KOE_POOL_WARMUP only, else NULL */
   float* expr_sigmoid;           /* [C] */
   float* expr_compact;           /* [C]: scratch of koe_stream_pool_set_egemaps */
   float* out;                    /* [C * H][52]: row r is the r-th frame emitted by the call */
   float* ema_state;              /* [C][52], or NULL: no temporal smoothing */
-  int32_t* tables;               /* [6][C * H] int32: the per-call tables */
+  int32_t* tables;               /* [6][C * H] int32 ([7][C * H] on a warm-up pool): the per-call tables */
   float alpha;                   /* sigmoid(smoothing_alpha) */
   int32_t precision;
 } koe_stream_pool_args;
@@ -348,6 +349,24 @@ int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_ff
  * capacity * max_hops <= 2^24): its rings hold R = window_frames + max_hops - 1 rows, because every row of a burst is
  * written before the core reads the burst's first window */
 int koe_stream_pool_create_ex(int capacity, int hop, int window_frames, int half_fft, int max_hops, koe_stream_pool_t** out);
+/* koe_stream_pool_create_ex with a flags word (any other bit set: KOE_E_INVALID).  flags = 0 is koe_stream_pool_create_ex.
+ *
+ * KOE_POOL_WARMUP: a warm-up pool.  Every pushed hop of every open stream emits a frame, from the stream's hop 0 on,
+ * instead of from its hop window_frames - 1 (W - 1): a new stream is animated after one hop instead of 8.5 s.
+ *   - hops h >= W - 1: the unsmoothed frame is bit for bit the one a pool without the flag gives (the same rows,
+ *     window-start variants included);
+ *   - hops h < W - 1: the unsmoothed frame is SimplifiedDualStreamModel.forward on the stream's first (h + 1) * hop
+ *     samples (up to the rounding of the frontend): T = h + 2 frames, frames 0 .. T - 1 - n_edge from the plain ring
+ *     rows, the last n_edge from that hop's window-end rows, no window-start variants -- the long-term part is those
+ *     frames zero-padded, the short-term detail their last three, the dB reference their maximum;
+ *   - smoothing (ema_state != NULL) runs over every frame since the stream was opened: the hop-0 frame passes
+ *     unchanged and every later one is smoothed onto the one before, so from hop W - 1 on the smoothed frames are the
+ *     smoothing of this pool's own frames, not those of a pool without the flag.
+ * koe_stream_pool_push on a warm-up pool is koe_stream_pool_push_hops with every count 1, whatever max_hops is; rings
+ * keep R = W + max_hops - 1 rows, and the tables take [7][C * H] int32. */
+#define KOE_POOL_WARMUP 1
+int koe_stream_pool_create_ex2(int capacity, int hop, int window_frames, int half_fft, int max_hops, int flags,
+                               koe_stream_pool_t** out);
 int koe_stream_pool_destroy(koe_stream_pool_t* pool);
 /* takes the n lowest free slots into slots_host[n]; their clocks start at zero (their expression input is unset until
  * koe_stream_pool_set_egemaps) */
@@ -360,15 +379,15 @@ int koe_stream_pool_set_egemaps(koe_stream_pool_t* pool, const koe_stream_pool_a
  * emitted_host[0..*n_emitted) (capacity entries), in call order, and their frames to out rows 0..*n_emitted.  Queues the
  * tail update, the frontend launches of koe_stream_push on the pushing streams (2 at 30 fps, 4 at 60 fps), the scatter
  * into their rings and, when a stream emits, the core over the emitting streams and the smoothing: 6 kernels (8 at
- * 60 fps), 4 (6) when no stream emits, none for n = 0.  On a pool with max_hops > 1 this is koe_stream_pool_push_hops
- * with every count 1 (the same frames, the same number of kernels). */
+ * 60 fps), 4 (6) when no stream emits, none for n = 0.  On a pool with max_hops > 1 or KOE_POOL_WARMUP this is
+ * koe_stream_pool_push_hops with every count 1 (the same frames, the same number of kernels). */
 int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const int32_t* slots_host, int n,
                          int32_t* emitted_host, int* n_emitted, void* stream);
 /* advances the n open streams slots_host[0..n) by counts_host[i] hops each, 1 <= counts_host[i] <= max_hops (host
  * memory): hop_audio holds sum(counts) hops, stream 0's in order, then stream 1's, ...  Every frame is bit for bit the
  * frame that one koe_stream_pool_push per hop would give.  *n_emitted frames come out: row r of out is a frame of stream
  * emitted_slot_host[r], the one that completes at its hop emitted_hop_host[r] (counted from 0 since the stream was opened:
- * the first frame comes at hop window_frames - 1); rows are grouped by stream in call order, hops ascending within a
+ * the first frame comes at hop window_frames - 1, or at hop 0 on a KOE_POOL_WARMUP pool); rows are grouped by stream in call order, hops ascending within a
  * stream (both host arrays take C * H entries).  All windows of a burst use the stream's expression value at the time of
  * the call: a koe_stream_pool_set_egemaps meant to take effect between two hops of a stream needs two calls.  Queues
  * the same kernels as koe_stream_pool_push, whatever the counts: a tail kernel that writes the tail after every pushed

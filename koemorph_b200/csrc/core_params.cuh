@@ -45,6 +45,10 @@ struct CoreParams {
   const int* hop_slot;
   const int* hop_row;
   int hop_base_shift;
+  // stream-pool warm-up (csrc/stream_pool.cu; CoreMode::PoolWarm only): window w has hop_frames[w] frames, 2 ..
+  // frames_per_window; a window shorter than frames_per_window starts at its stream's sample 0 and has no window-start
+  // variants.  Everything else as PoolHops.
+  const int* hop_frames;
 };
 
 // Which flavour of the core a launch runs.  Each is a separate instantiation of both kernels (the fp32 kernel has no
@@ -56,7 +60,9 @@ struct CoreParams {
 //   Varlen   a packed variable-length batch: window w belongs to the clip c with vl_window_base[c] <= w < vl_window_base[c + 1]
 //   PoolHops a stream-pool burst: window w reads the rings of stream hop_slot[hop_end[w]] (ring_frames rows each) and
 //            the window-end rows that hop hop_end[w] staged
-enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops };
+//   PoolWarm a burst of a warm-up pool: PoolHops with hop_frames[w] frames in window w; below frames_per_window the
+//            window is the stream's whole audio so far: plain rows, then the n_edge window-end rows, no window-start rows
+enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops, PoolWarm };
 
 // frame k of a window: which buffer (variant) holds it (see koe_dual_stream_windows in the header)
 __device__ __forceinline__ int window_variant(const CoreParams& p, int k) {
@@ -97,7 +103,8 @@ struct CoreWindow {
   int pos;          // where in them: the window within its clip (Windows, Early), the ring base (Pool, PoolHops), or the
                     // global window, which is also the window's row in every edge-variant buffer (Varlen)
   bool plain_only;  // Varlen: the clip has no edge variants, every frame comes from the plain rows
-  int hop;          // PoolHops: the staged hop at which the window completes (its window-end rows)
+  int hop;          // PoolHops, PoolWarm: the staged hop at which the window completes (its window-end rows)
+  int frames;       // PoolWarm: the window's frame count
 };
 
 // The window resolver of each mode: work item `item` is output row `item` and reads the window window<kWarp>(p, item);
@@ -113,6 +120,12 @@ struct CoreRows {
       const int e = p.hop_end[item];
       const int base = p.hop_row[e] + p.hop_base_shift;  // both < ring_frames
       return {p.hop_slot[e], base >= p.ring_frames ? base - p.ring_frames : base, false, e};
+    } else if constexpr (M == CoreMode::PoolWarm) {
+      const int e = p.hop_end[item], T = p.hop_frames[item];
+      // frame 0 is T - 2 - lag rows before the hop's newest plain row: hop_base_shift + frames_per_window - T is that
+      // distance mod ring_frames (PoolHops' shift when T = frames_per_window), and the sum stays below 2 ring_frames
+      const int base = (p.hop_row[e] + p.hop_base_shift + p.frames_per_window - T) % p.ring_frames;
+      return {p.hop_slot[e], base, false, e, T};
     } else if constexpr (M == CoreMode::Varlen) {
       const int c = varlen_clip<kWarp>(p, item);
       return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, item,
@@ -127,7 +140,7 @@ struct CoreRows {
     } else if constexpr (M == CoreMode::Pool) {
       return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
                                                : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
-    } else if constexpr (M == CoreMode::PoolHops) {
+    } else if constexpr (M == CoreMode::PoolHops || M == CoreMode::PoolWarm) {
       return variant > 0 && (variant & 1) == 0 ? (long long)w.hop * (1 + 2 * p.n_edge)
                                                : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
     } else {
@@ -138,18 +151,36 @@ struct CoreRows {
                           : (long long)w.owner * p.n_out + w.pos;
     }
   }
+  // the window's frame count: T, the launch's frames_per_window, in every mode but PoolWarm
+  static __device__ __forceinline__ int frames(const CoreWindow& w, int T) {
+    if constexpr (M == CoreMode::PoolWarm) return w.frames;
+    return T;
+  }
+  // whether the window's first n_edge frames have window-start variants (see window_variant); not in a PoolWarm
+  // window shorter than frames_per_window: it starts at sample 0 of its stream, and its plain rows see zeros before that
+  static __device__ __forceinline__ bool window_starts(const CoreParams& p, const CoreWindow& w) {
+    if constexpr (M == CoreMode::PoolWarm) return w.frames == p.frames_per_window;
+    return true;
+  }
+  // frame k of window w with frames(w, T) = T: which buffer (variant) holds it
+  static __device__ __forceinline__ int variant(const CoreParams& p, const CoreWindow& w, int T, int k) {
+    if constexpr (M == CoreMode::PoolWarm) {
+      if (T < p.frames_per_window) return k >= T - p.n_edge ? 2 + 2 * (T - 1 - k) : 0;
+    }
+    return window_variant(p, k);
+  }
   // ring modes (ring_frames > 0, n_out == 1): the ring slot of the window's frame 0
   static __device__ __forceinline__ int ring_base(const CoreParams& p, const CoreWindow& w) {
-    return M == CoreMode::Pool || M == CoreMode::PoolHops ? w.pos : p.ring_base;
+    return M == CoreMode::Pool || M == CoreMode::PoolHops || M == CoreMode::PoolWarm ? w.pos : p.ring_base;
   }
   // ring modes: the stream whose ring and frame maxima window `item` reads (the L2 prefetch of the next window)
   static __device__ __forceinline__ int ring_stream(const CoreParams& p, int item) {
-    if constexpr (M == CoreMode::PoolHops) return p.hop_slot[p.hop_end[item]];
+    if constexpr (M == CoreMode::PoolHops || M == CoreMode::PoolWarm) return p.hop_slot[p.hop_end[item]];
     return M == CoreMode::Pool ? p.pool_slot[item] : item;
   }
   // the clip or stream whose expression value (expr_sigmoid) output row `item` takes
   static __device__ __forceinline__ int expr_row(const CoreParams& p, int item) {
-    if constexpr (M == CoreMode::PoolHops) return p.hop_slot[p.hop_end[item]];
+    if constexpr (M == CoreMode::PoolHops || M == CoreMode::PoolWarm) return p.hop_slot[p.hop_end[item]];
     return M == CoreMode::Pool ? p.pool_slot[item] : item / p.n_out;
   }
   // the L2 policy of a window's plain rows: `reread` where other windows read them again (the overlapping windows of a
@@ -177,10 +208,11 @@ int launch_dual_stream_pool(const koe_core_weights* w, const float* const* power
 // the core over the windows of a stream-pool burst (csrc/stream_pool.cu): window w completes at staged hop hop_end[w] (device
 // tables as CoreParams::hop_*), rings of ring_frames rows, window-end rows power[2], power[4] at row hop * (1 + 2 n_edge);
 // output row w
+// hop_frames != NULL (a warm-up pool, CoreMode::PoolWarm): window w has hop_frames[w] frames (CoreParams::hop_frames)
 int launch_dual_stream_pool_hops(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
                                  int n_edge, int n_windows, int ring_frames, const int* hop_end, const int* hop_slot,
-                                 const int* hop_row, int hop_base_shift, const float* expr_sigmoid, float* out, int precision,
-                                 void* stream);
+                                 const int* hop_row, int hop_base_shift, const int* hop_frames, const float* expr_sigmoid,
+                                 float* out, int precision, void* stream);
 // the core over the windows of a packed variable-length batch (csrc/session.cu): window `item` of the n_windows belongs to
 // the clip c with window_base[c] <= item < window_base[c + 1] and writes output row `item`; plain rows from
 // frame_base[c] + (item - window_base[c]) * stride_frames, edge rows at `item` unless plain_only[c]; expression entries

@@ -120,11 +120,12 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
 
   const int tid = threadIdx.x, tx = tid & 31, ty = tid >> 5;
   const koe_core_weights& W = p.w;
-  const int T = p.frames_per_window;
+  const int T_launch = p.frames_per_window;
   const int n_items = p.n_clips * p.n_out;
 
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
     const CoreWindow win = CoreRows<M>::template window<true>(p, item);
+    const int T = CoreRows<M>::frames(win, T_launch);
     const bool prenorm = p.mel_long != nullptr;
 
     // ---- P0: dB reference of this window -------------------------------------------------------
@@ -132,7 +133,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
     if (!prenorm) {
       float mx = -INFINITY;
       for (int k = tid; k < T; k += kCoreThreads) {
-        const int v = win.plain_only ? 0 : window_variant(p, k);
+        const int v = win.plain_only ? 0 : CoreRows<M>::variant(p, win, T, k);
         mx = fmaxf(mx, p.fmax[v][CoreRows<M>::row(p, win, v, k)]);
       }
       mx = warp_max(mx);
@@ -173,7 +174,7 @@ __global__ void __launch_bounds__(kCoreThreads, 1) dual_stream_fp32_kernel(CoreP
           else if (t < p.n_long)
             v = __ldg(reinterpret_cast<const float4*>(p.mel_long + ((size_t)win.owner * p.n_frames + t) * kTok) + q);
         } else if (k >= 0) {
-          const int var = win.plain_only ? 0 : window_variant(p, k);
+          const int var = win.plain_only ? 0 : CoreRows<M>::variant(p, win, T, k);
           const float4 pw = __ldg(reinterpret_cast<const float4*>(p.power[var] + CoreRows<M>::row(p, win, var, k) * kTok) + q);
           v.x = normalise_db(pw.x, ref_db, true);
           v.y = normalise_db(pw.y, ref_db, true);
@@ -817,6 +818,7 @@ static int launch_core(const CoreParams& p_in, CoreMode mode, int precision, cud
     case CoreMode::Pool: return launch_fp32<CoreMode::Pool>(p, stream);
     case CoreMode::Varlen: return launch_fp32<CoreMode::Varlen>(p, stream);
     case CoreMode::PoolHops: return launch_fp32<CoreMode::PoolHops>(p, stream);
+    case CoreMode::PoolWarm: return launch_fp32<CoreMode::PoolWarm>(p, stream);
     case CoreMode::Early: break;
   }
   return fail(KOE_E_INVALID, "early release needs the tensor-core core (precision 2)");
@@ -941,8 +943,8 @@ int koe::launch_dual_stream_pool(const koe_core_weights* w, const float* const* 
 
 int koe::launch_dual_stream_pool_hops(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
                                       int n_edge, int n_windows, int ring_frames, const int* hop_end, const int* hop_slot,
-                                      const int* hop_row, int hop_base_shift, const float* expr_sigmoid, float* out,
-                                      int precision, void* stream) {
+                                      const int* hop_row, int hop_base_shift, const int* hop_frames,
+                                      const float* expr_sigmoid, float* out, int precision, void* stream) {
   if (int rc = validate_weights(w)) return rc;
   KOE_REQUIRE(power != nullptr && frame_max != nullptr && hop_end != nullptr && hop_slot != nullptr && hop_row != nullptr &&
                   expr_sigmoid != nullptr && out != nullptr,
@@ -962,7 +964,8 @@ int koe::launch_dual_stream_pool_hops(const koe_core_weights* w, const float* co
   p.hop_slot = hop_slot;
   p.hop_row = hop_row;
   p.hop_base_shift = hop_base_shift;
-  return launch_core(p, CoreMode::PoolHops, precision, (cudaStream_t)stream);
+  p.hop_frames = hop_frames;
+  return launch_core(p, hop_frames != nullptr ? CoreMode::PoolWarm : CoreMode::PoolHops, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,

@@ -320,6 +320,12 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
   const bool tma_mel = p.mel_long == nullptr;
   const int Tl = min(T, p.mel_seq);                              // long-term frames actually present
   const int n_mel_stages = tma_mel ? (Tl + kMelRows - 1) / kMelRows : 0;
+  // the same for a window of wT = Rows::frames(win, T) frames: the launch's own except in PoolWarm, where every window
+  // has its own count (the mel-row producer and the SIMT warps derive the stage count from the same window)
+  auto long_frames = [&](int wT) { return M == CoreMode::PoolWarm ? min(wT, p.mel_seq) : Tl; };
+  auto mel_stages = [&](int wTl) {
+    return M == CoreMode::PoolWarm ? (tma_mel ? (wTl + kMelRows - 1) / kMelRows : 0) : n_mel_stages;
+  };
 
   if (warp == 8) {
     // =========================================================== weight producer ========================
@@ -356,6 +362,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         long long* dp = (p.dbg != nullptr && blockIdx.x == 0 && item < 2 * (int)gridDim.x) ? p.dbg + 32 + 16 * (item / gridDim.x) : nullptr;
         const CoreWindow win = Rows::template window<false>(p, item);
+        const int wTl = long_frames(Rows::frames(win, T)), w_stages = mel_stages(wTl);
         if (M == CoreMode::Early && (item == (int)blockIdx.x || item == first_late_item)) {
           if (item == first_late_item) pdl_wait();
           asm volatile("fence.proxy.async.global;" ::: "memory");  // generic-proxy acquire / wait above -> TMA reads below
@@ -375,13 +382,13 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           if (fm_bytes > 0 && ((reinterpret_cast<uintptr_t>(p.fmax[0]) | ((size_t)nb * p.ring_frames * 4)) & 15) == 0)
             bulk_prefetch_l2(p.fmax[0] + (size_t)nb * p.ring_frames, fm_bytes);
         }
-        for (int s = 0; s < n_mel_stages; ++s) {
-          const int n = min(kMelRows, Tl - kMelRows * s);
+        for (int s = 0; s < w_stages; ++s) {
+          const int n = min(kMelRows, wTl - kMelRows * s);
           const uint32_t bytes = (uint32_t)n * kTok * 4;
           const uint32_t dst = sbase + kOffRing + slot * kStageBytes;
           mbar_wait(bar_empty + 8 * slot, phase ^ 1);
           if (s == 0) stamp(dp, 8);
-          if (s == n_mel_stages - 1) stamp(dp, 9);
+          if (s == w_stages - 1) stamp(dp, 9);
           mbar_expect_tx(bar_full + 8 * slot, bytes);
           if (p.ring_frames > 0) {
             const int r0 = (Rows::ring_base(p, win) + kMelRows * s) % p.ring_frames;
@@ -512,14 +519,15 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
       float mx = -INFINITY;
       if (!prenorm) {
         const CoreWindow win = Rows::template window<true>(p, item);
-        for (int k0 = tid; k0 < T; k0 += 3 * kSimt) {
+        const int wT = Rows::frames(win, T);
+        for (int k0 = tid; k0 < wT; k0 += 3 * kSimt) {
           float f[3];
 #pragma unroll
           for (int u = 0; u < 3; ++u) {
             const int k = k0 + u * kSimt;
             f[u] = -INFINITY;
-            if (k < T) {
-              const int v = win.plain_only ? 0 : window_variant(p, k);
+            if (k < wT) {
+              const int v = win.plain_only ? 0 : Rows::variant(p, win, wT, k);
               f[u] = p.fmax[v][Rows::row(p, win, v, k)];
             }
           }
@@ -530,6 +538,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
     };
     auto stage_window = [&](const int item, float mx, long long* ds) {
       const CoreWindow win = Rows::template window<true>(p, item);
+      const int wT = Rows::frames(win, T), wTl = long_frames(wT), w_stages = mel_stages(wTl);
       // ---- window dB reference
       float ref_db = 0.0f;
       if (!prenorm) {
@@ -548,23 +557,23 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
         if (tid < kTok) {
 #pragma unroll
           for (int e = 0; e < 3; ++e) {
-            const int k = T >= 3 ? T - 3 + e : (e < T ? e : -1);
+            const int k = wT >= 3 ? wT - 3 + e : (e < wT ? e : -1);
             if (k >= 0) {
-              const int var = win.plain_only ? 0 : window_variant(p, k);
+              const int var = win.plain_only ? 0 : Rows::variant(p, win, wT, k);
               extra[e] = p.power[var][Rows::row(p, win, var, k) * kTok + tid];
             } else {
               extra[e] = -INFINITY;
             }
           }
           if (!win.plain_only && p.n_edge > 0) {
-            extra[3] = __ldg(p.power[1] + Rows::row(p, win, 1, 0) * kTok + tid);
-            if (T - 1 < Tl) extra[4] = __ldg(p.power[2] + Rows::row(p, win, 2, T - 1) * kTok + tid);
+            if (Rows::window_starts(p, win)) extra[3] = __ldg(p.power[1] + Rows::row(p, win, 1, 0) * kTok + tid);
+            if (wT - 1 < wTl) extra[4] = __ldg(p.power[2] + Rows::row(p, win, 2, wT - 1) * kTok + tid);
           }
         }
-        for (int s = 0; s < n_mel_stages; ++s) {
+        for (int s = 0; s < w_stages; ++s) {
           mbar_wait(bar_full + 8 * slot, phase);
           const float* raw = reinterpret_cast<const float*>(smem + kOffRing + slot * kStageBytes);
-          const int rows = min(kMelRows, Tl - kMelRows * s);
+          const int rows = min(kMelRows, wTl - kMelRows * s);
           const int chunks = (rows + 7) >> 3;
           if (rows == kMelRows) {
             // full stage: 6 chunks x 80 channels = 480 items of 8 frames; a thread's two items are loaded together
@@ -600,7 +609,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           simt_barrier();                                   // every thread is done reading this ring slot
           if (s == 0) stamp(ds, 11);
           if (s == 2) stamp(ds, 12);
-          if (s == n_mel_stages - 1) stamp(ds, 13);
+          if (s == w_stages - 1) stamp(ds, 13);
           if (tid == 0) mbar_arrive(bar_empty + 8 * slot);
           if (++slot == kRing) slot = kWRing, phase ^= 1;
         }
@@ -608,7 +617,7 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           const int j = tid;
           unsigned char* arow = smem + kOffX + (j >> 3) * kA1Sbo + (j & 7) * 16;
           // K chunks past the long-term frames: zeros up to frame 255, then [short-term x3, 0 x5], then zeros
-          for (int c = (Tl + 7) >> 3; c < kLongChunks; ++c) *reinterpret_cast<uint4*>(arow + c * 128) = make_uint4(0, 0, 0, 0);
+          for (int c = (wTl + 7) >> 3; c < kLongChunks; ++c) *reinterpret_cast<uint4*>(arow + c * 128) = make_uint4(0, 0, 0, 0);
           float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll
           for (int e = 0; e < 3; ++e) v[e] = normalise_bf16(extra[e], ref_db, true);
@@ -618,11 +627,13 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
           // edge frames inside the long-term range see zeros beyond the window edge: patch them in place
           // (frame m and frame T-1-m for m < n_edge: one per side at 30 fps, two at 60 fps)
           for (int m = 0; !win.plain_only && m < p.n_edge; ++m) {
-            const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + Rows::row(p, win, 1 + 2 * m, m) * kTok + j);
-            *reinterpret_cast<__nv_bfloat16*>(arow + (m >> 3) * 128 + (m & 7) * 2) =
-                __float2bfloat16_rn(normalise_bf16(lo, ref_db, true));
-            const int k = T - 1 - m;
-            if (k < Tl) {
+            if (Rows::window_starts(p, win)) {
+              const float lo = m == 0 ? extra[3] : __ldg(p.power[1 + 2 * m] + Rows::row(p, win, 1 + 2 * m, m) * kTok + j);
+              *reinterpret_cast<__nv_bfloat16*>(arow + (m >> 3) * 128 + (m & 7) * 2) =
+                  __float2bfloat16_rn(normalise_bf16(lo, ref_db, true));
+            }
+            const int k = wT - 1 - m;
+            if (k < wTl) {
               const float x = m == 0 ? extra[4] : __ldg(p.power[2 + 2 * m] + Rows::row(p, win, 2 + 2 * m, k) * kTok + j);
               *reinterpret_cast<__nv_bfloat16*>(arow + (k >> 3) * 128 + (k & 7) * 2) =
                   __float2bfloat16_rn(normalise_bf16(x, ref_db, true));
@@ -952,7 +963,7 @@ int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t strea
                 "tensor-core path: bad early-release parameters");
   if (mode == CoreMode::Varlen)
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames == 0 && p.expr_sigmoid == nullptr, "tensor-core path: bad varlen parameters");
-  if (mode == CoreMode::Pool || mode == CoreMode::PoolHops)
+  if (mode == CoreMode::Pool || mode == CoreMode::PoolHops || mode == CoreMode::PoolWarm)
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
   if (p.attn_out != nullptr)  // head-average is accumulated with atomics
     KOE_CUDA(cudaMemsetAsync(p.attn_out, 0, (size_t)p.n_clips * p.n_out * KOE_N_MOUTH * tc::kTok * sizeof(float),
@@ -964,6 +975,7 @@ int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t strea
     case CoreMode::Pool: rc = launch_tc<CoreMode::Pool>(p, grid, stream); break;
     case CoreMode::Varlen: rc = launch_tc<CoreMode::Varlen>(p, grid, stream); break;
     case CoreMode::PoolHops: rc = launch_tc<CoreMode::PoolHops>(p, grid, stream); break;
+    case CoreMode::PoolWarm: rc = launch_tc<CoreMode::PoolWarm>(p, grid, stream); break;
   }
   if (rc != KOE_OK) return rc;
   count_launch();

@@ -20,6 +20,15 @@
 // rows from the newest one, which is why the rings hold W + max_hops - 1.  Window-end rows are read by the one window that
 // completes at their hop only, so the core reads them in the staging rows.  The smoothing runs each stream's frames of the
 // call one after the other with the roundings of one push per hop (a scan would round differently).
+//
+// A warm-up pool (KOE_POOL_WARMUP) emits from every stream's hop 0: the frame at hop h < W - 1 is the forward of
+// SimplifiedDualStreamModel on the h + 1 hops heard so far, T = h + 2 frames.  Those are frames 0 .. h + 1 of the
+// stream's own clock, which the rings and the hop's staging already hold: plain rows F[0 .. h - lag] in ring rows
+// 0 .. h - lag, and the hop's window-end rows for the last n_edge frames (they see zeros from sample (h + 1) hop on, as
+// the prefix does).  Every frame before sample 0 reads zeros there too, because a stream's tail starts at zero, so the
+// plain rows are the right first frames and no window-start variant is read.  A warm-up pool always runs the burst path
+// (koe_stream_pool_push is koe_stream_pool_push_hops with counts of 1), its core is CoreMode::PoolWarm with one more
+// table column (each window's T), and from hop W - 1 on its windows are those of PoolHops.
 #include <algorithm>
 #include <vector>
 
@@ -28,6 +37,7 @@
 struct koe_stream_pool {
   int capacity, hop, window_frames, half_fft, n_edge, tail_len;
   int max_hops, ring_frames;      // hops one stream may advance per call; rows per ring, window_frames + max_hops - 1
+  bool warmup;                    // KOE_POOL_WARMUP: every hop emits, from each stream's hop 0 on
   std::vector<unsigned char> open;
   std::vector<int64_t> hops;      // hops pushed since the slot was opened
   std::vector<int64_t> frames;    // frames emitted since the slot was opened
@@ -35,7 +45,7 @@ struct koe_stream_pool {
                                   // a counter, so that a push of thousands of streams does no division on the host
   std::vector<uint32_t> listed;   // duplicate check: the call that last listed the slot
   uint32_t call = 0;
-  std::vector<int32_t> ones;      // koe_stream_pool_push on a pool with max_hops > 1: counts of 1 ...
+  std::vector<int32_t> ones;      // koe_stream_pool_push on a pool with max_hops > 1 or warm-up: counts of 1 ...
   std::vector<int64_t> emit_hop;  // ... and the emitting hops it does not return
 };
 
@@ -209,10 +219,11 @@ int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* 
 
 using namespace koe;
 
-extern "C" int koe_stream_pool_create_ex(int capacity, int hop, int window_frames, int half_fft, int max_hops,
-                                         koe_stream_pool_t** out) {
+extern "C" int koe_stream_pool_create_ex2(int capacity, int hop, int window_frames, int half_fft, int max_hops, int flags,
+                                          koe_stream_pool_t** out) {
   KOE_REQUIRE(out != nullptr, "koe_stream_pool_create: NULL argument");
   *out = nullptr;
+  KOE_REQUIRE((flags & ~KOE_POOL_WARMUP) == 0, "koe_stream_pool_create: unknown flags 0x%x", (unsigned)flags);
   KOE_REQUIRE(capacity >= 1 && capacity <= (1 << 24) && hop > 0 && window_frames > 0 && half_fft > 0,
               "koe_stream_pool_create: bad geometry");
   KOE_REQUIRE(max_hops >= 1 && (int64_t)capacity * max_hops <= (1 << 24) && (int64_t)window_frames + max_hops - 1 <= INT32_MAX,
@@ -226,12 +237,13 @@ extern "C" int koe_stream_pool_create_ex(int capacity, int hop, int window_frame
   p->tail_len = half_fft + n_edge * hop;
   p->max_hops = max_hops;
   p->ring_frames = window_frames + max_hops - 1;
+  p->warmup = (flags & KOE_POOL_WARMUP) != 0;
   p->open.assign(capacity, 0);
   p->hops.assign(capacity, 0);
   p->frames.assign(capacity, 0);
   p->row.assign(capacity, 0);
   p->listed.assign(capacity, 0);
-  if (max_hops > 1) {
+  if (max_hops > 1 || p->warmup) {
     p->ones.assign(capacity, 1);
     p->emit_hop.assign(capacity, 0);
   }
@@ -239,8 +251,13 @@ extern "C" int koe_stream_pool_create_ex(int capacity, int hop, int window_frame
   return KOE_OK;
 }
 
+extern "C" int koe_stream_pool_create_ex(int capacity, int hop, int window_frames, int half_fft, int max_hops,
+                                         koe_stream_pool_t** out) {
+  return koe_stream_pool_create_ex2(capacity, hop, window_frames, half_fft, max_hops, 0, out);
+}
+
 extern "C" int koe_stream_pool_create(int capacity, int hop, int window_frames, int half_fft, koe_stream_pool_t** out) {
-  return koe_stream_pool_create_ex(capacity, hop, window_frames, half_fft, 1, out);
+  return koe_stream_pool_create_ex2(capacity, hop, window_frames, half_fft, 1, 0, out);
 }
 
 extern "C" int koe_stream_pool_destroy(koe_stream_pool_t* pool) {
@@ -299,7 +316,7 @@ extern "C" int koe_stream_pool_push(koe_stream_pool_t* pool, const koe_stream_po
   KOE_REQUIRE(pool != nullptr && a != nullptr && n_emitted != nullptr && emitted_host != nullptr,
               "koe_stream_pool_push: NULL argument");
   *n_emitted = 0;
-  if (pool->max_hops > 1)  // rings of W + max_hops - 1 rows: a burst of one hop per stream
+  if (pool->max_hops > 1 || pool->warmup)  // rings of W + max_hops - 1 rows, or warm-up: a burst of one hop per stream
     return koe_stream_pool_push_hops(pool, a, slots_host, pool->ones.data(), n, emitted_host, pool->emit_hop.data(),
                                      n_emitted, stream);
   if (int rc = check_slots(pool, slots_host, n, "koe_stream_pool_push")) return rc;
@@ -410,13 +427,18 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
   KOE_REQUIRE(counts_host != nullptr, "koe_stream_pool_push_hops: NULL counts");
   const int W = pool->window_frames, R = pool->ring_frames, H = pool->max_hops, n_edge = pool->n_edge;
   const int tail_len = pool->tail_len, hop = pool->hop, half = pool->half_fft, V = 1 + 2 * n_edge, lag = n_edge - 1;
+  const bool warm = pool->warmup;
+  // the windows a stream's c hops complete when it has pushed `age` hops before: at hops W - 1, W, ... -- or, warm-up,
+  // at every hop
+  auto completing = [&](int64_t age, int c) -> int {
+    return warm ? c : (int)std::min<int64_t>(c, std::max<int64_t>(0, age + c - (W - 1)));
+  };
   int n_hops = 0, k = 0;  // staged hops, windows that complete (<= capacity * max_hops <= 2^24)
   for (int i = 0; i < n; ++i) {
     const int c = counts_host[i];
     KOE_REQUIRE(c >= 1 && c <= H, "koe_stream_pool_push_hops: count %d for slot %d outside [1, %d]", c, slots_host[i], H);
-    const int64_t after = pool->hops[slots_host[i]] + c;  // hops after this call; windows complete at hops W - 1, W, ...
     n_hops += c;
-    k += (int)std::min<int64_t>(c, std::max<int64_t>(0, after - (W - 1)));
+    k += completing(pool->hops[slots_host[i]], c);
   }
   KOE_REQUIRE(a->frontend != nullptr && a->weights != nullptr, "koe_stream_pool_push_hops: NULL frontend / weights");
   KOE_REQUIRE(a->weights->k_mel == W + 3, "koe_stream_pool_push_hops: weights for k_mel %d, pool of window_frames %d",
@@ -433,9 +455,10 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
   cudaStream_t st = (cudaStream_t)stream;
 
   // ---- the per-call tables: [hop slot | hop ring row] per staged hop, [first staged hop | first hop since open] per
-  // pushing stream, [staged hop | has smoothing state] per window; 2 n_hops + 2 n + 2 k <= 6 capacity * max_hops
+  // pushing stream, [staged hop | has smoothing state] per window -- and on a warm-up pool [frames] per window;
+  // 2 n_hops + 2 n + 2 k <= 6 capacity * max_hops, with the frames <= 7 capacity * max_hops
   TableStaging* b = nullptr;
-  const size_t ints = 2 * (size_t)n_hops + 2 * (size_t)n + 2 * (size_t)k;
+  const size_t ints = 2 * (size_t)n_hops + 2 * (size_t)n + (warm ? 3 : 2) * (size_t)k;
   if (int rc = acquire_table_staging(stream, ints, &b)) return rc;
   int32_t* const h_slot = b->host;
   int32_t* const h_row = h_slot + n_hops;
@@ -443,6 +466,7 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
   int32_t* const h_fresh = h_first + n;
   int32_t* const h_end = h_fresh + n;
   int32_t* const h_has = h_end + k;
+  int32_t* const h_frames = h_has + k;  // (warm-up pools only)
   for (int i = 0, e = 0, w = 0; i < n; ++i) {
     const int s = slots_host[i], c = counts_host[i];
     const int64_t age = pool->hops[s];  // hops before this call
@@ -454,7 +478,8 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
       h_slot[e] = s;
       h_row[e] = r;
       if (++r == R) r = 0;
-      if (age + j + 1 >= W) {  // hop age + j completes a window
+      if (warm || age + j + 1 >= W) {  // hop age + j completes a window
+        if (warm) h_frames[w] = (int32_t)std::min<int64_t>(age + j + 2, W + 1);
         h_end[w] = e;
         h_has[w] = frames++ > 0 ? 1 : 0;
         emitted_slot_host[w] = s;
@@ -469,6 +494,7 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
   const int* fresh = first + n;
   const int* hop_end = fresh + n;
   const int* has_state = hop_end + k;
+  const int* hop_frames = warm ? has_state + k : nullptr;
 
   // ---- 1. one compact tail per staged hop, each slot's tail after its last hop
   {
@@ -500,9 +526,10 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
                                                  n_edge == 2 ? a->stage + 4 * KOE_N_MELS : nullptr};
     const float* cfmax[1 + 2 * KOE_MAX_EDGE] = {a->fmax_f, a->fmax_r, a->stage_max + 2, a->fmax_r2,
                                                 n_edge == 2 ? a->stage_max + 4 : nullptr};
-    // the window that completes at hop n starts at frame n + 1 - W = g + lag + 1 - W: ring row (row + lag + H) mod R
+    // the window that completes at hop n starts at frame n + 1 - W = g + lag + 1 - W: ring row (row + lag + H) mod R (a
+    // warm-up window at frame 0, which the core derives from its frame count)
     if (int rc = launch_dual_stream_pool_hops(a->weights, cpower, cfmax, n_edge, k, R, hop_end, hop_slot, hop_row, lag + H,
-                                              a->expr_sigmoid, a->out, a->precision, stream))
+                                              hop_frames, a->expr_sigmoid, a->out, a->precision, stream))
       return rc;
     if (a->ema_state != nullptr) {
       pool_hops_ema_kernel<<<(k * KOE_N_BLENDSHAPES + 255) / 256, 256, 0, st>>>(a->out, k, a->alpha, a->ema_state, hop_end,
@@ -514,9 +541,8 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
   // ---- the clocks advance once everything is queued
   for (int i = 0; i < n; ++i) {
     const int s = slots_host[i], c = counts_host[i];
-    const int64_t after = pool->hops[s] + c;
-    pool->frames[s] += std::min<int64_t>(c, std::max<int64_t>(0, after - (W - 1)));
-    pool->hops[s] = after;
+    pool->frames[s] += completing(pool->hops[s], c);
+    pool->hops[s] += c;
     pool->row[s] += c;
     if (pool->row[s] >= R) pool->row[s] -= R;
   }

@@ -17,7 +17,8 @@ L0[n+1] -- 5 FFTs per hop against 513.  F and R rows go into per-stream rings of
 rings directly (``koe_dual_stream_ring``).  After the 256th hop every step emits the frame that
 ``SequentialDualStreamModel.forward`` would produce for the window ending at the newest sample, EMA included.
 All streams of a StreamingEngine advance in lockstep (one hop per step each); in a StreamPool every stream opens,
-closes and advances on its own clock, by one hop per push or by several in one push_hops.
+closes and advances on its own clock, by one hop per push or by several in one push_hops, and a warm-up StreamPool
+emits from each stream's first hop on, computed on the audio heard so far.
 """
 from __future__ import annotations
 
@@ -222,9 +223,22 @@ class StreamPool:
 
     ``max_hops`` > 1 lets :meth:`push_hops` advance a stream by up to that many hops in one call (late packets after a
     jitter buffer drains, chunked audio, a backlog): the rings then hold ``W + max_hops - 1`` rows, and the per-call
-    buffers are sized for ``capacity * max_hops`` hops."""
+    buffers are sized for ``capacity * max_hops`` hops.
 
-    def __init__(self, model, capacity: int, max_hops: int = 1):
+    ``warmup=True`` makes every pushed hop of every stream emit a frame from the stream's hop 0 on, instead of after
+    8.5 s (``KOE_POOL_WARMUP``):
+
+    * at hops h >= W - 1 the unsmoothed frame is bit for bit the one a pool without warm-up gives;
+    * at hops h < W - 1 it is :meth:`SimplifiedDualStreamModel.forward` (smoothing off) on the audio heard so far, the
+      stream's first ``(h + 1) * hop`` samples (up to the frontend's rounding): ``h + 2`` frames, the long-term part
+      those frames zero-padded, the short-term detail their last three;
+    * the temporal smoothing runs over every frame since the stream opened: its hop-0 frame passes unchanged and each
+      later frame is smoothed onto the one before, so with smoothing on the frames from hop W - 1 on are the smoothing
+      of this pool's own frames and differ from those of a pool without warm-up.
+
+    :meth:`push` on a warm-up pool runs the burst path with counts of 1, whatever ``max_hops`` is."""
+
+    def __init__(self, model, capacity: int, max_hops: int = 1, warmup: bool = False):
         self.model = model
         self.capacity = int(capacity)
         if self.capacity < 1:
@@ -235,6 +249,9 @@ class StreamPool:
             raise ValueError(f"max_hops must be an integer, got {type(max_hops).__name__}") from None
         if isinstance(max_hops, bool) or self.max_hops < 1:
             raise ValueError(f"max_hops must be an integer >= 1, got {max_hops!r}")
+        if not isinstance(warmup, bool):
+            raise ValueError(f"warmup must be a bool, got {type(warmup).__name__}")
+        self.warmup = warmup
         self.dev = next(model.parameters()).device
         if self.dev.type != "cuda":
             raise RuntimeError("StreamPool needs the model on a CUDA device")
@@ -271,15 +288,16 @@ class StreamPool:
         self.expr_compact = torch.empty(cap, **f32)
         self.state = torch.zeros(cap, 52, **f32)
         self.out = torch.zeros(hops, 52, **f32)
-        self.tables = torch.empty(6 * hops, dtype=torch.int32, device=self.dev)
+        self.tables = torch.empty((7 if warmup else 6) * hops, dtype=torch.int32, device=self.dev)
         self._emitted = torch.empty(hops, dtype=torch.int32)     # host: the slots of the last push's frames
         self._emitted_hop = torch.empty(hops, dtype=torch.int64)  # host: the hop of each (push_hops)
         self._n_emitted = C.c_int(0)
         self._n_emitted_ref = C.byref(self._n_emitted)
         self._lib = _lib.load()
         h = C.c_void_p()
-        self._check(self._lib.koe_stream_pool_create_ex(cap, self.hop, self.W, self.half, self.max_hops, C.byref(h)),
-                    "koe_stream_pool_create_ex")
+        flags = _lib.POOL_WARMUP if warmup else 0
+        self._check(self._lib.koe_stream_pool_create_ex2(cap, self.hop, self.W, self.half, self.max_hops, flags,
+                                                         C.byref(h)), "koe_stream_pool_create_ex2")
         self._h = h
         self._fe = model._frontend(self.dev)
         self._alpha, self._alpha_key = 0.0, None
@@ -328,7 +346,8 @@ class StreamPool:
     def push(self, slots, hop_audio: torch.Tensor):
         """Advances exactly the listed open streams by one hop each: hop_audio (n, hop) float32 on the model's device,
         row i the next hop of slots[i].  Returns (emitted_slots, frames): a CPU int64 tensor of the streams that emitted
-        a frame in this call, in call order, and their (k, 52) smoothed frames -- a view reused by the next call."""
+        a frame in this call, in call order, and their (k, 52) smoothed frames -- a view reused by the next call.  A
+        stream emits from its hop W - 1 on; on a warm-up pool every listed stream emits, from its hop 0 on."""
         s = self._slots(slots)
         n = s.numel()
         if not isinstance(hop_audio, torch.Tensor):
@@ -353,8 +372,8 @@ class StreamPool:
         stream in call order -- a 1-D tensor of sum(counts) * hop samples or an (sum(counts), hop) tensor.  Every frame
         is bit for bit what one :meth:`push` per hop gives.  Returns (slots, hops, frames): two CPU int64 tensors and a
         (k, 52) view reused by the next call; row r is the frame of stream slots[r] that completes at its hop hops[r]
-        (counted from 0 since the stream was opened; its first frame comes at hop W - 1).  Rows are grouped by stream in
-        call order, hops ascending.  All frames of the call use each stream's expression input as it is now."""
+        (counted from 0 since the stream was opened; its first frame comes at hop W - 1, or at hop 0 on a warm-up pool,
+        where every hop emits).  Rows are grouped by stream in call order, hops ascending.  All frames of the call use each stream's expression input as it is now."""
         s = self._slots(slots)
         n = s.numel()
         c = counts if isinstance(counts, torch.Tensor) else torch.as_tensor(counts, dtype=torch.int64)
