@@ -454,7 +454,8 @@ int koe_forward_windows(const koe_forward_args* args, void* stream);
  * cannot be captured into a CUDA graph.  Queues the kernels of koe_forward_windows, chained the same way (no early
  * release): frontend, 2 * n_edge edge-variant launches (none when no clip uses them), emotion stream, core and, when
  * smooth != 0 and some clip has more than one frame, the smoothing.  Only the default filterbank (sr 16000, 80 mels,
- * 80..8000 Hz) is implemented; other banks return KOE_E_UNSUPPORTED.
+ * 80..8000 Hz) is implemented; other banks return KOE_E_UNSUPPORTED.  koe_forward_varlen_ex below adds the warm-up
+ * frames: a frame at every hop of the output grid from the clip's first hop on.
  */
 typedef struct {
   const koe_frontend_t* frontend;
@@ -477,6 +478,33 @@ typedef struct {
 int koe_forward_varlen_size(const koe_forward_varlen_args* args, int64_t* n_windows, int64_t* n_frames,
                             int64_t* workspace_bytes);
 int koe_forward_varlen(const koe_forward_varlen_args* args, void* stream);
+
+/*
+ * The same with a flags word; flags = 0 is koe_forward_varlen / koe_forward_varlen_size, any bit but KOE_VARLEN_WARMUP
+ * returns KOE_E_INVALID.
+ *
+ * KOE_VARLEN_WARMUP: the frames a KOE_POOL_WARMUP stream pool would emit for each clip, in one call.  With W =
+ * window_frames, s = stride_frames and n_c = L_c / hop complete hops, the output grid is the hops h = W - 1 (mod s) from
+ * r = (W - 1) mod s on, and clip c gets one row per grid hop it completes: h = r, r + s, .. <= n_c - 1, ascending (rows
+ * [sum of the rows of the clips < c, + those of clip c); n_windows of koe_forward_varlen_size_ex counts them).
+ *   - Rows at h >= W - 1 are the windows of koe_forward_varlen (n_out_c of them when n_c >= W, else none), from the same
+ *     frontend rows: bit for bit its rows when smooth = 0.  The padded single window of a clip with n_c < W is not a row.
+ *   - Rows at h < W - 1 (lead windows) are SimplifiedDualStreamModel.forward on the clip's first (h + 1) * hop samples:
+ *     T = h + 2 frames, the last n_edge of them window-end variants that see zeros from sample (h + 1) * hop on, no
+ *     window-start variants; long-term part zero padded to mel_seq, short-term detail the last three frames, dB
+ *     reference their maximum -- the frames of a warm-up pool at those hops.
+ *   - smooth != 0: the EMA restarts at each clip's first row and runs over all of its rows, so rows from W - 1 on are
+ *     the smoothing of this call's own rows (as a warm-up pool's frames differ from a plain pool's).
+ *   - A clip that completes no grid hop (L_c < (r + 1) * hop) returns KOE_E_INVALID before anything is queued.
+ * Launches: those of koe_forward_varlen (the plain and the 2 * n_edge steady edge-variant launches unchanged: the same
+ * frames per clip, the same frame pairs), plus n_edge lead-variant frontend launches when some clip has a lead window
+ * (any clip, when s < W), before the emotion stream; the core and the smoothing run over the rows above.  The workspace
+ * grows by n_edge window-end buffers of one row per lead window.
+ */
+#define KOE_VARLEN_WARMUP 1
+int koe_forward_varlen_size_ex(const koe_forward_varlen_args* args, int flags, int64_t* n_windows, int64_t* n_frames,
+                               int64_t* workspace_bytes);
+int koe_forward_varlen_ex(const koe_forward_varlen_args* args, int flags, void* stream);
 
 /*
  * Learnable-alpha exponential smoothing along the frame axis, in place

@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libkoemorph_b200.so")
 KOE_NO_EDGE = -1000000
 MAX_EDGE = 2
 POOL_WARMUP = 1       # KOE_POOL_WARMUP: koe_stream_pool_create_ex2 flag
+VARLEN_WARMUP = 1     # KOE_VARLEN_WARMUP: koe_forward_varlen_ex / koe_forward_varlen_size_ex flag
 # 1 was reserved for a tf32 tensor-core core that was never built: the ABI rejects it
 PRECISIONS = {"fp32": 0, "bf16": 2}
 
@@ -136,6 +137,9 @@ _SIGNATURES = {
     "koe_forward_varlen_size": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
                                           C.POINTER(C.c_int64)]),
     "koe_forward_varlen": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.c_void_p]),
+    "koe_forward_varlen_size_ex": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.c_int, C.POINTER(C.c_int64),
+                                             C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "koe_forward_varlen_ex": (C.c_int, [C.POINTER(ForwardVarlenArgs), C.c_int, C.c_void_p]),
     "koe_stream_pool_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "koe_stream_pool_create_ex": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "koe_stream_pool_create_ex2": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,

@@ -49,6 +49,12 @@ struct CoreParams {
   // frames_per_window; a window shorter than frames_per_window starts at its stream's sample 0 and has no window-start
   // variants.  Everything else as PoolHops.
   const int* hop_frames;
+  // packed warm-up batch (csrc/session.cu; CoreMode::VarlenWarm only): vl_window_base[c] is clip c's first output row;
+  // its first vl_lead_base[c + 1] - vl_lead_base[c] rows are lead windows, whose window-end rows (variants 2, 4) are rows
+  // vl_lead_base[c] .. of power[2] / power[4]; the rest are the windows of CoreMode::Varlen, whose edge rows start at
+  // vl_edge_base[c]
+  const int* vl_edge_base;
+  const int* vl_lead_base;
 };
 
 // Which flavour of the core a launch runs.  Each is a separate instantiation of both kernels (the fp32 kernel has no
@@ -62,7 +68,9 @@ struct CoreParams {
 //            the window-end rows that hop hop_end[w] staged
 //   PoolWarm a burst of a warm-up pool: PoolHops with hop_frames[w] frames in window w; below frames_per_window the
 //            window is the stream's whole audio so far: plain rows, then the n_edge window-end rows, no window-start rows
-enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops, PoolWarm };
+//   VarlenWarm a packed warm-up batch: Varlen with a clip's lead windows first -- the window at grid hop h < W - 1 is the
+//            clip's first h + 2 frames, shaped as a PoolWarm window below frames_per_window
+enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops, PoolWarm, VarlenWarm };
 
 // frame k of a window: which buffer (variant) holds it (see koe_dual_stream_windows in the header)
 __device__ __forceinline__ int window_variant(const CoreParams& p, int k) {
@@ -104,13 +112,15 @@ struct CoreWindow {
                     // global window, which is also the window's row in every edge-variant buffer (Varlen)
   bool plain_only;  // Varlen: the clip has no edge variants, every frame comes from the plain rows
   int hop;          // PoolHops, PoolWarm: the staged hop at which the window completes (its window-end rows)
-  int frames;       // PoolWarm: the window's frame count
+  int frames;       // PoolWarm, VarlenWarm: the window's frame count
 };
 
 // The window resolver of each mode: work item `item` is output row `item` and reads the window window<kWarp>(p, item);
 // frame k of it, variant v, is row row(p, w, v, k) of p.power[v] / p.fmax[v].
 template <CoreMode M>
 struct CoreRows {
+  // every window carries its own frame count (CoreWindow::frames), from 2 to frames_per_window
+  static constexpr bool kWindowFrames = M == CoreMode::PoolWarm || M == CoreMode::VarlenWarm;
   // kWarp: every lane of a converged warp calls with the same item (Varlen searches the clip with the whole warp)
   template <bool kWarp>
   static __device__ __forceinline__ CoreWindow window(const CoreParams& p, int item) {
@@ -130,12 +140,22 @@ struct CoreRows {
       const int c = varlen_clip<kWarp>(p, item);
       return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, item,
               __ldg(p.vl_plain_only + c) != 0};
+    } else if constexpr (M == CoreMode::VarlenWarm) {
+      const int c = varlen_clip<kWarp>(p, item);
+      const int local = item - __ldg(p.vl_window_base + c), lead0 = __ldg(p.vl_lead_base + c);
+      const int leads = __ldg(p.vl_lead_base + c + 1) - lead0;
+      if (local < leads)  // grid hop h = r + local * stride, r = (W - 1) mod stride: T = h + 2 frames from the clip's frame 0
+        return {__ldg(p.vl_frame_base + c), lead0 + local, false, 0,
+                (p.frames_per_window - 2) % p.stride_frames + local * p.stride_frames + 2};
+      const int j = local - leads;  // steady window j: as Varlen
+      return {__ldg(p.vl_frame_base + c) + j * p.stride_frames, __ldg(p.vl_edge_base + c) + j,
+              __ldg(p.vl_plain_only + c) != 0, 0, p.frames_per_window};
     } else {
       return {item / p.n_out, item % p.n_out, false};
     }
   }
   static __device__ __forceinline__ long long row(const CoreParams& p, const CoreWindow& w, int variant, int k) {
-    if constexpr (M == CoreMode::Varlen) {
+    if constexpr (M == CoreMode::Varlen || M == CoreMode::VarlenWarm) {
       return variant == 0 ? (long long)w.owner + k : (long long)w.pos;
     } else if constexpr (M == CoreMode::Pool) {
       return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
@@ -151,20 +171,21 @@ struct CoreRows {
                           : (long long)w.owner * p.n_out + w.pos;
     }
   }
-  // the window's frame count: T, the launch's frames_per_window, in every mode but PoolWarm
+  // the window's frame count: T, the launch's frames_per_window, unless kWindowFrames
   static __device__ __forceinline__ int frames(const CoreWindow& w, int T) {
-    if constexpr (M == CoreMode::PoolWarm) return w.frames;
+    if constexpr (kWindowFrames) return w.frames;
     return T;
   }
-  // whether the window's first n_edge frames have window-start variants (see window_variant); not in a PoolWarm
-  // window shorter than frames_per_window: it starts at sample 0 of its stream, and its plain rows see zeros before that
+  // whether the window's first n_edge frames have window-start variants (see window_variant); not in a kWindowFrames
+  // window shorter than frames_per_window: it starts at sample 0 of its stream or clip, and its plain rows see zeros
+  // before that
   static __device__ __forceinline__ bool window_starts(const CoreParams& p, const CoreWindow& w) {
-    if constexpr (M == CoreMode::PoolWarm) return w.frames == p.frames_per_window;
+    if constexpr (kWindowFrames) return w.frames == p.frames_per_window;
     return true;
   }
   // frame k of window w with frames(w, T) = T: which buffer (variant) holds it
   static __device__ __forceinline__ int variant(const CoreParams& p, const CoreWindow& w, int T, int k) {
-    if constexpr (M == CoreMode::PoolWarm) {
+    if constexpr (kWindowFrames) {
       if (T < p.frames_per_window) return k >= T - p.n_edge ? 2 + 2 * (T - 1 - k) : 0;
     }
     return window_variant(p, k);
@@ -186,7 +207,7 @@ struct CoreRows {
   // the L2 policy of a window's plain rows: `reread` where other windows read them again (the overlapping windows of a
   // sequence or of a varlen clip), else `once`
   static __device__ __forceinline__ uint64_t plain_rows_policy(const CoreParams& p, uint64_t reread, uint64_t once) {
-    return M == CoreMode::Varlen || p.n_out > 1 ? reread : once;
+    return M == CoreMode::Varlen || M == CoreMode::VarlenWarm || p.n_out > 1 ? reread : once;
   }
 };
 
@@ -221,6 +242,15 @@ int launch_dual_stream_varlen(const koe_core_weights* w, const float* const* pow
                               int n_edge, int n_windows, int n_frames, int stride_frames, int frames_per_window, int n_clips,
                               const int* window_base, const int* frame_base, const int* plain_only, float* out,
                               float* sigmoid_out, float* attn_out, int precision, void* stream);
+// the core over the rows of a packed warm-up batch (csrc/session.cu, CoreMode::VarlenWarm): output row `item` of the
+// n_rows belongs to the clip c with row_base[c] <= item < row_base[c + 1]; the clip's first lead_base[c + 1] -
+// lead_base[c] rows are its lead windows (window-end rows power[2], power[4] from lead_base[c]), the rest its windows of
+// launch_dual_stream_varlen with edge rows from edge_base[c]; expression entries are written by the emotion kernel
+int launch_dual_stream_varlen_warm(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
+                                   int n_edge, int n_rows, int n_frames, int stride_frames, int frames_per_window,
+                                   int n_clips, const int* row_base, const int* frame_base, const int* edge_base,
+                                   const int* lead_base, const int* plain_only, float* out, float* sigmoid_out,
+                                   float* attn_out, int precision, void* stream);
 // segmented EMA of a packed variable-length batch: clip c's frames are rows [row_base[c], row_base[c + 1]) of `frames`
 int launch_ema_scan_varlen(float* frames, int n_clips, const int* row_base, float alpha, void* stream);
 // how many SMs' worth of CTAs the tensor-core core launches for n_items windows (the early-release split follows it)

@@ -320,11 +320,11 @@ __global__ void __launch_bounds__(kThreads, 1) dual_stream_tc_kernel(CoreParams 
   const bool tma_mel = p.mel_long == nullptr;
   const int Tl = min(T, p.mel_seq);                              // long-term frames actually present
   const int n_mel_stages = tma_mel ? (Tl + kMelRows - 1) / kMelRows : 0;
-  // the same for a window of wT = Rows::frames(win, T) frames: the launch's own except in PoolWarm, where every window
-  // has its own count (the mel-row producer and the SIMT warps derive the stage count from the same window)
-  auto long_frames = [&](int wT) { return M == CoreMode::PoolWarm ? min(wT, p.mel_seq) : Tl; };
+  // the same for a window of wT = Rows::frames(win, T) frames: the launch's own unless every window has its own count
+  // (Rows::kWindowFrames; the mel-row producer and the SIMT warps derive the stage count from the same window)
+  auto long_frames = [&](int wT) { return Rows::kWindowFrames ? min(wT, p.mel_seq) : Tl; };
   auto mel_stages = [&](int wTl) {
-    return M == CoreMode::PoolWarm ? (tma_mel ? (wTl + kMelRows - 1) / kMelRows : 0) : n_mel_stages;
+    return Rows::kWindowFrames ? (tma_mel ? (wTl + kMelRows - 1) / kMelRows : 0) : n_mel_stages;
   };
 
   if (warp == 8) {
@@ -961,7 +961,7 @@ int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t strea
   if (mode == CoreMode::Early)
     KOE_REQUIRE(p.n_out == 1 && p.early_items > 0 && p.early_items % grid == 0 && p.early_target > 0,
                 "tensor-core path: bad early-release parameters");
-  if (mode == CoreMode::Varlen)
+  if (mode == CoreMode::Varlen || mode == CoreMode::VarlenWarm)
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames == 0 && p.expr_sigmoid == nullptr, "tensor-core path: bad varlen parameters");
   if (mode == CoreMode::Pool || mode == CoreMode::PoolHops || mode == CoreMode::PoolWarm)
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
@@ -976,6 +976,7 @@ int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t strea
     case CoreMode::Varlen: rc = launch_tc<CoreMode::Varlen>(p, grid, stream); break;
     case CoreMode::PoolHops: rc = launch_tc<CoreMode::PoolHops>(p, grid, stream); break;
     case CoreMode::PoolWarm: rc = launch_tc<CoreMode::PoolWarm>(p, grid, stream); break;
+    case CoreMode::VarlenWarm: rc = launch_tc<CoreMode::VarlenWarm>(p, grid, stream); break;
   }
   if (rc != KOE_OK) return rc;
   count_launch();

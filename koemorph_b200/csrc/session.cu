@@ -256,29 +256,40 @@ extern "C" int koe_forward_windows(const koe_forward_args* a, void* stream) {
   return KOE_OK;
 }
 
-// ---- packed variable-length batch (see koe_forward_varlen in the header) -------------------------------------------------
+// ---- packed variable-length batch (see koe_forward_varlen and koe_forward_varlen_ex in the header) ----------------------
 // Per-clip tables, int32 words (the int64 sample offsets first, so that they are 8-byte aligned):
 //   sample_off [B] int64 | length [B] | frame_base [B + 1] | window_base [B + 1] | pair_base [B + 1] | edge_pair_base [B + 1]
 //   | plain_only [B]
+// and with KOE_VARLEN_WARMUP | row_base [B + 1] | lead_base [B + 1] | lead_pair_base [B + 1].
 // pair_base counts the frame pairs of the plain launch (ceil(n_frames_c / 2) per clip), edge_pair_base those of each
-// edge-variant launch (ceil(n_out_c / 2), none for a clip that reads its window from the plain rows).
+// edge-variant launch (ceil(n_out_c / 2), none for a clip that reads its window from the plain rows).  Warm-up: clip c
+// has K_c lead windows (the grid hops h <= min(W - 2, n_c - 1)) and its steady windows (n_out_c when n_c >= W, else
+// none); row_base is the first output row, lead_base the first lead row of the window-end buffers, lead_pair_base counts
+// the frame pairs of each lead-variant launch (ceil(K_c / 2)).  The plain and edge-variant launches and their tables are
+// those of the plain call.
 // Workspace (16-byte aligned regions): power[0] [F][80] | power[1 .. 2 n_edge] [N][80] each | frame_max[0] [F] |
-// frame_max[1 .. 2 n_edge] [N] each | tables.
+// frame_max[1 .. 2 n_edge] [N] each | tables.  Warm-up: the window-end buffers power[2 + 2m] / frame_max[2 + 2m] hold the
+// Sum K_c lead rows after their N steady rows (N = 0 when no clip uses steady edge variants), and there are as many
+// variant buffers as the steady or the lead windows need.
 namespace {
-constexpr int kVarlenTableWords = 8;  // table words per clip (+ 4)
+constexpr int kVarlenTableWords = 8;      // table words per clip (+ 4)
+constexpr int kVarlenWarmTableWords = 3;  // more with KOE_VARLEN_WARMUP (+ 3)
 
 struct VarlenPlan {
-  int n_edge = 0;            // edge variants per window side (0: no clip uses them)
-  int max_out = 0;           // most frames of one clip
+  int n_edge = 0;            // edge variants per window side of the steady windows (0: no clip uses them)
+  int lead_edge = 0;         // window-end variants of the lead windows (0: no clip has one)
+  int max_out = 0;           // most output rows of one clip
   long long windows = 0, frames = 0, pairs = 0, edge_pairs = 0;
+  long long rows = 0, leads = 0, lead_pairs = 0;  // output rows; warm-up: lead windows and their frame pairs per launch
   size_t off_power[1 + 2 * KOE_MAX_EDGE] = {}, off_fmax[1 + 2 * KOE_MAX_EDGE] = {}, off_tables = 0, bytes = 0;
+  size_t table_words = 0;
 };
 
 size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
-// Validates the lengths and geometry of `a`, sums up the per-clip geometry (the rules of SequentialDualStreamModel) and lays
-// out the workspace; with tables != NULL also writes the per-clip tables.
-int plan_varlen(const koe_forward_varlen_args* a, VarlenPlan* pl, int32_t* tables) {
+// Validates the lengths and geometry of `a`, sums up the per-clip geometry (the rules of SequentialDualStreamModel; with
+// `warm`, the grid of KOE_VARLEN_WARMUP) and lays out the workspace; with tables != NULL also writes the per-clip tables.
+int plan_varlen(const koe_forward_varlen_args* a, bool warm, VarlenPlan* pl, int32_t* tables) {
   KOE_REQUIRE(a != nullptr && pl != nullptr, "koe_forward_varlen: NULL argument");
   KOE_REQUIRE(a->n_clips >= 0 && (a->n_clips == 0 || a->lengths_host != nullptr), "koe_forward_varlen: bad n_clips / lengths");
   KOE_REQUIRE(a->n_clips < (1 << 26), "koe_forward_varlen: %d clips (at most 2^26)", a->n_clips);
@@ -288,9 +299,10 @@ int plan_varlen(const koe_forward_varlen_args* a, VarlenPlan* pl, int32_t* table
   const int n_edge = (a->half_fft + hop - 1) / hop;
   KOE_REQUIRE(n_edge <= KOE_MAX_EDGE && W + 1 > 2 * n_edge,
               "koe_forward_varlen: hop %d needs %d edge frames per window side (max %d)", hop, n_edge, KOE_MAX_EDGE);
+  const int r = (W - 1) % stride;  // the first hop of the output grid h = W - 1 (mod stride)
   int64_t* sample_off = nullptr;
   int32_t *length = nullptr, *frame_base = nullptr, *window_base = nullptr, *pair_base = nullptr, *edge_pair_base = nullptr,
-          *plain_only = nullptr;
+          *plain_only = nullptr, *row_base = nullptr, *lead_base = nullptr, *lead_pair_base = nullptr;
   if (tables != nullptr) {
     sample_off = reinterpret_cast<int64_t*>(tables);
     length = tables + 2 * (size_t)B;
@@ -299,18 +311,23 @@ int plan_varlen(const koe_forward_varlen_args* a, VarlenPlan* pl, int32_t* table
     pair_base = window_base + B + 1;
     edge_pair_base = pair_base + B + 1;
     plain_only = edge_pair_base + B + 1;
+    if (warm) {
+      row_base = plain_only + B;
+      lead_base = row_base + B + 1;
+      lead_pair_base = lead_base + B + 1;
+    }
   }
   *pl = VarlenPlan();
   long long samples = 0;
   bool any_edge = false;
-  for (int c = 0; c <= B; ++c) {
+  for (int c = 0; c < B; ++c) {
     if (tables != nullptr) {
       frame_base[c] = (int32_t)pl->frames;
       window_base[c] = (int32_t)pl->windows;
       pair_base[c] = (int32_t)pl->pairs;
       edge_pair_base[c] = (int32_t)pl->edge_pairs;
+      if (warm) row_base[c] = (int32_t)pl->rows, lead_pair_base[c] = (int32_t)pl->lead_pairs;
     }
-    if (c == B) break;
     const int64_t L = a->lengths_host[c];
     KOE_REQUIRE(L >= 0 && L < (1ll << 30), "koe_forward_varlen: length %lld of clip %d outside [0, 2^30)", (long long)L, c);
     // num_output_frames: max(1, floor((L // hop - W) / stride) + 1) -- a negative numerator gives 1 either way
@@ -318,44 +335,90 @@ int plan_varlen(const koe_forward_varlen_args* a, VarlenPlan* pl, int32_t* table
     const long long n_out = rel < 0 ? 1 : rel / stride + 1;
     const long long n_frames = (n_out - 1) * stride + W + 1;
     const bool plain = n_out == 1 && L <= (long long)W * hop;  // one window spanning the whole clip: no interior edges
+    // warm-up: the grid hops r, r + stride, .. the clip completes; below W - 1 they are lead windows
+    long long leads = 0, clip_rows = n_out;
+    if (warm) {
+      const long long last_lead = std::min<long long>(W - 2, L / hop - 1);
+      leads = last_lead < r ? 0 : (last_lead - r) / stride + 1;
+      clip_rows = leads + (rel < 0 ? 0 : n_out);
+      KOE_REQUIRE(clip_rows > 0,
+                  "koe_forward_varlen_ex: clip %d of %lld samples completes no hop of the output grid (hop %d, first "
+                  "output at %d complete hops)", c, (long long)L, hop, r + 1);
+    }
     any_edge = any_edge || !plain;
     if (tables != nullptr) {
       sample_off[c] = samples;
       length[c] = (int32_t)L;
       plain_only[c] = plain ? 1 : 0;
+      if (warm) lead_base[c] = (int32_t)pl->leads;  // (+ the steady window-end rows, below)
     }
     samples += L;
     pl->windows += n_out;
     pl->frames += n_frames;
     pl->pairs += (n_frames + 1) / 2;
     pl->edge_pairs += plain ? 0 : (n_out + 1) / 2;
-    pl->max_out = (int)std::max<long long>(pl->max_out, n_out);
-    KOE_REQUIRE(pl->frames < (1ll << 31) - 32 && pl->windows < (1ll << 31), "koe_forward_varlen: more than 2^31 frames or windows");
+    pl->rows += clip_rows;
+    pl->leads += leads;
+    pl->lead_pairs += (leads + 1) / 2;
+    pl->max_out = (int)std::max<long long>(pl->max_out, clip_rows);
+    KOE_REQUIRE(pl->frames < (1ll << 31) - 32 && pl->windows < (1ll << 31) && pl->rows < (1ll << 31),
+                "koe_forward_varlen: more than 2^31 frames or windows");
   }
   pl->n_edge = any_edge ? n_edge : 0;
+  pl->lead_edge = pl->leads > 0 ? n_edge : 0;
+  const long long steady_rows = pl->n_edge > 0 ? pl->windows : 0;  // rows of each steady edge-variant buffer
+  KOE_REQUIRE(steady_rows + pl->leads < (1ll << 31), "koe_forward_varlen: more than 2^31 edge-variant rows");
+  if (tables != nullptr) {
+    frame_base[B] = (int32_t)pl->frames;
+    window_base[B] = (int32_t)pl->windows;
+    pair_base[B] = (int32_t)pl->pairs;
+    edge_pair_base[B] = (int32_t)pl->edge_pairs;
+    if (warm) {
+      row_base[B] = (int32_t)pl->rows, lead_pair_base[B] = (int32_t)pl->lead_pairs;
+      for (int c = 0; c < B; ++c) lead_base[c] += (int32_t)steady_rows;
+      lead_base[B] = (int32_t)(steady_rows + pl->leads);
+    }
+  }
+  const int n_var = 2 * std::max(pl->n_edge, pl->lead_edge);
+  // (window-start variants 1, 3: steady rows only; window-end variants 2, 4: steady rows, then the lead rows)
+  auto var_rows = [&](int j) { return (size_t)(steady_rows + (j % 2 == 0 ? pl->leads : 0)); };
   size_t off = 0;
   pl->off_power[0] = off, off += align16((size_t)pl->frames * KOE_N_MELS * sizeof(float));
-  for (int j = 1; j <= 2 * pl->n_edge; ++j) pl->off_power[j] = off, off += align16((size_t)pl->windows * KOE_N_MELS * sizeof(float));
+  for (int j = 1; j <= n_var; ++j) pl->off_power[j] = off, off += align16(var_rows(j) * KOE_N_MELS * sizeof(float));
   pl->off_fmax[0] = off, off += align16((size_t)pl->frames * sizeof(float));
-  for (int j = 1; j <= 2 * pl->n_edge; ++j) pl->off_fmax[j] = off, off += align16((size_t)pl->windows * sizeof(float));
-  pl->off_tables = off, off += align16(((size_t)kVarlenTableWords * B + 4) * sizeof(int32_t));
+  for (int j = 1; j <= n_var; ++j) pl->off_fmax[j] = off, off += align16(var_rows(j) * sizeof(float));
+  pl->table_words = (size_t)kVarlenTableWords * B + 4 + (warm ? (size_t)kVarlenWarmTableWords * B + 3 : 0);
+  pl->off_tables = off, off += align16(pl->table_words * sizeof(int32_t));
   pl->bytes = off;
+  return KOE_OK;
+}
+
+int varlen_flags(int flags, const char* what) {
+  KOE_REQUIRE((flags & ~KOE_VARLEN_WARMUP) == 0, "%s: unknown flags 0x%x", what, (unsigned)flags);
   return KOE_OK;
 }
 }  // namespace
 
-extern "C" int koe_forward_varlen_size(const koe_forward_varlen_args* a, int64_t* n_windows, int64_t* n_frames,
-                                       int64_t* workspace_bytes) {
+extern "C" int koe_forward_varlen_size_ex(const koe_forward_varlen_args* a, int flags, int64_t* n_windows,
+                                          int64_t* n_frames, int64_t* workspace_bytes) {
   KOE_REQUIRE(n_windows != nullptr && n_frames != nullptr && workspace_bytes != nullptr, "koe_forward_varlen_size: NULL argument");
+  if (int rc = varlen_flags(flags, "koe_forward_varlen_size_ex")) return rc;
   VarlenPlan pl;
-  if (int rc = plan_varlen(a, &pl, nullptr)) return rc;
-  *n_windows = pl.windows, *n_frames = pl.frames, *workspace_bytes = (int64_t)pl.bytes;
+  if (int rc = plan_varlen(a, flags & KOE_VARLEN_WARMUP, &pl, nullptr)) return rc;
+  *n_windows = pl.rows, *n_frames = pl.frames, *workspace_bytes = (int64_t)pl.bytes;
   return KOE_OK;
 }
 
-extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream) {
+extern "C" int koe_forward_varlen_size(const koe_forward_varlen_args* a, int64_t* n_windows, int64_t* n_frames,
+                                       int64_t* workspace_bytes) {
+  return koe_forward_varlen_size_ex(a, 0, n_windows, n_frames, workspace_bytes);
+}
+
+extern "C" int koe_forward_varlen_ex(const koe_forward_varlen_args* a, int flags, void* stream) {
+  if (int rc = varlen_flags(flags, "koe_forward_varlen_ex")) return rc;
+  const bool warm = flags & KOE_VARLEN_WARMUP;
   VarlenPlan pl;
-  if (int rc = plan_varlen(a, &pl, nullptr)) return rc;
+  if (int rc = plan_varlen(a, warm, &pl, nullptr)) return rc;
   if (a->n_clips == 0) return KOE_OK;
   KOE_REQUIRE(a->frontend != nullptr && a->weights != nullptr, "koe_forward_varlen: NULL frontend / weights");
   KOE_REQUIRE(a->weights->k_mel == a->window_frames + 3, "koe_forward_varlen: weights for k_mel %d, window_frames %d",
@@ -370,16 +433,17 @@ extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream
     return fail(KOE_E_UNSUPPORTED, "koe_forward_varlen: implemented for the default filterbank only");
   if (int rc = check_capture(stream, "koe_forward_varlen")) return rc;
   const int B = a->n_clips;
+  const int core_edge = std::max(pl.n_edge, pl.lead_edge);
   char* ws = static_cast<char*>(a->workspace);
   float* power[1 + 2 * KOE_MAX_EDGE] = {};
   float* fmax[1 + 2 * KOE_MAX_EDGE] = {};
-  for (int j = 0; j <= 2 * pl.n_edge; ++j)
+  for (int j = 0; j <= 2 * core_edge; ++j)
     power[j] = reinterpret_cast<float*>(ws + pl.off_power[j]), fmax[j] = reinterpret_cast<float*>(ws + pl.off_fmax[j]);
   int32_t* dev_tables = reinterpret_cast<int32_t*>(ws + pl.off_tables);
-  const size_t words = (size_t)kVarlenTableWords * B + 4;
+  const size_t words = pl.table_words;
   TableStaging* stage = nullptr;
   if (int rc = acquire_table_staging(stream, words, &stage)) return rc;
-  if (int rc = plan_varlen(a, &pl, stage->host)) return rc;
+  if (int rc = plan_varlen(a, warm, &pl, stage->host)) return rc;
   if (int rc = upload_tables(stage, dev_tables, words, (cudaStream_t)stream)) return rc;
   const long long* sample_off = reinterpret_cast<const long long*>(dev_tables);
   const int* length = dev_tables + 2 * (size_t)B;
@@ -388,6 +452,9 @@ extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream
   const int* pair_base = window_base + B + 1;
   const int* edge_pair_base = pair_base + B + 1;
   const int* plain_only = edge_pair_base + B + 1;
+  const int* row_base = warm ? plain_only + B : window_base;  // each clip's first output row
+  const int* lead_base = row_base + B + 1;                    // (warm-up only)
+  const int* lead_pair_base = lead_base + B + 1;
   const int T = a->window_frames + 1;
 
   koe_logmel_args f = {};
@@ -415,17 +482,39 @@ extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream
                                &edges))
       return rc;
   }
+  // warm-up: the lead window at grid hop h = r + j * stride ends on the window-end variants m < n_edge, frame h + 1 - m
+  // with zeros from sample (h + 1) * hop on -- frame j of a launch with frame_offset r + 1 - m
+  if (pl.lead_edge > 0) {
+    const VarlenTables leads = {sample_off, length, lead_pair_base, lead_base, B, pl.lead_pairs};
+    const int r = (a->window_frames - 1) % a->stride_frames;
+    for (int m = 0; m < pl.lead_edge; ++m) {
+      f.frame_step = a->stride_frames;
+      f.frame_offset = r + 1 - m, f.lo_rel_hops = KOE_NO_EDGE, f.hi_rel_hops = m;
+      f.power = power[2 + 2 * m], f.frame_max = fmax[2 + 2 * m];
+      if (int rc = launch_logmel(a->frontend, &f, FrontendMode::Varlen, /*follows_frontend_launch=*/true, stream, nullptr,
+                                 &leads))
+        return rc;
+    }
+  }
   // as in koe_forward_windows: the emotion kernel writes the expression entries of each clip's rows, the core the rest
   if (int rc = launch_emotion_stream(a->weights, a->egemaps, B, nullptr, a->out, a->sigmoid_out, 1, stream,
-                                     /*after_frontend=*/true, window_base))
+                                     /*after_frontend=*/true, row_base))
     return rc;
   const float* cpower[1 + 2 * KOE_MAX_EDGE] = {power[0], power[1], power[2], power[3], power[4]};
   const float* cfmax[1 + 2 * KOE_MAX_EDGE] = {fmax[0], fmax[1], fmax[2], fmax[3], fmax[4]};
-  if (int rc = launch_dual_stream_varlen(a->weights, cpower, cfmax, pl.n_edge, (int)pl.windows, (int)pl.frames,
-                                         a->stride_frames, T, B, window_base, frame_base, plain_only, a->out, a->sigmoid_out,
-                                         a->attn_out, a->precision, stream))
+  if (warm) {
+    if (int rc = launch_dual_stream_varlen_warm(a->weights, cpower, cfmax, core_edge, (int)pl.rows, (int)pl.frames,
+                                                a->stride_frames, T, B, row_base, frame_base, window_base, lead_base,
+                                                plain_only, a->out, a->sigmoid_out, a->attn_out, a->precision, stream))
+      return rc;
+  } else if (int rc = launch_dual_stream_varlen(a->weights, cpower, cfmax, pl.n_edge, (int)pl.windows, (int)pl.frames,
+                                                a->stride_frames, T, B, window_base, frame_base, plain_only, a->out,
+                                                a->sigmoid_out, a->attn_out, a->precision, stream)) {
     return rc;
+  }
   if (a->smooth && pl.max_out > 1)
-    if (int rc = launch_ema_scan_varlen(a->out, B, window_base, a->alpha, stream)) return rc;
+    if (int rc = launch_ema_scan_varlen(a->out, B, row_base, a->alpha, stream)) return rc;
   return KOE_OK;
 }
+
+extern "C" int koe_forward_varlen(const koe_forward_varlen_args* a, void* stream) { return koe_forward_varlen_ex(a, 0, stream); }

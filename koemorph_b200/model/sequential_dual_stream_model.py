@@ -75,7 +75,8 @@ class SequentialDualStreamModel(SimplifiedDualStreamModel):
 
     @torch.no_grad()
     def forward_varlen(self, audio: torch.Tensor, lengths, egemaps: Optional[torch.Tensor] = None,
-                       return_attention: bool = False, out: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+                       return_attention: bool = False, out: Optional[torch.Tensor] = None,
+                       warmup: bool = False) -> Dict[str, torch.Tensor]:
         """A packed batch of clips of different lengths as one native forward (koe_forward_varlen).
 
         ``audio``: 1-D float32 CUDA tensor with the clips back to back, ``audio.numel() == sum(lengths)``; ``lengths``:
@@ -83,7 +84,19 @@ class SequentialDualStreamModel(SimplifiedDualStreamModel):
         ``num_output_frames(lengths[c])`` frames are rows ``frame_offsets[c]:frame_offsets[c + 1]`` of ``blendshapes``
         (N, 52) (and of the attention / sigmoid outputs), each equal to ``forward`` on that clip alone, smoothing
         included.  ``out``: a preallocated contiguous (N, 52) float32 tensor.  Afterwards ``prev_blendshapes`` holds every
-        clip's last frame, (B, 52)."""
+        clip's last frame, (B, 52).
+
+        ``warmup=True`` (koe_forward_varlen_ex with KOE_VARLEN_WARMUP) gives the frames a warm-up ``StreamPool`` would
+        emit for each clip, from its first hop on.  With W = ``mel_sequence_length``, s = ``stride_frames`` and
+        n = ``lengths[c] // hop`` complete hops, clip c gets one row per hop h = W - 1 (mod s) that it completes: h = r,
+        r + s, ... <= n - 1 with r = (W - 1) % s (every hop 0 .. n - 1 when s = 1), ascending.  Rows at h >= W - 1 are,
+        with smoothing off, bit for bit the rows of ``warmup=False``; rows at h < W - 1 are
+        ``SimplifiedDualStreamModel.forward`` on the clip's first (h + 1) * hop samples.  A clip of fewer than W hops
+        gets no padded window.  Smoothing restarts at each clip's first row and runs over all of its rows, so with
+        smoothing on the rows from W - 1 on are the smoothing of these rows, not those of ``warmup=False``.  A clip that
+        completes no grid hop (``lengths[c] < (r + 1) * hop``) raises ``ValueError``."""
+        if not isinstance(warmup, bool):
+            raise ValueError(f"warmup must be a bool, got {type(warmup).__name__}")
         if not isinstance(audio, torch.Tensor) or not audio.is_cuda:
             raise ValueError("audio must be a 1-D float32 CUDA tensor holding the clips back to back")
         audio = _lib.require_cuda(audio, "audio")
@@ -94,7 +107,7 @@ class SequentialDualStreamModel(SimplifiedDualStreamModel):
         dev = audio.device
         eg = self._check_egemaps(egemaps, B, dev)
         hop, W, stride = self.hop_length, self.window_frames, self.stride_frames
-        n_out = torch.clamp((lens // hop - W) // stride + 1, min=1)     # num_output_frames, per clip
+        n_out = self.varlen_rows(lens, warmup)
         offsets = torch.zeros(B + 1, dtype=torch.int64)
         torch.cumsum(n_out, 0, out=offsets[1:])
         N = int(offsets[-1])
@@ -116,18 +129,19 @@ class SequentialDualStreamModel(SimplifiedDualStreamModel):
             a.smooth = 1 if self.use_temporal_smoothing else 0
             a.alpha = self._alpha() if self.use_temporal_smoothing else 0.0
             a.precision = _lib.PRECISIONS[self.precision]
+            flags = _lib.VARLEN_WARMUP if warmup else 0
             n_win, n_frames, ws_bytes = C.c_int64(), C.c_int64(), C.c_int64()
-            _lib.check(lib.koe_forward_varlen_size(C.byref(a), C.byref(n_win), C.byref(n_frames), C.byref(ws_bytes)),
-                       "koe_forward_varlen_size")
+            _lib.check(lib.koe_forward_varlen_size_ex(C.byref(a), flags, C.byref(n_win), C.byref(n_frames),
+                                                      C.byref(ws_bytes)), "koe_forward_varlen_size_ex")
             if n_win.value != N:
-                raise RuntimeError(f"koe_forward_varlen_size: {n_win.value} windows, the model counts {N}")
+                raise RuntimeError(f"koe_forward_varlen_size_ex: {n_win.value} windows, the model counts {N}")
             ws = torch.empty(ws_bytes.value, dtype=torch.uint8, device=dev)
             a.egemaps, a.workspace, a.workspace_bytes = eg.data_ptr(), ws.data_ptr(), ws_bytes.value
             a.out = out.data_ptr()
             a.sigmoid_out = sig.data_ptr() if sig is not None else None
             a.attn_out = attn.data_ptr() if attn is not None else None
             with torch.cuda.device(dev):
-                _lib.check(lib.koe_forward_varlen(C.byref(a), _lib.stream_ptr(dev)), "koe_forward_varlen")
+                _lib.check(lib.koe_forward_varlen_ex(C.byref(a), flags, _lib.stream_ptr(dev)), "koe_forward_varlen_ex")
         # as forward: the smoothing state is each clip's last frame
         self.prev_blendshapes = None
         if self.use_temporal_smoothing:
@@ -140,6 +154,25 @@ class SequentialDualStreamModel(SimplifiedDualStreamModel):
         res["emotion_backend"] = "egemaps_input"
         res["emotion_processing_time"] = 0.0
         return res
+
+    def varlen_rows(self, lengths: torch.Tensor, warmup: bool = False) -> torch.Tensor:
+        """Output rows of each clip of ``forward_varlen`` for the CPU int64 ``lengths``: ``num_output_frames`` per clip,
+        or with ``warmup`` the hops h = W - 1 (mod stride) from r = (W - 1) % stride on that the clip completes (raises
+        ``ValueError`` for a clip that completes none)."""
+        hop, W, stride = self.hop_length, self.window_frames, self.stride_frames
+        n_out = torch.clamp((lengths // hop - W) // stride + 1, min=1)     # num_output_frames, per clip
+        if not warmup:
+            return n_out
+        r = (W - 1) % stride
+        n_hops = lengths // hop
+        last_lead = torch.clamp(n_hops - 1, max=W - 2)                  # the last hop a lead window can end on
+        leads = torch.where(last_lead >= r, torch.div(last_lead - r, stride, rounding_mode="floor") + 1, 0)
+        rows = leads + torch.where(n_hops >= W, n_out, 0)
+        if rows.numel() > 0 and int(rows.min()) == 0:
+            c = int(torch.nonzero(rows == 0)[0, 0])
+            raise ValueError(f"clip {c} of {int(lengths[c])} samples completes no hop of the output grid: warm-up rows "
+                             f"start at {r + 1} complete hops of {hop} samples")
+        return rows
 
     @staticmethod
     def _check_lengths(lengths, n_samples: int) -> torch.Tensor:
