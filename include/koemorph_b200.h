@@ -474,7 +474,26 @@ typedef struct {
   float* attn_out;                   /* [n_windows][28][80], or NULL */
 } koe_forward_varlen_args;
 /* host only (no device work): total output rows, total global frames and the workspace koe_forward_varlen needs for
- * the lengths and geometry in args (the buffer and output fields are not read); KOE_E_INVALID on the same misuse */
+ * the lengths and geometry in args (the buffer and output fields are not read); KOE_E_INVALID on the same misuse.
+ *
+ * Workspace layout (what a caller may read back after the call; koe_forward_varlen_ex with the same flags).  With
+ * n_edge = ceil(half_fft / hop), W = window_frames, s = stride_frames, n_out_c and n_frames_c as above, and prefix sums
+ * over the clips before c: frame_base_c = sum n_frames, window_base_c = sum n_out, lead_base_c = sum K (K_c: the lead
+ * windows of KOE_VARLEN_WARMUP below, 0 without the flag).  E = n_edge when some clip is not a plain single window or
+ * (warm-up) some clip has a lead window, else 0; N = sum n_out over all clips when some clip is not a plain single
+ * window, else 0.  Regions follow each other, each rounded up to a multiple of 16 bytes, in this order:
+ *   power[0]           [sum n_frames][80]  clip c's global frame g at row frame_base_c + g (pad: frames past the clip
+ *                                          read zeros)
+ *   power[1 + 2m]      [N][80]             m < E: window-start variant m of window i of clip c at row window_base_c + i:
+ *                                          frame i * s + m with everything before (i * s) * hop zeroed
+ *   power[2 + 2m]      [N + sum K][80]     window-end variant m of window i at row window_base_c + i: frame
+ *                                          i * s + W - m with everything from (i * s + W) * hop on zeroed; then the lead
+ *                                          window at grid hop h = r + k * s (k < K_c) at row N + lead_base_c + k: frame
+ *                                          h + 1 - m with everything from (h + 1) * hop on zeroed
+ *   frame_max[0], frame_max[1 .. 2E]       the same rows without the 80: each row's largest band
+ *   the per-clip tables the call uploads (not part of the interface)
+ * Rows of a clip that reads its window from the plain rows are not written in power[1 .. 2E].  Within each launch the
+ * frontend transforms a clip's rows 2j and 2j + 1 (of that buffer, counted from the clip's first row) as one pair. */
 int koe_forward_varlen_size(const koe_forward_varlen_args* args, int64_t* n_windows, int64_t* n_frames,
                             int64_t* workspace_bytes);
 int koe_forward_varlen(const koe_forward_varlen_args* args, void* stream);
