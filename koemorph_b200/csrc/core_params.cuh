@@ -30,10 +30,10 @@ struct CoreParams {
   // stream pool_slot[w] with ring base pool_base[w], and writes output row w
   const int* pool_slot;
   const int* pool_base;
-  // packed variable-length batch (csrc/session.cu; CoreMode::Varlen only): n_clips counts windows (n_out = 1),
-  // item is the global window = output row; clip c owns windows [vl_window_base[c], vl_window_base[c + 1]) and its plain
-  // rows start at vl_frame_base[c]; vl_plain_only[c] != 0: the clip's window reads every frame from the plain rows
-  const int* vl_window_base;
+  // packed variable-length batch (csrc/session.cu; CoreMode::Varlen only): n_clips counts output rows (n_out = 1), item
+  // is the output row; clip c owns rows [vl_row_base[c], vl_row_base[c + 1]) and its plain rows start at
+  // vl_frame_base[c]; vl_plain_only[c] != 0: the clip's windows read every frame from the plain rows
+  const int* vl_row_base;
   const int* vl_frame_base;
   const int* vl_plain_only;
   int vl_clips;
@@ -45,14 +45,13 @@ struct CoreParams {
   const int* hop_slot;
   const int* hop_row;
   int hop_base_shift;
-  // stream-pool warm-up (csrc/stream_pool.cu; CoreMode::PoolWarm only): window w has hop_frames[w] frames, 2 ..
-  // frames_per_window; a window shorter than frames_per_window starts at its stream's sample 0 and has no window-start
-  // variants.  Everything else as PoolHops.
+  // a warm-up pool's burst (PoolHops): window w has hop_frames[w] frames, 2 .. frames_per_window; a window shorter than
+  // frames_per_window starts at its stream's sample 0 and has no window-start variants.  NULL: every window has
+  // frames_per_window frames.
   const int* hop_frames;
-  // packed warm-up batch (csrc/session.cu; CoreMode::VarlenWarm only): vl_window_base[c] is clip c's first output row;
-  // its first vl_lead_base[c + 1] - vl_lead_base[c] rows are lead windows, whose window-end rows (variants 2, 4) are rows
-  // vl_lead_base[c] .. of power[2] / power[4]; the rest are the windows of CoreMode::Varlen, whose edge rows start at
-  // vl_edge_base[c]
+  // packed batch (Varlen): clip c's first vl_lead_base[c + 1] - vl_lead_base[c] rows are lead windows (warm-up), whose
+  // window-end rows (variants 2, 4) are rows vl_lead_base[c] .. of power[2] / power[4]; vl_lead_base == NULL: none.  The
+  // rest are the clip's windows, stride_frames apart, whose edge rows start at vl_edge_base[c].
   const int* vl_edge_base;
   const int* vl_lead_base;
 };
@@ -63,14 +62,14 @@ struct CoreParams {
 //            the streaming step's per-stream rings (ring_frames > 0) and prenormalised features (mel_long != NULL)
 //   Early    Windows with one window per clip, released early by the frontend (the fused forward; early_flag)
 //   Pool     a stream-pool push: window w reads the rings of stream pool_slot[w] from ring base pool_base[w]
-//   Varlen   a packed variable-length batch: window w belongs to the clip c with vl_window_base[c] <= w < vl_window_base[c + 1]
+//   Varlen   a packed variable-length batch: output row w belongs to the clip c with vl_row_base[c] <= w < vl_row_base[c + 1];
+//            with warm-up the clip's lead windows come first -- the window at grid hop h < W - 1 is the clip's first
+//            h + 2 frames, shaped as a PoolHops window below frames_per_window
 //   PoolHops a stream-pool burst: window w reads the rings of stream hop_slot[hop_end[w]] (ring_frames rows each) and
-//            the window-end rows that hop hop_end[w] staged
-//   PoolWarm a burst of a warm-up pool: PoolHops with hop_frames[w] frames in window w; below frames_per_window the
-//            window is the stream's whole audio so far: plain rows, then the n_edge window-end rows, no window-start rows
-//   VarlenWarm a packed warm-up batch: Varlen with a clip's lead windows first -- the window at grid hop h < W - 1 is the
-//            clip's first h + 2 frames, shaped as a PoolWarm window below frames_per_window
-enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops, PoolWarm, VarlenWarm };
+//            the window-end rows that hop hop_end[w] staged; on a warm-up pool it has hop_frames[w] frames, and below
+//            frames_per_window it is the stream's whole audio so far: plain rows, then the n_edge window-end rows, no
+//            window-start rows
+enum class CoreMode { Windows, Early, Pool, Varlen, PoolHops };
 
 // frame k of a window: which buffer (variant) holds it (see koe_dual_stream_windows in the header)
 __device__ __forceinline__ int window_variant(const CoreParams& p, int k) {
@@ -79,11 +78,11 @@ __device__ __forceinline__ int window_variant(const CoreParams& p, int k) {
   return 0;
 }
 
-// varlen: the clip of window `item` (window_base[c] <= item < window_base[c + 1]; every clip has a window).  Scalar binary
+// varlen: the clip of output row `item` (row_base[c] <= item < row_base[c + 1]; every clip has a row).  Scalar binary
 // search, or -- every lane of a warp calling with the same item -- a 32-ary search with one table load per lane and round.
 template <bool kWarp>
 __device__ __forceinline__ int varlen_clip(const CoreParams& p, int item) {
-  const int* wb = p.vl_window_base;
+  const int* wb = p.vl_row_base;
   int lo = 0, n = p.vl_clips;  // the clip is in [lo, lo + n)
   if constexpr (kWarp) {
     while (n > 1) {
@@ -109,10 +108,10 @@ struct CoreWindow {
   int owner;        // whose rows: the clip (Windows, Early; ring mode: the stream), the stream slot (Pool, PoolHops), or
                     // the window's first plain row (Varlen)
   int pos;          // where in them: the window within its clip (Windows, Early), the ring base (Pool, PoolHops), or the
-                    // global window, which is also the window's row in every edge-variant buffer (Varlen)
+                    // window's row in every edge-variant buffer it reads (Varlen)
   bool plain_only;  // Varlen: the clip has no edge variants, every frame comes from the plain rows
-  int hop;          // PoolHops, PoolWarm: the staged hop at which the window completes (its window-end rows)
-  int frames;       // PoolWarm, VarlenWarm: the window's frame count
+  int hop;          // PoolHops: the staged hop at which the window completes (its window-end rows)
+  int frames;       // PoolHops, Varlen: the window's frame count
 };
 
 // The window resolver of each mode: work item `item` is output row `item` and reads the window window<kWarp>(p, item);
@@ -120,34 +119,27 @@ struct CoreWindow {
 template <CoreMode M>
 struct CoreRows {
   // every window carries its own frame count (CoreWindow::frames), from 2 to frames_per_window
-  static constexpr bool kWindowFrames = M == CoreMode::PoolWarm || M == CoreMode::VarlenWarm;
+  static constexpr bool kWindowFrames = M == CoreMode::Varlen || M == CoreMode::PoolHops;
   // kWarp: every lane of a converged warp calls with the same item (Varlen searches the clip with the whole warp)
   template <bool kWarp>
   static __device__ __forceinline__ CoreWindow window(const CoreParams& p, int item) {
     if constexpr (M == CoreMode::Pool) {
       return {p.pool_slot[item], p.pool_base[item], false};
     } else if constexpr (M == CoreMode::PoolHops) {
-      const int e = p.hop_end[item];
-      const int base = p.hop_row[e] + p.hop_base_shift;  // both < ring_frames
-      return {p.hop_slot[e], base >= p.ring_frames ? base - p.ring_frames : base, false, e};
-    } else if constexpr (M == CoreMode::PoolWarm) {
-      const int e = p.hop_end[item], T = p.hop_frames[item];
+      const int e = p.hop_end[item], T = p.hop_frames != nullptr ? p.hop_frames[item] : p.frames_per_window;
       // frame 0 is T - 2 - lag rows before the hop's newest plain row: hop_base_shift + frames_per_window - T is that
-      // distance mod ring_frames (PoolHops' shift when T = frames_per_window), and the sum stays below 2 ring_frames
+      // distance mod ring_frames, and the sum stays below 2 ring_frames
       const int base = (p.hop_row[e] + p.hop_base_shift + p.frames_per_window - T) % p.ring_frames;
       return {p.hop_slot[e], base, false, e, T};
     } else if constexpr (M == CoreMode::Varlen) {
       const int c = varlen_clip<kWarp>(p, item);
-      return {__ldg(p.vl_frame_base + c) + (item - __ldg(p.vl_window_base + c)) * p.stride_frames, item,
-              __ldg(p.vl_plain_only + c) != 0};
-    } else if constexpr (M == CoreMode::VarlenWarm) {
-      const int c = varlen_clip<kWarp>(p, item);
-      const int local = item - __ldg(p.vl_window_base + c), lead0 = __ldg(p.vl_lead_base + c);
-      const int leads = __ldg(p.vl_lead_base + c + 1) - lead0;
+      const int local = item - __ldg(p.vl_row_base + c);
+      int lead0 = 0, leads = 0;
+      if (p.vl_lead_base != nullptr) lead0 = __ldg(p.vl_lead_base + c), leads = __ldg(p.vl_lead_base + c + 1) - lead0;
       if (local < leads)  // grid hop h = r + local * stride, r = (W - 1) mod stride: T = h + 2 frames from the clip's frame 0
         return {__ldg(p.vl_frame_base + c), lead0 + local, false, 0,
                 (p.frames_per_window - 2) % p.stride_frames + local * p.stride_frames + 2};
-      const int j = local - leads;  // steady window j: as Varlen
+      const int j = local - leads;  // the clip's window j
       return {__ldg(p.vl_frame_base + c) + j * p.stride_frames, __ldg(p.vl_edge_base + c) + j,
               __ldg(p.vl_plain_only + c) != 0, 0, p.frames_per_window};
     } else {
@@ -155,12 +147,12 @@ struct CoreRows {
     }
   }
   static __device__ __forceinline__ long long row(const CoreParams& p, const CoreWindow& w, int variant, int k) {
-    if constexpr (M == CoreMode::Varlen || M == CoreMode::VarlenWarm) {
+    if constexpr (M == CoreMode::Varlen) {
       return variant == 0 ? (long long)w.owner + k : (long long)w.pos;
     } else if constexpr (M == CoreMode::Pool) {
       return variant > 0 && (variant & 1) == 0 ? (long long)w.owner
                                                : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
-    } else if constexpr (M == CoreMode::PoolHops || M == CoreMode::PoolWarm) {
+    } else if constexpr (M == CoreMode::PoolHops) {
       return variant > 0 && (variant & 1) == 0 ? (long long)w.hop * (1 + 2 * p.n_edge)
                                                : (long long)w.owner * p.ring_frames + (w.pos + k) % p.ring_frames;
     } else {
@@ -192,22 +184,22 @@ struct CoreRows {
   }
   // ring modes (ring_frames > 0, n_out == 1): the ring slot of the window's frame 0
   static __device__ __forceinline__ int ring_base(const CoreParams& p, const CoreWindow& w) {
-    return M == CoreMode::Pool || M == CoreMode::PoolHops || M == CoreMode::PoolWarm ? w.pos : p.ring_base;
+    return M == CoreMode::Pool || M == CoreMode::PoolHops ? w.pos : p.ring_base;
   }
   // ring modes: the stream whose ring and frame maxima window `item` reads (the L2 prefetch of the next window)
   static __device__ __forceinline__ int ring_stream(const CoreParams& p, int item) {
-    if constexpr (M == CoreMode::PoolHops || M == CoreMode::PoolWarm) return p.hop_slot[p.hop_end[item]];
+    if constexpr (M == CoreMode::PoolHops) return p.hop_slot[p.hop_end[item]];
     return M == CoreMode::Pool ? p.pool_slot[item] : item;
   }
   // the clip or stream whose expression value (expr_sigmoid) output row `item` takes
   static __device__ __forceinline__ int expr_row(const CoreParams& p, int item) {
-    if constexpr (M == CoreMode::PoolHops || M == CoreMode::PoolWarm) return p.hop_slot[p.hop_end[item]];
+    if constexpr (M == CoreMode::PoolHops) return p.hop_slot[p.hop_end[item]];
     return M == CoreMode::Pool ? p.pool_slot[item] : item / p.n_out;
   }
   // the L2 policy of a window's plain rows: `reread` where other windows read them again (the overlapping windows of a
   // sequence or of a varlen clip), else `once`
   static __device__ __forceinline__ uint64_t plain_rows_policy(const CoreParams& p, uint64_t reread, uint64_t once) {
-    return M == CoreMode::Varlen || M == CoreMode::VarlenWarm || p.n_out > 1 ? reread : once;
+    return M == CoreMode::Varlen || p.n_out > 1 ? reread : once;
   }
 };
 
@@ -228,29 +220,21 @@ int launch_dual_stream_pool(const koe_core_weights* w, const float* const* power
                             float* out, int precision, void* stream);
 // the core over the windows of a stream-pool burst (csrc/stream_pool.cu): window w completes at staged hop hop_end[w] (device
 // tables as CoreParams::hop_*), rings of ring_frames rows, window-end rows power[2], power[4] at row hop * (1 + 2 n_edge);
-// output row w
-// hop_frames != NULL (a warm-up pool, CoreMode::PoolWarm): window w has hop_frames[w] frames (CoreParams::hop_frames)
+// output row w; hop_frames != NULL (a warm-up pool): window w has hop_frames[w] frames (CoreParams::hop_frames)
 int launch_dual_stream_pool_hops(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
                                  int n_edge, int n_windows, int ring_frames, const int* hop_end, const int* hop_slot,
                                  const int* hop_row, int hop_base_shift, const int* hop_frames, const float* expr_sigmoid,
                                  float* out, int precision, void* stream);
-// the core over the windows of a packed variable-length batch (csrc/session.cu): window `item` of the n_windows belongs to
-// the clip c with window_base[c] <= item < window_base[c + 1] and writes output row `item`; plain rows from
-// frame_base[c] + (item - window_base[c]) * stride_frames, edge rows at `item` unless plain_only[c]; expression entries
-// are written by the emotion kernel
+// the core over the rows of a packed variable-length batch (csrc/session.cu): output row `item` of the n_rows belongs to
+// the clip c with row_base[c] <= item < row_base[c + 1]; the clip's first lead_base[c + 1] - lead_base[c] rows are its
+// lead windows (window-end rows power[2], power[4] from lead_base[c]; lead_base == NULL: none), the rest its windows j =
+// 0, 1, .. with plain rows from frame_base[c] + j * stride_frames and edge rows at edge_base[c] + j unless plain_only[c];
+// expression entries are written by the emotion kernel
 int launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
-                              int n_edge, int n_windows, int n_frames, int stride_frames, int frames_per_window, int n_clips,
-                              const int* window_base, const int* frame_base, const int* plain_only, float* out,
-                              float* sigmoid_out, float* attn_out, int precision, void* stream);
-// the core over the rows of a packed warm-up batch (csrc/session.cu, CoreMode::VarlenWarm): output row `item` of the
-// n_rows belongs to the clip c with row_base[c] <= item < row_base[c + 1]; the clip's first lead_base[c + 1] -
-// lead_base[c] rows are its lead windows (window-end rows power[2], power[4] from lead_base[c]), the rest its windows of
-// launch_dual_stream_varlen with edge rows from edge_base[c]; expression entries are written by the emotion kernel
-int launch_dual_stream_varlen_warm(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
-                                   int n_edge, int n_rows, int n_frames, int stride_frames, int frames_per_window,
-                                   int n_clips, const int* row_base, const int* frame_base, const int* edge_base,
-                                   const int* lead_base, const int* plain_only, float* out, float* sigmoid_out,
-                                   float* attn_out, int precision, void* stream);
+                              int n_edge, int n_rows, int n_frames, int stride_frames, int frames_per_window, int n_clips,
+                              const int* row_base, const int* frame_base, const int* edge_base, const int* lead_base,
+                              const int* plain_only, float* out, float* sigmoid_out, float* attn_out, int precision,
+                              void* stream);
 // segmented EMA of a packed variable-length batch: clip c's frames are rows [row_base[c], row_base[c + 1]) of `frames`
 int launch_ema_scan_varlen(float* frames, int n_clips, const int* row_base, float alpha, void* stream);
 // how many SMs' worth of CTAs the tensor-core core launches for n_items windows (the early-release split follows it)

@@ -818,8 +818,6 @@ static int launch_core(const CoreParams& p_in, CoreMode mode, int precision, cud
     case CoreMode::Pool: return launch_fp32<CoreMode::Pool>(p, stream);
     case CoreMode::Varlen: return launch_fp32<CoreMode::Varlen>(p, stream);
     case CoreMode::PoolHops: return launch_fp32<CoreMode::PoolHops>(p, stream);
-    case CoreMode::PoolWarm: return launch_fp32<CoreMode::PoolWarm>(p, stream);
-    case CoreMode::VarlenWarm: return launch_fp32<CoreMode::VarlenWarm>(p, stream);
     case CoreMode::Early: break;
   }
   return fail(KOE_E_INVALID, "early release needs the tensor-core core (precision 2)");
@@ -966,61 +964,35 @@ int koe::launch_dual_stream_pool_hops(const koe_core_weights* w, const float* co
   p.hop_row = hop_row;
   p.hop_base_shift = hop_base_shift;
   p.hop_frames = hop_frames;
-  return launch_core(p, hop_frames != nullptr ? CoreMode::PoolWarm : CoreMode::PoolHops, precision, (cudaStream_t)stream);
+  return launch_core(p, CoreMode::PoolHops, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_dual_stream_varlen(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
-                                   int n_edge, int n_windows, int n_frames, int stride_frames, int frames_per_window,
-                                   int n_clips, const int* window_base, const int* frame_base, const int* plain_only,
-                                   float* out, float* sigmoid_out, float* attn_out, int precision, void* stream) {
-  if (int rc = validate_weights(w)) return rc;
-  KOE_REQUIRE(power != nullptr && frame_max != nullptr && window_base != nullptr && frame_base != nullptr &&
-                  plain_only != nullptr && out != nullptr,
-              "varlen core: NULL argument");
-  KOE_REQUIRE(n_edge >= 0 && n_edge <= KOE_MAX_EDGE && n_windows >= 0 && n_clips >= 0 && stride_frames >= 1 &&
-                  frames_per_window > 2 * n_edge && frames_per_window == w->k_mel - 2,
-              "varlen core: bad sizes");
-  if (n_windows == 0) return KOE_OK;
-  CoreParams p;
-  if (int rc = core_params("varlen core", w, power, frame_max, n_edge, nullptr, out, sigmoid_out, attn_out, &p)) return rc;
-  p.n_clips = n_windows;
-  p.n_frames = n_frames;
-  p.stride_frames = stride_frames;
-  p.frames_per_window = frames_per_window;
-  p.vl_window_base = window_base;
-  p.vl_frame_base = frame_base;
-  p.vl_plain_only = plain_only;
-  p.vl_clips = n_clips;
-  return launch_core(p, CoreMode::Varlen, precision, (cudaStream_t)stream);
-}
-
-int koe::launch_dual_stream_varlen_warm(const koe_core_weights* w, const float* const* power, const float* const* frame_max,
-                                        int n_edge, int n_rows, int n_frames, int stride_frames, int frames_per_window,
-                                        int n_clips, const int* row_base, const int* frame_base, const int* edge_base,
-                                        const int* lead_base, const int* plain_only, float* out, float* sigmoid_out,
-                                        float* attn_out, int precision, void* stream) {
+                                   int n_edge, int n_rows, int n_frames, int stride_frames, int frames_per_window,
+                                   int n_clips, const int* row_base, const int* frame_base, const int* edge_base,
+                                   const int* lead_base, const int* plain_only, float* out, float* sigmoid_out,
+                                   float* attn_out, int precision, void* stream) {
   if (int rc = validate_weights(w)) return rc;
   KOE_REQUIRE(power != nullptr && frame_max != nullptr && row_base != nullptr && frame_base != nullptr &&
-                  edge_base != nullptr && lead_base != nullptr && plain_only != nullptr && out != nullptr,
-              "varlen warm-up core: NULL argument");
+                  edge_base != nullptr && plain_only != nullptr && out != nullptr,
+              "varlen core: NULL argument");
   KOE_REQUIRE(n_edge >= 0 && n_edge <= KOE_MAX_EDGE && n_rows >= 0 && n_clips >= 0 && stride_frames >= 1 &&
                   frames_per_window > 2 * n_edge && frames_per_window == w->k_mel - 2,
-              "varlen warm-up core: bad sizes");
+              "varlen core: bad sizes");
   if (n_rows == 0) return KOE_OK;
   CoreParams p;
-  if (int rc = core_params("varlen warm-up core", w, power, frame_max, n_edge, nullptr, out, sigmoid_out, attn_out, &p))
-    return rc;
+  if (int rc = core_params("varlen core", w, power, frame_max, n_edge, nullptr, out, sigmoid_out, attn_out, &p)) return rc;
   p.n_clips = n_rows;
   p.n_frames = n_frames;
   p.stride_frames = stride_frames;
   p.frames_per_window = frames_per_window;
-  p.vl_window_base = row_base;
+  p.vl_row_base = row_base;
   p.vl_frame_base = frame_base;
   p.vl_plain_only = plain_only;
   p.vl_clips = n_clips;
   p.vl_edge_base = edge_base;
   p.vl_lead_base = lead_base;
-  return launch_core(p, CoreMode::VarlenWarm, precision, (cudaStream_t)stream);
+  return launch_core(p, CoreMode::Varlen, precision, (cudaStream_t)stream);
 }
 
 int koe::launch_ema_scan_varlen(float* frames, int n_clips, const int* row_base, float alpha, void* stream) {

@@ -961,9 +961,9 @@ int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t strea
   if (mode == CoreMode::Early)
     KOE_REQUIRE(p.n_out == 1 && p.early_items > 0 && p.early_items % grid == 0 && p.early_target > 0,
                 "tensor-core path: bad early-release parameters");
-  if (mode == CoreMode::Varlen || mode == CoreMode::VarlenWarm)
+  if (mode == CoreMode::Varlen)
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames == 0 && p.expr_sigmoid == nullptr, "tensor-core path: bad varlen parameters");
-  if (mode == CoreMode::Pool || mode == CoreMode::PoolHops || mode == CoreMode::PoolWarm)
+  if (mode == CoreMode::Pool || mode == CoreMode::PoolHops)
     KOE_REQUIRE(p.n_out == 1 && p.ring_frames > 0 && p.attn_out == nullptr, "tensor-core path: bad stream-pool parameters");
   if (p.attn_out != nullptr)  // head-average is accumulated with atomics
     KOE_CUDA(cudaMemsetAsync(p.attn_out, 0, (size_t)p.n_clips * p.n_out * KOE_N_MOUTH * tc::kTok * sizeof(float),
@@ -975,8 +975,6 @@ int launch_dual_stream_tc(const CoreParams& p, CoreMode mode, cudaStream_t strea
     case CoreMode::Pool: rc = launch_tc<CoreMode::Pool>(p, grid, stream); break;
     case CoreMode::Varlen: rc = launch_tc<CoreMode::Varlen>(p, grid, stream); break;
     case CoreMode::PoolHops: rc = launch_tc<CoreMode::PoolHops>(p, grid, stream); break;
-    case CoreMode::PoolWarm: rc = launch_tc<CoreMode::PoolWarm>(p, grid, stream); break;
-    case CoreMode::VarlenWarm: rc = launch_tc<CoreMode::VarlenWarm>(p, grid, stream); break;
   }
   if (rc != KOE_OK) return rc;
   count_launch();

@@ -273,7 +273,7 @@ extern "C" int koe_forward_windows(const koe_forward_args* a, void* stream) {
 // variant buffers as the steady or the lead windows need.
 namespace {
 constexpr int kVarlenTableWords = 8;      // table words per clip (+ 4)
-constexpr int kVarlenWarmTableWords = 3;  // more with KOE_VARLEN_WARMUP (+ 3)
+constexpr int kWarmupTableWords = 3;      // more with KOE_VARLEN_WARMUP (+ 3)
 
 struct VarlenPlan {
   int n_edge = 0;            // edge variants per window side of the steady windows (0: no clip uses them)
@@ -387,7 +387,7 @@ int plan_varlen(const koe_forward_varlen_args* a, bool warm, VarlenPlan* pl, int
   for (int j = 1; j <= n_var; ++j) pl->off_power[j] = off, off += align16(var_rows(j) * KOE_N_MELS * sizeof(float));
   pl->off_fmax[0] = off, off += align16((size_t)pl->frames * sizeof(float));
   for (int j = 1; j <= n_var; ++j) pl->off_fmax[j] = off, off += align16(var_rows(j) * sizeof(float));
-  pl->table_words = (size_t)kVarlenTableWords * B + 4 + (warm ? (size_t)kVarlenWarmTableWords * B + 3 : 0);
+  pl->table_words = (size_t)kVarlenTableWords * B + 4 + (warm ? (size_t)kWarmupTableWords * B + 3 : 0);
   pl->off_tables = off, off += align16(pl->table_words * sizeof(int32_t));
   pl->bytes = off;
   return KOE_OK;
@@ -502,16 +502,11 @@ extern "C" int koe_forward_varlen_ex(const koe_forward_varlen_args* a, int flags
     return rc;
   const float* cpower[1 + 2 * KOE_MAX_EDGE] = {power[0], power[1], power[2], power[3], power[4]};
   const float* cfmax[1 + 2 * KOE_MAX_EDGE] = {fmax[0], fmax[1], fmax[2], fmax[3], fmax[4]};
-  if (warm) {
-    if (int rc = launch_dual_stream_varlen_warm(a->weights, cpower, cfmax, core_edge, (int)pl.rows, (int)pl.frames,
-                                                a->stride_frames, T, B, row_base, frame_base, window_base, lead_base,
-                                                plain_only, a->out, a->sigmoid_out, a->attn_out, a->precision, stream))
-      return rc;
-  } else if (int rc = launch_dual_stream_varlen(a->weights, cpower, cfmax, pl.n_edge, (int)pl.windows, (int)pl.frames,
-                                                a->stride_frames, T, B, window_base, frame_base, plain_only, a->out,
-                                                a->sigmoid_out, a->attn_out, a->precision, stream)) {
+  if (int rc = launch_dual_stream_varlen(a->weights, cpower, cfmax, core_edge, (int)pl.rows, (int)pl.frames,
+                                         a->stride_frames, T, B, row_base, frame_base, window_base,
+                                         warm ? lead_base : nullptr, plain_only, a->out, a->sigmoid_out, a->attn_out,
+                                         a->precision, stream))
     return rc;
-  }
   if (a->smooth && pl.max_out > 1)
     if (int rc = launch_ema_scan_varlen(a->out, B, row_base, a->alpha, stream)) return rc;
   return KOE_OK;

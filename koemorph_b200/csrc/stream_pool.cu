@@ -27,8 +27,8 @@
 // 0 .. h - lag, and the hop's window-end rows for the last n_edge frames (they see zeros from sample (h + 1) hop on, as
 // the prefix does).  Every frame before sample 0 reads zeros there too, because a stream's tail starts at zero, so the
 // plain rows are the right first frames and no window-start variant is read.  A warm-up pool always runs the burst path
-// (koe_stream_pool_push is koe_stream_pool_push_hops with counts of 1), its core is CoreMode::PoolWarm with one more
-// table column (each window's T), and from hop W - 1 on its windows are those of PoolHops.
+// (koe_stream_pool_push is koe_stream_pool_push_hops with counts of 1), with one more table column (each window's T) for
+// the core, and from hop W - 1 on its windows are those of a pool without warm-up.
 #include <algorithm>
 #include <vector>
 
