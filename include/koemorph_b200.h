@@ -399,6 +399,56 @@ int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stream_pool_arg
                               int* n_emitted, void* stream);
 
 /*
+ * Snapshots: a stream's whole state as one fixed-size float32 record, so that it can leave its slot -- into a pool of
+ * another capacity or max_hops (a pool that grows), onto another GPU (load balancing, draining a GPU), or through host
+ * memory (a restart of the serving process) -- and continue there bit for bit.
+ *
+ * koe_stream_pool_snapshot writes the records of the n open streams slots_host[0..n) to records[n][state_floats]
+ * (caller-owned device memory, 16-byte aligned) and each stream's clock -- the hops pushed since it was opened -- to
+ * hops_host[n].  The streams stay open and are not changed: their later frames are those they would have given without
+ * the snapshot.  The record holds the state after every call queued before it on `stream`.
+ * koe_stream_pool_restore takes the n lowest free slots (as koe_stream_pool_open) into slots_host[n], writes record i into
+ * slot i and sets its clock to hops_host[i]; with hops_host[i] == 0 that is exactly an open.
+ *
+ * Equality: a stream snapshotted after a hops in pool A and restored into pool B, then pushed the same hops a, a + 1, ...
+ * in B as in A -- any mix of koe_stream_pool_push and koe_stream_pool_push_hops -- gives bit for bit the frames (the
+ * unsmoothed and the smoothed ones) and the hops the stream gives in A, when both pools run the same weights at the same
+ * precision.  This holds whatever B's capacity and max_hops are and whatever B's slots held before.  A and B must have
+ * the same hop, window_frames, half_fft and KOE_POOL_WARMUP flag: the record does not carry them, and a record of another
+ * geometry is the caller's error (the Python layer, StreamSnapshot, refuses it).
+ *
+ * Only the hops travel; restore derives the rest as the pushes count them: frames = max(0, hops - W + 1) (hops on a
+ * warm-up pool) and the ring row of frame g = g mod R_B.  The expression value and the smoothing row travel in the
+ * record: no koe_stream_pool_set_egemaps is needed after a restore.  A snapshot with args->ema_state == NULL stores a
+ * zero smoothing row; a restore with args->ema_state == NULL does not write one.
+ *
+ * Record layout, with W = window_frames, lag = n_edge - 1, a = the stream's hops, P = W - 1 - lag (the frames a later
+ * window can still read: the window that completes at hop a starts at frame a + 1 - W, the newest complete frame is
+ * a - 1 - lag) and V_r = 1 + n_edge ring variants (plain, window-start 0, at hop < n_fft/2 window-start 1):
+ *   rows          [V_r][P][80]   variant v's row of frame a + 1 - W + i at row i (ring row (a + 1 - W + i) mod R)
+ *   row maxima    [V_r][P]
+ *   tail          [half_fft + n_edge * hop]
+ *   expr_sigmoid  [1]
+ *   ema_state     [52]
+ *   zero padding  to a multiple of 4 floats (state_floats in all)
+ * Rows of frames < 0 (a stream younger than W - 1 hops) are zeros and are not written back: no window reads them.
+ * Window-end rows are not state (the pushes write and read them in one call).  30 fps: 42,408 floats (170 KB); 60 fps:
+ * 125,028 floats (500 KB).
+ *
+ * Each call uploads a table of 3 n int32 through the pool's tables and queues one kernel; neither can be captured into a
+ * CUDA graph.  Misuse returns KOE_E_INVALID before anything is queued and leaves every clock as it was: snapshot -- a slot
+ * out of range, not open or listed twice, NULL records / hops; restore -- more records than free slots, a negative hops,
+ * NULL records / hops / slots.  Of args only the rings (ring_f, ring_r, ring_r2 and their maxima), tail, expr_sigmoid,
+ * ema_state and tables are used.  n = 0 is a no-op.
+ */
+/* floats per record for this pool's geometry (host only) */
+int koe_stream_pool_state_floats(const koe_stream_pool_t* pool);
+int koe_stream_pool_snapshot(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const int32_t* slots_host, int n,
+                             float* records, int64_t* hops_host, void* stream);
+int koe_stream_pool_restore(koe_stream_pool_t* pool, const koe_stream_pool_args* args, const float* records,
+                            const int64_t* hops_host, int n, int32_t* slots_host, void* stream);
+
+/*
  * The whole forward of SequentialDualStreamModel.forward (src/model/sequential_dual_stream_model.py:63-167) -- or, with
  * n_out = 1 and n_edge = 0, of SimplifiedDualStreamModel.forward (src/model/simplified_dual_stream_model.py:370-415) --
  * as ONE call: koe_logmel_power on the clip's global frames, the 2 * n_edge edge-variant launches on the window grid,

@@ -153,6 +153,11 @@ _SIGNATURES = {
                                        C.POINTER(C.c_int), C.c_void_p]),
     "koe_stream_pool_push_hops": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_void_p, C.c_int,
                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
+    "koe_stream_pool_state_floats": (C.c_int, [C.c_void_p]),
+    "koe_stream_pool_snapshot": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_int, C.c_void_p,
+                                           C.c_void_p, C.c_void_p]),
+    "koe_stream_pool_restore": (C.c_int, [C.c_void_p, C.POINTER(StreamPoolArgs), C.c_void_p, C.c_void_p, C.c_int,
+                                          C.c_void_p, C.c_void_p]),
     "koe_affine_rows": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "koe_emotion_stream": (C.c_int, [C.POINTER(CoreWeightsStruct), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "koe_dual_stream_windows": (C.c_int, [C.POINTER(CoreWeightsStruct), C.POINTER(C.c_void_p),

@@ -2,7 +2,7 @@
 #include "common.cuh"
 
 extern "C" const char* koe_last_error(void) { return koe::err_buf(); }
-extern "C" int koe_version(void) { return 100; }
+extern "C" int koe_version(void) { return 101; }
 extern "C" int64_t koe_launch_count(void) { return koe::launch_counter().load(); }
 extern "C" void koe_reset_launch_count(void) { koe::launch_counter().store(0); }
 extern "C" int koe_sizeof_struct(int which) {

@@ -194,7 +194,139 @@ __global__ void __launch_bounds__(256) pool_hops_ema_kernel(float* __restrict__ 
   *st = y;
 }
 
+// ---- snapshots (koe_stream_pool_snapshot / koe_stream_pool_restore).  A record is a stream's whole state, in the layout
+// of the header: rows [V_r][P][80], maxima [V_r][P], tail [tail_len], expression [1], smoothing row [52], zero padding to
+// rec_floats (a multiple of 4).  Record row i of variant v is the stream's frame a + 1 - W + i (a: its hops), ring row
+// row0 + i (mod R) of its slot; the first `skip` of them are frames < 0, which no window reads: zeros in the record, not
+// written back.  Per stream i the tables hold [slot | row0 | skip].  CTA (x, y) copies part x of the records of streams
+// y, y + gridDim.y, ...: the rows as float4s, kStateUnroll of them in flight per thread (all loads before any store), then
+// the other fields as floats.
+constexpr int kStateUnroll = 4;
+
+struct PoolState {
+  float* power[1 + KOE_MAX_EDGE];  // plain ring, window-start ring 0, window-start ring 1
+  float* fmax[1 + KOE_MAX_EDGE];
+  float* tail;
+  float* expr;
+  float* ema;  // or NULL
+  // ring variant v's buffers, selected without indexing the parameter arrays (which would copy them to the stack)
+  __device__ __forceinline__ float* ring(int v) const { return v == 0 ? power[0] : v == 1 ? power[1] : power[2]; }
+  __device__ __forceinline__ float* ring_max(int v) const { return v == 0 ? fmax[0] : v == 1 ? fmax[1] : fmax[2]; }
+};
+
+__global__ void __launch_bounds__(256) pool_snapshot_kernel(PoolState b, const int* __restrict__ tab, int n, int n_ring,
+                                                             int P, int R, int tail_len, int rec_floats,
+                                                             float* __restrict__ records) {
+  constexpr int kQuads = KOE_N_MELS / 4;
+  const int quads = n_ring * P * kQuads, rows = n_ring * P;
+  const int rest = rec_floats - rows * KOE_N_MELS;  // maxima, tail, expression, smoothing row, padding
+  const int t0 = blockIdx.x * blockDim.x + threadIdx.x, dt = gridDim.x * blockDim.x;
+  for (int i = blockIdx.y; i < n; i += gridDim.y) {
+    const long long s = __ldg(tab + i);
+    const int row0 = __ldg(tab + n + i), skip = __ldg(tab + 2 * n + i);
+    float* rec = records + (long long)i * rec_floats;
+    for (int u0 = t0; u0 < quads; u0 += kStateUnroll * dt) {
+      float4 x[kStateUnroll];
+#pragma unroll
+      for (int k = 0; k < kStateUnroll; ++k) {
+        const int u = u0 + k * dt;
+        const int q = u % kQuads, vr = u / kQuads, r = vr % P, v = vr / P;
+        x[k] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        if (u < quads && r >= skip) {
+          const int rr = row0 + r < R ? row0 + r : row0 + r - R;
+          x[k] = __ldcs(reinterpret_cast<const float4*>(b.ring(v) + (s * R + rr) * KOE_N_MELS) + q);
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < kStateUnroll; ++k)
+        if (u0 + k * dt < quads) __stcs(reinterpret_cast<float4*>(rec) + u0 + k * dt, x[k]);
+    }
+    float* tail_rec = rec + rows * KOE_N_MELS;
+    for (int u = t0; u < rest; u += dt) {
+      float x = 0.0f;
+      if (u < rows) {
+        const int r = u % P, v = u / P;
+        const int rr = row0 + r < R ? row0 + r : row0 + r - R;
+        if (r >= skip) x = __ldcs(b.ring_max(v) + s * R + rr);
+      } else if (u < rows + tail_len) {
+        x = __ldcs(b.tail + s * tail_len + (u - rows));
+      } else if (u == rows + tail_len) {
+        x = b.expr[s];
+      } else if (u < rows + tail_len + 1 + KOE_N_BLENDSHAPES && b.ema != nullptr) {
+        x = b.ema[s * KOE_N_BLENDSHAPES + (u - rows - tail_len - 1)];
+      }
+      __stcs(tail_rec + u, x);
+    }
+  }
+}
+
+// the inverse of pool_snapshot_kernel into the slots of the tables: the rows of frames >= 0, the maxima, the tail, the
+// expression value and -- when b.ema is non-NULL -- the smoothing row
+__global__ void __launch_bounds__(256) pool_restore_kernel(PoolState b, const int* __restrict__ tab, int n, int n_ring,
+                                                            int P, int R, int tail_len, int rec_floats,
+                                                            const float* __restrict__ records) {
+  constexpr int kQuads = KOE_N_MELS / 4;
+  const int quads = n_ring * P * kQuads, rows = n_ring * P;
+  const int rest = rows + tail_len + 1 + KOE_N_BLENDSHAPES;
+  const int t0 = blockIdx.x * blockDim.x + threadIdx.x, dt = gridDim.x * blockDim.x;
+  for (int i = blockIdx.y; i < n; i += gridDim.y) {
+    const long long s = __ldg(tab + i);
+    const int row0 = __ldg(tab + n + i), skip = __ldg(tab + 2 * n + i);
+    const float* rec = records + (long long)i * rec_floats;
+    for (int u0 = t0; u0 < quads; u0 += kStateUnroll * dt) {
+      float4 x[kStateUnroll];
+#pragma unroll
+      for (int k = 0; k < kStateUnroll; ++k) {
+        x[k] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        if (u0 + k * dt < quads) x[k] = __ldcs(reinterpret_cast<const float4*>(rec) + u0 + k * dt);
+      }
+#pragma unroll
+      for (int k = 0; k < kStateUnroll; ++k) {
+        const int u = u0 + k * dt;
+        const int q = u % kQuads, vr = u / kQuads, r = vr % P, v = vr / P;
+        const int rr = row0 + r < R ? row0 + r : row0 + r - R;
+        if (u < quads && r >= skip) reinterpret_cast<float4*>(b.ring(v) + (s * R + rr) * KOE_N_MELS)[q] = x[k];
+      }
+    }
+    const float* tail_rec = rec + rows * KOE_N_MELS;
+    for (int u = t0; u < rest; u += dt) {
+      if (u < rows) {
+        const int r = u % P, v = u / P;
+        const int rr = row0 + r < R ? row0 + r : row0 + r - R;
+        if (r >= skip) b.ring_max(v)[s * R + rr] = __ldcs(tail_rec + u);
+      } else if (u < rows + tail_len) {
+        b.tail[s * tail_len + (u - rows)] = __ldcs(tail_rec + u);
+      } else if (u == rows + tail_len) {
+        b.expr[s] = __ldcs(tail_rec + u);
+      } else if (b.ema != nullptr) {
+        b.ema[s * KOE_N_BLENDSHAPES + (u - rows - tail_len - 1)] = __ldcs(tail_rec + u);
+      }
+    }
+  }
+}
+
 namespace {
+// floats per snapshot record: rows and maxima of 1 + n_edge ring variants for the P = W - n_edge frames a later window
+// can still read, the tail, the expression value and the smoothing row, rounded up to whole float4s
+int64_t state_floats(const koe_stream_pool* p) {
+  const int64_t P = p->window_frames - p->n_edge, rows = (int64_t)(1 + p->n_edge) * P;
+  const int64_t f = rows * (KOE_N_MELS + 1) + p->tail_len + 1 + KOE_N_BLENDSHAPES;
+  return (f + 3) / 4 * 4;
+}
+
+// the grid of both snapshot kernels: enough CTAs per stream for its rows at kStateUnroll float4s per thread (10 at
+// 30 fps, 30 at 60 fps), streams over gridDim.y
+dim3 state_grid(const koe_stream_pool* p, int n) {
+  const int quads = (1 + p->n_edge) * (p->window_frames - p->n_edge) * (KOE_N_MELS / 4);
+  const int per_cta = 256 * kStateUnroll;
+  return dim3((unsigned)std::max(1, std::min((quads + per_cta - 1) / per_cta, 64)), (unsigned)std::min(n, 65535));
+}
+
+PoolState pool_state(const koe_stream_pool_args* a) {
+  return PoolState{{a->ring_f, a->ring_r, a->ring_r2}, {a->fmax_f, a->fmax_r, a->fmax_r2}, a->tail, a->expr_sigmoid,
+                   a->ema_state};
+}
+
 // every slot of slots[0, n) in range, open and listed once
 int check_slots(koe_stream_pool* pool, const int32_t* slots, int n, const char* what) {
   KOE_REQUIRE(n >= 0 && n <= pool->capacity, "%s: %d streams for a pool of %d", what, n, pool->capacity);
@@ -547,5 +679,96 @@ extern "C" int koe_stream_pool_push_hops(koe_stream_pool_t* pool, const koe_stre
     if (pool->row[s] >= R) pool->row[s] -= R;
   }
   *n_emitted = k;
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_state_floats(const koe_stream_pool_t* pool) {
+  KOE_REQUIRE(pool != nullptr, "koe_stream_pool_state_floats: NULL pool");
+  const int64_t f = state_floats(pool);
+  KOE_REQUIRE(f <= INT32_MAX, "koe_stream_pool_state_floats: %lld floats per record", (long long)f);
+  return (int)f;
+}
+
+extern "C" int koe_stream_pool_snapshot(koe_stream_pool_t* pool, const koe_stream_pool_args* a, const int32_t* slots_host,
+                                        int n, float* records, int64_t* hops_host, void* stream) {
+  KOE_REQUIRE(pool != nullptr && a != nullptr, "koe_stream_pool_snapshot: NULL argument");
+  if (int rc = check_slots(pool, slots_host, n, "koe_stream_pool_snapshot")) return rc;
+  if (n == 0) return KOE_OK;
+  KOE_REQUIRE(records != nullptr && hops_host != nullptr, "koe_stream_pool_snapshot: NULL records / hops");
+  KOE_REQUIRE(((uintptr_t)records & 15) == 0, "koe_stream_pool_snapshot: records not 16-byte aligned");
+  const int n_edge = pool->n_edge, R = pool->ring_frames, P = pool->window_frames - n_edge;
+  KOE_REQUIRE(a->tail && a->ring_f && a->fmax_f && a->ring_r && a->fmax_r && a->expr_sigmoid && a->tables &&
+                  (n_edge == 1 || (a->ring_r2 && a->fmax_r2)),
+              "koe_stream_pool_snapshot: NULL buffer");
+  const int rec = koe_stream_pool_state_floats(pool);
+  if (rec < 0) return rec;
+  if (int rc = check_capture(stream, "koe_stream_pool_snapshot")) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  // ---- [slot | ring row of the record's row 0 | leading rows of frames < 0] per stream
+  TableStaging* b = nullptr;
+  if (int rc = acquire_table_staging(stream, 3 * (size_t)n, &b)) return rc;
+  for (int i = 0; i < n; ++i) {
+    const int s = slots_host[i];
+    const int r0 = pool->row[s] - P;  // row[s]: ring row of frame hops - lag = the record's row P
+    b->host[i] = s;
+    b->host[n + i] = r0 < 0 ? r0 + R : r0;
+    b->host[2 * n + i] = (int)std::min<int64_t>(P, std::max<int64_t>(0, pool->window_frames - 1 - pool->hops[s]));
+  }
+  if (int rc = upload_tables(b, a->tables, 3 * (size_t)n, st)) return rc;
+  pool_snapshot_kernel<<<state_grid(pool, n), 256, 0, st>>>(pool_state(a), a->tables, n, 1 + n_edge, P, R, pool->tail_len,
+                                                            rec, records);
+  count_launch();
+  KOE_CUDA(cudaGetLastError());
+  for (int i = 0; i < n; ++i) hops_host[i] = pool->hops[slots_host[i]];
+  return KOE_OK;
+}
+
+extern "C" int koe_stream_pool_restore(koe_stream_pool_t* pool, const koe_stream_pool_args* a, const float* records,
+                                       const int64_t* hops_host, int n, int32_t* slots_host, void* stream) {
+  KOE_REQUIRE(pool != nullptr && a != nullptr, "koe_stream_pool_restore: NULL argument");
+  KOE_REQUIRE(n >= 0, "koe_stream_pool_restore: negative count");
+  if (n == 0) return KOE_OK;
+  KOE_REQUIRE(records != nullptr && hops_host != nullptr && slots_host != nullptr,
+              "koe_stream_pool_restore: NULL records / hops / slots");
+  KOE_REQUIRE(((uintptr_t)records & 15) == 0, "koe_stream_pool_restore: records not 16-byte aligned");
+  std::vector<int32_t> slots;  // the n lowest free slots, as koe_stream_pool_open takes them
+  for (int s = 0; s < pool->capacity && (int)slots.size() < n; ++s)
+    if (!pool->open[s]) slots.push_back(s);
+  KOE_REQUIRE((int)slots.size() == n, "koe_stream_pool_restore: %d streams, %d of %d slots free", n, (int)slots.size(),
+              pool->capacity);
+  for (int i = 0; i < n; ++i)
+    KOE_REQUIRE(hops_host[i] >= 0, "koe_stream_pool_restore: record %d has %lld hops", i, (long long)hops_host[i]);
+  const int W = pool->window_frames, n_edge = pool->n_edge, R = pool->ring_frames, P = W - n_edge, lag = n_edge - 1;
+  KOE_REQUIRE(a->tail && a->ring_f && a->fmax_f && a->ring_r && a->fmax_r && a->expr_sigmoid && a->tables &&
+                  (n_edge == 1 || (a->ring_r2 && a->fmax_r2)),
+              "koe_stream_pool_restore: NULL buffer");
+  const int rec = koe_stream_pool_state_floats(pool);
+  if (rec < 0) return rec;
+  if (int rc = check_capture(stream, "koe_stream_pool_restore")) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  auto mod = [](int64_t x, int m) { return (int32_t)(((x % m) + m) % m); };
+  TableStaging* b = nullptr;
+  if (int rc = acquire_table_staging(stream, 3 * (size_t)n, &b)) return rc;
+  for (int i = 0; i < n; ++i) {
+    const int64_t h = hops_host[i];
+    b->host[i] = slots[i];
+    b->host[n + i] = mod(h + 1 - W, R);  // frame g lives in ring row g mod R in every pool
+    b->host[2 * n + i] = (int)std::min<int64_t>(P, std::max<int64_t>(0, W - 1 - h));
+  }
+  if (int rc = upload_tables(b, a->tables, 3 * (size_t)n, st)) return rc;
+  pool_restore_kernel<<<state_grid(pool, n), 256, 0, st>>>(pool_state(a), a->tables, n, 1 + n_edge, P, R, pool->tail_len,
+                                                           rec, records);
+  count_launch();
+  KOE_CUDA(cudaGetLastError());
+  // ---- the clocks, once the launch is queued: derived from the hops, as the pushes count them
+  for (int i = 0; i < n; ++i) {
+    const int s = slots[i];
+    const int64_t h = hops_host[i];
+    pool->open[s] = 1;
+    pool->hops[s] = h;
+    pool->frames[s] = pool->warmup ? h : std::max<int64_t>(0, h - W + 1);
+    pool->row[s] = mod(h - lag, R);
+    slots_host[i] = s;
+  }
   return KOE_OK;
 }

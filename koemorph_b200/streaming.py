@@ -212,6 +212,38 @@ class StreamingEngine:
         return self.out
 
 
+class StreamSnapshot:
+    """The state of k streams of a :class:`StreamPool` (:meth:`StreamPool.snapshot`), to continue them in another pool
+    (:meth:`StreamPool.restore`): a pool of another capacity or ``max_hops``, on another GPU, or in a later process.
+
+    * ``hop``, ``window_frames``, ``half_fft``, ``warmup``: the geometry of the pool it was taken from; a pool restores
+      only a snapshot of its own geometry and warm-up flag;
+    * ``hops``: CPU int64 ``[k]``, each stream's hops since it was opened;
+    * ``records``: float32 ``[k][state_floats]``, one record per stream (layout in ``koe_stream_pool_snapshot``,
+      include/koemorph_b200.h), on the source pool's device until moved with :meth:`to`.
+
+    Tensors and ints only: ``torch.save`` / ``torch.load`` keep it as it is."""
+
+    def __init__(self, hop: int, window_frames: int, half_fft: int, warmup: bool, hops: torch.Tensor,
+                 records: torch.Tensor):
+        self.hop, self.window_frames, self.half_fft, self.warmup = int(hop), int(window_frames), int(half_fft), bool(warmup)
+        self.hops, self.records = hops, records
+
+    def __len__(self) -> int:
+        return int(self.hops.numel())
+
+    def to(self, device) -> "StreamSnapshot":
+        """A copy with the records on `device` (another GPU, or "cpu" to keep them in host memory)."""
+        return StreamSnapshot(self.hop, self.window_frames, self.half_fft, self.warmup, self.hops.clone(),
+                              self.records.to(device, copy=True))
+
+
+# Intended, process-wide: importing the package adds StreamSnapshot to torch's weights-only allowlist, so that
+# torch.load(path) with its default weights_only=True loads a saved snapshot.  The class holds tensors and ints only, so
+# the allowlist admits nothing that could run code on load.
+torch.serialization.add_safe_globals([StreamSnapshot])
+
+
 class StreamPool:
     """Up to ``capacity`` concurrent streams that open, close and advance on their own clocks (``koe_stream_pool_*`` in
     include/koemorph_b200.h): a real-time service whose users connect and leave at any time and whose packets arrive
@@ -236,7 +268,10 @@ class StreamPool:
       later frame is smoothed onto the one before, so with smoothing on the frames from hop W - 1 on are the smoothing
       of this pool's own frames and differ from those of a pool without warm-up.
 
-    :meth:`push` on a warm-up pool runs the burst path with counts of 1, whatever ``max_hops`` is."""
+    :meth:`push` on a warm-up pool runs the burst path with counts of 1, whatever ``max_hops`` is.
+
+    :meth:`snapshot` and :meth:`restore` move streams with their whole state (audio tail, mel rings, expression input,
+    smoothing state) into another pool: one of another capacity or ``max_hops``, on another GPU, or in a later process."""
 
     def __init__(self, model, capacity: int, max_hops: int = 1, warmup: bool = False):
         self.model = model
@@ -299,6 +334,9 @@ class StreamPool:
         self._check(self._lib.koe_stream_pool_create_ex2(cap, self.hop, self.W, self.half, self.max_hops, flags,
                                                          C.byref(h)), "koe_stream_pool_create_ex2")
         self._h = h
+        self.state_floats = self._lib.koe_stream_pool_state_floats(h)   # floats per StreamSnapshot record
+        if self.state_floats < 0:
+            self._check(self.state_floats, "koe_stream_pool_state_floats")
         self._fe = model._frontend(self.dev)
         self._alpha, self._alpha_key = 0.0, None
         self._args, self._args_key, self._w_tensors = None, None, []
@@ -404,7 +442,61 @@ class StreamPool:
         k = self._n_emitted.value
         return self._emitted[:k].to(torch.int64), self._emitted_hop[:k].clone(), self.out[:k]
 
+    @torch.no_grad()
+    def snapshot(self, slots) -> StreamSnapshot:
+        """The state of the listed open streams after every call queued so far on the current stream (where the
+        snapshot is queued, as :meth:`push`).  The streams stay open and unchanged.  Restored into a pool of the same
+        geometry and warm-up flag that runs the same weights at the same precision, each of them gives bit for bit the
+        frames and hops it gives here when both are pushed the same audio from here on, with :meth:`push` or
+        :meth:`push_hops` in any mix.  Without temporal smoothing the records carry a zero smoothing state."""
+        s = self._slots(slots)
+        k = s.numel()
+        records = torch.empty(k, self.state_floats, dtype=torch.float32, device=self.dev)
+        hops = torch.zeros(k, dtype=torch.int64)
+        self._current_args()
+        self._call(self._lib.koe_stream_pool_snapshot, self._h, self._args_ref, s.data_ptr(), k, records.data_ptr(),
+                   hops.data_ptr(), what="koe_stream_pool_snapshot")
+        return StreamSnapshot(self.hop, self.W, self.half, self.warmup, hops, records)
+
+    @torch.no_grad()
+    def restore(self, snapshot: StreamSnapshot) -> list:
+        """Opens one stream per record of `snapshot` in the lowest free slots and returns them, in record order: each
+        continues from its recorded hop with its recorded state, expression input included (no :meth:`set_egemaps`
+        needed).  The equality of :meth:`snapshot` holds whatever this pool's capacity and ``max_hops`` are and
+        whatever its slots held before.  The restore is queued on the current stream: records written on another CUDA
+        stream (a snapshot there, a copy from another device) need the caller's synchronisation first.  Raises
+        ValueError for a snapshot of another hop, window, FFT size or warm-up flag, records that are not float32 on
+        this pool's device or whose shapes disagree, or more records than free slots -- before anything is queued."""
+        records, hops = self._check_snapshot(snapshot)
+        k = hops.numel()
+        slots = torch.empty(k, dtype=torch.int32)
+        self._current_args()
+        self._call(self._lib.koe_stream_pool_restore, self._h, self._args_ref, records.data_ptr(), hops.data_ptr(), k,
+                   slots.data_ptr(), what="koe_stream_pool_restore")
+        return slots.tolist()
+
     # ---- helpers ----------------------------------------------------------------------------------------------------
+    def _check_snapshot(self, snap):
+        if not isinstance(snap, StreamSnapshot):
+            raise ValueError(f"restore takes a StreamSnapshot, got {type(snap).__name__}")
+        mine = (self.hop, self.W, self.half, self.warmup)
+        theirs = (snap.hop, snap.window_frames, snap.half_fft, snap.warmup)
+        if theirs != mine:
+            raise ValueError(f"snapshot of a pool with (hop, window_frames, half_fft, warmup) = {theirs}, this pool has "
+                             f"{mine}")
+        h, r = snap.hops, snap.records
+        if not isinstance(h, torch.Tensor) or h.device.type != "cpu" or h.dtype != torch.int64 or h.dim() != 1:
+            raise ValueError("snapshot hops must be a 1-D CPU int64 tensor")
+        if not isinstance(r, torch.Tensor) or r.device != self.dev or r.dtype != torch.float32:
+            raise ValueError(f"snapshot records must be float32 on {self.dev}, got "
+                             f"{getattr(r, 'dtype', type(r).__name__)} on {getattr(r, 'device', None)}")
+        if tuple(r.shape) != (h.numel(), self.state_floats):
+            raise ValueError(f"snapshot records must be ({h.numel()}, {self.state_floats}) for {h.numel()} hops, got "
+                             f"{tuple(r.shape)}")
+        if h.numel() and int(h.min()) < 0:
+            raise ValueError("snapshot hops must be >= 0")
+        return r.contiguous(), h.contiguous()
+
     def _check(self, rc: int, what: str) -> None:
         if rc == -1:   # KOE_E_INVALID: misuse (slot out of range / not open / listed twice, pool full)
             msg = self._lib.koe_last_error()
